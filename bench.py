@@ -13,7 +13,7 @@ from PINNED host buffers + on-device createCorrespondenceMatrix — and then run
 CUDA events on the device, max over ranks.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config cfg3_1000v]
-                    [--verify N] [--dump-tuples FILE]
+                    [--verify N] [--dump-tuples FILE] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -250,6 +250,24 @@ def emit(line):
 _REAL_STDOUT = 1
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, edges, budget=DUMP_BYTES):
+    """--dump-outputs: the pose graph the last timed step returned to its caller, its committed edges in commit order,
+    as one float64 array per field of builder.EDGE_DTYPE (path/edges_<field>.npy) and the rows' positions in the edge
+    list (edges_row.npy).  When the edges exceed `budget` bytes, a fixed seeded sample of rows, still in commit order."""
+    fields = [f for f in edges.dtype.names if f != "pad"]
+    row_bytes = 8 * (1 + sum(int(np.prod(edges.dtype[f].shape)) for f in fields))
+    rows = np.arange(len(edges))
+    if len(rows) * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(0).choice(len(edges), budget // row_bytes, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "edges_row.npy"), rows.astype(np.float64))
+    for f in fields:
+        np.save(os.path.join(path, "edges_%s.npy" % f), edges[f][rows].astype(np.float64))
+
+
 def verify_run(scene, log, n_tuples, replay_pairs):
     """--verify: the finished run against the CPU oracle at benchmark scale (pose_graph_initialization_b200/verify.py)."""
     from oracle import pgo_oracle as O
@@ -300,7 +318,13 @@ def main():
     ap.add_argument("--verify-replay", type=int, default=-1, help="queue positions replayed by the oracle host (-1 = whole queue up to 400 views, else 20000; 0 = whole queue)")
     ap.add_argument("--dump-tuples", default="", help="write N evenly spaced (pair, hypothesis) tuples of the last run (npz)")
     ap.add_argument("--dump-n", type=int, default=8192)
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the pose graph of the last step as float64 .npy files under DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm builds no pose graph")
     if args.cv2_yardstick:  # child mode of cv2_yardstick(): no torch, no CUDA
         sys.exit(cv2_yardstick_child(args.cv2_yardstick, args.workers))
 
@@ -365,7 +389,7 @@ def main():
     fp64_peak = pgb.engine.fp64_peak(fused=False)
     fp64_peak_fma = pgb.engine.fp64_peak(fused=True)
 
-    K = max(args.steps, 1)
+    K = args.steps
     batch_steps = args.step == "batch"
     batch = -(-P // K)  # queue positions per step in batch mode (cut at the next wave boundary)
     if batch_steps:
@@ -405,6 +429,10 @@ def main():
                         next(gen)
                 except StopIteration as done:
                     graph, gen = done.value, None
+                    if k < K - 1:  # the remaining steps would be timed with nothing in them
+                        sampler.stop()
+                        raise SystemExit("--steps %d: the pass over %d queue positions ended in step %d (waves of %d "
+                                         "positions); use fewer steps or a smaller --wave" % (K, P, k + 1, args.wave))
         barrier()
         evs[k][2].record()
         step_wall["e2e"].append(round((time.perf_counter() - ts) * 1e3, 1))
@@ -510,6 +538,8 @@ def main():
         verify = verify_run(scene, log, args.verify, replay)
     if args.dump_tuples and rank == 0:
         np.savez_compressed(args.dump_tuples, **tuples_from_log(log, args.dump_n))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, graph.edges)
 
     if rank == 0:
         cores = os.cpu_count() or 1

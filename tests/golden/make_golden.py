@@ -11,7 +11,7 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
-from helpers import two_view  # noqa: E402
+from helpers import two_view, two_view_keypoints  # noqa: E402
 
 cv2.setNumThreads(1)
 rng = np.random.default_rng(2024)
@@ -69,4 +69,23 @@ np.savez_compressed(os.path.join(HERE, "cv_usac_magsac.npz"), n=len(us),
                     **{f"c{i}": u[0] for i, u in enumerate(us)}, **{f"E{i}": u[1] for i, u in enumerate(us)},
                     **{f"m{i}": u[2] for i, u in enumerate(us)}, **{f"R{i}": u[3] for i, u in enumerate(us)},
                     **{f"t{i}": u[4] for i, u in enumerate(us)})
+
+# --- matchFeatures (feature_utils.h:103-210): BFMatcher(NORM_L2SQR) 2-NN both ways, 0.90 ratio test, mutual check,
+#     survivors sorted by ratio -> (ratio, query, train) on the descriptors of tests/test_oracle_features.py
+mf = {}
+for n, seed in ((200, 0), (900, 1)):
+    d = two_view_keypoints(n, np.random.default_rng(seed))
+    fw = cv2.BFMatcher(cv2.NORM_L2SQR).knnMatch(d["desc_src"], d["desc_dst"], 2)
+    bw = cv2.BFMatcher(cv2.NORM_L2SQR).knnMatch(d["desc_dst"], d["desc_src"], 2)
+    good = []
+    for i, m in enumerate(fw):
+        if len(m) < 2 or len(bw[m[0].trainIdx]) < 2:
+            continue
+        if m[0].distance < 0.90 * m[1].distance and m[0].queryIdx == bw[m[0].trainIdx][0].trainIdx:
+            good.append((m[0].distance / m[1].distance, i, m[0].trainIdx))
+    good.sort()
+    mf[f"ratio_{n}_{seed}"] = np.array([g[0] for g in good])
+    mf[f"query_{n}_{seed}"] = np.array([g[1] for g in good], dtype=np.int32)
+    mf[f"train_{n}_{seed}"] = np.array([g[2] for g in good], dtype=np.int32)
+np.savez_compressed(os.path.join(HERE, "cv_match_features.npz"), **mf)
 print("golden vectors written to", HERE, "with cv2", cv2.__version__)
