@@ -90,6 +90,10 @@ typedef struct pgi_stats {
     uint64_t fallback_models;   /* minimal + LO models scored by the fallback         */
     uint64_t h2d_bytes;         /* bytes copied host->device                          */
     uint64_t d2h_bytes;         /* bytes copied device->host                          */
+    double ms_match;            /* K9 batched descriptor matching (all chunks)        */
+    uint64_t dist_evals;        /* K9 descriptor distances (each pair's n_src x n_dst once) */
+    uint64_t match_pairs;       /* pairs matched by K9                                */
+    uint64_t match_rows;        /* matches K9 produced                                */
 } pgi_stats;
 
 const char *pgi_version(void);
@@ -115,6 +119,19 @@ pgi_status pgi_register_scene(pgi_ctx *ctx, uint64_t n_views, const double *foca
                               const uint64_t *kp_offset, const float *kp_xy, uint64_t n_pairs,
                               const uint32_t *pair_views, const uint64_t *m_offset, const uint32_t *matches,
                               double thr_px);
+
+/* matchFeatures (feature_utils.h:103-210) for every pair on the device (K9), then createCorrespondenceMatrix (K0) from the
+ * device-resident matches: pgi_register_scene with descriptors in place of matches.  desc[sum K][dim] float (dim 64 or
+ * 128, every value finite), row-aligned with kp_xy; at most 16384 keypoints per view (PGI_ERR_INVALID beyond).  Each
+ * pair's matches are the rows pgi_match_features returns for it, in the same order.  m_offset_out[n_pairs + 1] receives
+ * the match counts as offsets.  Device scratch is bounded by a chunk of pairs; the match list itself stays on the device. */
+pgi_status pgi_register_scene_descriptors(pgi_ctx *ctx, uint64_t n_views, const double *focal, const double *size_wh,
+                                          const uint64_t *kp_offset, const float *kp_xy, const float *desc, uint32_t dim,
+                                          uint64_t n_pairs, const uint32_t *pair_views, double thr_px,
+                                          uint64_t *m_offset_out);
+/* Copy the (srcIdx, dstIdx) rows and, if non-null, the ratios of the last pgi_register_scene_descriptors on this context
+ * (the correspondences.h5 cache): m_offset_out[n_pairs] rows.  PGI_ERR_STATE if a pgi_register_scene came after it. */
+pgi_status pgi_read_scene_matches(pgi_ctx *ctx, uint32_t *matches_out, double *ratios_or_null, uint64_t capacity_rows);
 
 /* Make `ctx` use the pairs registered in `owner` (same device) without copying them: a second context — its
  * own stream, wave buffers and statistics — can then verify waves concurrently with the first (used to overlap

@@ -306,6 +306,11 @@ def shard_scene(scene, rank, world_size):
     return sub
 
 
+def needs_matching(scene):
+    """A scene with keypoint descriptors and no matches yet: PoseGraphBuilder matches it on the device in prepare()."""
+    return "desc" in scene and "matches" not in scene
+
+
 def allgather_verdicts(local, counts, group=None, device=None):
     """All-gather variable-length verdict arrays (counts[r] records from rank r, known to every rank).
     Returns the list of per-rank arrays.  One collective; payload is padded to max(counts)."""
@@ -460,14 +465,23 @@ class PoseGraphBuilder:
     def prepare(self):
         if self.engine is None:
             self.engine = _engine.Engine(device=self.device, min_inliers=self.min_inliers)
+        registered = False
         if self.world == 1:
             sub = self.scene
+            if needs_matching(sub):  # keypoints + descriptors only: matchFeatures on the device, registered in the same call
+                self.engine.register_scene_descriptors(sub, self.thr_px)
+                registered = True
         else:
             # the rank's shard is cut once (a 32 GB scene's shard is gigabytes: not something to copy on every registration)
             if getattr(self, "_sub", None) is None:
-                self._sub = shard_scene(self.scene, self.rank, self.world)
+                if needs_matching(self.scene):
+                    self._sub = self._match_owned_pairs()
+                    registered = True
+                else:
+                    self._sub = shard_scene(self.scene, self.rank, self.world)
             sub = self._sub
-        self.engine.register_scene(sub, self.thr_px)
+        if not registered:
+            self.engine.register_scene(sub, self.thr_px)
         self.prepared = True
         if self.overlap:
             if self.engine_fb is None:
@@ -478,19 +492,47 @@ class PoseGraphBuilder:
                 if self.engine_fb2 is None:
                     self.engine_fb2 = _engine.Engine(device=self.device, min_inliers=self.min_inliers, background=True)
                 self.engine_fb2.share_pairs(self.engine)
-            if self.world > 1 and self.pf_group is None:
-                # The prefetch worker thread gathers its chunks' verdicts over its OWN communicator, and that communicator
-                # is gloo (CPU tensors, as in round 1) on purpose.  A second NCCL communicator driven from the worker thread
-                # was tried in round 2 and deadlocked on the 1 000-view scene at N=2 (all-gather #77 of the prefetch group
-                # against all-reduce #283 of the wave loop, both ranks in the watchdog after 600 s): two NCCL communicators
-                # used concurrently must enqueue their collectives in the same order on every rank, which two free-running
-                # threads do not, and on a GPU saturated by the fallback kernels the two collective kernels cannot
-                # co-schedule their way out of it.  (On the 300-view scene the same code happened to work.)  The payload is
-                # 330 KB per chunk; gloo moves it in about a millisecond.
-                import torch.distributed as dist
-                self.pf_group = dist.new_group(backend="gloo")
-                self.pf_device = None
-                self.pf_stream = None
+            if self.world > 1:
+                self._gloo_group()
+
+    def _gloo_group(self):
+        if self.pf_group is None:
+            # The prefetch worker thread gathers its chunks' verdicts over its OWN communicator, and that communicator
+            # is gloo (CPU tensors, as in round 1) on purpose.  A second NCCL communicator driven from the worker thread
+            # was tried in round 2 and deadlocked on the 1 000-view scene at N=2 (all-gather #77 of the prefetch group
+            # against all-reduce #283 of the wave loop, both ranks in the watchdog after 600 s): two NCCL communicators
+            # used concurrently must enqueue their collectives in the same order on every rank, which two free-running
+            # threads do not, and on a GPU saturated by the fallback kernels the two collective kernels cannot
+            # co-schedule their way out of it.  (On the 300-view scene the same code happened to work.)  The payload is
+            # 330 KB per chunk; gloo moves it in about a millisecond.
+            import torch.distributed as dist
+            self.pf_group = dist.new_group(backend="gloo")
+            self.pf_device = None
+            self.pf_stream = None
+        return self.pf_group
+
+    def _match_owned_pairs(self):
+        """world > 1 on a descriptor scene: match only the pairs this rank owns (the shard_scene pairs), registered as the
+        rank's shard; the per-pair counts are all-gathered over the gloo group so that every rank's host gets the global
+        m_offset (scene["m_offset"]).  The matches themselves stay with their owner."""
+        import torch
+        import torch.distributed as dist
+
+        P = len(self.scene["pair_views"])
+        sub = dict(self.scene)
+        sub["pair_views"] = np.ascontiguousarray(self.scene["pair_views"][self.rank::self.world])
+        self.engine.register_scene_descriptors(sub, self.thr_px)
+        counts = np.diff(sub["m_offset"].astype(np.int64))
+        per_rank = [len(range(r, P, self.world)) for r in range(self.world)]
+        send = torch.zeros(max(per_rank), dtype=torch.int64)
+        send[:len(counts)] = torch.from_numpy(counts)
+        parts = [torch.empty_like(send) for _ in range(self.world)]
+        dist.all_gather(parts, send, group=self._gloo_group())
+        n = np.zeros(P, dtype=np.int64)
+        for r in range(self.world):
+            n[r::self.world] = parts[r].numpy()[:per_rank[r]]
+        self.scene["m_offset"] = np.concatenate([[0], np.cumsum(n)]).astype(np.uint64)
+        return sub
 
     def engine_stats(self):
         st = self.engine.stats()

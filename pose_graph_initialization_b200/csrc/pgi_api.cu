@@ -17,6 +17,7 @@
 #include "pgi_astar.cuh"
 #include "pgi_matcher.cuh"
 #include "pgi_features.cuh"
+#include "pgi_match_scene.cuh"
 #include "pgi_nvtx.h"
 
 using namespace pgi;
@@ -63,6 +64,13 @@ struct pgi_ctx {
     float2 *d_stKp = nullptr;
     uint2 *d_stPv = nullptr, *d_stM = nullptr;
     size_t capStFocal = 0, capStSize = 0, capStKpOff = 0, capStKp = 0, capStPv = 0, capStM = 0;
+    // pgi_register_scene_descriptors: resident descriptors, the ratios beside d_stM, the per-chunk scratch of K9
+    float *d_stDesc = nullptr, *d_stRatio = nullptr;
+    size_t capStDesc = 0, capStRatio = 0;
+    unsigned char *d_k9Scratch = nullptr;
+    size_t capK9Scratch = 0;
+    uint64_t sceneRows = 0;
+    bool sceneMatches = false;  // d_stM / d_stRatio hold the matches of the last descriptor registration
     uint32_t *d_dkList = nullptr, *d_dkCtl = nullptr;  // work list of the split K4 (K4a -> K4b -> K4c)
     uint32_t k4aSmem = 0;  // PGI_K4A_SMEM: dynamic shared memory per K4a CTA, an occupancy throttle (L2 footprint of the 5 KB stacks)
     uint32_t k4bCtas = 2;  // K4b CTAs per SM (PGI_K4B_CTAS): fewer lanes = more polynomials per lane = better refill balance
@@ -477,6 +485,33 @@ pgi_status finishWave(pgi_ctx *ctx)
     return PGI_OK;
 }
 
+// K0 (createCorrespondenceMatrix) over the staged scene (ctx->d_st*: views, keypoints, pair views, matches) into r,
+// whose d_offset, h_offset, nPairs, nRows and maxN are set and whose d_corr / d_thr hold nRows / nPairs entries; then the
+// sampler tables.
+pgi_status buildCorrespondences(pgi_ctx *ctx, Registration &r, double thr_px)
+{
+    cudaStream_t s = ctx->stream;
+    const uint64_t n_pairs = r.nPairs;
+    if (n_pairs) {
+        CK(cudaEventRecord(ctx->evStart, s));
+        const uint32_t gx = std::max<uint32_t>(1, std::min<uint32_t>((r.maxN + 255) / 256, 64));
+        const uint32_t gy = (uint32_t)std::min<uint64_t>(n_pairs, 65535), gz = (uint32_t)((n_pairs + gy - 1) / gy);
+        k0_build_correspondences<<<dim3(gx, gy, gz), 256, 0, s>>>(ctx->d_stFocal, ctx->d_stSize, ctx->d_stKpOff, ctx->d_stKp,
+                                                                   n_pairs, ctx->d_stPv, r.d_offset, ctx->d_stM, thr_px,
+                                                                   reinterpret_cast<double4 *>(r.d_corr), r.d_thr);
+        CK(cudaEventRecord(ctx->evK1, s));
+        CK(cudaGetLastError());
+        ctx->stats.launches += 1;
+    }
+    CK(cudaStreamSynchronize(s));
+    if (n_pairs) {
+        float ms = 0;
+        CK(cudaEventElapsedTime(&ms, ctx->evStart, ctx->evK1));
+        ctx->stats.ms_correspondences += ms;
+    }
+    return buildTables(ctx, r);
+}
+
 }  // namespace
 
 extern "C" {
@@ -560,6 +595,7 @@ pgi_status pgi_destroy(pgi_ctx *ctx)
     cudaFree(ctx->d_verdicts); cudaFree(ctx->d_fbSols); cudaFree(ctx->d_fbSolsF); cudaFree(ctx->d_counters);
     cudaFree(ctx->d_k3Scratch); cudaFree(ctx->d_dkList); cudaFree(ctx->d_dkCtl);
     cudaFree(ctx->d_stFocal); cudaFree(ctx->d_stSize); cudaFree(ctx->d_stKpOff); cudaFree(ctx->d_stKp); cudaFree(ctx->d_stPv); cudaFree(ctx->d_stM);
+    cudaFree(ctx->d_stDesc); cudaFree(ctx->d_stRatio); cudaFree(ctx->d_k9Scratch);
     cudaFreeHost(ctx->h_pairId); cudaFreeHost(ctx->h_hypOffset); cudaFreeHost(ctx->h_hyp);
     cudaFreeHost(ctx->h_maskOffset); cudaFreeHost(ctx->h_verdicts); cudaFreeHost(ctx->h_counters);
     cudaEvent_t evs[] = {ctx->evBegin, ctx->evStart, ctx->evK1, ctx->evK2, ctx->evK3, ctx->evFbEnd};
@@ -638,25 +674,191 @@ pgi_status pgi_register_scene(pgi_ctx *ctx, uint64_t n_views, const double *foca
     CKC(cudaMemcpyAsync(d_m, matches, nRows * 8, cudaMemcpyHostToDevice, s));
     CKC(cudaMemcpyAsync(r.d_offset, m_offset, (n_pairs + 1) * 8, cudaMemcpyHostToDevice, s));
     ctx->stats.h2d_bytes += n_views * 24 + (n_views + 1) * 8 + nKp * 8 + n_pairs * 8 + nRows * 8 + (n_pairs + 1) * 8;
-    if (n_pairs) {
-        CKC(cudaEventRecord(ctx->evStart, s));
-        const uint32_t gx = std::max<uint32_t>(1, std::min<uint32_t>((r.maxN + 255) / 256, 64));
-        const uint32_t gy = (uint32_t)std::min<uint64_t>(n_pairs, 65535), gz = (uint32_t)((n_pairs + gy - 1) / gy);
-        k0_build_correspondences<<<dim3(gx, gy, gz), 256, 0, s>>>(d_focal, d_size, d_kpOff, d_kp, n_pairs, d_pv, r.d_offset,
-                                                                   d_m, thr_px, reinterpret_cast<double4 *>(r.d_corr), r.d_thr);
-        CKC(cudaEventRecord(ctx->evK1, s));
-        CKC(cudaGetLastError());
-        ctx->stats.launches += 1;
-    }
-    CKC(cudaStreamSynchronize(s));
-    if (n_pairs) {
-        float ms = 0;
-        CKC(cudaEventElapsedTime(&ms, ctx->evStart, ctx->evK1));
-        ctx->stats.ms_correspondences += ms;
-    }
+    ctx->sceneMatches = false;  // d_stM now holds the caller's matches
     cleanup();
 #undef CKC
-    return buildTables(ctx, r);
+    return buildCorrespondences(ctx, r, thr_px);
+}
+
+pgi_status pgi_register_scene_descriptors(pgi_ctx *ctx, uint64_t n_views, const double *focal, const double *size_wh,
+                                          const uint64_t *kp_offset, const float *kp_xy, const float *desc, uint32_t dim,
+                                          uint64_t n_pairs, const uint32_t *pair_views, double thr_px, uint64_t *m_offset_out)
+{
+    PgiNvtxRange nvtxRange("pgi:register_scene_descriptors (H2D + K9 match + K0)");
+    if (!ctx) return PGI_ERR_INVALID;
+    if (ctx->inFlight) { ctx->err = "a wave is in flight"; return PGI_ERR_STATE; }
+    if (!focal || !size_wh || !kp_offset || (!kp_xy && kp_offset[n_views]) || (!desc && kp_offset[n_views]) || !pair_views ||
+        !m_offset_out) {
+        ctx->err = "null argument";
+        return PGI_ERR_INVALID;
+    }
+    if (dim != 128 && dim != 64) { ctx->err = "descriptors must have 64 or 128 dimensions"; return PGI_ERR_INVALID; }
+    uint32_t maxK = 0;
+    if (kp_offset[0] != 0) { ctx->err = "kp_offset[0] must be 0"; return PGI_ERR_INVALID; }
+    for (uint64_t v = 0; v < n_views; v++) {
+        if (kp_offset[v + 1] < kp_offset[v]) { ctx->err = "kp_offset is not monotone"; return PGI_ERR_INVALID; }
+        const uint64_t k = kp_offset[v + 1] - kp_offset[v];
+        if (k > kK9MaxKp) {
+            char buf[160];
+            snprintf(buf, sizeof buf, "view %llu has %llu keypoints; batched matching supports at most %u per view",
+                     (unsigned long long)v, (unsigned long long)k, kK9MaxKp);
+            ctx->err = buf;
+            return PGI_ERR_INVALID;
+        }
+        maxK = std::max<uint32_t>(maxK, (uint32_t)k);
+    }
+    for (uint64_t p = 0; p < n_pairs; p++)
+        if (pair_views[2 * p] >= n_views || pair_views[2 * p + 1] >= n_views) { ctx->err = "view id out of range"; return PGI_ERR_INVALID; }
+    CK(cudaSetDevice(ctx->cfg.device));
+    if (ctx->reg.borrowed) ctx->reg = Registration();
+    Registration &r = ctx->reg;
+    cudaStream_t s = ctx->stream;
+    const uint64_t nKp = kp_offset[n_views];
+    ctx->sceneMatches = false;
+    pgi_status st;
+    if ((st = growDevice(ctx, &r.d_offset, r.capOffset, (size_t)n_pairs + 1)) != PGI_OK) return st;
+    if ((st = growDevice(ctx, &r.d_thr, r.capThr, (size_t)n_pairs)) != PGI_OK) return st;
+    if ((st = growDevice(ctx, &ctx->d_stFocal, ctx->capStFocal, (size_t)n_views)) != PGI_OK) return st;
+    if ((st = growDevice(ctx, &ctx->d_stSize, ctx->capStSize, (size_t)n_views * 2)) != PGI_OK) return st;
+    if ((st = growDevice(ctx, &ctx->d_stKpOff, ctx->capStKpOff, (size_t)n_views + 1)) != PGI_OK) return st;
+    if ((st = growDevice(ctx, &ctx->d_stKp, ctx->capStKp, (size_t)nKp)) != PGI_OK) return st;
+    if ((st = growDevice(ctx, &ctx->d_stPv, ctx->capStPv, (size_t)n_pairs)) != PGI_OK) return st;
+    if ((st = growDevice(ctx, &ctx->d_stDesc, ctx->capStDesc, (size_t)nKp * dim)) != PGI_OK) return st;
+    CK(cudaMemcpyAsync(ctx->d_stFocal, focal, n_views * 8, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(ctx->d_stSize, size_wh, n_views * 16, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(ctx->d_stKpOff, kp_offset, (n_views + 1) * 8, cudaMemcpyHostToDevice, s));
+    if (nKp) CK(cudaMemcpyAsync(ctx->d_stKp, kp_xy, nKp * 8, cudaMemcpyHostToDevice, s));
+    if (n_pairs) CK(cudaMemcpyAsync(ctx->d_stPv, pair_views, n_pairs * 8, cudaMemcpyHostToDevice, s));
+    // every view's descriptors once; they stay resident for all of its pairs
+    if (nKp) CK(cudaMemcpyAsync(ctx->d_stDesc, desc, nKp * dim * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemsetAsync(r.d_offset, 0, 8, s));
+    ctx->stats.h2d_bytes += n_views * 24 + (n_views + 1) * 8 + nKp * 8 + n_pairs * 8 + nKp * dim * 4;
+    // non-finite descriptors are rejected (a NaN distance never enters a 2-NN, so it would silently drop neighbours)
+    uint32_t *d_flag = reinterpret_cast<uint32_t *>(ctx->d_counters);
+    uint32_t flag = 0;
+    CK(cudaMemsetAsync(d_flag, 0, 4, s));
+    if (nKp) {
+        k9_check_finite<<<(uint32_t)std::min<uint64_t>((nKp * dim + 1023) / 1024, 4 * ctx->numSms), 1024, 0, s>>>(ctx->d_stDesc, nKp * dim, d_flag);
+        CK(cudaGetLastError());
+        ctx->stats.launches += 1;
+    }
+    CK(cudaMemcpyAsync(&flag, d_flag, 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    ctx->stats.d2h_bytes += 4;
+    if (flag) { ctx->err = "non-finite descriptor value"; return PGI_ERR_INVALID; }
+
+    // K9 per chunk of pairs: scratch (forward states, backward partials, staged sorted rows) sized for the chunk only
+    const uint32_t stride = std::max<uint32_t>(maxK, 1), maxSB = (stride + kK9Rows - 1) / kK9Rows;
+    uint32_t keyCap = 1;
+    while (keyCap < stride) keyCap <<= 1;
+    const size_t perPair = (size_t)maxSB * stride * sizeof(Nn2) + (size_t)stride * (sizeof(Nn2) + 8 + 4) + 4;
+    const size_t kScratchBudget = (size_t)512 << 20;
+    const uint64_t chunk = std::max<uint64_t>(1, std::min<uint64_t>({kScratchBudget / perPair, 65535, std::max<uint64_t>(n_pairs, 1)}));
+    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    const size_t oF = 0, oB = oF + al(chunk * stride * sizeof(Nn2)), oM = oB + al(chunk * maxSB * stride * sizeof(Nn2)),
+                 oR = oM + al(chunk * stride * 8), oC = oR + al(chunk * stride * 4), total = oC + al(chunk * 4);
+    if ((st = growDevice(ctx, &ctx->d_k9Scratch, ctx->capK9Scratch, total)) != PGI_OK) return st;
+    Nn2 *d_fwd = reinterpret_cast<Nn2 *>(ctx->d_k9Scratch + oF), *d_bpart = reinterpret_cast<Nn2 *>(ctx->d_k9Scratch + oB);
+    uint2 *d_sm = reinterpret_cast<uint2 *>(ctx->d_k9Scratch + oM);
+    float *d_sr = reinterpret_cast<float *>(ctx->d_k9Scratch + oR);
+    uint32_t *d_cnt = reinterpret_cast<uint32_t *>(ctx->d_k9Scratch + oC);
+    const size_t finishSmem = (size_t)keyCap * 8 + (size_t)stride * 4;
+    CK(cudaFuncSetAttribute(k9_finish, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)finishSmem));
+    // the match list is the one allocation that grows with the scene: doubled as needed, earlier rows kept
+    auto ensureRows = [&](uint64_t need, uint64_t keep) -> pgi_status {
+        if (need <= ctx->capStM && need <= ctx->capStRatio && ctx->d_stM && ctx->d_stRatio) return PGI_OK;
+        const size_t cap = std::max<size_t>({need, 2 * std::min(ctx->capStM, ctx->capStRatio), 1024});
+        uint2 *m = nullptr;
+        float *q = nullptr;
+        CK(cudaMalloc((void **)&m, cap * sizeof(uint2)));
+        if (cudaMalloc((void **)&q, cap * sizeof(float)) != cudaSuccess) { cudaFree(m); cudaGetLastError(); ctx->err = "out of device memory for the match list"; return PGI_ERR_NOMEM; }
+        if (keep) {
+            CK(cudaMemcpyAsync(m, ctx->d_stM, keep * sizeof(uint2), cudaMemcpyDeviceToDevice, s));
+            CK(cudaMemcpyAsync(q, ctx->d_stRatio, keep * sizeof(float), cudaMemcpyDeviceToDevice, s));
+            CK(cudaStreamSynchronize(s));
+        }
+        cudaFree(ctx->d_stM);
+        cudaFree(ctx->d_stRatio);
+        ctx->d_stM = m; ctx->d_stRatio = q;
+        ctx->capStM = ctx->capStRatio = cap;
+        return PGI_OK;
+    };
+    float msMatch = 0;
+    uint64_t rows = 0, dist = 0;
+    for (uint64_t c0 = 0; c0 < n_pairs; c0 += chunk) {
+        const uint32_t cp = (uint32_t)std::min<uint64_t>(chunk, n_pairs - c0);
+        uint32_t sbUsed = 0;
+        for (uint64_t p = c0; p < c0 + cp; p++) {
+            const uint64_t nS = kp_offset[pair_views[2 * p] + 1] - kp_offset[pair_views[2 * p]];
+            const uint64_t nD = kp_offset[pair_views[2 * p + 1] + 1] - kp_offset[pair_views[2 * p + 1]];
+            sbUsed = std::max<uint32_t>(sbUsed, (uint32_t)((nS + kK9Rows - 1) / kK9Rows));
+            dist += nS * nD;
+        }
+        CK(cudaEventRecord(ctx->evStart, s));
+        {
+            PgiNvtxRange chunkRange("pgi:k9 chunk");
+            if (sbUsed) {
+                if (dim == 128)
+                    k9_knn2_tile<128><<<dim3(sbUsed, cp), kK9Threads, 0, s>>>(ctx->d_stDesc, ctx->d_stKpOff, ctx->d_stPv, c0, stride, maxSB, d_fwd, d_bpart);
+                else
+                    k9_knn2_tile<64><<<dim3(sbUsed, cp), kK9Threads, 0, s>>>(ctx->d_stDesc, ctx->d_stKpOff, ctx->d_stPv, c0, stride, maxSB, d_fwd, d_bpart);
+                ctx->stats.launches += 1;
+            }
+            k9_finish<<<cp, kK9FinishThreads, finishSmem, s>>>(ctx->d_stKpOff, ctx->d_stPv, c0, stride, keyCap, maxSB, d_fwd, d_bpart, d_cnt, d_sm, d_sr);
+            k9_offsets<<<1, 1024, 0, s>>>(d_cnt, cp, r.d_offset, c0);
+            CK(cudaGetLastError());
+            ctx->stats.launches += 2;
+        }
+        uint64_t end = 0;
+        CK(cudaMemcpyAsync(&end, r.d_offset + c0 + cp, 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        ctx->stats.d2h_bytes += 8;
+        if ((st = ensureRows(end, rows)) != PGI_OK) return st;
+        k9_scatter<<<cp, 256, 0, s>>>(r.d_offset, c0, stride, d_cnt, d_sm, d_sr, ctx->d_stM, ctx->d_stRatio);
+        CK(cudaEventRecord(ctx->evK1, s));
+        CK(cudaGetLastError());
+        ctx->stats.launches += 1;
+        CK(cudaEventSynchronize(ctx->evK1));
+        float ms = 0;
+        CK(cudaEventElapsedTime(&ms, ctx->evStart, ctx->evK1));
+        msMatch += ms;
+        rows = end;
+    }
+    ctx->stats.ms_match += msMatch;
+    ctx->stats.dist_evals += dist;
+    ctx->stats.match_pairs += n_pairs;
+    ctx->stats.match_rows += rows;
+    // the offsets are the caller's m_offset and the registration's host copy; the matches stay on the device for K0
+    r.nPairs = n_pairs;
+    r.nRows = rows;
+    r.h_offset.resize(n_pairs + 1);
+    CK(cudaMemcpyAsync(r.h_offset.data(), r.d_offset, (n_pairs + 1) * 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    ctx->stats.d2h_bytes += (n_pairs + 1) * 8;
+    memcpy(m_offset_out, r.h_offset.data(), (n_pairs + 1) * 8);
+    r.maxN = 0;
+    for (uint64_t p = 0; p < n_pairs; p++) r.maxN = std::max<uint32_t>(r.maxN, (uint32_t)(r.h_offset[p + 1] - r.h_offset[p]));
+    if ((st = growDevice(ctx, &r.d_corr, r.capRows, (size_t)rows * 4)) != PGI_OK) return st;
+    ctx->sceneRows = rows;
+    ctx->sceneMatches = true;
+    return buildCorrespondences(ctx, r, thr_px);
+}
+
+pgi_status pgi_read_scene_matches(pgi_ctx *ctx, uint32_t *matches_out, double *ratios_or_null, uint64_t capacity_rows)
+{
+    if (!ctx) return PGI_ERR_INVALID;
+    if (!ctx->sceneMatches) { ctx->err = "no descriptor registration to read matches from"; return PGI_ERR_STATE; }
+    const uint64_t n = ctx->sceneRows;
+    if (capacity_rows < n || (!matches_out && n)) { ctx->err = "capacity too small"; return PGI_ERR_INVALID; }
+    CK(cudaSetDevice(ctx->cfg.device));
+    if (!n) return PGI_OK;
+    std::vector<float> r(ratios_or_null ? n : 0);
+    CK(cudaMemcpyAsync(matches_out, ctx->d_stM, n * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    if (ratios_or_null) CK(cudaMemcpyAsync(r.data(), ctx->d_stRatio, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    for (uint64_t i = 0; i < r.size(); i++) ratios_or_null[i] = (double)r[i];  // feature_utils.h:182: float widened
+    ctx->stats.d2h_bytes += n * 8 + r.size() * 4;
+    return PGI_OK;
 }
 
 pgi_status pgi_share_pairs(pgi_ctx *ctx, pgi_ctx *owner)

@@ -36,7 +36,8 @@ class PgiStats(C.Structure):
                 ("ms_fallback_solve", C.c_double), ("ms_fallback_score", C.c_double), ("ms_decompose", C.c_double),
                 ("ms_total", C.c_double), ("launches", C.c_uint64), ("pairs", C.c_uint64), ("corr_evals", C.c_uint64),
                 ("fallback_pairs", C.c_uint64), ("fallback_models", C.c_uint64), ("h2d_bytes", C.c_uint64),
-                ("d2h_bytes", C.c_uint64)]
+                ("d2h_bytes", C.c_uint64), ("ms_match", C.c_double), ("dist_evals", C.c_uint64), ("match_pairs", C.c_uint64),
+                ("match_rows", C.c_uint64)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
@@ -47,7 +48,8 @@ EXPORTS = [
     "pgi_register_scene", "pgi_share_pairs", "pgi_read_pair", "pgi_submit_wave", "pgi_wait_wave", "pgi_wait_wave_device",
     "pgi_estimate_pose", "pgi_test_pose", "pgi_graph_init", "pgi_graph_apply", "pgi_graph_search", "pgi_graph_stats",
     "pgi_guided_match", "pgi_match_features", "pgi_get_stats", "pgi_reset_stats", "pgi_dbg_sampson",
-    "pgi_dbg_five_point", "pgi_dbg_pose_from_essential", "pgi_dbg_fp64_peak",
+    "pgi_dbg_five_point", "pgi_dbg_pose_from_essential", "pgi_dbg_fp64_peak", "pgi_register_scene_descriptors",
+    "pgi_read_scene_matches",
 ]
 
 _lib = None
@@ -161,6 +163,33 @@ class Engine:
         self._ck(self.lib.pgi_register_scene(self.h, C.c_uint64(len(focal)), _ptr(focal), _ptr(size), _ptr(kpo), _ptr(kp),
                                              C.c_uint64(len(pv)), _ptr(pv), _ptr(mo), _ptr(mt), C.c_double(thr_px)))
         self.n_pairs, self.offset = len(pv), mo.copy()
+
+    def register_scene_descriptors(self, scene, thr_px=0.4):
+        """matchFeatures for every pair of `scene` on the device (K9), then the registration of register_scene from the
+        device-resident matches.  scene needs desc[sum K, dim] (float32, dim 64 or 128) beside the keys register_scene
+        reads, except m_offset / matches, which this fills in — with scene["ratios"], the scene's correspondences.h5."""
+        focal = _f64(scene["focal"]); size = _f64(scene["size"])
+        kpo = np.ascontiguousarray(scene["kp_offset"], dtype=np.uint64)
+        kp = np.ascontiguousarray(scene["kp"], dtype=np.float32)
+        desc = np.ascontiguousarray(scene["desc"], dtype=np.float32)
+        pv = np.ascontiguousarray(scene["pair_views"], dtype=np.uint32)
+        if desc.ndim != 2 or len(desc) != len(kp) or len(kpo) != len(focal) + 1 or int(kpo[-1]) != len(kp):
+            raise ValueError("desc must be a [sum K, dim] array row-aligned with kp / kp_offset")
+        mo = np.zeros(len(pv) + 1, dtype=np.uint64)
+        self._ck(self.lib.pgi_register_scene_descriptors(self.h, C.c_uint64(len(focal)), _ptr(focal), _ptr(size), _ptr(kpo),
+                                                         _ptr(kp), _ptr(desc), C.c_uint32(desc.shape[1]), C.c_uint64(len(pv)),
+                                                         _ptr(pv), C.c_double(thr_px), _ptr(mo)))
+        self.n_pairs, self.offset = len(pv), mo.copy()
+        matches, ratios = self.read_scene_matches(int(mo[-1]))
+        scene["m_offset"], scene["matches"], scene["ratios"] = mo, matches, ratios
+        return mo
+
+    def read_scene_matches(self, n_rows):
+        """(matches [n_rows, 2] u32, ratios [n_rows]) of the last register_scene_descriptors."""
+        m = np.zeros((n_rows, 2), dtype=np.uint32)
+        r = np.zeros(n_rows)
+        self._ck(self.lib.pgi_read_scene_matches(self.h, _ptr(m), _ptr(r), C.c_uint64(n_rows)))
+        return m, r
 
     def share_pairs(self, owner):
         """Use the pairs registered in `owner` (same device) without copying them."""

@@ -10,12 +10,15 @@ A scene is a dict of numpy arrays:
   pair_views[P,2] u32 (src<dst as the similarity queue emits them), m_offset[P+1] u64,
   matches[sum N,2] u32 (srcIdx,dstIdx) in the order matchFeatures would emit (sorted by ratio = shuffled),
   gt_q[V,4]/gt_t[V,3] world->camera ground truth (accuracy reporting only).
+A descriptor scene (make_descriptor_scene; the reference's keypoints.h5) has desc[sum K,dim] f32 row-aligned with kp and
+no matches until they are computed (Engine.register_scene_descriptors fills m_offset, matches and ratios[sum N] f64).
 """
 import struct
 
 import numpy as np
 
 MAGIC = b"PGISCN01"
+MAGIC_V2 = b"PGISCN02"  # + descriptors, matches and ratios optional
 
 
 def _rot_look_at(cam_pos, target, up=np.array([0.0, 0.0, 1.0])):
@@ -153,9 +156,87 @@ CONFIGS = {
 }
 
 
+def make_descriptor_scene(n_views=12, kp_range=(600, 2500), dim=128, seed=0, n_points=None, kp_counts=None, focal=800.0,
+                          width=1600.0, height=1200.0, noise_px=0.5, desc_noise=0.05, distractor_ratio=0.3, radius=6.0,
+                          arc=2.0 * np.pi, visible_half_angle=0.5 * np.pi):
+    """Keypoints and descriptors of every view, no matches (what matchFeatures starts from).  Cameras on a ring as in
+    make_scene.  Every 3-D point faces a random azimuth and is detectable only from cameras within visible_half_angle of
+    it, so overlap falls with the ring distance and far pairs end below kMinimumPointNumber.  View v keeps kp_counts[v]
+    keypoints (default: uniform in kp_range): a random subset of its detectable points plus distractor_ratio of unrelated
+    keypoints, in its own shuffled order.  A point's descriptor is a unit vector plus per-view Gaussian noise (desc_noise
+    per dimension, as tests/helpers.two_view_keypoints); a distractor's is an unrelated unit vector.  gt_point[sum K] holds
+    the 3-D point of each keypoint (-1 for distractors).  Uses its own RNG stream: make_scene is unaffected."""
+    rng = np.random.default_rng(seed)
+    V = n_views
+    counts = (np.asarray(kp_counts, dtype=np.int64) if kp_counts is not None
+              else rng.integers(int(kp_range[0]), int(kp_range[1]) + 1, V))
+    assert len(counts) == V
+    if n_points is None:
+        n_points = max(64, 2 * int(counts.max()) if V else 64)
+    pts = rng.standard_normal((n_points, 3))
+    facing = rng.uniform(0.0, 2.0 * np.pi, n_points)
+    base = rng.standard_normal((n_points, dim))
+    base /= np.linalg.norm(base, axis=1, keepdims=True)
+    ang = np.arange(V) * (arc / max(V, 1)) + rng.uniform(-0.2, 0.2, V) * (arc / max(V, 1))
+    elev = rng.uniform(-0.25, 0.25, V)
+    rad = radius * (1.0 + rng.uniform(-0.15, 0.15, V))
+    cam = np.stack([rad * np.cos(ang) * np.cos(elev), rad * np.sin(ang) * np.cos(elev), rad * np.sin(elev)], 1)
+    Rw = np.stack([_rot_look_at(cam[v], rng.standard_normal(3) * 0.15) for v in range(V)]) if V else np.zeros((0, 3, 3))
+    tw = -np.einsum("vij,vj->vi", Rw, cam)
+    kps, descs, pids = [], [], []
+    for v in range(V):
+        dphi = np.abs((facing - ang[v] + np.pi) % (2.0 * np.pi) - np.pi)
+        vis = np.flatnonzero(dphi < visible_half_angle)
+        n_real = min(len(vis), int(round(counts[v] * (1.0 - distractor_ratio))))
+        real = rng.choice(vis, n_real, replace=False) if n_real else np.zeros(0, dtype=np.int64)
+        m = int(counts[v]) - n_real
+        Xc = pts[real] @ Rw[v].T + tw[v]
+        uv = focal * Xc[:, :2] / Xc[:, 2:3] + np.array([width / 2.0, height / 2.0]) + rng.standard_normal((n_real, 2)) * noise_px
+        d = base[real] + rng.standard_normal((n_real, dim)) * desc_noise
+        de = rng.standard_normal((m, dim))
+        de /= np.linalg.norm(de, axis=1, keepdims=True)
+        uv = np.vstack([uv, rng.uniform([0.0, 0.0], [width, height], (m, 2))])
+        d = np.vstack([d, de])
+        pid = np.concatenate([real, np.full(m, -1)])
+        order = rng.permutation(int(counts[v]))
+        kps.append(uv[order].astype(np.float32)); descs.append(d[order].astype(np.float32)); pids.append(pid[order])
+    view_dir = Rw[:, 2, :]
+    sim = np.round(np.minimum(np.clip(view_dir @ view_dir.T, 0.0, 0.999), 0.999), 3)
+    sim = np.round((sim + sim.T) / 2.0, 3)
+    np.fill_diagonal(sim, 1.0)
+    iu, ju = np.triu_indices(V, 1)
+    gt_q = np.array([_quat_from_rot(Rw[v]) for v in range(V)]).reshape(V, 4)
+    return dict(focal=np.full(V, focal), size=np.tile(np.array([width, height]), (V, 1)), sim=sim,
+                kp_offset=np.concatenate([[0], np.cumsum(counts)]).astype(np.uint64),
+                kp=np.concatenate(kps).reshape(-1, 2) if V else np.zeros((0, 2), dtype=np.float32),
+                desc=np.concatenate(descs).reshape(-1, dim) if V else np.zeros((0, dim), dtype=np.float32),
+                pair_views=np.stack([iu, ju], 1).astype(np.uint32), gt_q=gt_q, gt_t=tw.copy(), gt_R=Rw.copy(),
+                gt_point=np.concatenate(pids).astype(np.int64) if V else np.zeros(0, dtype=np.int64))
+
+
 def save_scene(path, scene):
-    """Binary container of SURVEY App. D: header + arrays, little-endian."""
+    """Binary container of SURVEY App. D: header + arrays, little-endian.  A scene with descriptors is written as
+    version 2 (PGISCN02: the version-1 header plus dim and which of matches / ratios follow, then desc and those); any
+    other scene as version 1, byte for byte as before."""
     V, P = len(scene["focal"]), len(scene["pair_views"])
+    if "desc" in scene:
+        desc = np.ascontiguousarray(scene["desc"], dtype="<f4")
+        has_m = "matches" in scene and "m_offset" in scene
+        has_r = has_m and "ratios" in scene
+        M = len(scene["matches"]) if has_m else 0
+        with open(path, "wb") as f:
+            f.write(MAGIC_V2)
+            f.write(struct.pack("<QQQQQQ", V, P, len(scene["kp"]), M, desc.shape[1], int(has_m) | int(has_r) << 1))
+            for key, dt in (("focal", "<f8"), ("size", "<f8"), ("sim", "<f8"), ("kp_offset", "<u8"), ("kp", "<f4"),
+                            ("pair_views", "<u4")):
+                f.write(np.ascontiguousarray(scene[key], dtype=dt).tobytes())
+            f.write(desc.tobytes())
+            if has_m:
+                f.write(np.ascontiguousarray(scene["m_offset"], dtype="<u8").tobytes())
+                f.write(np.ascontiguousarray(scene["matches"], dtype="<u4").tobytes())
+            if has_r:
+                f.write(np.ascontiguousarray(scene["ratios"], dtype="<f8").tobytes())
+        return
     with open(path, "wb") as f:
         f.write(MAGIC)
         f.write(struct.pack("<QQQQ", V, P, len(scene["kp"]), len(scene["matches"])))
@@ -166,13 +247,23 @@ def save_scene(path, scene):
 
 def load_scene(path):
     with open(path, "rb") as f:
-        assert f.read(8) == MAGIC, "not a PGI scene container"
-        V, P, K, M = struct.unpack("<QQQQ", f.read(32))
+        magic = f.read(8)
+        assert magic in (MAGIC, MAGIC_V2), "not a PGI scene container"
 
         def rd(dt, shape):
             n = int(np.prod(shape))
             return np.frombuffer(f.read(n * np.dtype(dt).itemsize), dtype=dt).reshape(shape).copy()
 
+        if magic == MAGIC_V2:
+            V, P, K, M, D, flags = struct.unpack("<QQQQQQ", f.read(48))
+            sc = dict(focal=rd("<f8", (V,)), size=rd("<f8", (V, 2)), sim=rd("<f8", (V, V)), kp_offset=rd("<u8", (V + 1,)),
+                      kp=rd("<f4", (K, 2)), pair_views=rd("<u4", (P, 2)), desc=rd("<f4", (K, D)))
+            if flags & 1:
+                sc["m_offset"], sc["matches"] = rd("<u8", (P + 1,)), rd("<u4", (M, 2))
+            if flags & 2:
+                sc["ratios"] = rd("<f8", (M,))
+            return sc
+        V, P, K, M = struct.unpack("<QQQQ", f.read(32))
         return dict(focal=rd("<f8", (V,)), size=rd("<f8", (V, 2)), sim=rd("<f8", (V, V)),
                     kp_offset=rd("<u8", (V + 1,)), kp=rd("<f4", (K, 2)), pair_views=rd("<u4", (P, 2)),
                     m_offset=rd("<u8", (P + 1,)), matches=rd("<u4", (M, 2)))
