@@ -7,7 +7,9 @@
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include <cuda_runtime.h>
@@ -24,19 +26,170 @@ using namespace pgi;
 
 namespace {
 
+// A device (or pinned host) allocation of `capacity()` elements of T, freed with its owner. Move-only.
+template <typename T, bool Pinned>
+class CudaBuf {
+public:
+    CudaBuf() = default;
+    CudaBuf(CudaBuf &&o) noexcept : p_(std::exchange(o.p_, nullptr)), cap_(std::exchange(o.cap_, 0)) {}
+    CudaBuf &operator=(CudaBuf o) noexcept  // the old allocation leaves with `o`
+    {
+        std::swap(p_, o.p_);
+        std::swap(cap_, o.cap_);
+        return *this;
+    }
+    ~CudaBuf() { release(); }
+
+    T *data() const { return p_; }
+    size_t capacity() const { return cap_; }
+
+    // Room for n elements (at least one). The old allocation is freed before the new one is made, so peak memory does
+    // not rise, and its contents are lost. A failed grow leaves the buffer empty.
+    cudaError_t grow(size_t n)
+    {
+        if (p_ && n <= cap_) return cudaSuccess;
+        cudaError_t e = release();
+        if (e == cudaSuccess) {
+            const size_t bytes = std::max<size_t>(n, 1) * sizeof(T);
+            e = Pinned ? cudaMallocHost((void **)&p_, bytes) : cudaMalloc((void **)&p_, bytes);
+        }
+        if (e != cudaSuccess) {
+            p_ = nullptr;
+            cudaGetLastError();  // a failed allocation must not be reported again by a later launch check
+            return e;
+        }
+        cap_ = n;
+        return cudaSuccess;
+    }
+
+private:
+    cudaError_t release()
+    {
+        cudaError_t e = cudaSuccess;
+        if (p_) e = Pinned ? cudaFreeHost(p_) : cudaFree(p_);
+        p_ = nullptr;
+        cap_ = 0;
+        return e;
+    }
+
+    T *p_ = nullptr;
+    size_t cap_ = 0;
+};
+
+template <typename T>
+using DevBuf = CudaBuf<T, false>;
+template <typename T>
+using PinnedBuf = CudaBuf<T, true>;
+
+// A stream or event, destroyed with its owner; converts to the runtime handle.
+template <typename H, cudaError_t (*Destroy)(H)>
+struct Owned {
+    H h = nullptr;
+    Owned() = default;
+    Owned(const Owned &) = delete;
+    Owned &operator=(const Owned &) = delete;
+    ~Owned() { if (h) Destroy(h); }
+    operator H() const { return h; }
+};
+using Stream = Owned<cudaStream_t, cudaStreamDestroy>;
+using Event = Owned<cudaEvent_t, cudaEventDestroy>;
+
+// The pairs a context verifies: normalised correspondences (4 doubles per row), offsets, thresholds, sampler tables.
 struct Registration {
-    double *d_corr = nullptr;
-    uint64_t *d_offset = nullptr;
-    double *d_thr = nullptr;
-    uint32_t *d_pairTable = nullptr;
-    uint32_t *d_sampler = nullptr;
-    uint16_t *d_itersTab = nullptr;
-    uint64_t *d_itersOff = nullptr;
+    DevBuf<double> corr;
+    DevBuf<uint64_t> offset;
+    DevBuf<double> thr;
+    DevBuf<uint32_t> pairTable, sampler;
+    DevBuf<uint16_t> itersTab;
+    DevBuf<uint64_t> itersOff;
     uint64_t nPairs = 0, nRows = 0;
     uint32_t maxN = 0;
     std::vector<uint64_t> h_offset;
-    bool borrowed = false;  // device buffers belong to another context (pgi_share_pairs)
-    size_t capRows = 0, capOffset = 0, capThr = 0, capPairTable = 0, capSampler = 0, capIters = 0, capTables = 0;
+};
+
+// Device arrays with one entry per wave slot, re-created together when the slot count or the bit stride grows.
+struct DevSlots {
+    uint32_t cap = 0;  // slots; 0 until every array is allocated
+    DevBuf<uint32_t> pairId, hypOffset, bits;
+    DevBuf<SlotState> state;
+    DevBuf<uint64_t> maskOffset;
+    DevBuf<pgi_verdict> verdicts;
+    DevBuf<uint32_t> k3Scratch;  // K3 vote totals + arrival ticket (zero between launches)
+};
+
+// Pinned staging of the per-slot wave inputs and verdicts.
+struct HostSlots {
+    uint32_t cap = 0;
+    PinnedBuf<uint32_t> pairId, hypOffset;
+    PinnedBuf<uint64_t> maskOffset;
+    PinnedBuf<pgi_verdict> verdicts;
+};
+
+// Scratch of the fallback kernels (K4, K5), sized for DevSlots::cap; created by the first fallback wave.
+struct FallbackScratch {
+    DevBuf<double> sols;
+    DevBuf<uint8_t> counts;
+    DevBuf<float4> solsF;
+    DevBuf<uint32_t> dkList, dkCtl;  // work list of the split K4 (K4a -> K4b -> K4c)
+};
+
+// The compact inputs of the last scene registration. Kept between registrations: cudaMalloc / cudaFree of GB-sized
+// buffers costs up to hundreds of milliseconds and synchronises the device.
+struct SceneStaging {
+    DevBuf<double> focal, size;
+    DevBuf<uint64_t> kpOff;
+    DevBuf<float2> kp;
+    DevBuf<uint2> pv, m;
+    // pgi_register_scene_descriptors: resident descriptors, the ratios beside m, the per-chunk scratch of K9
+    DevBuf<float> desc, ratio;
+    DevBuf<unsigned char> k9Scratch;
+    uint64_t rows = 0;
+    bool matches = false;  // m / ratio hold the matches of the last descriptor registration
+
+    // The match list is the one allocation that grows while it is filled: to max(need, 2 x capacity, 1024) rows,
+    // with its first `keep` rows copied over.
+    cudaError_t growMatches(uint64_t need, uint64_t keep, cudaStream_t s)
+    {
+        if (need <= m.capacity() && need <= ratio.capacity() && m.data() && ratio.data()) return cudaSuccess;
+        const size_t cap = std::max<size_t>({need, 2 * std::min(m.capacity(), ratio.capacity()), 1024});
+        DevBuf<uint2> m2;
+        DevBuf<float> ratio2;
+        cudaError_t e;
+        if ((e = m2.grow(cap)) != cudaSuccess || (e = ratio2.grow(cap)) != cudaSuccess) return e;
+        if (keep && ((e = cudaMemcpyAsync(m2.data(), m.data(), keep * sizeof(uint2), cudaMemcpyDeviceToDevice, s)) != cudaSuccess ||
+                     (e = cudaMemcpyAsync(ratio2.data(), ratio.data(), keep * sizeof(float), cudaMemcpyDeviceToDevice, s)) != cudaSuccess ||
+                     (e = cudaStreamSynchronize(s)) != cudaSuccess))
+            return e;
+        m = std::move(m2);
+        ratio = std::move(ratio2);
+        return cudaSuccess;
+    }
+};
+
+// K6: device mirror of the pose graph and the per-search slabs (pgi_graph_*). V is 0 until pgi_graph_init built it.
+struct Graph {
+    uint32_t V = 0, cap = 0, words = 0, heapCap = 0, arenaCap = 0, slots = 0;
+    DevBuf<AdjDev> adj;
+    DevBuf<uint32_t> counts;  // [0, V): committed entries per vertex, [V, 2V): committed + predicted
+    PinnedBuf<uint32_t> hCounts;
+    DevBuf<double> simT;
+    DevBuf<HeapItemDev> heaps;
+    DevBuf<ArenaNodeDev> arenas;
+    DevBuf<uint32_t> nextQuery;
+    struct {
+        uint32_t cap = 0;
+        DevBuf<ApplyEntry> dev;
+        PinnedBuf<ApplyEntry> host;
+    } apply;
+    struct {
+        uint32_t cap = 0;
+        DevBuf<pgi_query> queries;
+        DevBuf<pgi_search_result> results;
+        DevBuf<uint32_t> expBits;
+        PinnedBuf<pgi_query> hQueries;
+        PinnedBuf<pgi_search_result> hResults;
+        PinnedBuf<uint32_t> hExpBits;
+    } search;
 };
 
 constexpr int kMaxChunks = 64;
@@ -44,83 +197,41 @@ constexpr uint32_t kK5MaxSmemPts = 11264;  // 176 KB of float4 + 22 KB of queues
 
 }  // namespace
 
+// Members are destroyed in reverse order: the buffers first, then the events and the stream.
 struct pgi_ctx {
     pgi_config cfg;
-    cudaStream_t stream = nullptr;
+    Stream stream;
+    Event evBegin, evStart, evK1, evK2, evK3, evFbEnd;
+    Event evChunk[kMaxChunks][2];
+    Event evS0, evS1;
     std::string err;
-    Registration reg, tmp;
+    Registration own, tmp;
+    const Registration *reg = &own;  // own, or the owner's after pgi_share_pairs
     // wave buffers
-    uint32_t waveCap = 0, hypCap = 0, bitsStride = 0;
-    bool fbScratch = false;
-    uint64_t maskCap = 0;
-    uint32_t *d_pairId = nullptr, *d_hypOffset = nullptr, *d_bits = nullptr;
-    double *d_hyp = nullptr;
-    SlotState *d_state = nullptr;
-    uint8_t *d_masks = nullptr, *d_fbCounts = nullptr;
-    // staging of pgi_register_scene's compact inputs; kept between registrations (cudaMalloc / cudaFree of GB-sized
-    // buffers costs up to hundreds of milliseconds and synchronises the device)
-    double *d_stFocal = nullptr, *d_stSize = nullptr;
-    uint64_t *d_stKpOff = nullptr;
-    float2 *d_stKp = nullptr;
-    uint2 *d_stPv = nullptr, *d_stM = nullptr;
-    size_t capStFocal = 0, capStSize = 0, capStKpOff = 0, capStKp = 0, capStPv = 0, capStM = 0;
-    // pgi_register_scene_descriptors: resident descriptors, the ratios beside d_stM, the per-chunk scratch of K9
-    float *d_stDesc = nullptr, *d_stRatio = nullptr;
-    size_t capStDesc = 0, capStRatio = 0;
-    unsigned char *d_k9Scratch = nullptr;
-    size_t capK9Scratch = 0;
-    uint64_t sceneRows = 0;
-    bool sceneMatches = false;  // d_stM / d_stRatio hold the matches of the last descriptor registration
-    uint32_t *d_dkList = nullptr, *d_dkCtl = nullptr;  // work list of the split K4 (K4a -> K4b -> K4c)
+    DevSlots slots;
+    HostSlots hostSlots;
+    FallbackScratch fb;
+    uint32_t bitsStride = 0;  // only grows
+    DevBuf<double> hyp;       // 7 per hypothesis
+    PinnedBuf<double> hHyp;
+    DevBuf<uint8_t> masks;
+    DevBuf<unsigned long long> counters;
+    PinnedBuf<unsigned long long> hCounters;
+    SceneStaging scene;
     uint32_t k4aSmem = 0;  // PGI_K4A_SMEM: dynamic shared memory per K4a CTA, an occupancy throttle (L2 footprint of the 5 KB stacks)
     uint32_t k4bCtas = 2;  // K4b CTAs per SM (PGI_K4B_CTAS): fewer lanes = more polynomials per lane = better refill balance
     bool k4Split = true;   // PGI_K4_SPLIT=0 selects the one-kernel k4_fallback_solve
     bool k1Tma = true;     // PGI_K1_TMA=0: always the direct-load K1
     uint32_t numSms = 148;
-    uint32_t *d_k3Scratch = nullptr;  // per wave slot: K3 vote totals + arrival ticket (zero between launches)
-    uint64_t *d_maskOffset = nullptr;
-    pgi_verdict *d_verdicts = nullptr;
-    double *d_fbSols = nullptr;
-    float4 *d_fbSolsF = nullptr;
-    unsigned long long *d_counters = nullptr;
-    // pinned staging
-    uint32_t *h_pairId = nullptr, *h_hypOffset = nullptr;
-    double *h_hyp = nullptr;
-    uint64_t *h_maskOffset = nullptr;
-    pgi_verdict *h_verdicts = nullptr;
-    unsigned long long *h_counters = nullptr;
-    uint32_t hWaveCap = 0, hHypCap = 0;
     // in flight
     bool inFlight = false;
     uint32_t waveN = 0, waveFlags = 0;
     uint64_t waveMaskRows = 0;
     int nChunks = 0;
-    cudaEvent_t evBegin = nullptr, evStart = nullptr, evK1 = nullptr, evK2 = nullptr, evK3 = nullptr, evFbEnd = nullptr;
-    cudaEvent_t evChunk[kMaxChunks][2];
     bool fbLaunched = false;
     pgi_stats stats;
-    // ---- K6: device mirror of the pose graph + per-search slabs (pgi_graph_*) ----
-    AdjDev *d_adj = nullptr;
-    uint32_t gV = 0, gCap = 0, gWords = 0;
-    uint32_t *d_gCounts = nullptr;   // [0, V): committed entries per vertex, [V, 2V): committed + predicted
-    double *d_simT = nullptr;
-    HeapItemDev *d_heaps = nullptr;
-    ArenaNodeDev *d_arenas = nullptr;
-    uint32_t heapCap = 0, arenaCap = 0, searchSlots = 0;
-    pgi_query *d_queries = nullptr;
-    pgi_search_result *d_results = nullptr;
-    uint32_t *d_expBits = nullptr, *d_nextQuery = nullptr;
-    uint32_t queryCap = 0;
-    ApplyEntry *d_apply = nullptr;
-    uint32_t applyCap = 0;
-    ApplyEntry *h_apply = nullptr;
-    uint32_t *h_gCounts = nullptr;
-    pgi_query *h_queries = nullptr;
-    pgi_search_result *h_results = nullptr;
-    uint32_t *h_expBits = nullptr;
-    uint32_t hApplyCap = 0, hQueryCap = 0;
+    Graph graph;
     int popLookahead = 1, stagedPush = 1;
-    cudaEvent_t evS0 = nullptr, evS1 = nullptr;
     pgi_search_stats sstats;
 };
 
@@ -137,26 +248,6 @@ namespace {
             return e__ == cudaErrorMemoryAllocation ? PGI_ERR_NOMEM : PGI_ERR_CUDA;                \
         }                                                                                          \
     } while (0)
-
-template <typename T>
-pgi_status growDevice(pgi_ctx *ctx, T **p, size_t &cap, size_t need)
-{
-    if (need <= cap && *p) return PGI_OK;
-    if (*p) CK(cudaFree(*p));
-    *p = nullptr;
-    cap = 0;
-    CK(cudaMalloc((void **)p, std::max<size_t>(need, 1) * sizeof(T)));
-    cap = need;
-    return PGI_OK;
-}
-
-void freeReg(Registration &r)
-{
-    if (r.borrowed) { r = Registration(); return; }
-    cudaFree(r.d_corr); cudaFree(r.d_offset); cudaFree(r.d_thr); cudaFree(r.d_pairTable);
-    cudaFree(r.d_sampler); cudaFree(r.d_itersTab); cudaFree(r.d_itersOff);
-    r = Registration();
-}
 
 // cv::RNG (multiply-with-carry) on the host, for the sampler tables.
 struct HostRng {
@@ -225,15 +316,14 @@ pgi_status buildTables(pgi_ctx *ctx, Registration &r)
             }
         }
     }
-    pgi_status st;
-    if ((st = growDevice(ctx, &r.d_pairTable, r.capPairTable, (size_t)r.nPairs)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &r.d_sampler, r.capSampler, sampler.size())) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &r.d_itersTab, r.capIters, itersTab.size())) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &r.d_itersOff, r.capTables, T)) != PGI_OK) return st;
-    CK(cudaMemcpyAsync(r.d_pairTable, pairTable.data(), pairTable.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(r.d_sampler, sampler.data(), sampler.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(r.d_itersTab, itersTab.data(), itersTab.size() * 2, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(r.d_itersOff, itersOff.data(), itersOff.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CK(r.pairTable.grow(r.nPairs));
+    CK(r.sampler.grow(sampler.size()));
+    CK(r.itersTab.grow(itersTab.size()));
+    CK(r.itersOff.grow(T));
+    CK(cudaMemcpyAsync(r.pairTable.data(), pairTable.data(), pairTable.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(r.sampler.data(), sampler.data(), sampler.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(r.itersTab.data(), itersTab.data(), itersTab.size() * 2, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(r.itersOff.data(), itersOff.data(), itersOff.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     ctx->stats.h2d_bytes += pairTable.size() * 4 + sampler.size() * 4 + itersTab.size() * 2 + itersOff.size() * 8;
     return PGI_OK;
@@ -250,13 +340,12 @@ pgi_status registerDense(pgi_ctx *ctx, Registration &r, uint64_t nPairs, const u
     r.h_offset.assign(offset, offset + nPairs + 1);
     r.maxN = 0;
     for (uint64_t p = 0; p < nPairs; p++) r.maxN = std::max<uint32_t>(r.maxN, (uint32_t)(offset[p + 1] - offset[p]));
-    pgi_status st;
-    if ((st = growDevice(ctx, &r.d_corr, r.capRows, (size_t)r.nRows * 4)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &r.d_offset, r.capOffset, (size_t)nPairs + 1)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &r.d_thr, r.capThr, (size_t)nPairs)) != PGI_OK) return st;
-    if (r.nRows) CK(cudaMemcpyAsync(r.d_corr, corr, r.nRows * 32, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(r.d_offset, offset, (nPairs + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
-    if (nPairs) CK(cudaMemcpyAsync(r.d_thr, thr, nPairs * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CK(r.corr.grow(r.nRows * 4));
+    CK(r.offset.grow(nPairs + 1));
+    CK(r.thr.grow(nPairs));
+    if (r.nRows) CK(cudaMemcpyAsync(r.corr.data(), corr, r.nRows * 32, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(r.offset.data(), offset, (nPairs + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
+    if (nPairs) CK(cudaMemcpyAsync(r.thr.data(), thr, nPairs * 8, cudaMemcpyHostToDevice, ctx->stream));
     ctx->stats.h2d_bytes += r.nRows * 32 + (nPairs + 1) * 8 + nPairs * 8;
     return buildTables(ctx, r);
 }
@@ -264,71 +353,44 @@ pgi_status registerDense(pgi_ctx *ctx, Registration &r, uint64_t nPairs, const u
 pgi_status ensureWave(pgi_ctx *ctx, const Registration &r, uint32_t n, uint32_t nHyp, uint32_t flags, uint64_t maskRows)
 {
     const uint32_t stride = (r.maxN + 31) / 32 + 1;
-    if (n > ctx->waveCap || stride > ctx->bitsStride) {
-        const uint32_t cap = std::max<uint32_t>(std::max(n, ctx->waveCap), 64);
-        cudaFree(ctx->d_pairId); cudaFree(ctx->d_hypOffset); cudaFree(ctx->d_state); cudaFree(ctx->d_bits);
-        cudaFree(ctx->d_maskOffset); cudaFree(ctx->d_verdicts); cudaFree(ctx->d_fbSols); cudaFree(ctx->d_fbCounts); cudaFree(ctx->d_fbSolsF);
-        cudaFree(ctx->d_k3Scratch); cudaFree(ctx->d_dkList);
-        ctx->d_fbSolsF = nullptr; ctx->d_k3Scratch = nullptr; ctx->d_dkList = nullptr;
-        ctx->d_pairId = ctx->d_hypOffset = ctx->d_bits = nullptr; ctx->d_state = nullptr; ctx->d_maskOffset = nullptr;
-        ctx->d_verdicts = nullptr; ctx->d_fbSols = nullptr; ctx->d_fbCounts = nullptr;
-        ctx->fbScratch = false;
-        ctx->waveCap = 0;
+    if (n > ctx->slots.cap || stride > ctx->bitsStride) {
+        const uint32_t cap = std::max<uint32_t>(std::max(n, ctx->slots.cap), 64);
+        // the fallback scratch is sized for the old slot count: released here, re-created by the next fallback wave
+        ctx->fb = FallbackScratch();
+        ctx->slots = DevSlots();
         ctx->bitsStride = std::max(stride, ctx->bitsStride);
-        CK(cudaMalloc((void **)&ctx->d_pairId, (size_t)cap * 4));
-        CK(cudaMalloc((void **)&ctx->d_hypOffset, ((size_t)cap + 1) * 4));
-        CK(cudaMalloc((void **)&ctx->d_state, (size_t)cap * sizeof(SlotState)));
-        CK(cudaMalloc((void **)&ctx->d_bits, (size_t)cap * 2 * ctx->bitsStride * 4));
-        CK(cudaMalloc((void **)&ctx->d_maskOffset, ((size_t)cap + 1) * 8));
-        CK(cudaMalloc((void **)&ctx->d_verdicts, (size_t)cap * sizeof(pgi_verdict)));
-        CK(cudaMalloc((void **)&ctx->d_k3Scratch, (size_t)cap * 8 * 4));
-        CK(cudaMemsetAsync(ctx->d_k3Scratch, 0, (size_t)cap * 8 * 4, ctx->stream));
-        ctx->waveCap = cap;
+        CK(ctx->slots.pairId.grow(cap));
+        CK(ctx->slots.hypOffset.grow((size_t)cap + 1));
+        CK(ctx->slots.state.grow(cap));
+        CK(ctx->slots.bits.grow((size_t)cap * 2 * ctx->bitsStride));
+        CK(ctx->slots.maskOffset.grow((size_t)cap + 1));
+        CK(ctx->slots.verdicts.grow(cap));
+        CK(ctx->slots.k3Scratch.grow((size_t)cap * 8));
+        CK(cudaMemsetAsync(ctx->slots.k3Scratch.data(), 0, (size_t)cap * 8 * 4, ctx->stream));
+        ctx->slots.cap = cap;
     }
-    if ((flags & PGI_WAVE_FALLBACK) && !ctx->fbScratch) {
-        // (after a failed attempt some of these may be allocated: release them first, cudaFree(nullptr) is a no-op)
-        cudaFree(ctx->d_fbSols); cudaFree(ctx->d_fbCounts); cudaFree(ctx->d_fbSolsF); cudaFree(ctx->d_dkList);
-        ctx->d_fbSols = nullptr; ctx->d_fbCounts = nullptr; ctx->d_fbSolsF = nullptr; ctx->d_dkList = nullptr;
-        CK(cudaMalloc((void **)&ctx->d_fbSols, (size_t)ctx->waveCap * kFbChunk * 90 * 8));
-        CK(cudaMalloc((void **)&ctx->d_fbCounts, (size_t)ctx->waveCap * kFbChunk));
-        CK(cudaMalloc((void **)&ctx->d_fbSolsF, (size_t)ctx->waveCap * kFbChunk * 30 * sizeof(float4)));
-        CK(cudaMalloc((void **)&ctx->d_dkList, (size_t)ctx->waveCap * kFbChunk * 4));
-        if (!ctx->d_dkCtl) CK(cudaMalloc((void **)&ctx->d_dkCtl, 2 * 4));
-        ctx->fbScratch = true;
+    if (flags & PGI_WAVE_FALLBACK) {
+        const size_t slots = (size_t)ctx->slots.cap * kFbChunk;
+        CK(ctx->fb.sols.grow(slots * 90));
+        CK(ctx->fb.counts.grow(slots));
+        CK(ctx->fb.solsF.grow(slots * 30));
+        CK(ctx->fb.dkList.grow(slots));
+        CK(ctx->fb.dkCtl.grow(2));
     }
-    if (nHyp > ctx->hypCap) {
-        cudaFree(ctx->d_hyp);
-        ctx->d_hyp = nullptr;
-        ctx->hypCap = 0;  // (a failed allocation below must not leave a stale capacity behind a null pointer)
-        const uint32_t cap = std::max<uint32_t>(nHyp, std::max<uint32_t>(ctx->waveCap, 64));
-        CK(cudaMalloc((void **)&ctx->d_hyp, (size_t)cap * 7 * 8));
-        ctx->hypCap = cap;
+    if ((size_t)nHyp * 7 > ctx->hyp.capacity())
+        CK(ctx->hyp.grow((size_t)std::max<uint32_t>(nHyp, std::max<uint32_t>(ctx->slots.cap, 64)) * 7));
+    if ((flags & PGI_WAVE_MASKS) && maskRows > ctx->masks.capacity()) CK(ctx->masks.grow(maskRows));
+    if (n > ctx->hostSlots.cap) {
+        const uint32_t cap = std::max<uint32_t>(std::max(n, ctx->hostSlots.cap), 64);
+        ctx->hostSlots = HostSlots();
+        CK(ctx->hostSlots.pairId.grow(cap));
+        CK(ctx->hostSlots.hypOffset.grow((size_t)cap + 1));
+        CK(ctx->hostSlots.maskOffset.grow((size_t)cap + 1));
+        CK(ctx->hostSlots.verdicts.grow(cap));
+        ctx->hostSlots.cap = cap;
     }
-    if ((flags & PGI_WAVE_MASKS) && maskRows > ctx->maskCap) {
-        cudaFree(ctx->d_masks);
-        ctx->d_masks = nullptr;
-        ctx->maskCap = 0;
-        CK(cudaMalloc((void **)&ctx->d_masks, (size_t)maskRows));
-        ctx->maskCap = maskRows;
-    }
-    if (n > ctx->hWaveCap) {
-        const uint32_t cap = std::max<uint32_t>(std::max(n, ctx->hWaveCap), 64);
-        cudaFreeHost(ctx->h_pairId); cudaFreeHost(ctx->h_hypOffset); cudaFreeHost(ctx->h_maskOffset); cudaFreeHost(ctx->h_verdicts);
-        ctx->h_pairId = ctx->h_hypOffset = nullptr; ctx->h_maskOffset = nullptr; ctx->h_verdicts = nullptr;
-        ctx->hWaveCap = 0;
-        CK(cudaMallocHost((void **)&ctx->h_pairId, (size_t)cap * 4));
-        CK(cudaMallocHost((void **)&ctx->h_hypOffset, ((size_t)cap + 1) * 4));
-        CK(cudaMallocHost((void **)&ctx->h_maskOffset, ((size_t)cap + 1) * 8));
-        CK(cudaMallocHost((void **)&ctx->h_verdicts, (size_t)cap * sizeof(pgi_verdict)));
-        ctx->hWaveCap = cap;
-    }
-    if (nHyp > ctx->hHypCap) {
-        cudaFreeHost(ctx->h_hyp);
-        ctx->h_hyp = nullptr;
-        const uint32_t cap = std::max<uint32_t>(nHyp, std::max<uint32_t>(ctx->hWaveCap, 64));
-        CK(cudaMallocHost((void **)&ctx->h_hyp, (size_t)cap * 7 * 8));
-        ctx->hHypCap = cap;
-    }
+    if ((size_t)nHyp * 7 > ctx->hHyp.capacity())
+        CK(ctx->hHyp.grow((size_t)std::max<uint32_t>(nHyp, std::max<uint32_t>(ctx->hostSlots.cap, 64)) * 7));
     return PGI_OK;
 }
 
@@ -338,7 +400,7 @@ pgi_status submitWave(pgi_ctx *ctx, const Registration &r, uint32_t n, const uin
     if (ctx->inFlight) { ctx->err = "a wave is already in flight"; return PGI_ERR_STATE; }
     if (n == 0) { ctx->waveN = 0; ctx->inFlight = true; ctx->fbLaunched = false; ctx->nChunks = 0; ctx->waveFlags = flags; return PGI_OK; }
     if (!pairId || !hypOffset) { ctx->err = "null argument"; return PGI_ERR_INVALID; }
-    if (!r.d_offset) { ctx->err = "no pairs registered"; return PGI_ERR_STATE; }
+    if (!r.offset.data()) { ctx->err = "no pairs registered"; return PGI_ERR_STATE; }
     const uint32_t nHyp = hypOffset[n];
     if (nHyp && !hyp) { ctx->err = "hypotheses missing"; return PGI_ERR_INVALID; }
     uint64_t maskRows = 0;
@@ -348,35 +410,37 @@ pgi_status submitWave(pgi_ctx *ctx, const Registration &r, uint32_t n, const uin
     }
     pgi_status st = ensureWave(ctx, r, n, nHyp, flags, 0);
     if (st != PGI_OK) return st;
+    const DevSlots &d = ctx->slots;
+    const HostSlots &h = ctx->hostSlots;
     for (uint32_t i = 0; i < n; i++) {
-        ctx->h_maskOffset[i] = maskRows;
+        h.maskOffset.data()[i] = maskRows;
         maskRows += r.h_offset[pairId[i] + 1] - r.h_offset[pairId[i]];
     }
-    ctx->h_maskOffset[n] = maskRows;
+    h.maskOffset.data()[n] = maskRows;
     if ((st = ensureWave(ctx, r, n, nHyp, flags, maskRows)) != PGI_OK) return st;
-    memcpy(ctx->h_pairId, pairId, (size_t)n * 4);
-    memcpy(ctx->h_hypOffset, hypOffset, ((size_t)n + 1) * 4);
-    if (nHyp) memcpy(ctx->h_hyp, hyp, (size_t)nHyp * 56);
+    memcpy(h.pairId.data(), pairId, (size_t)n * 4);
+    memcpy(h.hypOffset.data(), hypOffset, ((size_t)n + 1) * 4);
+    if (nHyp) memcpy(ctx->hHyp.data(), hyp, (size_t)nHyp * 56);
     cudaStream_t s = ctx->stream;
     CK(cudaEventRecord(ctx->evBegin, s));
-    CK(cudaMemcpyAsync(ctx->d_pairId, ctx->h_pairId, (size_t)n * 4, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(ctx->d_hypOffset, ctx->h_hypOffset, ((size_t)n + 1) * 4, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(ctx->d_maskOffset, ctx->h_maskOffset, ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, s));
-    if (nHyp) CK(cudaMemcpyAsync(ctx->d_hyp, ctx->h_hyp, (size_t)nHyp * 56, cudaMemcpyHostToDevice, s));
-    CK(cudaMemsetAsync(ctx->d_counters, 0, 3 * sizeof(unsigned long long), s));
+    CK(cudaMemcpyAsync(d.pairId.data(), h.pairId.data(), (size_t)n * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d.hypOffset.data(), h.hypOffset.data(), ((size_t)n + 1) * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d.maskOffset.data(), h.maskOffset.data(), ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, s));
+    if (nHyp) CK(cudaMemcpyAsync(ctx->hyp.data(), ctx->hHyp.data(), (size_t)nHyp * 56, cudaMemcpyHostToDevice, s));
+    CK(cudaMemsetAsync(ctx->counters.data(), 0, 3 * sizeof(unsigned long long), s));
     ctx->stats.h2d_bytes += (size_t)n * 4 + ((size_t)n + 1) * 12 + (size_t)nHyp * 56;
 
     WaveArgs a;
-    a.corr = r.d_corr; a.offset = r.d_offset; a.thr = r.d_thr; a.pairTable = r.d_pairTable;
-    a.samplerTab = r.d_sampler; a.itersTab = r.d_itersTab; a.itersTabOff = r.d_itersOff;
-    a.n = n; a.pairId = ctx->d_pairId; a.hypOffset = ctx->d_hypOffset; a.hyp = ctx->d_hyp; a.state = ctx->d_state;
-    a.bits = ctx->d_bits; a.bitsStride = ctx->bitsStride; a.masks = ctx->d_masks; a.maskOffset = ctx->d_maskOffset;
-    a.verdicts = ctx->d_verdicts; a.flags = flags; a.minInliers = ctx->cfg.min_inliers;
+    a.corr = r.corr.data(); a.offset = r.offset.data(); a.thr = r.thr.data(); a.pairTable = r.pairTable.data();
+    a.samplerTab = r.sampler.data(); a.itersTab = r.itersTab.data(); a.itersTabOff = r.itersOff.data();
+    a.n = n; a.pairId = d.pairId.data(); a.hypOffset = d.hypOffset.data(); a.hyp = ctx->hyp.data(); a.state = d.state.data();
+    a.bits = d.bits.data(); a.bitsStride = ctx->bitsStride; a.masks = ctx->masks.data(); a.maskOffset = d.maskOffset.data();
+    a.verdicts = d.verdicts.data(); a.flags = flags; a.minInliers = ctx->cfg.min_inliers;
     a.testMinInliers = testMinOverride ? testMinOverride : ctx->cfg.test_min_inliers;
     a.fbMaxIters = ctx->cfg.fallback_max_iters; a.thrMultiplier = ctx->cfg.threshold_multiplier;
     a.thrOverride = thrOverride;
-    a.fbSols = ctx->d_fbSols; a.fbSolsF = ctx->d_fbSolsF; a.fbCounts = ctx->d_fbCounts; a.counters = ctx->d_counters;
-    a.k3Scratch = ctx->d_k3Scratch; a.dkList = ctx->d_dkList; a.dkCtl = ctx->d_dkCtl;
+    a.fbSols = ctx->fb.sols.data(); a.fbSolsF = ctx->fb.solsF.data(); a.fbCounts = ctx->fb.counts.data(); a.counters = ctx->counters.data();
+    a.k3Scratch = d.k3Scratch.data(); a.dkList = ctx->fb.dkList.data(); a.dkCtl = ctx->fb.dkCtl.data();
 
     CK(cudaEventRecord(ctx->evStart, s));  // kernel-only timing: the wave's small H2D copies are before this event
     // full waves stream the correspondences through shared memory with bulk async copies (persistent CTAs, one per SM);
@@ -415,7 +479,7 @@ pgi_status submitWave(pgi_ctx *ctx, const Registration &r, uint32_t n, const uin
             for (int c = 0; c < ctx->nChunks; c++) {
                 const uint32_t threads = n * kFbChunk;
                 if (ctx->k4Split) {
-                    CK(cudaMemsetAsync(ctx->d_dkCtl, 0, 8, s));
+                    CK(cudaMemsetAsync(ctx->fb.dkCtl.data(), 0, 8, s));
                     k4a_polynomial<<<(threads + 127) / 128, 128, ctx->k4aSmem, s>>>(a, c);
                     k4b_roots<<<std::min<uint32_t>((threads + 127) / 128, ctx->numSms * ctx->k4bCtas), 128, 0, s>>>(a);
                     k4c_solutions<<<(threads + 127) / 128, 128, 0, s>>>(a, c);
@@ -478,27 +542,28 @@ pgi_status finishWave(pgi_ctx *ctx)
     }
     CK(cudaEventElapsedTime(&ms, ctx->evFbEnd, ctx->evK3)); ctx->stats.ms_decompose += ms;
     CK(cudaEventElapsedTime(&ms, ctx->evBegin, ctx->evK3)); ctx->stats.ms_total += ms;
-    ctx->stats.corr_evals += ctx->h_counters[0];
-    ctx->stats.fallback_pairs += ctx->h_counters[1];
-    ctx->stats.fallback_models += ctx->h_counters[2];
+    ctx->stats.corr_evals += ctx->hCounters.data()[0];
+    ctx->stats.fallback_pairs += ctx->hCounters.data()[1];
+    ctx->stats.fallback_models += ctx->hCounters.data()[2];
     ctx->inFlight = false;
     return PGI_OK;
 }
 
-// K0 (createCorrespondenceMatrix) over the staged scene (ctx->d_st*: views, keypoints, pair views, matches) into r,
-// whose d_offset, h_offset, nPairs, nRows and maxN are set and whose d_corr / d_thr hold nRows / nPairs entries; then the
+// K0 (createCorrespondenceMatrix) over the staged scene (ctx->scene: views, keypoints, pair views, matches) into r,
+// whose offset, h_offset, nPairs, nRows and maxN are set and whose corr / thr hold nRows / nPairs entries; then the
 // sampler tables.
 pgi_status buildCorrespondences(pgi_ctx *ctx, Registration &r, double thr_px)
 {
     cudaStream_t s = ctx->stream;
+    const SceneStaging &sc = ctx->scene;
     const uint64_t n_pairs = r.nPairs;
     if (n_pairs) {
         CK(cudaEventRecord(ctx->evStart, s));
         const uint32_t gx = std::max<uint32_t>(1, std::min<uint32_t>((r.maxN + 255) / 256, 64));
         const uint32_t gy = (uint32_t)std::min<uint64_t>(n_pairs, 65535), gz = (uint32_t)((n_pairs + gy - 1) / gy);
-        k0_build_correspondences<<<dim3(gx, gy, gz), 256, 0, s>>>(ctx->d_stFocal, ctx->d_stSize, ctx->d_stKpOff, ctx->d_stKp,
-                                                                   n_pairs, ctx->d_stPv, r.d_offset, ctx->d_stM, thr_px,
-                                                                   reinterpret_cast<double4 *>(r.d_corr), r.d_thr);
+        k0_build_correspondences<<<dim3(gx, gy, gz), 256, 0, s>>>(sc.focal.data(), sc.size.data(), sc.kpOff.data(), sc.kp.data(),
+                                                                   n_pairs, sc.pv.data(), r.offset.data(), sc.m.data(), thr_px,
+                                                                   reinterpret_cast<double4 *>(r.corr.data()), r.thr.data());
         CK(cudaEventRecord(ctx->evK1, s));
         CK(cudaGetLastError());
         ctx->stats.launches += 1;
@@ -512,11 +577,31 @@ pgi_status buildCorrespondences(pgi_ctx *ctx, Registration &r, double thr_px)
     return buildTables(ctx, r);
 }
 
+// Grows the staging both scene registrations share and queues its upload: focal lengths, image sizes, keypoint
+// offsets, keypoints and pair views.
+pgi_status stageScene(pgi_ctx *ctx, uint64_t n_views, const double *focal, const double *size_wh, const uint64_t *kp_offset,
+                      const float *kp_xy, uint64_t n_pairs, const uint32_t *pair_views)
+{
+    SceneStaging &sc = ctx->scene;
+    const uint64_t nKp = kp_offset[n_views];
+    CK(sc.focal.grow(n_views));
+    CK(sc.size.grow(n_views * 2));
+    CK(sc.kpOff.grow(n_views + 1));
+    CK(sc.kp.grow(nKp));
+    CK(sc.pv.grow(n_pairs));
+    cudaStream_t s = ctx->stream;
+    CK(cudaMemcpyAsync(sc.focal.data(), focal, n_views * 8, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(sc.size.data(), size_wh, n_views * 16, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(sc.kpOff.data(), kp_offset, (n_views + 1) * 8, cudaMemcpyHostToDevice, s));
+    if (nKp) CK(cudaMemcpyAsync(sc.kp.data(), kp_xy, nKp * 8, cudaMemcpyHostToDevice, s));
+    if (n_pairs) CK(cudaMemcpyAsync(sc.pv.data(), pair_views, n_pairs * 8, cudaMemcpyHostToDevice, s));
+    ctx->stats.h2d_bytes += n_views * 24 + (n_views + 1) * 8 + nKp * 8 + n_pairs * 8;
+    return PGI_OK;
+}
+
 }  // namespace
 
 extern "C" {
-
-static void freeGraph(pgi_ctx *ctx);
 
 const char *pgi_version(void) { return "pgi 0.1 (sm_100a)"; }
 
@@ -541,7 +626,8 @@ pgi_status pgi_create(const pgi_config *cfg, pgi_ctx **out)
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, cfg->device) != cudaSuccess) return PGI_ERR_CUDA;
     if (prop.major != 10) return PGI_ERR_CUDA;  // kernels are sm_100a-only; there is no other path
-    pgi_ctx *ctx = new pgi_ctx();
+    // until it is handed out, a failure destroys the half-built context
+    std::unique_ptr<pgi_ctx, decltype(&pgi_destroy)> ctx(new pgi_ctx(), pgi_destroy);
     ctx->cfg = *cfg;
     if (const char *e = getenv("PGI_K4_SPLIT")) ctx->k4Split = atoi(e) != 0;
     if (const char *e = getenv("PGI_K1_TMA")) ctx->k1Tma = atoi(e) != 0;
@@ -555,28 +641,25 @@ pgi_status pgi_create(const pgi_config *cfg, pgi_ctx **out)
     if (ctx->cfg.threshold_multiplier == 0.0) ctx->cfg.threshold_multiplier = 3.0 / 2.0;
     memset(&ctx->stats, 0, sizeof ctx->stats);
     memset(&ctx->sstats, 0, sizeof ctx->sstats);
-    auto fail = [&](pgi_status s) { pgi_destroy(ctx); return s; };
-    if (cudaSetDevice(cfg->device) != cudaSuccess) return fail(PGI_ERR_CUDA);
+    if (cudaSetDevice(cfg->device) != cudaSuccess) return PGI_ERR_CUDA;
     {
         // flags bit 0: background context (lowest stream priority) — used for the hypothesis-independent fallback
         // prefetch so that the latency-critical wave kernels of the foreground context get SM slots first
         int prioLow = 0, prioHigh = 0;
         cudaDeviceGetStreamPriorityRange(&prioLow, &prioHigh);
         const int prio = (ctx->cfg.flags & 1u) ? prioLow : prioHigh;
-        if (cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, prio) != cudaSuccess) return fail(PGI_ERR_CUDA);
+        if (cudaStreamCreateWithPriority(&ctx->stream.h, cudaStreamNonBlocking, prio) != cudaSuccess) return PGI_ERR_CUDA;
     }
-    cudaEvent_t *evs[] = {&ctx->evBegin, &ctx->evStart, &ctx->evK1, &ctx->evK2, &ctx->evK3, &ctx->evFbEnd};
-    for (auto e : evs)
-        if (cudaEventCreate(e) != cudaSuccess) return fail(PGI_ERR_CUDA);
-    for (int c = 0; c < kMaxChunks; c++)
-        for (int k = 0; k < 2; k++) {
-            ctx->evChunk[c][k] = nullptr;
-            if (cudaEventCreate(&ctx->evChunk[c][k]) != cudaSuccess) return fail(PGI_ERR_CUDA);
-        }
-    if (cudaMalloc((void **)&ctx->d_counters, 3 * sizeof(unsigned long long)) != cudaSuccess) return fail(PGI_ERR_NOMEM);
-    if (cudaMallocHost((void **)&ctx->h_counters, 3 * sizeof(unsigned long long)) != cudaSuccess) return fail(PGI_ERR_NOMEM);
-    memset(ctx->h_counters, 0, 3 * sizeof(unsigned long long));
-    *out = ctx;
+    Event *evs[] = {&ctx->evBegin, &ctx->evStart, &ctx->evK1, &ctx->evK2, &ctx->evK3, &ctx->evFbEnd};
+    for (Event *e : evs)
+        if (cudaEventCreate(&e->h) != cudaSuccess) return PGI_ERR_CUDA;
+    for (auto &chunk : ctx->evChunk)
+        for (Event &e : chunk)
+            if (cudaEventCreate(&e.h) != cudaSuccess) return PGI_ERR_CUDA;
+    if (ctx->counters.grow(3) != cudaSuccess) return PGI_ERR_NOMEM;
+    if (ctx->hCounters.grow(3) != cudaSuccess) return PGI_ERR_NOMEM;
+    memset(ctx->hCounters.data(), 0, 3 * sizeof(unsigned long long));
+    *out = ctx.release();
     return PGI_OK;
 }
 
@@ -584,29 +667,9 @@ pgi_status pgi_destroy(pgi_ctx *ctx)
 {
     if (!ctx) return PGI_OK;
     cudaSetDevice(ctx->cfg.device);
-    if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-    freeGraph(ctx);
-    if (ctx->evS0) cudaEventDestroy(ctx->evS0);
-    if (ctx->evS1) cudaEventDestroy(ctx->evS1);
-    freeReg(ctx->reg);
-    freeReg(ctx->tmp);
-    cudaFree(ctx->d_pairId); cudaFree(ctx->d_hypOffset); cudaFree(ctx->d_bits); cudaFree(ctx->d_hyp);
-    cudaFree(ctx->d_state); cudaFree(ctx->d_masks); cudaFree(ctx->d_fbCounts); cudaFree(ctx->d_maskOffset);
-    cudaFree(ctx->d_verdicts); cudaFree(ctx->d_fbSols); cudaFree(ctx->d_fbSolsF); cudaFree(ctx->d_counters);
-    cudaFree(ctx->d_k3Scratch); cudaFree(ctx->d_dkList); cudaFree(ctx->d_dkCtl);
-    cudaFree(ctx->d_stFocal); cudaFree(ctx->d_stSize); cudaFree(ctx->d_stKpOff); cudaFree(ctx->d_stKp); cudaFree(ctx->d_stPv); cudaFree(ctx->d_stM);
-    cudaFree(ctx->d_stDesc); cudaFree(ctx->d_stRatio); cudaFree(ctx->d_k9Scratch);
-    cudaFreeHost(ctx->h_pairId); cudaFreeHost(ctx->h_hypOffset); cudaFreeHost(ctx->h_hyp);
-    cudaFreeHost(ctx->h_maskOffset); cudaFreeHost(ctx->h_verdicts); cudaFreeHost(ctx->h_counters);
-    cudaEvent_t evs[] = {ctx->evBegin, ctx->evStart, ctx->evK1, ctx->evK2, ctx->evK3, ctx->evFbEnd};
-    for (auto e : evs)
-        if (e) cudaEventDestroy(e);
-    for (int c = 0; c < kMaxChunks; c++)
-        for (int k = 0; k < 2; k++)
-            if (ctx->evChunk[c][k]) cudaEventDestroy(ctx->evChunk[c][k]);
-    if (ctx->stream) cudaStreamDestroy(ctx->stream);
-    cudaGetLastError();
+    if (ctx->stream) cudaStreamSynchronize(ctx->stream);  // nothing still running may use a buffer freed below
     delete ctx;
+    cudaGetLastError();
     return PGI_OK;
 }
 
@@ -619,8 +682,8 @@ pgi_status pgi_register_pairs(pgi_ctx *ctx, uint64_t n_pairs, const uint64_t *co
     if (!ctx) return PGI_ERR_INVALID;
     if (ctx->inFlight) { ctx->err = "a wave is in flight"; return PGI_ERR_STATE; }
     CK(cudaSetDevice(ctx->cfg.device));
-    if (ctx->reg.borrowed) ctx->reg = Registration();
-    return registerDense(ctx, ctx->reg, n_pairs, corr_offset, corr_xy4, thr_norm);
+    ctx->reg = &ctx->own;
+    return registerDense(ctx, ctx->own, n_pairs, corr_offset, corr_xy4, thr_norm);
 }
 
 pgi_status pgi_register_scene(pgi_ctx *ctx, uint64_t n_views, const double *focal, const double *size_wh,
@@ -636,9 +699,9 @@ pgi_status pgi_register_scene(pgi_ctx *ctx, uint64_t n_views, const double *foca
         return PGI_ERR_INVALID;
     }
     CK(cudaSetDevice(ctx->cfg.device));
-    if (ctx->reg.borrowed) ctx->reg = Registration();
-    Registration &r = ctx->reg;
-    const uint64_t nKp = kp_offset[n_views], nRows = m_offset[n_pairs];
+    ctx->reg = &ctx->own;
+    Registration &r = ctx->own;
+    const uint64_t nRows = m_offset[n_pairs];
     for (uint64_t p = 0; p < n_pairs; p++) {
         if (pair_views[2 * p] >= n_views || pair_views[2 * p + 1] >= n_views) { ctx->err = "view id out of range"; return PGI_ERR_INVALID; }
         if (m_offset[p + 1] < m_offset[p] || m_offset[p + 1] - m_offset[p] > 0x7fffffffULL) { ctx->err = "bad m_offset"; return PGI_ERR_INVALID; }
@@ -648,35 +711,16 @@ pgi_status pgi_register_scene(pgi_ctx *ctx, uint64_t n_views, const double *foca
     r.h_offset.assign(m_offset, m_offset + n_pairs + 1);
     r.maxN = 0;
     for (uint64_t p = 0; p < n_pairs; p++) r.maxN = std::max<uint32_t>(r.maxN, (uint32_t)(m_offset[p + 1] - m_offset[p]));
-    pgi_status st;
-    if ((st = growDevice(ctx, &r.d_corr, r.capRows, (size_t)nRows * 4)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &r.d_offset, r.capOffset, (size_t)n_pairs + 1)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &r.d_thr, r.capThr, (size_t)n_pairs)) != PGI_OK) return st;
-    // staging buffers for the compact inputs (owned by the context, grown on demand)
-    if ((st = growDevice(ctx, &ctx->d_stFocal, ctx->capStFocal, (size_t)n_views)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &ctx->d_stSize, ctx->capStSize, (size_t)n_views * 2)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &ctx->d_stKpOff, ctx->capStKpOff, (size_t)n_views + 1)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &ctx->d_stKp, ctx->capStKp, (size_t)nKp)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &ctx->d_stPv, ctx->capStPv, (size_t)n_pairs)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &ctx->d_stM, ctx->capStM, (size_t)nRows)) != PGI_OK) return st;
-    double *d_focal = ctx->d_stFocal, *d_size = ctx->d_stSize;
-    uint64_t *d_kpOff = ctx->d_stKpOff;
-    float2 *d_kp = ctx->d_stKp;
-    uint2 *d_pv = ctx->d_stPv, *d_m = ctx->d_stM;
+    CK(r.corr.grow(nRows * 4));
+    CK(r.offset.grow(n_pairs + 1));
+    CK(r.thr.grow(n_pairs));
+    CK(ctx->scene.m.grow(nRows));
+    if (pgi_status st = stageScene(ctx, n_views, focal, size_wh, kp_offset, kp_xy, n_pairs, pair_views); st != PGI_OK) return st;
     cudaStream_t s = ctx->stream;
-    auto cleanup = [&]() {};
-#define CKC(call) do { cudaError_t e2__ = (call); if (e2__ != cudaSuccess) { cleanup(); ctx->err = std::string(#call) + ": " + cudaGetErrorString(e2__); return e2__ == cudaErrorMemoryAllocation ? PGI_ERR_NOMEM : PGI_ERR_CUDA; } } while (0)
-    CKC(cudaMemcpyAsync(d_focal, focal, n_views * 8, cudaMemcpyHostToDevice, s));
-    CKC(cudaMemcpyAsync(d_size, size_wh, n_views * 16, cudaMemcpyHostToDevice, s));
-    CKC(cudaMemcpyAsync(d_kpOff, kp_offset, (n_views + 1) * 8, cudaMemcpyHostToDevice, s));
-    CKC(cudaMemcpyAsync(d_kp, kp_xy, nKp * 8, cudaMemcpyHostToDevice, s));
-    CKC(cudaMemcpyAsync(d_pv, pair_views, n_pairs * 8, cudaMemcpyHostToDevice, s));
-    CKC(cudaMemcpyAsync(d_m, matches, nRows * 8, cudaMemcpyHostToDevice, s));
-    CKC(cudaMemcpyAsync(r.d_offset, m_offset, (n_pairs + 1) * 8, cudaMemcpyHostToDevice, s));
-    ctx->stats.h2d_bytes += n_views * 24 + (n_views + 1) * 8 + nKp * 8 + n_pairs * 8 + nRows * 8 + (n_pairs + 1) * 8;
-    ctx->sceneMatches = false;  // d_stM now holds the caller's matches
-    cleanup();
-#undef CKC
+    CK(cudaMemcpyAsync(ctx->scene.m.data(), matches, nRows * 8, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(r.offset.data(), m_offset, (n_pairs + 1) * 8, cudaMemcpyHostToDevice, s));
+    ctx->stats.h2d_bytes += nRows * 8 + (n_pairs + 1) * 8;
+    ctx->scene.matches = false;  // m now holds the caller's matches
     return buildCorrespondences(ctx, r, thr_px);
 }
 
@@ -710,35 +754,26 @@ pgi_status pgi_register_scene_descriptors(pgi_ctx *ctx, uint64_t n_views, const 
     for (uint64_t p = 0; p < n_pairs; p++)
         if (pair_views[2 * p] >= n_views || pair_views[2 * p + 1] >= n_views) { ctx->err = "view id out of range"; return PGI_ERR_INVALID; }
     CK(cudaSetDevice(ctx->cfg.device));
-    if (ctx->reg.borrowed) ctx->reg = Registration();
-    Registration &r = ctx->reg;
+    ctx->reg = &ctx->own;
+    Registration &r = ctx->own;
+    SceneStaging &sc = ctx->scene;
     cudaStream_t s = ctx->stream;
     const uint64_t nKp = kp_offset[n_views];
-    ctx->sceneMatches = false;
-    pgi_status st;
-    if ((st = growDevice(ctx, &r.d_offset, r.capOffset, (size_t)n_pairs + 1)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &r.d_thr, r.capThr, (size_t)n_pairs)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &ctx->d_stFocal, ctx->capStFocal, (size_t)n_views)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &ctx->d_stSize, ctx->capStSize, (size_t)n_views * 2)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &ctx->d_stKpOff, ctx->capStKpOff, (size_t)n_views + 1)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &ctx->d_stKp, ctx->capStKp, (size_t)nKp)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &ctx->d_stPv, ctx->capStPv, (size_t)n_pairs)) != PGI_OK) return st;
-    if ((st = growDevice(ctx, &ctx->d_stDesc, ctx->capStDesc, (size_t)nKp * dim)) != PGI_OK) return st;
-    CK(cudaMemcpyAsync(ctx->d_stFocal, focal, n_views * 8, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(ctx->d_stSize, size_wh, n_views * 16, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(ctx->d_stKpOff, kp_offset, (n_views + 1) * 8, cudaMemcpyHostToDevice, s));
-    if (nKp) CK(cudaMemcpyAsync(ctx->d_stKp, kp_xy, nKp * 8, cudaMemcpyHostToDevice, s));
-    if (n_pairs) CK(cudaMemcpyAsync(ctx->d_stPv, pair_views, n_pairs * 8, cudaMemcpyHostToDevice, s));
+    sc.matches = false;
+    CK(r.offset.grow(n_pairs + 1));
+    CK(r.thr.grow(n_pairs));
+    CK(sc.desc.grow(nKp * dim));
+    if (pgi_status st = stageScene(ctx, n_views, focal, size_wh, kp_offset, kp_xy, n_pairs, pair_views); st != PGI_OK) return st;
     // every view's descriptors once; they stay resident for all of its pairs
-    if (nKp) CK(cudaMemcpyAsync(ctx->d_stDesc, desc, nKp * dim * 4, cudaMemcpyHostToDevice, s));
-    CK(cudaMemsetAsync(r.d_offset, 0, 8, s));
-    ctx->stats.h2d_bytes += n_views * 24 + (n_views + 1) * 8 + nKp * 8 + n_pairs * 8 + nKp * dim * 4;
+    if (nKp) CK(cudaMemcpyAsync(sc.desc.data(), desc, nKp * dim * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemsetAsync(r.offset.data(), 0, 8, s));
+    ctx->stats.h2d_bytes += nKp * dim * 4;
     // non-finite descriptors are rejected (a NaN distance never enters a 2-NN, so it would silently drop neighbours)
-    uint32_t *d_flag = reinterpret_cast<uint32_t *>(ctx->d_counters);
+    uint32_t *d_flag = reinterpret_cast<uint32_t *>(ctx->counters.data());
     uint32_t flag = 0;
     CK(cudaMemsetAsync(d_flag, 0, 4, s));
     if (nKp) {
-        k9_check_finite<<<(uint32_t)std::min<uint64_t>((nKp * dim + 1023) / 1024, 4 * ctx->numSms), 1024, 0, s>>>(ctx->d_stDesc, nKp * dim, d_flag);
+        k9_check_finite<<<(uint32_t)std::min<uint64_t>((nKp * dim + 1023) / 1024, 4 * ctx->numSms), 1024, 0, s>>>(sc.desc.data(), nKp * dim, d_flag);
         CK(cudaGetLastError());
         ctx->stats.launches += 1;
     }
@@ -757,32 +792,13 @@ pgi_status pgi_register_scene_descriptors(pgi_ctx *ctx, uint64_t n_views, const 
     auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
     const size_t oF = 0, oB = oF + al(chunk * stride * sizeof(Nn2)), oM = oB + al(chunk * maxSB * stride * sizeof(Nn2)),
                  oR = oM + al(chunk * stride * 8), oC = oR + al(chunk * stride * 4), total = oC + al(chunk * 4);
-    if ((st = growDevice(ctx, &ctx->d_k9Scratch, ctx->capK9Scratch, total)) != PGI_OK) return st;
-    Nn2 *d_fwd = reinterpret_cast<Nn2 *>(ctx->d_k9Scratch + oF), *d_bpart = reinterpret_cast<Nn2 *>(ctx->d_k9Scratch + oB);
-    uint2 *d_sm = reinterpret_cast<uint2 *>(ctx->d_k9Scratch + oM);
-    float *d_sr = reinterpret_cast<float *>(ctx->d_k9Scratch + oR);
-    uint32_t *d_cnt = reinterpret_cast<uint32_t *>(ctx->d_k9Scratch + oC);
+    CK(sc.k9Scratch.grow(total));
+    Nn2 *d_fwd = reinterpret_cast<Nn2 *>(sc.k9Scratch.data() + oF), *d_bpart = reinterpret_cast<Nn2 *>(sc.k9Scratch.data() + oB);
+    uint2 *d_sm = reinterpret_cast<uint2 *>(sc.k9Scratch.data() + oM);
+    float *d_sr = reinterpret_cast<float *>(sc.k9Scratch.data() + oR);
+    uint32_t *d_cnt = reinterpret_cast<uint32_t *>(sc.k9Scratch.data() + oC);
     const size_t finishSmem = (size_t)keyCap * 8 + (size_t)stride * 4;
     CK(cudaFuncSetAttribute(k9_finish, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)finishSmem));
-    // the match list is the one allocation that grows with the scene: doubled as needed, earlier rows kept
-    auto ensureRows = [&](uint64_t need, uint64_t keep) -> pgi_status {
-        if (need <= ctx->capStM && need <= ctx->capStRatio && ctx->d_stM && ctx->d_stRatio) return PGI_OK;
-        const size_t cap = std::max<size_t>({need, 2 * std::min(ctx->capStM, ctx->capStRatio), 1024});
-        uint2 *m = nullptr;
-        float *q = nullptr;
-        CK(cudaMalloc((void **)&m, cap * sizeof(uint2)));
-        if (cudaMalloc((void **)&q, cap * sizeof(float)) != cudaSuccess) { cudaFree(m); cudaGetLastError(); ctx->err = "out of device memory for the match list"; return PGI_ERR_NOMEM; }
-        if (keep) {
-            CK(cudaMemcpyAsync(m, ctx->d_stM, keep * sizeof(uint2), cudaMemcpyDeviceToDevice, s));
-            CK(cudaMemcpyAsync(q, ctx->d_stRatio, keep * sizeof(float), cudaMemcpyDeviceToDevice, s));
-            CK(cudaStreamSynchronize(s));
-        }
-        cudaFree(ctx->d_stM);
-        cudaFree(ctx->d_stRatio);
-        ctx->d_stM = m; ctx->d_stRatio = q;
-        ctx->capStM = ctx->capStRatio = cap;
-        return PGI_OK;
-    };
     float msMatch = 0;
     uint64_t rows = 0, dist = 0;
     for (uint64_t c0 = 0; c0 < n_pairs; c0 += chunk) {
@@ -799,22 +815,22 @@ pgi_status pgi_register_scene_descriptors(pgi_ctx *ctx, uint64_t n_views, const 
             PgiNvtxRange chunkRange("pgi:k9 chunk");
             if (sbUsed) {
                 if (dim == 128)
-                    k9_knn2_tile<128><<<dim3(sbUsed, cp), kK9Threads, 0, s>>>(ctx->d_stDesc, ctx->d_stKpOff, ctx->d_stPv, c0, stride, maxSB, d_fwd, d_bpart);
+                    k9_knn2_tile<128><<<dim3(sbUsed, cp), kK9Threads, 0, s>>>(sc.desc.data(), sc.kpOff.data(), sc.pv.data(), c0, stride, maxSB, d_fwd, d_bpart);
                 else
-                    k9_knn2_tile<64><<<dim3(sbUsed, cp), kK9Threads, 0, s>>>(ctx->d_stDesc, ctx->d_stKpOff, ctx->d_stPv, c0, stride, maxSB, d_fwd, d_bpart);
+                    k9_knn2_tile<64><<<dim3(sbUsed, cp), kK9Threads, 0, s>>>(sc.desc.data(), sc.kpOff.data(), sc.pv.data(), c0, stride, maxSB, d_fwd, d_bpart);
                 ctx->stats.launches += 1;
             }
-            k9_finish<<<cp, kK9FinishThreads, finishSmem, s>>>(ctx->d_stKpOff, ctx->d_stPv, c0, stride, keyCap, maxSB, d_fwd, d_bpart, d_cnt, d_sm, d_sr);
-            k9_offsets<<<1, 1024, 0, s>>>(d_cnt, cp, r.d_offset, c0);
+            k9_finish<<<cp, kK9FinishThreads, finishSmem, s>>>(sc.kpOff.data(), sc.pv.data(), c0, stride, keyCap, maxSB, d_fwd, d_bpart, d_cnt, d_sm, d_sr);
+            k9_offsets<<<1, 1024, 0, s>>>(d_cnt, cp, r.offset.data(), c0);
             CK(cudaGetLastError());
             ctx->stats.launches += 2;
         }
         uint64_t end = 0;
-        CK(cudaMemcpyAsync(&end, r.d_offset + c0 + cp, 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(&end, r.offset.data() + c0 + cp, 8, cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
         ctx->stats.d2h_bytes += 8;
-        if ((st = ensureRows(end, rows)) != PGI_OK) return st;
-        k9_scatter<<<cp, 256, 0, s>>>(r.d_offset, c0, stride, d_cnt, d_sm, d_sr, ctx->d_stM, ctx->d_stRatio);
+        CK(sc.growMatches(end, rows, s));
+        k9_scatter<<<cp, 256, 0, s>>>(r.offset.data(), c0, stride, d_cnt, d_sm, d_sr, sc.m.data(), sc.ratio.data());
         CK(cudaEventRecord(ctx->evK1, s));
         CK(cudaGetLastError());
         ctx->stats.launches += 1;
@@ -832,29 +848,29 @@ pgi_status pgi_register_scene_descriptors(pgi_ctx *ctx, uint64_t n_views, const 
     r.nPairs = n_pairs;
     r.nRows = rows;
     r.h_offset.resize(n_pairs + 1);
-    CK(cudaMemcpyAsync(r.h_offset.data(), r.d_offset, (n_pairs + 1) * 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(r.h_offset.data(), r.offset.data(), (n_pairs + 1) * 8, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     ctx->stats.d2h_bytes += (n_pairs + 1) * 8;
     memcpy(m_offset_out, r.h_offset.data(), (n_pairs + 1) * 8);
     r.maxN = 0;
     for (uint64_t p = 0; p < n_pairs; p++) r.maxN = std::max<uint32_t>(r.maxN, (uint32_t)(r.h_offset[p + 1] - r.h_offset[p]));
-    if ((st = growDevice(ctx, &r.d_corr, r.capRows, (size_t)rows * 4)) != PGI_OK) return st;
-    ctx->sceneRows = rows;
-    ctx->sceneMatches = true;
+    CK(r.corr.grow(rows * 4));
+    sc.rows = rows;
+    sc.matches = true;
     return buildCorrespondences(ctx, r, thr_px);
 }
 
 pgi_status pgi_read_scene_matches(pgi_ctx *ctx, uint32_t *matches_out, double *ratios_or_null, uint64_t capacity_rows)
 {
     if (!ctx) return PGI_ERR_INVALID;
-    if (!ctx->sceneMatches) { ctx->err = "no descriptor registration to read matches from"; return PGI_ERR_STATE; }
-    const uint64_t n = ctx->sceneRows;
+    if (!ctx->scene.matches) { ctx->err = "no descriptor registration to read matches from"; return PGI_ERR_STATE; }
+    const uint64_t n = ctx->scene.rows;
     if (capacity_rows < n || (!matches_out && n)) { ctx->err = "capacity too small"; return PGI_ERR_INVALID; }
     CK(cudaSetDevice(ctx->cfg.device));
     if (!n) return PGI_OK;
     std::vector<float> r(ratios_or_null ? n : 0);
-    CK(cudaMemcpyAsync(matches_out, ctx->d_stM, n * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    if (ratios_or_null) CK(cudaMemcpyAsync(r.data(), ctx->d_stRatio, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(matches_out, ctx->scene.m.data(), n * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    if (ratios_or_null) CK(cudaMemcpyAsync(r.data(), ctx->scene.ratio.data(), n * 4, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     for (uint64_t i = 0; i < r.size(); i++) ratios_or_null[i] = (double)r[i];  // feature_utils.h:182: float widened
     ctx->stats.d2h_bytes += n * 8 + r.size() * 4;
@@ -867,9 +883,8 @@ pgi_status pgi_share_pairs(pgi_ctx *ctx, pgi_ctx *owner)
     if (ctx->inFlight) { ctx->err = "a wave is in flight"; return PGI_ERR_STATE; }
     if (ctx->cfg.device != owner->cfg.device) { ctx->err = "contexts are on different devices"; return PGI_ERR_INVALID; }
     if (ctx->cfg.fallback_max_iters != owner->cfg.fallback_max_iters) { ctx->err = "fallback_max_iters differ"; return PGI_ERR_INVALID; }
-    freeReg(ctx->reg);
-    ctx->reg = owner->reg;  // shallow copy of the device pointers and host offsets
-    ctx->reg.borrowed = true;
+    ctx->own = Registration();  // not used while shared; a later pgi_register_* starts it afresh
+    ctx->reg = owner->reg;
     return PGI_OK;
 }
 
@@ -877,16 +892,16 @@ pgi_status pgi_read_pair(pgi_ctx *ctx, uint32_t pair_id, double *corr_xy4, uint6
                          double *thr_norm)
 {
     if (!ctx) return PGI_ERR_INVALID;
-    const Registration &r = ctx->reg;
+    const Registration &r = *ctx->reg;
     if (pair_id >= r.nPairs) { ctx->err = "pair_id out of range"; return PGI_ERR_INVALID; }
     CK(cudaSetDevice(ctx->cfg.device));
     const uint64_t n = r.h_offset[pair_id + 1] - r.h_offset[pair_id];
     if (n_rows) *n_rows = n;
     if (corr_xy4) {
         if (capacity_rows < n) { ctx->err = "capacity too small"; return PGI_ERR_INVALID; }
-        CK(cudaMemcpyAsync(corr_xy4, r.d_corr + 4 * r.h_offset[pair_id], n * 32, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(corr_xy4, r.corr.data() + 4 * r.h_offset[pair_id], n * 32, cudaMemcpyDeviceToHost, ctx->stream));
     }
-    if (thr_norm) CK(cudaMemcpyAsync(thr_norm, r.d_thr + pair_id, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    if (thr_norm) CK(cudaMemcpyAsync(thr_norm, r.thr.data() + pair_id, 8, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return PGI_OK;
 }
@@ -897,7 +912,7 @@ pgi_status pgi_submit_wave(pgi_ctx *ctx, uint32_t n, const uint32_t *pair_id, co
     PgiNvtxRange nvtxRange("pgi:submit_wave (H2D hypotheses + K1/K2/K4/K5/K3 launches)");
     if (!ctx) return PGI_ERR_INVALID;
     CK(cudaSetDevice(ctx->cfg.device));
-    return submitWave(ctx, ctx->reg, n, pair_id, hyp_offset, hyp_q_t, flags, 0.0, 0, false);
+    return submitWave(ctx, *ctx->reg, n, pair_id, hyp_offset, hyp_q_t, flags, 0.0, 0, false);
 }
 
 pgi_status pgi_wait_wave(pgi_ctx *ctx, pgi_verdict *out, uint8_t *masks_or_null)
@@ -910,12 +925,12 @@ pgi_status pgi_wait_wave(pgi_ctx *ctx, pgi_verdict *out, uint8_t *masks_or_null)
     const uint32_t n = ctx->waveN;
     if (n) {
         if (!out) { ctx->err = "null output"; return PGI_ERR_INVALID; }
-        CK(cudaMemcpyAsync(ctx->h_verdicts, ctx->d_verdicts, (size_t)n * sizeof(pgi_verdict), cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(ctx->hostSlots.verdicts.data(), ctx->slots.verdicts.data(), (size_t)n * sizeof(pgi_verdict), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(ctx->hCounters.data(), ctx->counters.data(), 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
         if (masks_or_null && (ctx->waveFlags & PGI_WAVE_MASKS) && ctx->waveMaskRows)
-            CK(cudaMemcpyAsync(masks_or_null, ctx->d_masks, ctx->waveMaskRows, cudaMemcpyDeviceToHost, ctx->stream));
+            CK(cudaMemcpyAsync(masks_or_null, ctx->masks.data(), ctx->waveMaskRows, cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
-        memcpy(out, ctx->h_verdicts, (size_t)n * sizeof(pgi_verdict));
+        memcpy(out, ctx->hostSlots.verdicts.data(), (size_t)n * sizeof(pgi_verdict));
         ctx->stats.d2h_bytes += (size_t)n * sizeof(pgi_verdict) + 24 + ((masks_or_null && (ctx->waveFlags & PGI_WAVE_MASKS)) ? ctx->waveMaskRows : 0);
     }
     return finishWave(ctx);
@@ -931,8 +946,8 @@ pgi_status pgi_wait_wave_device(pgi_ctx *ctx, void *verdicts_device)
     const uint32_t n = ctx->waveN;
     if (n) {
         if (!verdicts_device) { ctx->err = "null output"; return PGI_ERR_INVALID; }
-        CK(cudaMemcpyAsync(verdicts_device, ctx->d_verdicts, (size_t)n * sizeof(pgi_verdict), cudaMemcpyDeviceToDevice, ctx->stream));
-        CK(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(verdicts_device, ctx->slots.verdicts.data(), (size_t)n * sizeof(pgi_verdict), cudaMemcpyDeviceToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(ctx->hCounters.data(), ctx->counters.data(), 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
         ctx->stats.d2h_bytes += 24;
     }
@@ -982,8 +997,8 @@ int32_t pgi_test_pose(pgi_ctx *ctx, const double *corr_xy4, uint64_t n, double t
     if (st != PGI_OK) return st;
     // score-only wave: read the slot state instead of a verdict
     SlotState s;
-    CK(cudaMemcpyAsync(&s, ctx->d_state, sizeof s, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&s, ctx->slots.state.data(), sizeof s, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->hCounters.data(), ctx->counters.data(), 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     st = finishWave(ctx);
     if (st != PGI_OK) return st;
@@ -992,20 +1007,6 @@ int32_t pgi_test_pose(pgi_ctx *ctx, const double *corr_xy4, uint64_t n, double t
 }
 
 // ---- K6: device pose graph + batched A* -------------------------------------------------------------------
-static void freeGraph(pgi_ctx *ctx)
-{
-    cudaFree(ctx->d_adj); cudaFree(ctx->d_gCounts); cudaFree(ctx->d_simT); cudaFree(ctx->d_heaps); cudaFree(ctx->d_arenas);
-    cudaFree(ctx->d_queries); cudaFree(ctx->d_results); cudaFree(ctx->d_expBits); cudaFree(ctx->d_nextQuery); cudaFree(ctx->d_apply);
-    cudaFreeHost(ctx->h_apply); cudaFreeHost(ctx->h_gCounts); cudaFreeHost(ctx->h_queries); cudaFreeHost(ctx->h_results);
-    cudaFreeHost(ctx->h_expBits);
-    ctx->d_adj = nullptr; ctx->d_gCounts = nullptr; ctx->d_simT = nullptr; ctx->d_heaps = nullptr; ctx->d_arenas = nullptr;
-    ctx->d_queries = nullptr; ctx->d_results = nullptr; ctx->d_expBits = nullptr; ctx->d_nextQuery = nullptr; ctx->d_apply = nullptr;
-    ctx->h_apply = nullptr; ctx->h_gCounts = nullptr; ctx->h_queries = nullptr; ctx->h_results = nullptr; ctx->h_expBits = nullptr;
-    ctx->gV = ctx->gCap = ctx->gWords = 0;
-    ctx->queryCap = ctx->applyCap = ctx->hApplyCap = ctx->hQueryCap = 0;
-    ctx->heapCap = ctx->arenaCap = ctx->searchSlots = 0;
-}
-
 pgi_status pgi_graph_init(pgi_ctx *ctx, uint32_t n_views, const double *sim_to_next)
 {
     if (!ctx) return PGI_ERR_INVALID;
@@ -1027,23 +1028,27 @@ pgi_status pgi_graph_init(pgi_ctx *ctx, uint32_t n_views, const double *sim_to_n
     }
     const uint32_t slots = (uint32_t)prop.multiProcessorCount * slotsPerSm;
     const uint32_t arenaCap = 16384;
-    if (ctx->gV != V || ctx->heapCap != heapCap || ctx->searchSlots != slots) {
-        freeGraph(ctx);
-        ctx->gV = V; ctx->gCap = V; ctx->gWords = (V + 31) / 32;
-        CK(cudaMalloc((void **)&ctx->d_adj, (size_t)V * ctx->gCap * sizeof(AdjDev)));
-        CK(cudaMalloc((void **)&ctx->d_gCounts, (size_t)2 * V * 4));
-        CK(cudaMalloc((void **)&ctx->d_simT, (size_t)V * V * 8));
-        CK(cudaMalloc((void **)&ctx->d_heaps, (size_t)slots * heapCap * sizeof(HeapItemDev)));
-        CK(cudaMalloc((void **)&ctx->d_arenas, (size_t)slots * arenaCap * sizeof(ArenaNodeDev)));
-        CK(cudaMalloc((void **)&ctx->d_nextQuery, 4));
-        CK(cudaMallocHost((void **)&ctx->h_gCounts, (size_t)2 * V * 4));
-        ctx->heapCap = heapCap; ctx->arenaCap = arenaCap; ctx->searchSlots = slots;
+    if (ctx->graph.V != V || ctx->graph.heapCap != heapCap || ctx->graph.slots != slots) {
+        // the old graph is released first; the new one only replaces it once every allocation succeeded
+        ctx->graph = Graph();
+        Graph g;
+        CK(g.adj.grow((size_t)V * V));
+        CK(g.counts.grow((size_t)2 * V));
+        CK(g.simT.grow((size_t)V * V));
+        CK(g.heaps.grow((size_t)slots * heapCap));
+        CK(g.arenas.grow((size_t)slots * arenaCap));
+        CK(g.nextQuery.grow(1));
+        CK(g.hCounts.grow((size_t)2 * V));
+        g.V = V; g.cap = V; g.words = (V + 31) / 32;
+        g.heapCap = heapCap; g.arenaCap = arenaCap; g.slots = slots;
+        ctx->graph = std::move(g);
     }
-    CK(cudaMemsetAsync(ctx->d_gCounts, 0, (size_t)2 * V * 4, ctx->stream));
-    CK(cudaMemcpyAsync(ctx->d_simT, sim_to_next, (size_t)V * V * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemsetAsync(ctx->graph.counts.data(), 0, (size_t)2 * V * 4, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->graph.simT.data(), sim_to_next, (size_t)V * V * 8, cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     ctx->sstats.h2d_bytes += (uint64_t)V * V * 8;
-    if (!ctx->evS0) { CK(cudaEventCreate(&ctx->evS0)); CK(cudaEventCreate(&ctx->evS1)); }
+    if (!ctx->evS0) CK(cudaEventCreate(&ctx->evS0.h));
+    if (!ctx->evS1) CK(cudaEventCreate(&ctx->evS1.h));
     return PGI_OK;
 }
 
@@ -1051,31 +1056,31 @@ pgi_status pgi_graph_apply(pgi_ctx *ctx, uint32_t n_entries, const pgi_adj_entry
                            const uint32_t *total_count)
 {
     if (!ctx) return PGI_ERR_INVALID;
-    if (!ctx->d_adj) { ctx->err = "pgi_graph_init has not been called"; return PGI_ERR_STATE; }
+    Graph &g = ctx->graph;
+    if (!g.V) { ctx->err = "pgi_graph_init has not been called"; return PGI_ERR_STATE; }
     if ((n_entries && !entries) || !committed_count || !total_count) { ctx->err = "null argument"; return PGI_ERR_INVALID; }
     CK(cudaSetDevice(ctx->cfg.device));
-    const uint32_t V = ctx->gV;
+    const uint32_t V = g.V;
     for (uint32_t v = 0; v < V; v++)
-        if (total_count[v] < committed_count[v] || total_count[v] > ctx->gCap) { ctx->err = "bad edge-list count"; return PGI_ERR_INVALID; }
+        if (total_count[v] < committed_count[v] || total_count[v] > g.cap) { ctx->err = "bad edge-list count"; return PGI_ERR_INVALID; }
     for (uint32_t i = 0; i < n_entries; i++)
-        if (entries[i].vertex >= V || entries[i].next >= V || entries[i].index >= ctx->gCap) { ctx->err = "edge-list entry out of range"; return PGI_ERR_INVALID; }
-    if (n_entries > ctx->hApplyCap) {
+        if (entries[i].vertex >= V || entries[i].next >= V || entries[i].index >= g.cap) { ctx->err = "edge-list entry out of range"; return PGI_ERR_INVALID; }
+    if (n_entries > g.apply.cap) {
         const uint32_t cap = std::max<uint32_t>(n_entries * 2, 4096);
-        cudaFreeHost(ctx->h_apply); ctx->h_apply = nullptr; ctx->hApplyCap = 0;
-        cudaFree(ctx->d_apply); ctx->d_apply = nullptr; ctx->applyCap = 0;
-        CK(cudaMallocHost((void **)&ctx->h_apply, (size_t)cap * sizeof(ApplyEntry)));
-        CK(cudaMalloc((void **)&ctx->d_apply, (size_t)cap * sizeof(ApplyEntry)));
-        ctx->hApplyCap = ctx->applyCap = cap;
+        g.apply = {};
+        CK(g.apply.host.grow(cap));
+        CK(g.apply.dev.grow(cap));
+        g.apply.cap = cap;
     }
     static_assert(sizeof(ApplyEntry) == sizeof(pgi_adj_entry), "apply entry layout");
     cudaStream_t s = ctx->stream;
-    memcpy(ctx->h_gCounts, committed_count, (size_t)V * 4);
-    memcpy(ctx->h_gCounts + V, total_count, (size_t)V * 4);
-    CK(cudaMemcpyAsync(ctx->d_gCounts, ctx->h_gCounts, (size_t)2 * V * 4, cudaMemcpyHostToDevice, s));
+    memcpy(g.hCounts.data(), committed_count, (size_t)V * 4);
+    memcpy(g.hCounts.data() + V, total_count, (size_t)V * 4);
+    CK(cudaMemcpyAsync(g.counts.data(), g.hCounts.data(), (size_t)2 * V * 4, cudaMemcpyHostToDevice, s));
     if (n_entries) {
-        memcpy(ctx->h_apply, entries, (size_t)n_entries * sizeof(ApplyEntry));
-        CK(cudaMemcpyAsync(ctx->d_apply, ctx->h_apply, (size_t)n_entries * sizeof(ApplyEntry), cudaMemcpyHostToDevice, s));
-        k6_graph_apply<<<(n_entries + 255) / 256, 256, 0, s>>>(ctx->d_adj, ctx->gCap, ctx->d_apply, n_entries);
+        memcpy(g.apply.host.data(), entries, (size_t)n_entries * sizeof(ApplyEntry));
+        CK(cudaMemcpyAsync(g.apply.dev.data(), g.apply.host.data(), (size_t)n_entries * sizeof(ApplyEntry), cudaMemcpyHostToDevice, s));
+        k6_graph_apply<<<(n_entries + 255) / 256, 256, 0, s>>>(g.adj.data(), g.cap, g.apply.dev.data(), n_entries);
         CK(cudaGetLastError());
         ctx->sstats.launches += 1;
     }
@@ -1089,52 +1094,50 @@ pgi_status pgi_graph_search(pgi_ctx *ctx, uint32_t n, const pgi_query *queries, 
 {
     PgiNvtxRange nvtxRange("pgi:graph_search (K6)");
     if (!ctx) return PGI_ERR_INVALID;
-    if (!ctx->d_adj) { ctx->err = "pgi_graph_init has not been called"; return PGI_ERR_STATE; }
+    Graph &g = ctx->graph;
+    if (!g.V) { ctx->err = "pgi_graph_init has not been called"; return PGI_ERR_STATE; }
     if (n == 0) return PGI_OK;
     if (!queries || !results || !expanded_bits || max_depth > 7) { ctx->err = "bad argument"; return PGI_ERR_INVALID; }
     CK(cudaSetDevice(ctx->cfg.device));
-    const uint32_t V = ctx->gV, words = ctx->gWords;
+    const uint32_t V = g.V, words = g.words;
     for (uint32_t i = 0; i < n; i++)
         if (queries[i].src >= V || queries[i].dst >= V) { ctx->err = "query vertex out of range"; return PGI_ERR_INVALID; }
-    if (n > ctx->queryCap) {
+    auto &q = g.search;
+    if (n > q.cap) {
         const uint32_t cap = std::max<uint32_t>(n, 4096);
-        cudaFree(ctx->d_queries); cudaFree(ctx->d_results); cudaFree(ctx->d_expBits);
-        cudaFreeHost(ctx->h_queries); cudaFreeHost(ctx->h_results); cudaFreeHost(ctx->h_expBits);
-        ctx->d_queries = nullptr; ctx->d_results = nullptr; ctx->d_expBits = nullptr;
-        ctx->h_queries = nullptr; ctx->h_results = nullptr; ctx->h_expBits = nullptr;
-        ctx->queryCap = ctx->hQueryCap = 0;
-        CK(cudaMalloc((void **)&ctx->d_queries, (size_t)cap * sizeof(pgi_query)));
-        CK(cudaMalloc((void **)&ctx->d_results, (size_t)cap * sizeof(pgi_search_result)));
-        CK(cudaMalloc((void **)&ctx->d_expBits, (size_t)cap * words * 4));
-        CK(cudaMallocHost((void **)&ctx->h_queries, (size_t)cap * sizeof(pgi_query)));
-        CK(cudaMallocHost((void **)&ctx->h_results, (size_t)cap * sizeof(pgi_search_result)));
-        CK(cudaMallocHost((void **)&ctx->h_expBits, (size_t)cap * words * 4));
-        ctx->queryCap = ctx->hQueryCap = cap;
+        q = {};
+        CK(q.queries.grow(cap));
+        CK(q.results.grow(cap));
+        CK(q.expBits.grow((size_t)cap * words));
+        CK(q.hQueries.grow(cap));
+        CK(q.hResults.grow(cap));
+        CK(q.hExpBits.grow((size_t)cap * words));
+        q.cap = cap;
     }
     cudaStream_t s = ctx->stream;
-    memcpy(ctx->h_queries, queries, (size_t)n * sizeof(pgi_query));
-    CK(cudaMemcpyAsync(ctx->d_queries, ctx->h_queries, (size_t)n * sizeof(pgi_query), cudaMemcpyHostToDevice, s));
-    CK(cudaMemsetAsync(ctx->d_nextQuery, 0, 4, s));
+    memcpy(q.hQueries.data(), queries, (size_t)n * sizeof(pgi_query));
+    CK(cudaMemcpyAsync(q.queries.data(), q.hQueries.data(), (size_t)n * sizeof(pgi_query), cudaMemcpyHostToDevice, s));
+    CK(cudaMemsetAsync(g.nextQuery.data(), 0, 4, s));
     SearchArgs a;
-    a.adj = ctx->d_adj; a.cap = ctx->gCap; a.ccnt = ctx->d_gCounts; a.cnt = ctx->d_gCounts + V; a.simT = ctx->d_simT;
-    a.V = V; a.words = words; a.n = n; a.queries = ctx->d_queries; a.maxDepth = max_depth;
+    a.adj = g.adj.data(); a.cap = g.cap; a.ccnt = g.counts.data(); a.cnt = g.counts.data() + V; a.simT = g.simT.data();
+    a.V = V; a.words = words; a.n = n; a.queries = q.queries.data(); a.maxDepth = max_depth;
     a.weight = weight; a.oneMinusWeight = 1.0 - weight;
-    a.heaps = ctx->d_heaps; a.heapCap = ctx->heapCap; a.arenas = ctx->d_arenas; a.arenaCap = ctx->arenaCap;
-    a.results = ctx->d_results; a.expandedBits = ctx->d_expBits; a.nextQuery = ctx->d_nextQuery;
+    a.heaps = g.heaps.data(); a.heapCap = g.heapCap; a.arenas = g.arenas.data(); a.arenaCap = g.arenaCap;
+    a.results = q.results.data(); a.expandedBits = q.expBits.data(); a.nextQuery = g.nextQuery.data();
     a.popLookahead = ctx->popLookahead;
     a.staged = ctx->stagedPush;
-    const uint32_t ctas = std::min<uint32_t>((n + kAstarWarps - 1) / kAstarWarps, ctx->searchSlots / kAstarWarps);
+    const uint32_t ctas = std::min<uint32_t>((n + kAstarWarps - 1) / kAstarWarps, g.slots / kAstarWarps);
     const size_t smem = (size_t)kAstarWarps * ((size_t)kStageItems * sizeof(HeapItemDev) + (size_t)kChunk * 2 + (size_t)2 * words * 4);
     CK(cudaFuncSetAttribute(k6_astar_search, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)));
     CK(cudaEventRecord(ctx->evS0, s));
     k6_astar_search<<<ctas, kAstarWarps * 32, smem, s>>>(a);
     CK(cudaEventRecord(ctx->evS1, s));
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(ctx->h_results, ctx->d_results, (size_t)n * sizeof(pgi_search_result), cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(ctx->h_expBits, ctx->d_expBits, (size_t)n * words * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(q.hResults.data(), q.results.data(), (size_t)n * sizeof(pgi_search_result), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(q.hExpBits.data(), q.expBits.data(), (size_t)n * words * 4, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
-    memcpy(results, ctx->h_results, (size_t)n * sizeof(pgi_search_result));
-    memcpy(expanded_bits, ctx->h_expBits, (size_t)n * words * 4);
+    memcpy(results, q.hResults.data(), (size_t)n * sizeof(pgi_search_result));
+    memcpy(expanded_bits, q.hExpBits.data(), (size_t)n * words * 4);
     float ms = 0;
     CK(cudaEventElapsedTime(&ms, ctx->evS0, ctx->evS1));
     pgi_search_stats &st = ctx->sstats;
@@ -1182,18 +1185,17 @@ pgi_status pgi_guided_match(pgi_ctx *ctx, uint32_t n_src, const float *kp_src, c
     cudaStream_t s = ctx->stream;
     const size_t bS = (size_t)n_src, bD = (size_t)n_dst;
     // one scratch allocation per call: this entry point is the reference-shaped single-pair call
-    unsigned char *d = nullptr;
     auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
     const size_t oKpS = 0, oDS = oKpS + al(bS * 8), oKpD = oDS + al(bS * dim * 4), oDD = oKpD + al(bD * 8), oBin = oDD + al(bD * dim * 4),
                  oList = oBin + al(bD), oCand = oList + al(bD * 4), oRatio = oCand + al(bS * 4), oM = oRatio + al(bS * 8),
                  oR = oM + al(bS * 8), oN = oR + al(bS * 8), oPrep = oN + 256, total = oPrep + 256;
-    CK(cudaMalloc((void **)&d, total));
-    auto fail = [&](cudaError_t e) { cudaFree(d); ctx->err = cudaGetErrorString(e); return PGI_ERR_CUDA; };
-    cudaError_t e;
-    if ((e = cudaMemcpyAsync(d + oKpS, kp_src, bS * 8, cudaMemcpyHostToDevice, s)) != cudaSuccess) return fail(e);
-    if ((e = cudaMemcpyAsync(d + oDS, desc_src, bS * dim * 4, cudaMemcpyHostToDevice, s)) != cudaSuccess) return fail(e);
-    if ((e = cudaMemcpyAsync(d + oKpD, kp_dst, bD * 8, cudaMemcpyHostToDevice, s)) != cudaSuccess) return fail(e);
-    if ((e = cudaMemcpyAsync(d + oDD, desc_dst, bD * dim * 4, cudaMemcpyHostToDevice, s)) != cudaSuccess) return fail(e);
+    DevBuf<unsigned char> scratch;
+    CK(scratch.grow(total));
+    unsigned char *d = scratch.data();
+    CK(cudaMemcpyAsync(d + oKpS, kp_src, bS * 8, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d + oDS, desc_src, bS * dim * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d + oKpD, kp_dst, bD * 8, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d + oDD, desc_dst, bD * dim * 4, cudaMemcpyHostToDevice, s));
     MatchArgs a;
     a.kpS = reinterpret_cast<const float2 *>(d + oKpS); a.dS = reinterpret_cast<const float *>(d + oDS);
     a.kpD = reinterpret_cast<const float2 *>(d + oKpD); a.dD = reinterpret_cast<const float *>(d + oDD);
@@ -1220,17 +1222,16 @@ pgi_status pgi_guided_match(pgi_ctx *ctx, uint32_t n_src, const float *kp_src, c
     a.ratios = reinterpret_cast<double *>(d + oR); a.nOut = reinterpret_cast<uint32_t *>(d + oN);
     a.prepOut = reinterpret_cast<double *>(d + oPrep);
     k7_guided_match<<<1, kMatchThreads, 0, s>>>(a);
-    if ((e = cudaGetLastError()) != cudaSuccess) return fail(e);
+    CK(cudaGetLastError());
     uint32_t n = 0;
-    if ((e = cudaMemcpyAsync(&n, d + oN, 4, cudaMemcpyDeviceToHost, s)) != cudaSuccess) return fail(e);
-    if ((e = cudaStreamSynchronize(s)) != cudaSuccess) return fail(e);
+    CK(cudaMemcpyAsync(&n, d + oN, 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
     if (n > n_src) n = n_src;
     if (n) {
-        if ((e = cudaMemcpy(matches_out, d + oM, (size_t)n * 8, cudaMemcpyDeviceToHost)) != cudaSuccess) return fail(e);
-        if ((e = cudaMemcpy(ratios_out, d + oR, (size_t)n * 8, cudaMemcpyDeviceToHost)) != cudaSuccess) return fail(e);
+        CK(cudaMemcpy(matches_out, d + oM, (size_t)n * 8, cudaMemcpyDeviceToHost));
+        CK(cudaMemcpy(ratios_out, d + oR, (size_t)n * 8, cudaMemcpyDeviceToHost));
     }
-    if (prepared_or_null && (e = cudaMemcpy(prepared_or_null, d + oPrep, 14 * 8, cudaMemcpyDeviceToHost)) != cudaSuccess) return fail(e);
-    cudaFree(d);
+    if (prepared_or_null) CK(cudaMemcpy(prepared_or_null, d + oPrep, 14 * 8, cudaMemcpyDeviceToHost));
     *n_out = n;
     ctx->stats.launches += 1;
     ctx->stats.h2d_bytes += bS * (8 + dim * 4) + bD * (8 + dim * 4);
@@ -1255,12 +1256,11 @@ pgi_status pgi_match_features(pgi_ctx *ctx, uint32_t n_src, const float *desc_sr
     const size_t bS = n_src, bD = n_dst;
     const size_t oA = 0, oB = oA + al(bS * dim * 4), oF = oB + al(bD * dim * 4), oG = oF + al(bS * sizeof(Knn2)),
                  oM = oG + al(bD * sizeof(Knn2)), oR = oM + al(bS * 8), oN = oR + al(bS * 8), total = oN + 256;
-    unsigned char *d = nullptr;
-    CK(cudaMalloc((void **)&d, total));
-    auto fail = [&](cudaError_t e) { cudaFree(d); ctx->err = cudaGetErrorString(e); return PGI_ERR_CUDA; };
-    cudaError_t e;
-    if ((e = cudaMemcpyAsync(d + oA, desc_src, bS * dim * 4, cudaMemcpyHostToDevice, s)) != cudaSuccess) return fail(e);
-    if ((e = cudaMemcpyAsync(d + oB, desc_dst, bD * dim * 4, cudaMemcpyHostToDevice, s)) != cudaSuccess) return fail(e);
+    DevBuf<unsigned char> scratch;
+    CK(scratch.grow(total));
+    unsigned char *d = scratch.data();
+    CK(cudaMemcpyAsync(d + oA, desc_src, bS * dim * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d + oB, desc_dst, bD * dim * 4, cudaMemcpyHostToDevice, s));
     const float *A = reinterpret_cast<const float *>(d + oA), *B = reinterpret_cast<const float *>(d + oB);
     Knn2 *F = reinterpret_cast<Knn2 *>(d + oF), *G = reinterpret_cast<Knn2 *>(d + oG);
     if (dim == 128) {
@@ -1272,18 +1272,17 @@ pgi_status pgi_match_features(pgi_ctx *ctx, uint32_t n_src, const float *desc_sr
     }
     k8_mutual<<<1, 1024, 0, s>>>(F, n_src, G, n_dst, reinterpret_cast<uint32_t *>(d + oM), reinterpret_cast<double *>(d + oR),
                                  reinterpret_cast<uint32_t *>(d + oN));
-    if ((e = cudaGetLastError()) != cudaSuccess) return fail(e);
+    CK(cudaGetLastError());
     uint32_t n = 0;
-    if ((e = cudaMemcpyAsync(&n, d + oN, 4, cudaMemcpyDeviceToHost, s)) != cudaSuccess) return fail(e);
-    if ((e = cudaStreamSynchronize(s)) != cudaSuccess) return fail(e);
+    CK(cudaMemcpyAsync(&n, d + oN, 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
     if (n > n_src) n = n_src;
     std::vector<uint32_t> m((size_t)2 * n);
     std::vector<double> r(n);
     if (n) {
-        if ((e = cudaMemcpy(m.data(), d + oM, (size_t)n * 8, cudaMemcpyDeviceToHost)) != cudaSuccess) return fail(e);
-        if ((e = cudaMemcpy(r.data(), d + oR, (size_t)n * 8, cudaMemcpyDeviceToHost)) != cudaSuccess) return fail(e);
+        CK(cudaMemcpy(m.data(), d + oM, (size_t)n * 8, cudaMemcpyDeviceToHost));
+        CK(cudaMemcpy(r.data(), d + oR, (size_t)n * 8, cudaMemcpyDeviceToHost));
     }
-    cudaFree(d);
     // std::sort of (ratio, &matches[i]) pairs (feature_utils.h:188): by ratio, then by the address of the query's
     // match vector, i.e. by query index
     std::vector<uint32_t> order(n);
@@ -1343,16 +1342,16 @@ pgi_status pgi_dbg_sampson(pgi_ctx *ctx, const double *corr_xy4, uint64_t n, con
 {
     if (!ctx || !corr_xy4 || !E || !out) return PGI_ERR_INVALID;
     CK(cudaSetDevice(ctx->cfg.device));
-    double *d_c = nullptr, *d_E = nullptr, *d_o = nullptr;
-    CK(cudaMalloc((void **)&d_c, std::max<uint64_t>(n, 1) * 32));
-    CK(cudaMalloc((void **)&d_E, 72));
-    CK(cudaMalloc((void **)&d_o, std::max<uint64_t>(n, 1) * 8));
-    CK(cudaMemcpy(d_c, corr_xy4, n * 32, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_E, E, 72, cudaMemcpyHostToDevice));
-    if (n) kdbg_sampson<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(reinterpret_cast<double4 *>(d_c), n, d_E, d_o);
+    DevBuf<double4> d_c;
+    DevBuf<double> d_E, d_o;
+    CK(d_c.grow(n));
+    CK(d_E.grow(9));
+    CK(d_o.grow(n));
+    CK(cudaMemcpy(d_c.data(), corr_xy4, n * 32, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(d_E.data(), E, 72, cudaMemcpyHostToDevice));
+    if (n) kdbg_sampson<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(d_c.data(), n, d_E.data(), d_o.data());
     CK(cudaStreamSynchronize(ctx->stream));
-    CK(cudaMemcpy(out, d_o, n * 8, cudaMemcpyDeviceToHost));
-    cudaFree(d_c); cudaFree(d_E); cudaFree(d_o);
+    CK(cudaMemcpy(out, d_o.data(), n * 8, cudaMemcpyDeviceToHost));
     ctx->stats.launches += 1;
     return PGI_OK;
 }
@@ -1362,22 +1361,21 @@ pgi_status pgi_dbg_five_point(pgi_ctx *ctx, const double *x1, const double *x2, 
 {
     if (!ctx || !x1 || !x2 || !E_out || !count_out) return PGI_ERR_INVALID;
     CK(cudaSetDevice(ctx->cfg.device));
-    double *d_a = nullptr, *d_b = nullptr, *d_E = nullptr;
-    int *d_c = nullptr;
+    DevBuf<double> d_a, d_b, d_E;
+    DevBuf<int> d_c;
     const size_t n = std::max<uint32_t>(n_problems, 1);
-    CK(cudaMalloc((void **)&d_a, n * 80));
-    CK(cudaMalloc((void **)&d_b, n * 80));
-    CK(cudaMalloc((void **)&d_E, n * 720));
-    CK(cudaMalloc((void **)&d_c, n * 4));
-    CK(cudaMemset(d_E, 0, n * 720));
-    CK(cudaMemcpy(d_a, x1, (size_t)n_problems * 80, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_b, x2, (size_t)n_problems * 80, cudaMemcpyHostToDevice));
-    if (n_problems) kdbg_five_point<<<(n_problems + 63) / 64, 64, 0, ctx->stream>>>(d_a, d_b, n_problems, dk_max_iters, dk_tol_sq, d_E, d_c);
+    CK(d_a.grow(n * 10));
+    CK(d_b.grow(n * 10));
+    CK(d_E.grow(n * 90));
+    CK(d_c.grow(n));
+    CK(cudaMemset(d_E.data(), 0, n * 720));
+    CK(cudaMemcpy(d_a.data(), x1, (size_t)n_problems * 80, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(d_b.data(), x2, (size_t)n_problems * 80, cudaMemcpyHostToDevice));
+    if (n_problems) kdbg_five_point<<<(n_problems + 63) / 64, 64, 0, ctx->stream>>>(d_a.data(), d_b.data(), n_problems, dk_max_iters, dk_tol_sq, d_E.data(), d_c.data());
     CK(cudaStreamSynchronize(ctx->stream));
     CK(cudaGetLastError());
-    CK(cudaMemcpy(E_out, d_E, (size_t)n_problems * 720, cudaMemcpyDeviceToHost));
-    CK(cudaMemcpy(count_out, d_c, (size_t)n_problems * 4, cudaMemcpyDeviceToHost));
-    cudaFree(d_a); cudaFree(d_b); cudaFree(d_E); cudaFree(d_c);
+    CK(cudaMemcpy(E_out, d_E.data(), (size_t)n_problems * 720, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(count_out, d_c.data(), (size_t)n_problems * 4, cudaMemcpyDeviceToHost));
     ctx->stats.launches += 1;
     return PGI_OK;
 }
@@ -1387,24 +1385,24 @@ pgi_status pgi_dbg_pose_from_essential(pgi_ctx *ctx, const double *E, const doub
 {
     if (!ctx || !E || !corr_xy4 || !R || !t || !votes || n > 0x7fffffffULL) return PGI_ERR_INVALID;
     CK(cudaSetDevice(ctx->cfg.device));
-    double *d_c = nullptr, *d_E = nullptr, *d_R = nullptr, *d_t = nullptr;
-    unsigned long long *d_v = nullptr;
-    CK(cudaMalloc((void **)&d_c, std::max<uint64_t>(n, 1) * 32));
-    CK(cudaMalloc((void **)&d_E, 72));
-    CK(cudaMalloc((void **)&d_R, 72));
-    CK(cudaMalloc((void **)&d_t, 24));
-    CK(cudaMalloc((void **)&d_v, 32));
-    CK(cudaMemcpy(d_c, corr_xy4, n * 32, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_E, E, 72, cudaMemcpyHostToDevice));
-    kdbg_pose_from_essential<<<1, kCtaThreads, 0, ctx->stream>>>(d_E, reinterpret_cast<double4 *>(d_c), (uint32_t)n, d_R, d_t, d_v);
+    DevBuf<double4> d_c;
+    DevBuf<double> d_E, d_R, d_t;
+    DevBuf<unsigned long long> d_v;
+    CK(d_c.grow(n));
+    CK(d_E.grow(9));
+    CK(d_R.grow(9));
+    CK(d_t.grow(3));
+    CK(d_v.grow(4));
+    CK(cudaMemcpy(d_c.data(), corr_xy4, n * 32, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(d_E.data(), E, 72, cudaMemcpyHostToDevice));
+    kdbg_pose_from_essential<<<1, kCtaThreads, 0, ctx->stream>>>(d_E.data(), d_c.data(), (uint32_t)n, d_R.data(), d_t.data(), d_v.data());
     CK(cudaStreamSynchronize(ctx->stream));
     CK(cudaGetLastError());
     unsigned long long hv[4];
-    CK(cudaMemcpy(R, d_R, 72, cudaMemcpyDeviceToHost));
-    CK(cudaMemcpy(t, d_t, 24, cudaMemcpyDeviceToHost));
-    CK(cudaMemcpy(hv, d_v, 32, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(R, d_R.data(), 72, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(t, d_t.data(), 24, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(hv, d_v.data(), 32, cudaMemcpyDeviceToHost));
     for (int k = 0; k < 4; k++) votes[k] = hv[k];
-    cudaFree(d_c); cudaFree(d_E); cudaFree(d_R); cudaFree(d_t); cudaFree(d_v);
     ctx->stats.launches += 1;
     return PGI_OK;
 }
@@ -1416,13 +1414,13 @@ pgi_status pgi_dbg_fp64_peak(pgi_ctx *ctx, int32_t fused, double *tflops_out)
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, ctx->cfg.device));
     const int blocks = prop.multiProcessorCount * 8, threads = 256, iters = 1 << 14;
-    double *d = nullptr;
-    CK(cudaMalloc((void **)&d, (size_t)blocks * threads * 8));
-    k_fp64_peak<<<blocks, threads, 0, ctx->stream>>>(d, 64, fused);  // warm-up
+    DevBuf<double> d;
+    CK(d.grow((size_t)blocks * threads));
+    k_fp64_peak<<<blocks, threads, 0, ctx->stream>>>(d.data(), 64, fused);  // warm-up
     double best = 0.0;
     for (int rep = 0; rep < 5; rep++) {
         CK(cudaEventRecord(ctx->evStart, ctx->stream));
-        k_fp64_peak<<<blocks, threads, 0, ctx->stream>>>(d, iters, fused);
+        k_fp64_peak<<<blocks, threads, 0, ctx->stream>>>(d.data(), iters, fused);
         CK(cudaEventRecord(ctx->evK1, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
         float ms = 0;
@@ -1430,7 +1428,6 @@ pgi_status pgi_dbg_fp64_peak(pgi_ctx *ctx, int32_t fused, double *tflops_out)
         const double flops = (double)blocks * threads * iters * 8.0 * 2.0;  // 8 chains x (mul + add)
         best = std::max(best, flops / (ms * 1e-3) / 1e12);
     }
-    cudaFree(d);
     ctx->stats.launches += 6;
     *tflops_out = best;
     return PGI_OK;
