@@ -148,6 +148,40 @@ typedef struct pgb_drive_stats {
 int32_t pgb_run_wave(pgb_builder *b, uint32_t wave_size, pgb_submit_fn submit, pgb_wait_fn wait, void *engine,
                      uint32_t flags, pgb_drive_stats *stats);
 
+/* ---- Epipolar-hashing mode (use_epipolar_hashing, cpp_example.cpp:38): exact sequential loop --------------------------
+ * processImages with core_number = 1 and the quick-matching branch (pose_graph_builder.h:492-547, :657-707): for every
+ * queue position (src, dst) that is not a duplicate edge, q = Tracklets::getCorrespondences(src, dst, maximum_tracklet_number);
+ * if |q| >= minimum_point_number the position is QUICK-matched on q (registered with pgi_register_extra_pairs, verified
+ * with PGI_WAVE_EXTRA), otherwise FULL-matched on the scene's matches (`matches`, rows as in pgb_create's m_offset);
+ * fewer than minimum_point_number rows skip it.  A* and the commit are those of the wave host; the edge score is
+ * inliers / rows of the chosen list.  After an accepted position the tracklets grow: a quick-matched one by the rows of
+ * guidedMatching with the committed pose (all inliers), a full-matched one by its matches under the estimatePose inlier
+ * mask.  Each position is one engine wave of one pair with PATH | FALLBACK | MASKS (plus EXTRA): the next position's
+ * matches depend on this one's tracks, so nothing is speculated.  The engine sits behind function pointers whose
+ * signatures are those of pgi_submit_wave, pgi_wait_wave, pgi_register_extra_pairs and pgi_guided_match_views.  Runs
+ * the whole queue of a builder on which no wave was run; returns 0 or the engine's negative status (-1: bad argument). */
+typedef struct pgb_hashing_config {
+    uint64_t maximum_tracklet_number;  /* kMaximumTrackletNumber_, cpp_example.cpp (5000)                   */
+    uint64_t maximum_point_number;     /* kMaximumPointNumberForEpipolarHashing_ (100)                      */
+    int32_t bin_number;                /* HashingBasedMatcherWithPose<false, 45>: 45                        */
+    int32_t pad;
+} pgb_hashing_config;
+typedef int32_t (*pgb_register_extra_fn)(void *engine, uint64_t n_pairs, const uint32_t *pair_views, const uint64_t *m_offset,
+                                         const uint32_t *matches);
+typedef int32_t (*pgb_guided_fn)(void *engine, uint32_t src, uint32_t dst, const double *pose_q_t, int32_t bin_number,
+                                 uint32_t max_points, uint32_t *matches_out, double *values_out, uint32_t *n_out);
+typedef struct pgb_hashing_stats {  /* accumulated by pgb_run_hashing */
+    uint64_t positions, quick_matched, full_matched, guided_calls, guided_rows, tracklet_adds;
+    double sec_astar, sec_engine, sec_guided, sec_tracklets;
+} pgb_hashing_stats;
+enum { PGB_MATCH_SKIPPED = 0, PGB_MATCH_QUICK = 1, PGB_MATCH_FULL = 2 };
+int32_t pgb_run_hashing(pgb_builder *b, const uint32_t *matches, const pgb_hashing_config *cfg, pgb_submit_fn submit,
+                        pgb_wait_fn wait, pgb_register_extra_fn register_extra, pgb_guided_fn guided, void *engine,
+                        pgb_hashing_stats *stats);
+/* Per log record of pgb_run_hashing: the match source (PGB_MATCH_*) and the rows guidedMatching added to the tracklets.
+ * Either output may be null.  Returns the number of records (0 for a builder driven by waves). */
+uint64_t pgb_copy_match_sources(pgb_builder *b, uint8_t *source_out, uint32_t *guided_rows_out);
+
 /* Device search backend: with it, the speculative A* searches of a wave round (graph_traversal.h:679-870) run as ONE
  * batched device call instead of on the host thread pool — the two function pointers have the signatures of
  * pgi_graph_apply / pgi_graph_search (pgi.h) and the product passes exactly those and its pgi_ctx, after

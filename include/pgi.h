@@ -43,7 +43,8 @@ enum {
     PGI_WAVE_PATH = 1u,     /* verify the supplied path hypotheses: test + getInliers + five-point (a3-a7) */
     PGI_WAVE_FALLBACK = 2u, /* run the robust fallback (a8) for pairs whose path branch did not succeed     */
     PGI_WAVE_MASKS = 4u,    /* also produce the per-correspondence inlier masks (PGB:1000-1009, :1034-1044)  */
-    PGI_WAVE_NO_TEST = 8u   /* hypotheses are estimatePose guesses: skip the InTraversalPoseTester gate      */
+    PGI_WAVE_NO_TEST = 8u,  /* hypotheses are estimatePose guesses: skip the InTraversalPoseTester gate      */
+    PGI_WAVE_EXTRA = 16u    /* pair ids index the pairs of pgi_register_extra_pairs, not the scene's         */
 };
 
 typedef struct pgi_config {
@@ -94,6 +95,8 @@ typedef struct pgi_stats {
     uint64_t dist_evals;        /* K9 descriptor distances (each pair's n_src x n_dst once) */
     uint64_t match_pairs;       /* pairs matched by K9                                */
     uint64_t match_rows;        /* matches K9 produced                                */
+    double ms_guided;           /* K7 guided matching (pgi_guided_match, pgi_guided_match_views) */
+    uint64_t guided_calls;      /* K7 launches timed in ms_guided                     */
 } pgi_stats;
 
 const char *pgi_version(void);
@@ -132,6 +135,23 @@ pgi_status pgi_register_scene_descriptors(pgi_ctx *ctx, uint64_t n_views, const 
 /* Copy the (srcIdx, dstIdx) rows and, if non-null, the ratios of the last pgi_register_scene_descriptors on this context
  * (the correspondences.h5 cache): m_offset_out[n_pairs] rows.  PGI_ERR_STATE if a pgi_register_scene came after it. */
 pgi_status pgi_read_scene_matches(pgi_ctx *ctx, uint32_t *matches_out, double *ratios_or_null, uint64_t capacity_rows);
+
+/* Descriptors for a scene registered with pgi_register_scene (which keeps none): desc[sum K][dim] float, row-aligned with
+ * that registration's kp_xy, dim 64 or 128, every value finite (PGI_ERR_INVALID otherwise).  They stay resident for
+ * pgi_guided_match_views.  PGI_ERR_STATE before any scene registration. */
+pgi_status pgi_set_scene_descriptors(pgi_ctx *ctx, const float *desc, uint32_t dim);
+
+/* Pairs whose matches the caller supplies (the quick matches the Tracklets hand out, pose_graph_builder.h:492-520), built
+ * into normalised correspondences on the device by K0 from the keypoints, focal lengths, image sizes and thr_px of the last
+ * scene registration.  pair_views[n_pairs][2]; m_offset[n_pairs + 1] (m_offset[0] = 0); matches[m_offset[n_pairs]][2]
+ * (srcIdx, dstIdx), each index below its view's keypoint count.  The rows go into a second registration of the context,
+ * replaced by the next call; waves address it with PGI_WAVE_EXTRA (pair id = row of this call).  The scene's own
+ * registration is neither copied nor changed.  PGI_ERR_STATE before any scene registration. */
+pgi_status pgi_register_extra_pairs(pgi_ctx *ctx, uint64_t n_pairs, const uint32_t *pair_views, const uint64_t *m_offset,
+                                    const uint32_t *matches);
+/* pgi_read_pair for the pairs of pgi_register_extra_pairs (testing). */
+pgi_status pgi_read_extra_pair(pgi_ctx *ctx, uint32_t pair_id, double *corr_xy4, uint64_t capacity_rows, uint64_t *n_rows,
+                               double *thr_norm);
 
 /* Make `ctx` use the pairs registered in `owner` (same device) without copying them: a second context — its
  * own stream, wave buffers and statistics — can then verify waves concurrently with the first (used to overlap
@@ -236,6 +256,15 @@ pgi_status pgi_guided_match(pgi_ctx *ctx, uint32_t n_src, const float *kp_src, c
                             const double *K_src, const double *K_dst, const int32_t *size_src, const int32_t *size_dst,
                             int32_t bin_number, uint32_t *matches_out, double *ratios_out, uint32_t *n_out,
                             double *prepared_or_null);
+
+/* PoseGraphBuilder::guidedMatching (pose_graph_builder.h:717-783) of views src -> dst of the registered scene: K7 on the
+ * device-resident keypoints and descriptors (pgi_register_scene_descriptors or pgi_set_scene_descriptors), K = [f 0 w/2;
+ * 0 f h/2; 0 0 1] of each view, then the selection of :760-782.  matches_out (capacity max_points x 2) and values_out
+ * (capacity max_points) receive the selected rows: the max_points smallest (value, index) entries in ascending order if
+ * match() returned more than max_points, else all of them in source order, each with the first match's value.  No
+ * allocation after the first calls and no descriptor copy.  PGI_ERR_STATE without a scene or without descriptors. */
+pgi_status pgi_guided_match_views(pgi_ctx *ctx, uint32_t src, uint32_t dst, const double *pose_q_t, int32_t bin_number,
+                                  uint32_t max_points, uint32_t *matches_out, double *values_out, uint32_t *n_out);
 
 /* ---- brute-force descriptor matching (K8) ------------------------------------------------------------------
  * matchFeatures (feature_utils.h:103-210) without its HDF5 cache: BRUTEFORCE_SL2 2-NN in both directions, ratio test

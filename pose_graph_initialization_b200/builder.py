@@ -62,7 +62,7 @@ PGB_EXPORTS = ["pgb_create", "pgb_destroy", "pgb_remaining", "pgb_set_fallback_v
                "pgb_export_records", "pgb_import_records", "pgb_next_wave", "pgb_set_search_backend", "pgb_copy_sim_table",
                "pgb_commit_wave", "pgb_edge_count", "pgb_copy_edges", "pgb_log_count", "pgb_copy_log", "pgb_get_counters",
                "pgb_astar", "pgb_tracklets_create", "pgb_tracklets_destroy", "pgb_tracklets_add",
-               "pgb_tracklets_get_correspondences", "pgb_tracklets_track_count"]
+               "pgb_tracklets_get_correspondences", "pgb_tracklets_track_count", "pgb_run_hashing", "pgb_copy_match_sources"]
 
 
 def _host_lib():
@@ -87,6 +87,8 @@ def _host_lib():
         lib.pgb_tracklets_add.restype = C.c_int32
         lib.pgb_tracklets_get_correspondences.restype = C.c_int64
         lib.pgb_tracklets_track_count.restype = C.c_uint64
+        lib.pgb_run_hashing.restype = C.c_int32
+        lib.pgb_copy_match_sources.restype = C.c_uint64
         for name in PGB_EXPORTS[1:]:
             getattr(lib, name).argtypes = None
         lib._pgb_ready = True
@@ -99,6 +101,24 @@ def _ptr(a):
 
 class DriveStats(C.Structure):
     _fields_ = [("engine_s", C.c_double), ("host_s", C.c_double), ("rounds", C.c_uint32), ("items", C.c_uint32)]
+
+
+class HashingConfig(C.Structure):
+    _fields_ = [("maximum_tracklet_number", C.c_uint64), ("maximum_point_number", C.c_uint64), ("bin_number", C.c_int32),
+                ("pad", C.c_int32)]
+
+
+class HashingStats(C.Structure):
+    _fields_ = [(k, C.c_uint64) for k in ("positions", "quick_matched", "full_matched", "guided_calls", "guided_rows",
+                                          "tracklet_adds")] + \
+               [(k, C.c_double) for k in ("sec_astar", "sec_engine", "sec_guided", "sec_tracklets")]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_ if k != "pad"}
+
+
+MATCH_SKIPPED, MATCH_QUICK, MATCH_FULL = 0, 1, 2
+SOURCE_DTYPE = np.dtype([("source", np.uint8), ("guided_rows", np.uint32)])
 
 
 class Tracklets:
@@ -209,6 +229,28 @@ class HostBuilder:
         rc = int(self.lib.pgb_run_wave(self.h, C.c_uint32(wave_size), submit_fn, wait_fn, engine_handle, C.c_uint32(flags),
                                        C.byref(st)))
         return rc
+
+    def run_hashing(self, matches, submit_fn, wait_fn, register_extra_fn, guided_fn, engine_handle, maximum_tracklet_number=5000,
+                    maximum_point_number=100, bin_number=45, stats=None):
+        """pgb_run_hashing: the whole queue in the exact sequential epipolar-hashing mode.  matches: the scene's match list
+        (rows as m_offset says).  The four function pointers have the signatures of pgi_submit_wave, pgi_wait_wave,
+        pgi_register_extra_pairs and pgi_guided_match_views.  Returns (status, HashingStats)."""
+        m = np.ascontiguousarray(matches, dtype=np.uint32).reshape(-1, 2)
+        cfg = HashingConfig(int(maximum_tracklet_number), int(maximum_point_number), int(bin_number), 0)
+        st = stats if stats is not None else HashingStats()
+        rc = int(self.lib.pgb_run_hashing(self.h, _ptr(m), C.byref(cfg), submit_fn, wait_fn, register_extra_fn, guided_fn,
+                                          engine_handle, C.byref(st)))
+        return rc, st
+
+    def match_sources(self):
+        """Per log record of run_hashing: (source: MATCH_SKIPPED / MATCH_QUICK / MATCH_FULL, guided_rows)."""
+        n = int(self.lib.pgb_copy_match_sources(self.h, None, None))
+        src, rows = np.zeros(n, dtype=np.uint8), np.zeros(n, dtype=np.uint32)
+        if n:
+            self.lib.pgb_copy_match_sources(self.h, _ptr(src), _ptr(rows))
+        out = np.zeros(n, dtype=SOURCE_DTYPE)
+        out["source"], out["guided_rows"] = src, rows
+        return out
 
     def commit_wave(self, verdicts):
         verdicts = np.ascontiguousarray(verdicts, dtype=VERDICT_DTYPE)
@@ -403,7 +445,9 @@ class PoseGraphBuilder:
     """Drop-in for reconstruction::PoseGraphBuilder (pose_graph_builder.h:27-71).  Argument names, order and
     defaults follow examples/cpp_example.cpp:86-103; the four path arguments are accepted and ignored (the
     data comes from `scene`), `kCoreNumber_` sizes the host thread pool of the speculative A*, and
-    `kUseGPU_` must be true (there is no CPU path)."""
+    `kUseGPU_` must be true (there is no CPU path).  kUseEpipolarHashing_=True runs the reference's quick matching from
+    point tracks and guided matching after accepted quick-matched pairs, exactly as the reference with core_number = 1
+    (pgb_run_hashing); it needs a scene with descriptors (`desc`) and one GPU, and does not use the device A* (K6)."""
 
     def __init__(self, kCoreNumber_=20, kMaximumTrackletNumber_=5000, kMaximumSearchDepth_=5, kMaximumPathNumber_=100,
                  kMinimumInlierNumber_=20, kMinimumPointNumber_=50, kMaximumPointNumberForEpipolarHashing_=100,
@@ -415,10 +459,18 @@ class PoseGraphBuilder:
                  group=None, rank=0, world_size=1):
         if not kUseGPU_:
             raise ValueError("the B200 path has no CPU implementation (kUseGPU_ must be true)")
-        if kUseEpipolarHashing_:
-            raise NotImplementedError("epipolar hashing (matcher.h) is outside the hot path (SURVEY §8f row 3)")
         if scene is None:
             raise ValueError("scene=... is required (the reference's HDF5/1DSfM inputs are replaced by scene.py)")
+        self.hashing = bool(kUseEpipolarHashing_)
+        if self.hashing:
+            # each position's matches come from the tracks the positions before it left: the mode is sequential
+            if "desc" not in scene:
+                raise ValueError("kUseEpipolarHashing_ needs a scene with descriptors (desc): guided matching reads them")
+            if world_size > 1:
+                raise ValueError("kUseEpipolarHashing_ runs on one GPU (world_size must be 1)")
+            if gpu_search:
+                raise ValueError("kUseEpipolarHashing_ searches on the host: gpu_search must be False")
+            prefetch_fallback = overlap_fallback = False
         if world_size > 1 and not prefetch_fallback:
             # the exchange records carry path verdicts only: a non-owner rank could never learn a remote pair's
             # fallback verdict and the ranks' wave loops would diverge
@@ -429,6 +481,8 @@ class PoseGraphBuilder:
                         traversal_heuristics_weight=kTraversalHeuristicsWeight_, use_path_finding=kUsePathFinding_,
                         host_threads=kCoreNumber_, research_window=research_window)
         self.thr_px = kInlierOutlierThreshold_
+        self.max_tracklets = kMaximumTrackletNumber_
+        self.max_points_hashing = kMaximumPointNumberForEpipolarHashing_
         self.min_inliers = kMinimumInlierNumber_
         self.device = device
         # measured on cfg2 (scripts/gpu_sweep.sh): 256 positions per wave is the optimum on one GPU (fewer A* re-searches
@@ -482,6 +536,8 @@ class PoseGraphBuilder:
             sub = self._sub
         if not registered:
             self.engine.register_scene(sub, self.thr_px)
+            if self.hashing:  # a scene that came with matches: guided matching still needs its descriptors on the device
+                self.engine.set_scene_descriptors(sub["desc"])
         self.prepared = True
         if self.overlap:
             if self.engine_fb is None:
@@ -593,6 +649,10 @@ class PoseGraphBuilder:
         first wave boundary after every further `batch` committed positions, so that a caller can bracket slices of ONE
         pass — bench.py's steps; the prefetch pipeline keeps running across the yields.  The PoseGraph is the generator's
         return value (StopIteration.value).  batch=None never yields: that is run()."""
+        if self.hashing:
+            if batch:
+                raise ValueError("kUseEpipolarHashing_ runs the queue in one pass: run_in_batches needs batch=None")
+            return self._run_hashing()
         t0 = time.perf_counter()
         if self.engine is None or not getattr(self, "prepared", False):
             self.prepare()
@@ -770,4 +830,28 @@ class PoseGraphBuilder:
         self.log = host.log()
         self.counters = host.counters()
         self.search_stats = self.engine.search_stats() if self.gpu_search else {}
+        return PoseGraph(len(self.scene["focal"]), edges)
+
+    def _run_hashing(self):
+        """The exact sequential epipolar-hashing loop (pgb_run_hashing) with the engine's own entry points."""
+        t0 = time.perf_counter()
+        if self.engine is None or not getattr(self, "prepared", False):
+            self.prepare()
+        t_reg = time.perf_counter()
+        host = HostBuilder(self.scene, lazy_fallback=True, **self.cfg)
+        self.host = host
+        lib = _engine.load_library()
+        fns = [C.cast(getattr(lib, n), C.c_void_p) for n in ("pgi_submit_wave", "pgi_wait_wave", "pgi_register_extra_pairs",
+                                                            "pgi_guided_match_views")]
+        rc, st = host.run_hashing(self.scene["matches"], *fns, self.engine.h, self.max_tracklets, self.max_points_hashing)
+        if rc < 0:
+            raise _engine.PgiError(f"status {rc}: {lib.pgi_last_error(self.engine.h).decode()}")
+        t_end = time.perf_counter()
+        self.hashing_stats = st.as_dict()
+        self.timing = dict(register_s=t_reg - t0, waves_s=t_end - t_reg, total_s=t_end - t0)
+        edges = host.edges()
+        self.log = host.log()
+        self.match_sources = host.match_sources()
+        self.counters = host.counters()
+        self.search_stats = {}
         return PoseGraph(len(self.scene["focal"]), edges)

@@ -32,6 +32,7 @@
 #include <condition_variable>
 #include <deque>
 #include <functional>
+#include <memory>
 #include <mutex>
 #include <queue>
 #include <thread>
@@ -41,6 +42,9 @@
 
 #include "../../include/pgb.h"
 #include "pgi_nvtx.h"
+// Tracklets share this translation unit with the hashing loop that drives them (pgb_run_hashing), so that the host
+// compiles and links as one file.
+#include "pgb_tracklets.cpp"
 
 #if defined(__x86_64__) && defined(__GNUC__)
 #include <immintrin.h>
@@ -830,6 +834,9 @@ struct pgb_builder {
     std::vector<uint32_t> gpuCommitted, gpuTotal, gpuBits, gpuTodo;
     std::vector<pgi_query> gpuQueries;
     std::vector<pgi_search_result> gpuResults;
+    // pgb_run_hashing: one entry per log record
+    std::vector<uint8_t> matchSource;
+    std::vector<uint32_t> guidedRows;
 };
 
 namespace {
@@ -1648,6 +1655,158 @@ int32_t pgb_run_wave(pgb_builder *b, uint32_t wave_size, pgb_submit_fn submit, p
     return status;
 }
 uint32_t pgb_wave_size(pgb_builder *b) { return b ? (uint32_t)b->wave.size() : 0; }
+
+int32_t pgb_run_hashing(pgb_builder *b, const uint32_t *matches, const pgb_hashing_config *hc, pgb_submit_fn submit,
+                        pgb_wait_fn wait, pgb_register_extra_fn register_extra, pgb_guided_fn guided, void *engine,
+                        pgb_hashing_stats *stats)
+{
+    PgiNvtxRange nvtxRange("pgb:run_hashing");
+    if (!b || !hc || !submit || !wait || !register_extra || !guided || (b->mOffset.back() && !matches)) return -1;
+    if (b->waveOpen || !b->pending.empty() || b->log.size() != b->matchSource.size()) return -1;
+    pgb_hashing_stats local;
+    memset(&local, 0, sizeof local);
+    pgb_hashing_stats &st = stats ? *stats : local;
+    std::unique_ptr<pgb_tracklets, void (*)(pgb_tracklets *)> tracklets(pgb_tracklets_create(b->V), pgb_tracklets_destroy);
+    const uint64_t maxTracks = hc->maximum_tracklet_number, maxGuided = hc->maximum_point_number;
+    std::vector<uint64_t> qS(maxTracks + 1), qD(maxTracks + 1), addS, addD;
+    std::vector<uint32_t> quick, gm((size_t)2 * maxGuided);
+    std::vector<double> gv(maxGuided);
+    std::vector<uint8_t> mask, ones;
+    AStarScratch &S = b->scratch[0];
+    const uint32_t flagsBase = PGI_WAVE_PATH | PGI_WAVE_FALLBACK | PGI_WAVE_MASKS;
+    while (b->nextInOrder < b->order.size()) {
+        Item it;
+        it.src = b->order[b->nextInOrder].first;
+        it.dst = b->order[b->nextInOrder].second;
+        ++b->nextInOrder;
+        ++st.positions;
+        uint8_t source = PGB_MATCH_SKIPPED;
+        uint32_t guidedAdded = 0;
+        const auto finish = [&]() {
+            commitPosition(b, it);
+            b->matchSource.push_back(source);
+            b->guidedRows.push_back(guidedAdded);
+        };
+        if (b->graph.hasEdge(it.src, it.dst) || b->graph.hasEdge(it.dst, it.src)) {  // pose_graph_builder.h:438-443
+            finish();
+            continue;
+        }
+        it.visible = b->vis.hasLink(it.src, it.dst);  // :456-457
+        auto pi = b->pairIndex.find(edgeKey(it.src, it.dst));
+        if (pi != b->pairIndex.end()) it.pairId = pi->second;
+        // quick matching from the tracks the two views share (:492-520)
+        double t0 = nowSec();
+        const int64_t nq = pgb_tracklets_get_correspondences(tracklets.get(), it.src, it.dst, maxTracks, qS.data(), qD.data(), qS.size());
+        st.sec_tracklets += nowSec() - t0;
+        if (nq < 0) return -1;
+        const bool isQuick = (uint64_t)nq >= b->cfg.minimum_point_number;
+        if (isQuick)
+            it.nCorr = (uint32_t)nq;
+        else  // matchFeatures' list (:522-547)
+            it.nCorr = it.pairId == UINT32_MAX ? 0u : (uint32_t)(b->mOffset[it.pairId + 1] - b->mOffset[it.pairId]);
+        if (it.nCorr < b->cfg.minimum_point_number) {  // :550-551
+            it.staticSkip = true;
+            finish();
+            continue;
+        }
+        source = isQuick ? PGB_MATCH_QUICK : PGB_MATCH_FULL;
+        ++(isQuick ? st.quick_matched : st.full_matched);
+        uint32_t flags = flagsBase, pid = it.pairId;
+        t0 = nowSec();
+        if (isQuick) {
+            quick.resize((size_t)2 * nq);
+            for (int64_t i = 0; i < nq; i++) { quick[2 * i] = (uint32_t)qS[i]; quick[2 * i + 1] = (uint32_t)qD[i]; }
+            const uint32_t pv[2] = {it.src, it.dst};
+            const uint64_t off[2] = {0, (uint64_t)nq};
+            const int32_t rc = register_extra(engine, 1, pv, off, quick.data());
+            if (rc < 0) return rc;
+            flags |= PGI_WAVE_EXTRA;
+            pid = 0;
+        }
+        st.sec_engine += nowSec() - t0;
+        // A* on the committed graph (:569-603)
+        if (b->cfg.use_path_finding && it.visible) {
+            t0 = nowSec();
+            AStarOut o;
+            GraphView gv0{&b->graph, nullptr, 0};
+            aStar(gv0, b->sim.data(), b->V, it.src, it.dst, (size_t)b->cfg.maximum_search_depth, b->cfg.traversal_heuristics_weight, S, o);
+            it.hasHyp = o.found;
+            it.hyp = o.pose;
+            it.touched = o.touched;
+            const double dt = nowSec() - t0;
+            st.sec_astar += dt;
+            b->ctr.sec_astar += dt;
+            b->ctr.astar_runs++;
+            b->ctr.astar_pops += o.touched;
+            b->ctr.astar_pushes += o.pushes;
+        }
+        // estimatePose on the chosen matches: a wave of one, with its inlier mask
+        t0 = nowSec();
+        double hyp[7];
+        memcpy(hyp, it.hyp.q, 32);
+        memcpy(hyp + 4, it.hyp.t, 24);
+        const uint32_t hoff[2] = {0, it.hasHyp ? 1u : 0u};
+        pgi_verdict v;
+        mask.assign(it.nCorr, 0);
+        int32_t rc = submit(engine, 1, &pid, hoff, it.hasHyp ? hyp : nullptr, flags);
+        if (rc < 0) return rc;
+        rc = wait(engine, &v, mask.data());
+        if (rc < 0) return rc;
+        st.sec_engine += nowSec() - t0;
+        b->ctr.waves++;
+        b->ctr.items_speculated++;
+        v.pair_id = it.pairId;
+        it.finalV = &v;
+        it.pathV = it.hasHyp ? &v : nullptr;
+        commitPosition(b, it);
+        if (v.accepted) {
+            uint64_t n = 0;
+            const uint8_t *m = nullptr;
+            if (isQuick) {  // guidedMatching with the committed pose (:663-676, :717-783)
+                t0 = nowSec();
+                double pose[7];
+                memcpy(pose, v.q, 32);
+                memcpy(pose + 4, v.t, 24);
+                uint32_t gn = 0;
+                rc = guided(engine, it.src, it.dst, pose, hc->bin_number, (uint32_t)maxGuided, gm.data(), gv.data(), &gn);
+                if (rc < 0) return rc;
+                st.sec_guided += nowSec() - t0;
+                st.guided_calls++;
+                st.guided_rows += gn;
+                guidedAdded = gn;
+                n = std::min<uint64_t>(gn, maxGuided);
+                addS.resize(n);
+                addD.resize(n);
+                for (uint64_t i = 0; i < n; i++) { addS[i] = gm[2 * i]; addD[i] = gm[2 * i + 1]; }
+                ones.assign(n, 1);
+                m = ones.data();
+            } else {  // the matchFeatures list under estimatePose's inlier mask (:697-703)
+                n = it.nCorr;
+                const uint32_t *pm = matches + 2 * b->mOffset[it.pairId];
+                addS.resize(n);
+                addD.resize(n);
+                for (uint64_t i = 0; i < n; i++) { addS[i] = pm[2 * i]; addD[i] = pm[2 * i + 1]; }
+                m = mask.data();
+            }
+            t0 = nowSec();
+            if (pgb_tracklets_add(tracklets.get(), it.src, it.dst, n, addS.data(), addD.data(), m) != 0) return -1;
+            st.sec_tracklets += nowSec() - t0;
+            st.tracklet_adds++;
+        }
+        b->matchSource.push_back(source);
+        b->guidedRows.push_back(guidedAdded);
+    }
+    return 0;
+}
+
+uint64_t pgb_copy_match_sources(pgb_builder *b, uint8_t *source_out, uint32_t *guided_rows_out)
+{
+    if (!b) return 0;
+    const size_t n = b->matchSource.size();
+    if (source_out && n) memcpy(source_out, b->matchSource.data(), n);
+    if (guided_rows_out && n) memcpy(guided_rows_out, b->guidedRows.data(), n * 4);
+    return n;
+}
 
 // One record per wave position; a rank fills the positions it owns and leaves the others zero, so a byte-wise SUM
 // all-reduce merges the ranks' buffers.

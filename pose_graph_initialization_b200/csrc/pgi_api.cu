@@ -145,6 +145,13 @@ struct SceneStaging {
     DevBuf<unsigned char> k9Scratch;
     uint64_t rows = 0;
     bool matches = false;  // m / ratio hold the matches of the last descriptor registration
+    // what pgi_register_extra_pairs and pgi_guided_match_views read on the host: the last registration's views
+    bool staged = false;   // a scene registration completed its upload
+    bool hasDesc = false;  // desc holds dim floats per keypoint of this scene
+    uint32_t dim = 0;
+    double thrPx = 0.0;
+    std::vector<uint64_t> hKpOff;
+    std::vector<double> hFocal, hSize;
 
     // The match list is the one allocation that grows while it is filled: to max(need, 2 x capacity, 1024) rows,
     // with its first `keep` rows copied over.
@@ -206,6 +213,12 @@ struct pgi_ctx {
     Event evS0, evS1;
     std::string err;
     Registration own, tmp;
+    Registration extra;            // pgi_register_extra_pairs: rows built from caller-supplied matches (PGI_WAVE_EXTRA)
+    DevBuf<uint2> extraPv, extraM; // their pair views and matches, as K0 reads them
+    DevBuf<unsigned char> guided;  // pgi_guided_match_views: K7 scratch
+    std::vector<uint32_t> guidedM;
+    std::vector<double> guidedR;
+    std::vector<uint32_t> guidedOrder;
     const Registration *reg = &own;  // own, or the owner's after pgi_share_pairs
     // wave buffers
     DevSlots slots;
@@ -549,10 +562,11 @@ pgi_status finishWave(pgi_ctx *ctx)
     return PGI_OK;
 }
 
-// K0 (createCorrespondenceMatrix) over the staged scene (ctx->scene: views, keypoints, pair views, matches) into r,
+// K0 (createCorrespondenceMatrix) over the staged scene's views and keypoints (ctx->scene) for the pair views pv and
+// matches m (device arrays: the scene's own, or the extra pairs') into r,
 // whose offset, h_offset, nPairs, nRows and maxN are set and whose corr / thr hold nRows / nPairs entries; then the
 // sampler tables.
-pgi_status buildCorrespondences(pgi_ctx *ctx, Registration &r, double thr_px)
+pgi_status buildCorrespondences(pgi_ctx *ctx, Registration &r, double thr_px, const uint2 *pv, const uint2 *m)
 {
     cudaStream_t s = ctx->stream;
     const SceneStaging &sc = ctx->scene;
@@ -562,7 +576,7 @@ pgi_status buildCorrespondences(pgi_ctx *ctx, Registration &r, double thr_px)
         const uint32_t gx = std::max<uint32_t>(1, std::min<uint32_t>((r.maxN + 255) / 256, 64));
         const uint32_t gy = (uint32_t)std::min<uint64_t>(n_pairs, 65535), gz = (uint32_t)((n_pairs + gy - 1) / gy);
         k0_build_correspondences<<<dim3(gx, gy, gz), 256, 0, s>>>(sc.focal.data(), sc.size.data(), sc.kpOff.data(), sc.kp.data(),
-                                                                   n_pairs, sc.pv.data(), r.offset.data(), sc.m.data(), thr_px,
+                                                                   n_pairs, pv, r.offset.data(), m, thr_px,
                                                                    reinterpret_cast<double4 *>(r.corr.data()), r.thr.data());
         CK(cudaEventRecord(ctx->evK1, s));
         CK(cudaGetLastError());
@@ -577,6 +591,33 @@ pgi_status buildCorrespondences(pgi_ctx *ctx, Registration &r, double thr_px)
     return buildTables(ctx, r);
 }
 
+// Uploads the scene's descriptors (nKp x dim, row-aligned with the staged keypoints); they stay resident for K9 and K7.
+// Non-finite values are rejected (a NaN distance never enters a 2-NN, so it would silently drop neighbours).
+pgi_status uploadDescriptors(pgi_ctx *ctx, const float *desc, uint64_t nKp, uint32_t dim)
+{
+    SceneStaging &sc = ctx->scene;
+    cudaStream_t s = ctx->stream;
+    sc.hasDesc = false;
+    CK(sc.desc.grow(nKp * dim));
+    if (nKp) CK(cudaMemcpyAsync(sc.desc.data(), desc, nKp * dim * 4, cudaMemcpyHostToDevice, s));
+    ctx->stats.h2d_bytes += nKp * dim * 4;
+    uint32_t *d_flag = reinterpret_cast<uint32_t *>(ctx->counters.data());
+    uint32_t flag = 0;
+    CK(cudaMemsetAsync(d_flag, 0, 4, s));
+    if (nKp) {
+        k9_check_finite<<<(uint32_t)std::min<uint64_t>((nKp * dim + 1023) / 1024, 4 * ctx->numSms), 1024, 0, s>>>(sc.desc.data(), nKp * dim, d_flag);
+        CK(cudaGetLastError());
+        ctx->stats.launches += 1;
+    }
+    CK(cudaMemcpyAsync(&flag, d_flag, 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    ctx->stats.d2h_bytes += 4;
+    if (flag) { ctx->err = "non-finite descriptor value"; return PGI_ERR_INVALID; }
+    sc.hasDesc = true;
+    sc.dim = dim;
+    return PGI_OK;
+}
+
 // Grows the staging both scene registrations share and queues its upload: focal lengths, image sizes, keypoint
 // offsets, keypoints and pair views.
 pgi_status stageScene(pgi_ctx *ctx, uint64_t n_views, const double *focal, const double *size_wh, const uint64_t *kp_offset,
@@ -584,6 +625,10 @@ pgi_status stageScene(pgi_ctx *ctx, uint64_t n_views, const double *focal, const
 {
     SceneStaging &sc = ctx->scene;
     const uint64_t nKp = kp_offset[n_views];
+    sc.staged = sc.hasDesc = false;
+    sc.hKpOff.assign(kp_offset, kp_offset + n_views + 1);
+    sc.hFocal.assign(focal, focal + n_views);
+    sc.hSize.assign(size_wh, size_wh + 2 * n_views);
     CK(sc.focal.grow(n_views));
     CK(sc.size.grow(n_views * 2));
     CK(sc.kpOff.grow(n_views + 1));
@@ -597,6 +642,33 @@ pgi_status stageScene(pgi_ctx *ctx, uint64_t n_views, const double *focal, const
     if (n_pairs) CK(cudaMemcpyAsync(sc.pv.data(), pair_views, n_pairs * 8, cudaMemcpyHostToDevice, s));
     ctx->stats.h2d_bytes += n_views * 24 + (n_views + 1) * 8 + nKp * 8 + n_pairs * 8;
     return PGI_OK;
+}
+
+// E = [t]x R of the pose (pose.h:46-55), as the matcher reads it from Pose::getEssentialMatrix (matcher.h:218)
+void essentialOfPose(const double *q, double *E)
+{
+    double R[9];
+    const double tx = 2.0 * q[0], ty = 2.0 * q[1], tz = 2.0 * q[2];
+    const double twx = tx * q[3], twy = ty * q[3], twz = tz * q[3], txx = tx * q[0], txy = ty * q[0], txz = tz * q[0];
+    const double tyy = ty * q[1], tyz = tz * q[1], tzz = tz * q[2];
+    R[0] = 1.0 - (tyy + tzz); R[1] = txy - twz; R[2] = txz + twy;
+    R[3] = txy + twz; R[4] = 1.0 - (txx + tzz); R[5] = tyz - twx;
+    R[6] = txz - twy; R[7] = tyz + twx; R[8] = 1.0 - (txx + tyy);
+    const double Cx[9] = {0.0, -q[6], q[5], q[6], 0.0, -q[4], -q[5], q[4], 0.0};
+    for (int i = 0; i < 3; i++)
+        for (int j = 0; j < 3; j++) E[i * 3 + j] = Cx[i * 3 + 0] * R[j] + (Cx[i * 3 + 1] * R[3 + j] + Cx[i * 3 + 2] * R[6 + j]);
+}
+
+// K7's device time (evStart -> evK1 around its launch), after the stream was synchronised.
+cudaError_t addGuidedTime(pgi_ctx *ctx)
+{
+    float ms = 0;
+    const cudaError_t e = cudaEventElapsedTime(&ms, ctx->evStart, ctx->evK1);
+    if (e == cudaSuccess) {
+        ctx->stats.ms_guided += ms;
+        ctx->stats.guided_calls += 1;
+    }
+    return e;
 }
 
 }  // namespace
@@ -721,7 +793,9 @@ pgi_status pgi_register_scene(pgi_ctx *ctx, uint64_t n_views, const double *foca
     CK(cudaMemcpyAsync(r.offset.data(), m_offset, (n_pairs + 1) * 8, cudaMemcpyHostToDevice, s));
     ctx->stats.h2d_bytes += nRows * 8 + (n_pairs + 1) * 8;
     ctx->scene.matches = false;  // m now holds the caller's matches
-    return buildCorrespondences(ctx, r, thr_px);
+    ctx->scene.staged = true;
+    ctx->scene.thrPx = thr_px;
+    return buildCorrespondences(ctx, r, thr_px, ctx->scene.pv.data(), ctx->scene.m.data());
 }
 
 pgi_status pgi_register_scene_descriptors(pgi_ctx *ctx, uint64_t n_views, const double *focal, const double *size_wh,
@@ -762,25 +836,9 @@ pgi_status pgi_register_scene_descriptors(pgi_ctx *ctx, uint64_t n_views, const 
     sc.matches = false;
     CK(r.offset.grow(n_pairs + 1));
     CK(r.thr.grow(n_pairs));
-    CK(sc.desc.grow(nKp * dim));
     if (pgi_status st = stageScene(ctx, n_views, focal, size_wh, kp_offset, kp_xy, n_pairs, pair_views); st != PGI_OK) return st;
-    // every view's descriptors once; they stay resident for all of its pairs
-    if (nKp) CK(cudaMemcpyAsync(sc.desc.data(), desc, nKp * dim * 4, cudaMemcpyHostToDevice, s));
     CK(cudaMemsetAsync(r.offset.data(), 0, 8, s));
-    ctx->stats.h2d_bytes += nKp * dim * 4;
-    // non-finite descriptors are rejected (a NaN distance never enters a 2-NN, so it would silently drop neighbours)
-    uint32_t *d_flag = reinterpret_cast<uint32_t *>(ctx->counters.data());
-    uint32_t flag = 0;
-    CK(cudaMemsetAsync(d_flag, 0, 4, s));
-    if (nKp) {
-        k9_check_finite<<<(uint32_t)std::min<uint64_t>((nKp * dim + 1023) / 1024, 4 * ctx->numSms), 1024, 0, s>>>(sc.desc.data(), nKp * dim, d_flag);
-        CK(cudaGetLastError());
-        ctx->stats.launches += 1;
-    }
-    CK(cudaMemcpyAsync(&flag, d_flag, 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    ctx->stats.d2h_bytes += 4;
-    if (flag) { ctx->err = "non-finite descriptor value"; return PGI_ERR_INVALID; }
+    if (pgi_status st = uploadDescriptors(ctx, desc, nKp, dim); st != PGI_OK) return st;
 
     // K9 per chunk of pairs: scratch (forward states, backward partials, staged sorted rows) sized for the chunk only
     const uint32_t stride = std::max<uint32_t>(maxK, 1), maxSB = (stride + kK9Rows - 1) / kK9Rows;
@@ -857,7 +915,9 @@ pgi_status pgi_register_scene_descriptors(pgi_ctx *ctx, uint64_t n_views, const 
     CK(r.corr.grow(rows * 4));
     sc.rows = rows;
     sc.matches = true;
-    return buildCorrespondences(ctx, r, thr_px);
+    sc.staged = true;
+    sc.thrPx = thr_px;
+    return buildCorrespondences(ctx, r, thr_px, ctx->scene.pv.data(), ctx->scene.m.data());
 }
 
 pgi_status pgi_read_scene_matches(pgi_ctx *ctx, uint32_t *matches_out, double *ratios_or_null, uint64_t capacity_rows)
@@ -888,11 +948,10 @@ pgi_status pgi_share_pairs(pgi_ctx *ctx, pgi_ctx *owner)
     return PGI_OK;
 }
 
-pgi_status pgi_read_pair(pgi_ctx *ctx, uint32_t pair_id, double *corr_xy4, uint64_t capacity_rows, uint64_t *n_rows,
-                         double *thr_norm)
+namespace {
+pgi_status readPair(pgi_ctx *ctx, const Registration &r, uint32_t pair_id, double *corr_xy4, uint64_t capacity_rows,
+                    uint64_t *n_rows, double *thr_norm)
 {
-    if (!ctx) return PGI_ERR_INVALID;
-    const Registration &r = *ctx->reg;
     if (pair_id >= r.nPairs) { ctx->err = "pair_id out of range"; return PGI_ERR_INVALID; }
     CK(cudaSetDevice(ctx->cfg.device));
     const uint64_t n = r.h_offset[pair_id + 1] - r.h_offset[pair_id];
@@ -905,6 +964,76 @@ pgi_status pgi_read_pair(pgi_ctx *ctx, uint32_t pair_id, double *corr_xy4, uint6
     CK(cudaStreamSynchronize(ctx->stream));
     return PGI_OK;
 }
+}  // namespace
+
+pgi_status pgi_read_pair(pgi_ctx *ctx, uint32_t pair_id, double *corr_xy4, uint64_t capacity_rows, uint64_t *n_rows,
+                         double *thr_norm)
+{
+    if (!ctx) return PGI_ERR_INVALID;
+    return readPair(ctx, *ctx->reg, pair_id, corr_xy4, capacity_rows, n_rows, thr_norm);
+}
+
+pgi_status pgi_read_extra_pair(pgi_ctx *ctx, uint32_t pair_id, double *corr_xy4, uint64_t capacity_rows, uint64_t *n_rows,
+                               double *thr_norm)
+{
+    if (!ctx) return PGI_ERR_INVALID;
+    return readPair(ctx, ctx->extra, pair_id, corr_xy4, capacity_rows, n_rows, thr_norm);
+}
+
+pgi_status pgi_register_extra_pairs(pgi_ctx *ctx, uint64_t n_pairs, const uint32_t *pair_views, const uint64_t *m_offset,
+                                    const uint32_t *matches)
+{
+    PgiNvtxRange nvtxRange("pgi:register_extra_pairs (H2D + K0)");
+    if (!ctx) return PGI_ERR_INVALID;
+    if (ctx->inFlight) { ctx->err = "a wave is in flight"; return PGI_ERR_STATE; }
+    const SceneStaging &sc = ctx->scene;
+    if (!sc.staged) { ctx->err = "pgi_register_extra_pairs needs a scene registration first"; return PGI_ERR_STATE; }
+    if ((n_pairs && !pair_views) || !m_offset || (!matches && m_offset[n_pairs])) { ctx->err = "null argument"; return PGI_ERR_INVALID; }
+    if (m_offset[0] != 0) { ctx->err = "m_offset[0] must be 0"; return PGI_ERR_INVALID; }
+    const uint64_t V = sc.hFocal.size();
+    for (uint64_t p = 0; p < n_pairs; p++) {
+        const uint32_t s = pair_views[2 * p], d = pair_views[2 * p + 1];
+        if (s >= V || d >= V) { ctx->err = "view id out of range"; return PGI_ERR_INVALID; }
+        if (m_offset[p + 1] < m_offset[p] || m_offset[p + 1] - m_offset[p] > 0x7fffffffULL) { ctx->err = "bad m_offset"; return PGI_ERR_INVALID; }
+        // K0 reads the keypoints the indices name: an index past the view's keypoints is rejected here
+        const uint64_t nS = sc.hKpOff[s + 1] - sc.hKpOff[s], nD = sc.hKpOff[d + 1] - sc.hKpOff[d];
+        for (uint64_t i = m_offset[p]; i < m_offset[p + 1]; i++)
+            if (matches[2 * i] >= nS || matches[2 * i + 1] >= nD) { ctx->err = "keypoint index out of range"; return PGI_ERR_INVALID; }
+    }
+    CK(cudaSetDevice(ctx->cfg.device));
+    Registration &r = ctx->extra;
+    const uint64_t nRows = m_offset[n_pairs];
+    r.nPairs = n_pairs;
+    r.nRows = nRows;
+    r.h_offset.assign(m_offset, m_offset + n_pairs + 1);
+    r.maxN = 0;
+    for (uint64_t p = 0; p < n_pairs; p++) r.maxN = std::max<uint32_t>(r.maxN, (uint32_t)(m_offset[p + 1] - m_offset[p]));
+    CK(r.corr.grow(nRows * 4));
+    CK(r.offset.grow(n_pairs + 1));
+    CK(r.thr.grow(n_pairs));
+    CK(ctx->extraPv.grow(n_pairs));
+    CK(ctx->extraM.grow(nRows));
+    cudaStream_t s = ctx->stream;
+    if (n_pairs) CK(cudaMemcpyAsync(ctx->extraPv.data(), pair_views, n_pairs * 8, cudaMemcpyHostToDevice, s));
+    if (nRows) CK(cudaMemcpyAsync(ctx->extraM.data(), matches, nRows * 8, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(r.offset.data(), m_offset, (n_pairs + 1) * 8, cudaMemcpyHostToDevice, s));
+    ctx->stats.h2d_bytes += n_pairs * 8 + nRows * 8 + (n_pairs + 1) * 8;
+    return buildCorrespondences(ctx, r, sc.thrPx, ctx->extraPv.data(), ctx->extraM.data());
+}
+
+pgi_status pgi_set_scene_descriptors(pgi_ctx *ctx, const float *desc, uint32_t dim)
+{
+    PgiNvtxRange nvtxRange("pgi:set_scene_descriptors (H2D)");
+    if (!ctx) return PGI_ERR_INVALID;
+    if (ctx->inFlight) { ctx->err = "a wave is in flight"; return PGI_ERR_STATE; }
+    SceneStaging &sc = ctx->scene;
+    if (!sc.staged) { ctx->err = "pgi_set_scene_descriptors needs a scene registration first"; return PGI_ERR_STATE; }
+    if (dim != 128 && dim != 64) { ctx->err = "descriptors must have 64 or 128 dimensions"; return PGI_ERR_INVALID; }
+    const uint64_t nKp = sc.hKpOff.back();
+    if (!desc && nKp) { ctx->err = "null argument"; return PGI_ERR_INVALID; }
+    CK(cudaSetDevice(ctx->cfg.device));
+    return uploadDescriptors(ctx, desc, nKp, dim);
+}
 
 pgi_status pgi_submit_wave(pgi_ctx *ctx, uint32_t n, const uint32_t *pair_id, const uint32_t *hyp_offset,
                            const double *hyp_q_t, uint32_t flags)
@@ -912,7 +1041,9 @@ pgi_status pgi_submit_wave(pgi_ctx *ctx, uint32_t n, const uint32_t *pair_id, co
     PgiNvtxRange nvtxRange("pgi:submit_wave (H2D hypotheses + K1/K2/K4/K5/K3 launches)");
     if (!ctx) return PGI_ERR_INVALID;
     CK(cudaSetDevice(ctx->cfg.device));
-    return submitWave(ctx, *ctx->reg, n, pair_id, hyp_offset, hyp_q_t, flags, 0.0, 0, false);
+    // PGI_WAVE_EXTRA selects the registration of pgi_register_extra_pairs; the kernels never see the bit
+    const Registration &r = (flags & PGI_WAVE_EXTRA) ? ctx->extra : *ctx->reg;
+    return submitWave(ctx, r, n, pair_id, hyp_offset, hyp_q_t, flags & ~(uint32_t)PGI_WAVE_EXTRA, 0.0, 0, false);
 }
 
 pgi_status pgi_wait_wave(pgi_ctx *ctx, pgi_verdict *out, uint8_t *masks_or_null)
@@ -1200,32 +1331,21 @@ pgi_status pgi_guided_match(pgi_ctx *ctx, uint32_t n_src, const float *kp_src, c
     a.kpS = reinterpret_cast<const float2 *>(d + oKpS); a.dS = reinterpret_cast<const float *>(d + oDS);
     a.kpD = reinterpret_cast<const float2 *>(d + oKpD); a.dD = reinterpret_cast<const float *>(d + oDD);
     a.nS = n_src; a.nD = n_dst; a.dim = dim;
-    {
-        double E[9];
-        // E = [t]x R of the pose (pose.h:46-55), as the matcher reads it from Pose::getEssentialMatrix (matcher.h:218)
-        double R[9];
-        const double *q = pose_q_t;
-        const double tx = 2.0 * q[0], ty = 2.0 * q[1], tz = 2.0 * q[2];
-        const double twx = tx * q[3], twy = ty * q[3], twz = tz * q[3], txx = tx * q[0], txy = ty * q[0], txz = tz * q[0];
-        const double tyy = ty * q[1], tyz = tz * q[1], tzz = tz * q[2];
-        R[0] = 1.0 - (tyy + tzz); R[1] = txy - twz; R[2] = txz + twy;
-        R[3] = txy + twz; R[4] = 1.0 - (txx + tzz); R[5] = tyz - twx;
-        R[6] = txz - twy; R[7] = tyz + twx; R[8] = 1.0 - (txx + tyy);
-        const double Cx[9] = {0.0, -q[6], q[5], q[6], 0.0, -q[4], -q[5], q[4], 0.0};
-        for (int i = 0; i < 3; i++)
-            for (int j = 0; j < 3; j++) E[i * 3 + j] = Cx[i * 3 + 0] * R[j] + (Cx[i * 3 + 1] * R[3 + j] + Cx[i * 3 + 2] * R[6 + j]);
-        for (int k = 0; k < 9; k++) { a.E[k] = E[k]; a.Ks[k] = K_src[k]; a.Kd[k] = K_dst[k]; }
-    }
+    essentialOfPose(pose_q_t, a.E);
+    for (int k = 0; k < 9; k++) { a.Ks[k] = K_src[k]; a.Kd[k] = K_dst[k]; }
     a.wS = size_src[0]; a.hS = size_src[1]; a.wD = size_dst[0]; a.hD = size_dst[1]; a.binNumber = bin_number;
     a.binOfD = d + oBin; a.binList = reinterpret_cast<uint32_t *>(d + oList); a.cand = reinterpret_cast<uint32_t *>(d + oCand);
     a.candRatio = reinterpret_cast<double *>(d + oRatio); a.matches = reinterpret_cast<uint32_t *>(d + oM);
     a.ratios = reinterpret_cast<double *>(d + oR); a.nOut = reinterpret_cast<uint32_t *>(d + oN);
     a.prepOut = reinterpret_cast<double *>(d + oPrep);
+    CK(cudaEventRecord(ctx->evStart, s));
     k7_guided_match<<<1, kMatchThreads, 0, s>>>(a);
+    CK(cudaEventRecord(ctx->evK1, s));
     CK(cudaGetLastError());
     uint32_t n = 0;
     CK(cudaMemcpyAsync(&n, d + oN, 4, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
+    CK(addGuidedTime(ctx));
     if (n > n_src) n = n_src;
     if (n) {
         CK(cudaMemcpy(matches_out, d + oM, (size_t)n * 8, cudaMemcpyDeviceToHost));
@@ -1236,6 +1356,95 @@ pgi_status pgi_guided_match(pgi_ctx *ctx, uint32_t n_src, const float *kp_src, c
     ctx->stats.launches += 1;
     ctx->stats.h2d_bytes += bS * (8 + dim * 4) + bD * (8 + dim * 4);
     ctx->stats.d2h_bytes += (size_t)n * 16 + 4;
+    return PGI_OK;
+}
+
+pgi_status pgi_guided_match_views(pgi_ctx *ctx, uint32_t src, uint32_t dst, const double *pose_q_t, int32_t bin_number,
+                                  uint32_t max_points, uint32_t *matches_out, double *values_out, uint32_t *n_out)
+{
+    PgiNvtxRange nvtxRange("pgi:guided_match_views (K7 on the resident scene)");
+    if (!ctx) return PGI_ERR_INVALID;
+    if (ctx->inFlight) { ctx->err = "a wave is in flight"; return PGI_ERR_STATE; }
+    const SceneStaging &sc = ctx->scene;
+    if (!sc.staged) { ctx->err = "pgi_guided_match_views needs a scene registration first"; return PGI_ERR_STATE; }
+    if (!sc.hasDesc) {
+        ctx->err = "the registered scene has no descriptors (pgi_register_scene_descriptors or pgi_set_scene_descriptors)";
+        return PGI_ERR_STATE;
+    }
+    const uint64_t V = sc.hFocal.size();
+    if (src >= V || dst >= V) { ctx->err = "view id out of range"; return PGI_ERR_INVALID; }
+    if (!pose_q_t || !n_out || (max_points && (!matches_out || !values_out)) || bin_number > kMatchMaxBins) {
+        ctx->err = "bad argument";
+        return PGI_ERR_INVALID;
+    }
+    CK(cudaSetDevice(ctx->cfg.device));
+    *n_out = 0;
+    const uint64_t nS = sc.hKpOff[src + 1] - sc.hKpOff[src], nD = sc.hKpOff[dst + 1] - sc.hKpOff[dst];
+    if (nS == 0 || nD == 0 || max_points == 0) return PGI_OK;
+    cudaStream_t s = ctx->stream;
+    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    const size_t oBin = 0, oList = oBin + al(nD), oCand = oList + al(nD * 4), oRatio = oCand + al(nS * 4), oM = oRatio + al(nS * 8),
+                 oR = oM + al(nS * 8), oN = oR + al(nS * 8), total = oN + 256;
+    CK(ctx->guided.grow(total));
+    unsigned char *d = ctx->guided.data();
+    MatchArgs a;
+    a.kpS = sc.kp.data() + sc.hKpOff[src]; a.dS = sc.desc.data() + sc.hKpOff[src] * sc.dim;
+    a.kpD = sc.kp.data() + sc.hKpOff[dst]; a.dD = sc.desc.data() + sc.hKpOff[dst] * sc.dim;
+    a.nS = (uint32_t)nS; a.nD = (uint32_t)nD; a.dim = sc.dim;
+    essentialOfPose(pose_q_t, a.E);
+    // K = [f 0 w/2; 0 f h/2; 0 0 1] of each view (pose_graph_builder.h:284-286)
+    const double fS = sc.hFocal[src], wS = sc.hSize[2 * src], hS = sc.hSize[2 * src + 1];
+    const double fD = sc.hFocal[dst], wD = sc.hSize[2 * dst], hD = sc.hSize[2 * dst + 1];
+    const double Ks[9] = {fS, 0.0, wS / 2.0, 0.0, fS, hS / 2.0, 0.0, 0.0, 1.0};
+    const double Kd[9] = {fD, 0.0, wD / 2.0, 0.0, fD, hD / 2.0, 0.0, 0.0, 1.0};
+    for (int k = 0; k < 9; k++) { a.Ks[k] = Ks[k]; a.Kd[k] = Kd[k]; }
+    a.wS = (int)wS; a.hS = (int)hS; a.wD = (int)wD; a.hD = (int)hD; a.binNumber = bin_number;
+    a.binOfD = d + oBin; a.binList = reinterpret_cast<uint32_t *>(d + oList); a.cand = reinterpret_cast<uint32_t *>(d + oCand);
+    a.candRatio = reinterpret_cast<double *>(d + oRatio); a.matches = reinterpret_cast<uint32_t *>(d + oM);
+    a.ratios = reinterpret_cast<double *>(d + oR); a.nOut = reinterpret_cast<uint32_t *>(d + oN);
+    a.prepOut = nullptr;
+    CK(cudaEventRecord(ctx->evStart, s));
+    k7_guided_match<<<1, kMatchThreads, 0, s>>>(a);
+    CK(cudaEventRecord(ctx->evK1, s));
+    CK(cudaGetLastError());
+    uint32_t n = 0;
+    CK(cudaMemcpyAsync(&n, d + oN, 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    CK(addGuidedTime(ctx));
+    if (n > nS) n = (uint32_t)nS;
+    ctx->guidedM.resize((size_t)2 * n);
+    ctx->guidedR.resize(n);
+    if (n) {
+        CK(cudaMemcpyAsync(ctx->guidedM.data(), d + oM, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(ctx->guidedR.data(), d + oR, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+    }
+    ctx->stats.launches += 1;
+    ctx->stats.d2h_bytes += (size_t)n * 16 + 4;
+    // guidedMatching's selection (pose_graph_builder.h:760-782): above max_points matches, the max_points smallest
+    // (value, index) entries in the min-heap's pop order; otherwise every match, each carrying the first value (:777-779)
+    const std::vector<uint32_t> &m = ctx->guidedM;
+    const std::vector<double> &r = ctx->guidedR;
+    if (n > max_points) {
+        std::vector<uint32_t> &order = ctx->guidedOrder;
+        order.resize(n);
+        for (uint32_t i = 0; i < n; i++) order[i] = i;
+        const auto less = [&](uint32_t x, uint32_t y) { return r[x] != r[y] ? r[x] < r[y] : x < y; };
+        std::partial_sort(order.begin(), order.begin() + max_points, order.end(), less);
+        for (uint32_t k = 0; k < max_points; k++) {
+            matches_out[2 * k] = m[2 * order[k]];
+            matches_out[2 * k + 1] = m[2 * order[k] + 1];
+            values_out[k] = r[order[k]];
+        }
+        *n_out = max_points;
+    } else {
+        for (uint32_t k = 0; k < n; k++) {
+            matches_out[2 * k] = m[2 * k];
+            matches_out[2 * k + 1] = m[2 * k + 1];
+            values_out[k] = r[0];
+        }
+        *n_out = n;
+    }
     return PGI_OK;
 }
 

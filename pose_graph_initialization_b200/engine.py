@@ -11,7 +11,7 @@ import numpy as np
 from . import build as _build
 
 PGI_OK = 0
-WAVE_PATH, WAVE_FALLBACK, WAVE_MASKS, WAVE_NO_TEST = 1, 2, 4, 8
+WAVE_PATH, WAVE_FALLBACK, WAVE_MASKS, WAVE_NO_TEST, WAVE_EXTRA = 1, 2, 4, 8, 16
 
 VERDICT_DTYPE = np.dtype(
     [
@@ -37,7 +37,7 @@ class PgiStats(C.Structure):
                 ("ms_total", C.c_double), ("launches", C.c_uint64), ("pairs", C.c_uint64), ("corr_evals", C.c_uint64),
                 ("fallback_pairs", C.c_uint64), ("fallback_models", C.c_uint64), ("h2d_bytes", C.c_uint64),
                 ("d2h_bytes", C.c_uint64), ("ms_match", C.c_double), ("dist_evals", C.c_uint64), ("match_pairs", C.c_uint64),
-                ("match_rows", C.c_uint64)]
+                ("match_rows", C.c_uint64), ("ms_guided", C.c_double), ("guided_calls", C.c_uint64)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
@@ -49,7 +49,8 @@ EXPORTS = [
     "pgi_estimate_pose", "pgi_test_pose", "pgi_graph_init", "pgi_graph_apply", "pgi_graph_search", "pgi_graph_stats",
     "pgi_guided_match", "pgi_match_features", "pgi_get_stats", "pgi_reset_stats", "pgi_dbg_sampson",
     "pgi_dbg_five_point", "pgi_dbg_pose_from_essential", "pgi_dbg_fp64_peak", "pgi_register_scene_descriptors",
-    "pgi_read_scene_matches",
+    "pgi_read_scene_matches", "pgi_set_scene_descriptors", "pgi_register_extra_pairs", "pgi_read_extra_pair",
+    "pgi_guided_match_views",
 ]
 
 _lib = None
@@ -126,6 +127,7 @@ class Engine:
         self.h = h
         self.n_pairs = 0
         self.offset = None
+        self.extra_offset = None
         self._wave_n = 0
         self._wave_rows = 0
 
@@ -191,6 +193,32 @@ class Engine:
         self._ck(self.lib.pgi_read_scene_matches(self.h, _ptr(m), _ptr(r), C.c_uint64(n_rows)))
         return m, r
 
+    def set_scene_descriptors(self, desc):
+        """Descriptors [sum K, dim] (float32, dim 64 or 128) of the scene registered by register_scene, row-aligned with its
+        keypoints; they stay on the device for guided_match_views."""
+        desc = np.ascontiguousarray(desc, dtype=np.float32)
+        if desc.ndim != 2:
+            raise ValueError("desc must be a [sum K, dim] array")
+        self._ck(self.lib.pgi_set_scene_descriptors(self.h, _ptr(desc), C.c_uint32(desc.shape[1])))
+
+    def register_extra_pairs(self, pair_views, m_offset, matches):
+        """Correspondences of caller-supplied matches (pair_views [n, 2], m_offset [n + 1], matches [M, 2]) built on the
+        device from the registered scene's keypoints; waves address them with WAVE_EXTRA."""
+        pv = np.ascontiguousarray(pair_views, dtype=np.uint32).reshape(-1, 2)
+        mo = np.ascontiguousarray(m_offset, dtype=np.uint64)
+        mt = np.ascontiguousarray(matches, dtype=np.uint32).reshape(-1, 2)
+        if len(mo) != len(pv) + 1 or int(mo[-1]) != len(mt):
+            raise ValueError("m_offset must have n_pairs + 1 entries ending at len(matches)")
+        self._ck(self.lib.pgi_register_extra_pairs(self.h, C.c_uint64(len(pv)), _ptr(pv), _ptr(mo), _ptr(mt)))
+        self.extra_offset = mo.copy()
+
+    def read_extra_pair(self, pair_id):
+        n = int(self.extra_offset[pair_id + 1] - self.extra_offset[pair_id])
+        corr = np.empty((n, 4))
+        rows, thr = C.c_uint64(0), C.c_double(0)
+        self._ck(self.lib.pgi_read_extra_pair(self.h, C.c_uint32(pair_id), _ptr(corr), C.c_uint64(n), C.byref(rows), C.byref(thr)))
+        return corr, thr.value
+
     def share_pairs(self, owner):
         """Use the pairs registered in `owner` (same device) without copying them."""
         self._ck(self.lib.pgi_share_pairs(self.h, owner.h))
@@ -213,7 +241,8 @@ class Engine:
         hyp = _f64(hyp).reshape(-1, 7) if hyp is not None and len(hyp) else np.zeros((0, 7))
         self._ck(self.lib.pgi_submit_wave(self.h, C.c_uint32(n), _ptr(pair_ids), _ptr(hyp_offset), _ptr(hyp), C.c_uint32(flags)))
         self._wave_n = n
-        self._wave_rows = int(sum(int(self.offset[p + 1] - self.offset[p]) for p in pair_ids)) if flags & WAVE_MASKS else 0
+        off = self.extra_offset if flags & WAVE_EXTRA else self.offset
+        self._wave_rows = int(sum(int(off[p + 1] - off[p]) for p in pair_ids)) if flags & WAVE_MASKS else 0
 
     def wait_wave(self, want_masks=False):
         out = np.zeros(self._wave_n, dtype=VERDICT_DTYPE)
@@ -314,6 +343,19 @@ class Engine:
         else:
             selected = [(int(a), int(b), float(ratios[0])) for a, b in matches]
         return dict(matches=matches, ratios=ratios, selected=selected, prepared=prep)
+
+    def guided_match_views(self, src, dst, pose_qt, bin_number=45, max_points=100):
+        """guidedMatching (pose_graph_builder.h:717-783) of views src -> dst of the registered scene on its device-resident
+        keypoints and descriptors -> the selected rows [(src idx, dst idx, value)], as guided_match(...)["selected"]."""
+        cap = max(int(max_points), 1)
+        m = np.zeros((cap, 2), dtype=np.uint32)
+        r = np.zeros(cap)
+        n = C.c_uint32(0)
+        pose = _f64(pose_qt).reshape(7)
+        self._ck(self.lib.pgi_guided_match_views(self.h, C.c_uint32(src), C.c_uint32(dst), _ptr(pose), C.c_int32(bin_number),
+                                                 C.c_uint32(max_points), _ptr(m), _ptr(r), C.byref(n)))
+        k = int(n.value)
+        return [(int(m[i, 0]), int(m[i, 1]), float(r[i])) for i in range(k)]
 
     def match_features(self, desc_src, desc_dst):
         """matchFeatures (feature_utils.h:103-210) on the device: -> (matches [n, 2] (queryIdx, trainIdx), ratios [n]),
