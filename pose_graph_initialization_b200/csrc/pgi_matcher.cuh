@@ -17,6 +17,7 @@
 // what glibc returns for all but ~2.5e-4 of arguments (CUDA's own atan2 is a 2-ulp function and differed from the host
 // in the angular range of one of five test scenes).
 #pragma once
+#include <climits>
 #include <cstdint>
 #include <cuda_runtime.h>
 
@@ -74,7 +75,9 @@ PGI_DEV double lineAngle(double ny, double nx)
 PGI_DEV int binOfAngle(double angle, double minAngle, double angularRange, int binNumber)
 {
     angle = (binNumber - 1) * (angle - minAngle) / angularRange;
-    const int b = (int)round(angle);
+    const double r = round(angle);
+    // the host's conversion (x86 cvttsd2si): NaN and out-of-range values become INT_MIN, i.e. bin 0 (cvt.rzi saturates)
+    const int b = (r >= -2147483648.0 && r < 2147483648.0) ? (int)r : INT_MIN;
     const int lo = b < 0 ? 0 : b;  // MAX(0, .)
     return lo < binNumber - 1 ? lo : binNumber - 1;
 }

@@ -84,3 +84,133 @@ def two_view_keypoints(n, rng, f=800.0, w=1600, h=1200, noise_px=0.3, desc_noise
     truth = np.full(len(kp_s), -1, dtype=np.int64)
     truth[inv_s[:n]] = inv_d[:n]
     return dict(kp_src=kp_s, desc_src=d_s, kp_dst=kp_d, desc_dst=d_d, pose=pose_qt(R, t), K=K, size=(w, h), truth=truth)
+
+
+def intrinsics(f, size):
+    """K = [f 0 w/2; 0 f h/2; 0 0 1], the camera the reference builds for every view (pose_graph_builder.h:284-286)."""
+    return np.array([[f, 0.0, size[0] / 2.0], [0.0, f, size[1] / 2.0], [0.0, 0.0, 1.0]])
+
+
+def _project(K, X):
+    return (X @ K.T)[:, :2] / X[:, 2:]
+
+
+def _inside(uv, size):
+    return (uv[:, 0] >= 0) & (uv[:, 0] < size[0]) & (uv[:, 1] >= 0) & (uv[:, 1] < size[1])
+
+
+def two_view_keypoints_posed(n, rng, R, t, K_src, K_dst, size_src, size_dst, noise_px=0.3, desc_noise=0.05, extra=0.3,
+                             dim=128, depth=7.0):
+    """two_view_keypoints with a given relative pose (x_dst ~ R x_src + t) and each view's own intrinsics and image size.
+    The n shared points lie in front of both cameras and project inside both images (before the keypoint noise); the
+    `extra`*n unrelated keypoints per view are uniform in that view's image.  Returns two_view_keypoints' dict with
+    K_src / K_dst and size_src / size_dst in place of K and size."""
+    R, t = np.asarray(R, dtype=np.float64), np.asarray(t, dtype=np.float64)
+    K_src, K_dst = np.asarray(K_src, dtype=np.float64), np.asarray(K_dst, dtype=np.float64)
+    X = np.zeros((0, 3))
+    for _ in range(200):
+        if len(X) >= n:
+            break
+        C = rng.standard_normal((4 * n, 3)) * np.array([1.5, 1.0, 1.0]) + np.array([0, 0, depth])
+        C2 = C @ R.T + t
+        ok = (C[:, 2] > 0.5) & (C2[:, 2] > 0.5) & _inside(_project(K_src, C), size_src) & _inside(_project(K_dst, C2), size_dst)
+        X = np.vstack([X, C[ok]])
+    assert len(X) >= n, "the two cameras do not share enough of the point cloud"
+    X = X[:n]
+    base = rng.standard_normal((n, dim))
+    base /= np.linalg.norm(base, axis=1, keepdims=True)
+
+    def view(Xc, K, size):
+        uv = _project(K, Xc) + rng.standard_normal((n, 2)) * noise_px
+        d = base + rng.standard_normal((n, dim)) * desc_noise
+        m = int(extra * n)
+        uv = np.vstack([uv, rng.uniform([0, 0], size, (m, 2))])
+        de = rng.standard_normal((m, dim))
+        d = np.vstack([d, de / np.linalg.norm(de, axis=1, keepdims=True)])
+        p = rng.permutation(n + m)
+        inv = np.empty(n + m, dtype=np.int64)
+        inv[p] = np.arange(n + m)
+        return uv[p].astype(np.float32), d[p].astype(np.float32), inv
+
+    kp_s, d_s, inv_s = view(X, K_src, size_src)
+    kp_d, d_d, inv_d = view(X @ R.T + t, K_dst, size_dst)
+    truth = np.full(len(kp_s), -1, dtype=np.int64)
+    truth[inv_s[:n]] = inv_d[:n]
+    return dict(kp_src=kp_s, desc_src=d_s, kp_dst=kp_d, desc_dst=d_d, pose=pose_qt(R, t), K_src=K_src, K_dst=K_dst,
+                size_src=tuple(size_src), size_dst=tuple(size_dst), truth=truth)
+
+
+# (focal length px, (width, height)): landscape, portrait, small, large and odd sizes (w/2 or h/2 not an integer).  The
+# focal lengths are exact in binary, so thr_px / ((f + f + f + f) / 4) == thr_px / f.
+CAMERAS = ((1200.0, (1601, 1199)), (450.0, (640, 480)), (2400.0, (3000, 4000)), (912.5, (1200, 1600)),
+           (1636.25, (2048, 1535)), (700.0, (1023, 767)))
+
+
+def per_view_camera_scene(n_views=12, seed=0, cameras=CAMERAS, group=3, n_points=1500, kp_max=1200, dim=128, noise_px=0.2,
+                          desc_noise=0.01, distractor_ratio=0.2, radius=6.0, arc=np.pi, with_matches=False,
+                          outlier_ratio=0.25):
+    """A scene in scene.py's dict layout in which each view has its own camera: view v uses cameras[(v // group) %
+    len(cameras)], so neighbouring views of one group share a camera and neighbours across groups do not.  Cameras on a
+    ring arc looking at a Gaussian blob, as scene.make_descriptor_scene; view v keeps at most kp_max keypoints: points that
+    project inside its image (projected with its own K, plus noise_px), plus distractor_ratio of unrelated keypoints, in
+    its own shuffled order, each with a `dim`-d descriptor (a unit vector per point plus desc_noise per dimension).
+    with_matches adds m_offset / matches for every pair: its shared points in random order, outlier_ratio of them with a
+    wrong destination keypoint.  gt_point[sum K] holds each keypoint's 3-D point (-1 for distractors)."""
+    rng = np.random.default_rng(seed)
+    V = n_views
+    cam_of = [cameras[(v // group) % len(cameras)] for v in range(V)]
+    pts = rng.standard_normal((n_points, 3))
+    base = rng.standard_normal((n_points, dim))
+    base /= np.linalg.norm(base, axis=1, keepdims=True)
+    ang = np.arange(V) * (arc / V) + rng.uniform(-0.2, 0.2, V) * (arc / V)
+    elev = rng.uniform(-0.2, 0.2, V)
+    rad = radius * (1.0 + rng.uniform(-0.1, 0.1, V))
+    cam = np.stack([rad * np.cos(ang) * np.cos(elev), rad * np.sin(ang) * np.cos(elev), rad * np.sin(elev)], 1)
+    Rw = np.empty((V, 3, 3))
+    for v in range(V):
+        z = rng.standard_normal(3) * 0.15 - cam[v]
+        z /= np.linalg.norm(z)
+        x = np.cross(z, [0.0, 0.0, 1.0])
+        x /= np.linalg.norm(x)
+        Rw[v] = np.stack([x, np.cross(z, x), z])  # rows: camera axes in world coordinates (world -> camera)
+    tw = -np.einsum("vij,vj->vi", Rw, cam)
+    kps, descs, pids = [], [], []
+    for v in range(V):
+        f, size = cam_of[v]
+        Xc = pts @ Rw[v].T + tw[v]
+        uv = _project(intrinsics(f, size), Xc)
+        vis = np.flatnonzero((Xc[:, 2] > 0.5) & _inside(uv, size))
+        n_real = min(len(vis), int(round(kp_max * (1.0 - distractor_ratio))))
+        real = np.sort(rng.choice(vis, n_real, replace=False))
+        m = int(round(n_real * distractor_ratio / (1.0 - distractor_ratio)))
+        de = rng.standard_normal((m, dim))
+        xy = np.vstack([uv[real] + rng.standard_normal((n_real, 2)) * noise_px, rng.uniform([0.0, 0.0], size, (m, 2))])
+        d = np.vstack([base[real] + rng.standard_normal((n_real, dim)) * desc_noise, de / np.linalg.norm(de, axis=1, keepdims=True)])
+        pid = np.concatenate([real, np.full(m, -1)])
+        order = rng.permutation(len(pid))
+        kps.append(xy[order].astype(np.float32)); descs.append(d[order].astype(np.float32)); pids.append(pid[order])
+    view_dir = Rw[:, 2, :]
+    sim = np.round(np.minimum(np.clip(view_dir @ view_dir.T, 0.0, 0.999), 0.999), 3)
+    sim = np.round((sim + sim.T) / 2.0, 3)
+    np.fill_diagonal(sim, 1.0)
+    iu, ju = np.triu_indices(V, 1)
+    counts = np.array([len(k) for k in kps])
+    sc = dict(focal=np.array([c[0] for c in cam_of]), size=np.array([c[1] for c in cam_of], dtype=np.float64), sim=sim,
+              kp_offset=np.concatenate([[0], np.cumsum(counts)]).astype(np.uint64), kp=np.concatenate(kps).reshape(-1, 2),
+              desc=np.concatenate(descs).reshape(-1, dim), pair_views=np.stack([iu, ju], 1).astype(np.uint32),
+              gt_q=np.array([quat_from_rot(R) for R in Rw]), gt_t=tw.copy(), gt_R=Rw.copy(),
+              gt_point=np.concatenate(pids).astype(np.int64))
+    if with_matches:
+        mo, rows = [0], []
+        for s, d in zip(iu, ju):
+            ps, pd = pids[s], pids[d]
+            where_d = {int(p): k for k, p in enumerate(pd) if p >= 0}
+            m = np.array([(k, where_d[int(p)]) for k, p in enumerate(ps) if p >= 0 and int(p) in where_d], dtype=np.int64).reshape(-1, 2)
+            m = m[rng.permutation(len(m))]
+            bad = rng.random(len(m)) < outlier_ratio
+            m[bad, 1] = rng.integers(0, len(pd), int(bad.sum()))
+            rows.append(m)
+            mo.append(mo[-1] + len(m))
+        sc["m_offset"] = np.array(mo, dtype=np.uint64)
+        sc["matches"] = np.concatenate(rows).astype(np.uint32).reshape(-1, 2)
+    return sc
