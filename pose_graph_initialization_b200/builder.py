@@ -12,7 +12,6 @@ NVLink on device buffers, gloo on CPU tensors in the tests) so that every rank r
 commit.  With world_size == 1 no collective is issued.
 """
 import ctypes as C
-import os
 import threading
 import time
 
@@ -485,10 +484,14 @@ class PoseGraphBuilder:
         self.max_points_hashing = kMaximumPointNumberForEpipolarHashing_
         self.min_inliers = kMinimumInlierNumber_
         self.device = device
+        # gpu_search=True: the speculative A* searches of a wave round run as one batched device call (K6) beside the host
+        # thread pool.  Exact, but measured no faster than the pool alone on the benchmark scenes (DESIGN.md section 4): a
+        # round lasts as long as its longest search and a search is a chain of dependent heap operations, so it is off by
+        # default.
+        self.gpu_search = bool(gpu_search)
         # measured on cfg2 (scripts/gpu_sweep.sh): 256 positions per wave is the optimum on one GPU (fewer A* re-searches
         # per position, rounds are cheap); with several ranks every round also costs a record exchange
-        use_gpu_search = bool(gpu_search) and os.environ.get("PGI_GPU_SEARCH", "1") != "0"
-        self.wave_size = wave_size if wave_size else default_wave_size(len(scene["focal"]), world_size, use_gpu_search)
+        self.wave_size = wave_size if wave_size else default_wave_size(len(scene["focal"]), world_size, self.gpu_search)
         self.prefetch_fallback = prefetch_fallback
         self.fallback_wave = fallback_wave
         self.group, self.rank, self.world = group, rank, world_size
@@ -497,8 +500,6 @@ class PoseGraphBuilder:
         # gloo group so that it never shares a communicator (or NCCL's ordering requirements) with the wave loop
         self.overlap = bool(overlap_fallback and prefetch_fallback)
         self.pf_group = None
-        self.pf_device = None
-        self.pf_stream = None
         self.engine = None
         self.engine_fb = None
         self.engine_fb2 = None
@@ -506,11 +507,6 @@ class PoseGraphBuilder:
         # one rank: the wave loop itself runs in C++ (pgb_run_wave calling pgi_submit_wave / pgi_wait_wave directly);
         # several ranks: the Python loop below, because the record exchange goes through torch.distributed
         self.native_loop = bool(native_loop)
-        # gpu_search=True: the speculative A* searches of a wave round run as one batched device call (K6) beside the host
-        # thread pool.  Exact, but measured no faster than the pool alone on the benchmark scenes (DESIGN.md section 4): a
-        # round lasts as long as its longest search and a search is a chain of dependent heap operations, so it is off by
-        # default.
-        self.gpu_search = bool(gpu_search) and os.environ.get("PGI_GPU_SEARCH", "1") != "0"
         self.gpu_search_min_batch = int(gpu_search_min_batch)
         self.prefetch_streams = int(prefetch_streams)
         self.timing = {}
@@ -563,8 +559,6 @@ class PoseGraphBuilder:
             # 330 KB per chunk; gloo moves it in about a millisecond.
             import torch.distributed as dist
             self.pf_group = dist.new_group(backend="gloo")
-            self.pf_device = None
-            self.pf_stream = None
         return self.pf_group
 
     def _match_owned_pairs(self):
@@ -674,9 +668,6 @@ class PoseGraphBuilder:
 
             def prefetch_worker():
                 try:
-                    if self.pf_device is not None:
-                        import torch
-                        torch.cuda.set_device(self.pf_device)
                     chunk = self.fallback_wave * self.world
                     engines = [e for e in (self.engine_fb, self.engine_fb2) if e is not None]
                     pending = []  # submitted chunks, oldest first: one in flight per background engine
@@ -687,12 +678,7 @@ class PoseGraphBuilder:
                         v["pair_id"] = mine.astype(np.uint32)
                         if self.world > 1:  # every rank needs every pair's fallback verdict (predictions + commit)
                             counts = [int(np.count_nonzero(own == r)) for r in range(self.world)]
-                            if self.pf_device is not None:
-                                import torch
-                                with torch.cuda.stream(self.pf_stream):
-                                    parts = allgather_verdicts(v, counts, self.pf_group, self.pf_device)
-                            else:
-                                parts = allgather_verdicts(v, counts, self.pf_group, None)
+                            parts = allgather_verdicts(v, counts, self.pf_group)
                             merged = np.zeros(len(ids), dtype=VERDICT_DTYPE)
                             for r in range(self.world):
                                 merged[np.nonzero(own == r)[0]] = parts[r]

@@ -195,10 +195,6 @@ struct Visibility {
     }
 };
 
-// PGB_EXPAND selects the expansion loop of the host A* (identical results; for measurements): 0 one pass, 1 two passes,
-// 2 (default) two passes with the AVX2 evaluation and batched sift-up flags
-static const int kExpandVariant = getenv("PGB_EXPAND") ? atoi(getenv("PGB_EXPAND")) : 2;
-
 struct AStarOut {
     bool valid = true;        // false: an entry below the cost floor reached the top of the queue (the caller repeats the search without a floor)
     double minPoppedF = 2.0;  // smallest combined cost among the popped nodes (the start node aside): the floor the search needed
@@ -528,8 +524,7 @@ void aStar(const GraphView &gv, const double *sim /*transposed*/, uint32_t V, ui
             uint32_t entry = 0;
             // Two passes over the edge list.  Pass 1 evaluates every entry without a data-dependent branch (admissible
             // children are compacted into a scratch array by a predicated store); pass 2 replays std::push_heap for them
-            // in list order.  Same operations on the same operands as the one-pass loop, but the sift-up's unpredictable
-            // exit no longer sits between two gathers.
+            // in list order, so the sift-up's unpredictable exit does not sit between two gathers.
             const size_t listLen = rl.size() + (ol ? ol->size() : 0);
             if (S.childF.size() < listLen + 8) { S.childF.resize(listLen + 8); S.childE.resize(listLen + 8); }  // (+8: a compress store may be issued at the very end)
             double *cf = S.childF.data();
@@ -549,39 +544,9 @@ void aStar(const GraphView &gv, const double *sim /*transposed*/, uint32_t V, ui
             };
             const Adj *ra = rl.data();
             const uint32_t nr = (uint32_t)rl.size();
-            if (kExpandVariant == 0) {
-                // the one-pass form (kept for A/B measurements, PGB_EXPAND=0): evaluate and push entry by entry
-                auto push1 = [&](const Adj &e, uint32_t ent) __attribute__((always_inline)) {
-                    if (e.score < 0.0) return;
-                    uint32_t next = e.next;
-                    if (lv != v) next = e.next == v ? lv : e.next;
-                    if (mark[next] == epoch) return;
-                    const double edgeCost = c0 > e.score ? e.score : c0;
-                    const double h = simTo[next];
-                    const double nextToDest = c1 < h ? h : c1;
-                    const double combined = wgt * edgeCost + oneMinusWeight * nextToDest;
-                    size_t hole = hs++;
-                    if (combined >= floorF)
-                        while (hole > 0) {
-                            const size_t parent = (hole - 1) / 2;
-                            if (!(first[parent].f < combined)) break;
-                            first[hole] = first[parent];
-                            hole = parent;
-                        }
-                    first[hole] = HeapItem{combined, ni, ent};
-                };
-                for (; entry < nr; ++entry) push1(ra[entry], entry);
-                if (ol)
-                    for (const OvAdj &oe : *ol) {
-                        if (oe.pos >= gv.cutoff) break;
-                        push1(oe.a, entry++);
-                    }
-                out.pushes += (uint32_t)(hs - hs0);
-                continue;
-            }
 #ifdef PGB_HAVE_AVX2_PATH
-            if (kExpandVariant >= 2 && kUseAvx512 && lv == v) cnt = evalEntriesAvx512(ra, nr, mark, epoch, simTo, c0, c1, wgt, oneMinusWeight, cf, ce, cnt, entry);
-            else if (kExpandVariant >= 2 && kUseAvx2 && lv == v) cnt = evalEntriesAvx2(ra, nr, mark, epoch, simTo, c0, c1, wgt, oneMinusWeight, cf, ce, cnt, entry);
+            if (kUseAvx512 && lv == v) cnt = evalEntriesAvx512(ra, nr, mark, epoch, simTo, c0, c1, wgt, oneMinusWeight, cf, ce, cnt, entry);
+            else if (kUseAvx2 && lv == v) cnt = evalEntriesAvx2(ra, nr, mark, epoch, simTo, c0, c1, wgt, oneMinusWeight, cf, ce, cnt, entry);
 #endif
             for (; entry < nr; ++entry) eval(ra[entry], entry);
             if (ol)
@@ -593,7 +558,7 @@ void aStar(const GraphView &gv, const double *sim /*transposed*/, uint32_t V, ui
             // heap before this expansion can only grow while its children are pushed, so a child that is not larger than
             // its parent NOW stays where it is appended.  All children are appended first, the ones that move are then
             // replayed in list order (when the heap is smaller than the batch, parents may be new slots: replay them all).
-            if (kExpandVariant >= 2 && hs >= cnt) {
+            if (hs >= cnt) {
                 size_t nMove = 0;
                 uint32_t *mv = S.childMove.size() < cnt ? (S.childMove.resize(listLen), S.childMove.data()) : S.childMove.data();
                 for (size_t i = 0; i < cnt; i++) {
@@ -677,8 +642,6 @@ struct Change {  // a wave position whose actual outcome differs from the predic
     bool existence;      // the edge appears or disappears (otherwise only its score / pose changes)
     double sOld, sNew;   // inlier ratios of the predicted and of the actual edge
 };
-// PGB_FINE_STALENESS=0: a changed edge at an expanded vertex always invalidates the search (the coarse rule)
-static const bool kFineStaleness = !(getenv("PGB_FINE_STALENESS") && atoi(getenv("PGB_FINE_STALENESS")) == 0);
 
 // The fine staleness rule for ONE expansion of a search: the expansion's node had the cost tuple (c0, c1), `h` is the
 // heuristic of the changed edge's other endpoint, the edge's score goes sOld -> sNew, tauMin is the smallest combined cost
@@ -825,7 +788,7 @@ struct pgb_builder {
     int32_t searchError = 0;     // first engine status of a failed device search (surfaced by pgb_run_wave)
     bool gpuCheck = false;       // PGB_SEARCH_CHECK=1: every device search is repeated on the host and compared
     bool ovDirty = true;         // the overlay changed since it was last mirrored to the device
-    double hybridShare = 0.3;    // share of a round's estimated search work the host pool takes beside the device (0: none)
+    double hybridShare = 0.3;    // share of a round's estimated search work the host pool takes beside the device
     uint32_t gpuBudget = 0;      // push budget of the round's device queries (0: unlimited)
     std::vector<double> srcFloor, dstFloor;  // per view: smallest popped cost of the last search from / to it (floor guesses)
     std::vector<uint32_t> srcCost;  // per source view: pushes of the last search that started there (cost estimate)
@@ -934,8 +897,8 @@ void rebuildOverlay(pgb_builder *b, uint32_t from = 0)
     b->ctr.sec_visibility += nowSec() - t0;
 }
 
-// Margin under the remembered floors for the next guess; PGB_FLOOR_MARGIN < 0 switches the cost floor off.
-static const double kFloorMargin = getenv("PGB_FLOOR_MARGIN") ? atof(getenv("PGB_FLOOR_MARGIN")) : 0.01;
+// Margin under the remembered floors for the next guess.
+static const double kFloorMargin = 0.01;
 
 void searchPosition(pgb_builder *b, uint32_t k, AStarScratch &S)
 {
@@ -952,11 +915,9 @@ void searchPosition(pgb_builder *b, uint32_t k, AStarScratch &S)
         // same source view and to the same destination view needed (neighbouring queue positions behave alike), minus a
         // margin.  The tables are hints shared by the pool threads without synchronisation — any value is a valid guess.
         double floorF = -1.0;
-        if (kFloorMargin >= 0.0) {
-            double g = it.floorSeen;
-            if (g < 0.0 && b->srcFloor[it.src] >= 0.0 && b->dstFloor[it.dst] >= 0.0) g = std::min(b->srcFloor[it.src], b->dstFloor[it.dst]);
-            if (g >= 0.0) floorF = g - kFloorMargin;
-        }
+        double g = it.floorSeen;
+        if (g < 0.0 && b->srcFloor[it.src] >= 0.0 && b->dstFloor[it.dst] >= 0.0) g = std::min(b->srcFloor[it.src], b->dstFloor[it.dst]);
+        if (g >= 0.0) floorF = g - kFloorMargin;
         aStar(gv, b->sim.data(), b->V, it.src, it.dst, (size_t)b->cfg.maximum_search_depth,
               b->cfg.traversal_heuristics_weight, S, o, floorF);
         if (!o.valid && floorF - 0.05 > 0.0) {  // guessed too high: once more with a wide margin, then without a floor
@@ -1133,7 +1094,7 @@ void searchStale(pgb_builder *b, uint32_t limit)
         // searches expected to be the longest — a position's previous search is the estimate — up to a share of the
         // estimated work that is adapted round by round until both finish together.
         std::vector<uint32_t> hostPart, devPart;
-        if (b->hybridShare > 0.0 && b->cfg.host_threads > 1) {
+        if (b->cfg.host_threads > 1) {
             std::vector<std::pair<uint64_t, uint32_t>> est;
             est.reserve(todo.size());
             uint64_t total = 0;
@@ -1354,7 +1315,7 @@ uint32_t advanceWave(pgb_builder *b)
             for (uint32_t m = firstChanged + 1; m < n; m++) {
                 Item &it = b->wave[m];
                 if (!it.mine || !it.searched) continue;
-                const bool fine = kFineStaleness && it.expCost.size() == 2 * it.expanded.size();
+                const bool fine = it.expCost.size() == 2 * it.expanded.size();
                 const double *simTo = b->sim.data() + (size_t)it.dst * b->V;
                 for (size_t x = 0; x < it.expanded.size() && it.searched; x++) {
                     const uint32_t v = it.expanded[x];
@@ -1589,7 +1550,6 @@ int32_t pgb_set_search_backend(pgb_builder *b, pgb_graph_apply_fn apply, pgb_gra
     b->gpuMinBatch = min_batch;
     b->ovDirty = true;
     if (const char *e = getenv("PGB_SEARCH_CHECK")) b->gpuCheck = atoi(e) != 0;
-    if (const char *e = getenv("PGB_HYBRID_SHARE")) b->hybridShare = std::min(0.9, std::max(0.0, atof(e)));
     if (!apply) return 0;
     // bring the device graph up to the committed graph (normally empty at this point)
     std::vector<pgi_adj_entry> entries;

@@ -130,7 +130,7 @@ struct FallbackScratch {
     DevBuf<double> sols;
     DevBuf<uint8_t> counts;
     DevBuf<float4> solsF;
-    DevBuf<uint32_t> dkList, dkCtl;  // work list of the split K4 (K4a -> K4b -> K4c)
+    DevBuf<uint32_t> dkList, dkCtl;  // work list of K4b (K4a -> K4b -> K4c)
 };
 
 // The compact inputs of the last scene registration. Kept between registrations: cudaMalloc / cudaFree of GB-sized
@@ -201,6 +201,9 @@ struct Graph {
 
 constexpr int kMaxChunks = 64;
 constexpr uint32_t kK5MaxSmemPts = 11264;  // 176 KB of float4 + 22 KB of queues; also keeps point slots per thread <= 64 (mask bits)
+constexpr uint32_t kK4bCtasPerSm = 2;       // fewer lanes = more polynomials per lane = better refill balance
+constexpr uint32_t kAstarSlotsPerSm = 16;   // K6 searches resident per SM (heap + arena slabs each)
+static_assert(kAstarSlotsPerSm % kAstarWarps == 0, "K6 slots come in whole CTAs");
 
 }  // namespace
 
@@ -231,10 +234,6 @@ struct pgi_ctx {
     DevBuf<unsigned long long> counters;
     PinnedBuf<unsigned long long> hCounters;
     SceneStaging scene;
-    uint32_t k4aSmem = 0;  // PGI_K4A_SMEM: dynamic shared memory per K4a CTA, an occupancy throttle (L2 footprint of the 5 KB stacks)
-    uint32_t k4bCtas = 2;  // K4b CTAs per SM (PGI_K4B_CTAS): fewer lanes = more polynomials per lane = better refill balance
-    bool k4Split = true;   // PGI_K4_SPLIT=0 selects the one-kernel k4_fallback_solve
-    bool k1Tma = true;     // PGI_K1_TMA=0: always the direct-load K1
     uint32_t numSms = 148;
     // in flight
     bool inFlight = false;
@@ -244,7 +243,6 @@ struct pgi_ctx {
     bool fbLaunched = false;
     pgi_stats stats;
     Graph graph;
-    int popLookahead = 1, stagedPush = 1;
     pgi_search_stats sstats;
 };
 
@@ -458,7 +456,7 @@ pgi_status submitWave(pgi_ctx *ctx, const Registration &r, uint32_t n, const uin
     CK(cudaEventRecord(ctx->evStart, s));  // kernel-only timing: the wave's small H2D copies are before this event
     // full waves stream the correspondences through shared memory with bulk async copies (persistent CTAs, one per SM);
     // small waves and waves that want byte masks take the one-CTA-per-pair kernel
-    if (ctx->k1Tma && n >= 2u * ctx->numSms && !(flags & PGI_WAVE_MASKS)) {
+    if (n >= 2u * ctx->numSms && !(flags & PGI_WAVE_MASKS)) {
         const int k1Smem = kK1Stages * kK1TileRows * 32 + (int)sizeof(K1Meta);
         CK(cudaFuncSetAttribute(k1_score_hypotheses_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, k1Smem));
         k1_score_hypotheses_tma<<<std::min<uint32_t>(n, ctx->numSms), kK1TmaThreads, k1Smem, s>>>(a);
@@ -486,23 +484,17 @@ pgi_status submitWave(pgi_ctx *ctx, const Registration &r, uint32_t n, const uin
                                   (size_t)((smemPts + 31) / 32) * 4;  // + inlier bit mask of the LO refit
             if (k5Smem > 40 * 1024)  // static shared memory (~4 KB) counts towards the 48 KB default limit
                 CK(cudaFuncSetAttribute(k5_fallback_score, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k5Smem));
-            if (ctx->k4aSmem > 40 * 1024)
-                CK(cudaFuncSetAttribute(k4a_polynomial, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->k4aSmem));
             ctx->nChunks = std::min(chunks, kMaxChunks);
             for (int c = 0; c < ctx->nChunks; c++) {
                 const uint32_t threads = n * kFbChunk;
-                if (ctx->k4Split) {
-                    CK(cudaMemsetAsync(ctx->fb.dkCtl.data(), 0, 8, s));
-                    k4a_polynomial<<<(threads + 127) / 128, 128, ctx->k4aSmem, s>>>(a, c);
-                    k4b_roots<<<std::min<uint32_t>((threads + 127) / 128, ctx->numSms * ctx->k4bCtas), 128, 0, s>>>(a);
-                    k4c_solutions<<<(threads + 127) / 128, 128, 0, s>>>(a, c);
-                    ctx->stats.launches += 2;
-                } else
-                    k4_fallback_solve<<<(threads + 127) / 128, 128, 0, s>>>(a, c);
+                CK(cudaMemsetAsync(ctx->fb.dkCtl.data(), 0, 8, s));
+                k4a_polynomial<<<(threads + 127) / 128, 128, 0, s>>>(a, c);
+                k4b_roots<<<std::min<uint32_t>((threads + 127) / 128, ctx->numSms * kK4bCtasPerSm), 128, 0, s>>>(a);
+                k4c_solutions<<<(threads + 127) / 128, 128, 0, s>>>(a, c);
                 CK(cudaEventRecord(ctx->evChunk[c][0], s));
                 k5_fallback_score<<<n, kCtaThreads, k5Smem, s>>>(a, c, c == ctx->nChunks - 1 ? 1 : 0, smemPts);
                 CK(cudaEventRecord(ctx->evChunk[c][1], s));
-                ctx->stats.launches += 2;
+                ctx->stats.launches += 4;
             }
             ctx->fbLaunched = true;
         }
@@ -701,11 +693,7 @@ pgi_status pgi_create(const pgi_config *cfg, pgi_ctx **out)
     // until it is handed out, a failure destroys the half-built context
     std::unique_ptr<pgi_ctx, decltype(&pgi_destroy)> ctx(new pgi_ctx(), pgi_destroy);
     ctx->cfg = *cfg;
-    if (const char *e = getenv("PGI_K4_SPLIT")) ctx->k4Split = atoi(e) != 0;
-    if (const char *e = getenv("PGI_K1_TMA")) ctx->k1Tma = atoi(e) != 0;
     ctx->numSms = (uint32_t)std::max(1, prop.multiProcessorCount);
-    if (const char *e = getenv("PGI_K4A_SMEM")) ctx->k4aSmem = (uint32_t)std::max(0, std::min(200 * 1024, atoi(e)));
-    if (const char *e = getenv("PGI_K4B_CTAS")) ctx->k4bCtas = (uint32_t)std::max(1, std::min(4, atoi(e)));
     if (ctx->cfg.min_inliers == 0) ctx->cfg.min_inliers = 20;
     if (ctx->cfg.test_min_inliers == 0) ctx->cfg.test_min_inliers = 5;
     if (ctx->cfg.fallback_max_iters == 0) ctx->cfg.fallback_max_iters = 1000;
@@ -1147,17 +1135,13 @@ pgi_status pgi_graph_init(pgi_ctx *ctx, uint32_t n_views, const double *sim_to_n
     const uint32_t V = n_views;
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, ctx->cfg.device));
-    uint32_t slotsPerSm = 16, heapCap = 0;
-    if (const char *e = getenv("PGI_ASTAR_SLOTS_PER_SM")) slotsPerSm = (uint32_t)std::max(4, std::min(48, atoi(e)));
-    slotsPerSm = (slotsPerSm / kAstarWarps) * kAstarWarps;
+    uint32_t heapCap = 0;
     if (const char *e = getenv("PGI_ASTAR_HEAP")) heapCap = (uint32_t)std::max(1024, atoi(e));
-    if (const char *e = getenv("PGI_ASTAR_POP")) ctx->popLookahead = atoi(e) != 0;
-    if (const char *e = getenv("PGI_ASTAR_STAGED")) ctx->stagedPush = atoi(e) != 0;
     if (!heapCap) {
         const uint64_t want = (uint64_t)V * V / 2;
         heapCap = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(want, 65536), 1u << 20);
     }
-    const uint32_t slots = (uint32_t)prop.multiProcessorCount * slotsPerSm;
+    const uint32_t slots = (uint32_t)prop.multiProcessorCount * kAstarSlotsPerSm;
     const uint32_t arenaCap = 16384;
     if (ctx->graph.V != V || ctx->graph.heapCap != heapCap || ctx->graph.slots != slots) {
         // the old graph is released first; the new one only replaces it once every allocation succeeded
@@ -1255,8 +1239,6 @@ pgi_status pgi_graph_search(pgi_ctx *ctx, uint32_t n, const pgi_query *queries, 
     a.weight = weight; a.oneMinusWeight = 1.0 - weight;
     a.heaps = g.heaps.data(); a.heapCap = g.heapCap; a.arenas = g.arenas.data(); a.arenaCap = g.arenaCap;
     a.results = q.results.data(); a.expandedBits = q.expBits.data(); a.nextQuery = g.nextQuery.data();
-    a.popLookahead = ctx->popLookahead;
-    a.staged = ctx->stagedPush;
     const uint32_t ctas = std::min<uint32_t>((n + kAstarWarps - 1) / kAstarWarps, g.slots / kAstarWarps);
     const size_t smem = (size_t)kAstarWarps * ((size_t)kStageItems * sizeof(HeapItemDev) + (size_t)kChunk * 2 + (size_t)2 * words * 4);
     CK(cudaFuncSetAttribute(k6_astar_search, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)));

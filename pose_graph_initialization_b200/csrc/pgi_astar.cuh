@@ -76,8 +76,6 @@ struct SearchArgs {
     pgi_search_result *results;
     uint32_t *expandedBits;  // n x words
     uint32_t *nextQuery;     // work counter (zeroed before the launch)
-    int popLookahead;        // 1: warp-cooperative pop (4 levels per round trip); 0: lane 0 walks alone
-    int staged;              // 1: expansions are replayed in shared memory (expandStaged); 0: directly on the heap in HBM
 };
 
 __device__ __forceinline__ HeapItemDev ldItem(const HeapItemDev *p)
@@ -107,23 +105,11 @@ __device__ __forceinline__ void touchL1(const HeapItemDev *p)
     (void)sink;
 }
 
-// std::__push_heap(first, hole, 0, value, less-on-f): libstdc++ bits/stl_heap.h
-__device__ __forceinline__ void siftUp(HeapItemDev *H, uint32_t hole, const HeapItemDev &value)
-{
-    while (hole > 0) {
-        const uint32_t parent = (hole - 1) >> 1;
-        const HeapItemDev p = ldItem(H + parent);
-        if (!(p.f < value.f)) break;
-        stItem(H + hole, p);
-        hole = parent;
-    }
-    stItem(H + hole, value);
-}
-
-// The same std::__push_heap by the whole warp, in one memory round trip whatever the depth.  The path from a slot to
-// the root is non-decreasing in f (heap property), so the ancestors smaller than `value` are the first L of the path:
-// lane j loads the j-th ancestor, a ballot yields L, ancestors 1..L each move one level down (lane j stores what it
-// loaded) and `value` lands on level L — exactly the moves of the sequential loop.  (A child that out-ranks most of a
+// std::__push_heap(first, hole, 0, value, less-on-f) (libstdc++ bits/stl_heap.h) by the whole warp, in one memory
+// round trip whatever the depth.  The path from a slot to the root is non-decreasing in f (heap property), so the
+// ancestors smaller than `value` are the first L of the path: lane j loads the j-th ancestor, a ballot yields L,
+// ancestors 1..L each move one level down (lane j stores what it loaded) and `value` lands on level L — exactly the
+// moves of libstdc++'s sequential loop.  (A child that out-ranks most of a
 // 10^5-entry heap climbs ~15 levels; one lane walking them costs 15 dependent loads.)  All lanes pass the same
 // arguments; the caller separates consecutive calls with __syncwarp().
 __device__ __forceinline__ void siftUpWarp(HeapItemDev *H, uint32_t hole, const HeapItemDev &value, int lane)
@@ -147,34 +133,10 @@ __device__ __forceinline__ HeapItemDev shflItem(const HeapItemDev &it, int src)
     return r;
 }
 
-// std::pop_heap(H, H + hs) by one thread: __pop_heap -> __adjust_heap -> __push_heap.
-__device__ inline void popHeapSerial(HeapItemDev *H, uint32_t hs)
-{
-    if (hs <= 1) return;
-    const uint32_t len = hs - 1;
-    const HeapItemDev value = ldItem(H + len);
-    uint32_t hole = 0, second = 0;
-    while (second < (len - 1) / 2) {
-        second = 2 * (second + 1);
-        const HeapItemDev r = ldItem(H + second), l = ldItem(H + second - 1);
-        if (r.f < l.f) {
-            --second;
-            stItem(H + hole, l);
-        } else
-            stItem(H + hole, r);
-        hole = second;
-    }
-    if ((len & 1u) == 0 && second == (len - 2) / 2) {
-        second = 2 * (second + 1);
-        stItem(H + hole, ldItem(H + second - 1));
-        hole = second - 1;
-    }
-    siftUp(H, hole, value);
-}
-
-// The same pop by the whole warp.  Per step the hole's 2 + 4 + 8 + 16 descendants of the next four levels are loaded by
-// lanes 0..29 (lane (2^j - 2) + i holds descendant i of level j), the walk "larger child, ties to the right" is resolved
-// with shuffles, and the chosen items are stored one level up — the moves __adjust_heap makes, four levels at a time.
+// std::pop_heap(H, H + hs) (__pop_heap -> __adjust_heap -> __push_heap) by the whole warp.  Per step the hole's
+// 2 + 4 + 8 + 16 descendants of the next four levels are loaded by lanes 0..29 (lane (2^j - 2) + i holds descendant i
+// of level j), the walk "larger child, ties to the right" is resolved with shuffles, and the chosen items are stored
+// one level up — the moves __adjust_heap makes, four levels at a time.
 __device__ inline void popHeapWarp(HeapItemDev *H, uint32_t hs, int lane)
 {
     if (hs <= 1) return;
@@ -495,10 +457,7 @@ __global__ void __launch_bounds__(kAstarWarps * 32) k6_astar_search(SearchArgs a
             const HeapItemDev top = ldItem(H);
             ++touched;  // :750
             __syncwarp();
-            if (a.popLookahead)
-                popHeapWarp(H, hs, lane);
-            else if (lane == 0)
-                popHeapSerial(H, hs);
+            popHeapWarp(H, hs, lane);
             --hs;
             __syncwarp();
             uint32_t v, depth;
@@ -538,17 +497,10 @@ __global__ void __launch_bounds__(kAstarWarps * 32) k6_astar_search(SearchArgs a
             if (total == 0) { status = SEARCH_STALE_LIST; break; }
             if (depth < a.maxDepth) {  // :820
                 const AdjDev *list = a.adj + (size_t)v * a.cap;
-                bool overflow = false;
-                if (a.staged) {
-                    overflow = !expandStaged(a, H, hs, pushes, list, total, nc, cutoff, bits, simTo, c0, c1, ni, sStage, sList, lane);
-                } else {
-                    for (uint32_t base = 0; base < total; base += 32) {
-                        bool hidden = false;
-                        if (!pushBatchGlobal(a, H, hs, pushes, list, total, nc, cutoff, bits, simTo, c0, c1, ni, base, lane, hidden)) { overflow = true; break; }
-                        if (hidden) break;  // predicted entries are in position order: everything behind is hidden too
-                    }
+                if (!expandStaged(a, H, hs, pushes, list, total, nc, cutoff, bits, simTo, c0, c1, ni, sStage, sList, lane)) {
+                    status = SEARCH_HEAP_OVERFLOW;
+                    break;
                 }
-                if (overflow) { status = SEARCH_HEAP_OVERFLOW; break; }
                 if (budget && pushes > budget) { status = SEARCH_BUDGET; break; }
             }
         }

@@ -618,52 +618,19 @@ __global__ void __launch_bounds__(64) k2_fivept_first_solution(WaveArgs a, int o
 }
 
 // ---------------------------------------------------------------------------------------------
-// K4: minimal solves of the fallback.  One thread per (wave pair, iteration of the current chunk).
+// K4: minimal solves of the fallback, one per (wave pair, iteration of the current chunk).
 // The uniform sampler's sequence depends on N only (persistent-pool partial Fisher-Yates driven by
 // cv::RNG(0), SURVEY App. B.5), so the samples come from a per-N table built at registration.
-// ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128, 4) k4_fallback_solve(WaveArgs a, int chunk)
-{
-    const uint32_t g = blockIdx.x * blockDim.x + threadIdx.x;
-    const uint32_t w = g / kFbChunk, j = g % kFbChunk;
-    if (w >= a.n) return;
-    const SlotState &s = a.state[w];
-    if (!(s.flags & ST_FB_ACTIVE)) return;
-    const int it = chunk * kFbChunk + (int)j;
-    if (it >= s.maxIters) return;
-    const uint32_t pid = a.pairId[w];
-    const double4 *rows = reinterpret_cast<const double4 *>(a.corr) + a.offset[pid];
-    const uint32_t *smp = a.samplerTab + ((size_t)s.tableIdx * a.fbMaxIters + it) * 5;
-    double x1[10], x2[10];
-#pragma unroll
-    for (int i = 0; i < 5; i++) {
-        const double4 c = rows[smp[i]];
-        x1[2 * i] = c.x; x1[2 * i + 1] = c.y; x2[2 * i] = c.z; x2[2 * i + 1] = c.w;
-    }
-    double *out = a.fbSols + ((size_t)w * kFbChunk + j) * 90;
-    const int n = fivePoint<false>(x1, x2, out, 10, kDkMaxSweeps, kDkTolSq);
-    a.fbCounts[(size_t)w * kFbChunk + j] = (uint8_t)n;
-    float4 *outF = a.fbSolsF + ((size_t)w * kFbChunk + j) * 30;
-    for (int q = 0; q < n; q++) {
-        const double *e = out + q * 9;
-        outF[q * 3 + 0] = make_float4((float)e[0], (float)e[1], (float)e[2], (float)e[3]);
-        outF[q * 3 + 1] = make_float4((float)e[4], (float)e[5], (float)e[6], (float)e[7]);
-        outF[q * 3 + 2] = make_float4((float)e[8], 0.f, 0.f, 0.f);
-    }
-}
-
-
-// ---------------------------------------------------------------------------------------------
-// K4 as three kernels (the default): the Durand-Kerner root solve is ~45 % of a minimal solve and its sweep count
-// differs from polynomial to polynomial, so with one thread per solve a warp runs as long as its slowest lane
-// (17 of 32 lanes active in the sweeps of k4_fallback_solve).  Here
+// The Durand-Kerner root solve is ~45 % of a minimal solve and its sweep count differs from polynomial to
+// polynomial, so with one thread per solve a warp runs as long as its slowest lane (17 of 32 lanes active in the
+// sweeps, measured).  K4 is therefore three kernels:
 //   K4a  one thread per (pair, iteration): sample -> null space -> elimination -> polynomial; parks EE (36), b (39),
 //        c (11) and the degree in the slot's 90-double solution record and appends the slot to a work list;
 //   K4b  persistent lanes: every lane pulls the next polynomial from the list the moment its current one has
 //        converged (register-resident roots, the same dkSweep sequence per polynomial) -> roots into the slot's
 //        FP32-record area (20 doubles);
 //   K4c  one thread per (pair, iteration): roots -> essential matrices, overwriting the parked data with the
-//        solutions + their FP32 copies, exactly what k4_fallback_solve leaves behind.
+//        solutions (9 doubles each, as fivePoint() returns them) and their FP32 copies for K5.
 // Per polynomial the arithmetic is the same sequence of operations as fivePoint(): bit-identical solutions.
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ bool k4SlotActive(const WaveArgs &a, int chunk, uint32_t g, uint32_t &w, uint32_t &j)
@@ -676,10 +643,7 @@ __device__ __forceinline__ bool k4SlotActive(const WaveArgs &a, int chunk, uint3
     return chunk * kFbChunk + (int)j < s.maxIters;
 }
 
-#ifndef PGI_K4A_MINB
-#define PGI_K4A_MINB 4
-#endif
-__global__ void __launch_bounds__(128, PGI_K4A_MINB) k4a_polynomial(WaveArgs a, int chunk)
+__global__ void __launch_bounds__(128, 4) k4a_polynomial(WaveArgs a, int chunk)
 {
     const uint32_t g = blockIdx.x * blockDim.x + threadIdx.x;
     uint32_t w, j;
@@ -1382,10 +1346,7 @@ __device__ __forceinline__ void k5Body(const WaveArgs &a, int chunk, int lastChu
     }
 }
 
-#ifndef PGI_K5_MINB
-#define PGI_K5_MINB 3
-#endif
-__global__ void __launch_bounds__(kCtaThreads, PGI_K5_MINB) k5_fallback_score(WaveArgs a, int chunk, int lastChunk, uint32_t smemPts)
+__global__ void __launch_bounds__(kCtaThreads, 3) k5_fallback_score(WaveArgs a, int chunk, int lastChunk, uint32_t smemPts)
 {
     extern __shared__ float4 sPts[];  // smemPts float4 slots (FP32 copy of the pair's correspondences)
     const uint32_t w = blockIdx.x;
@@ -1453,14 +1414,11 @@ __device__ inline void decomposeVoteBlock(const double E[9], const double4 *rows
 // integer counts, so merging them through global atomics is exact.  The last CTA of a pair to arrive picks the
 // first maximum, converts to a unit quaternion and packs the 160-byte verdict.
 // ---------------------------------------------------------------------------------------------
-#ifndef PGI_K3_MINB
-#define PGI_K3_MINB 2
-#endif
 #ifndef PGI_K3_THREADS
 #define PGI_K3_THREADS 256
 #endif
 constexpr int kK3Threads = PGI_K3_THREADS;
-__global__ void __launch_bounds__(kK3Threads, PGI_K3_MINB) k3_decompose_vote(WaveArgs a, uint32_t split)
+__global__ void __launch_bounds__(kK3Threads, 2) k3_decompose_vote(WaveArgs a, uint32_t split)
 {
     const uint32_t w = blockIdx.x / split, part = blockIdx.x % split;
     if (w >= a.n) return;

@@ -8,4 +8,3 @@ timeout 1500 python -m pytest tests -m gpu -x -q --deselect tests/test_gpu_astar
 for args in "300 1024 44850 host" "300 1024 44850 gpu" "1000 1024 60000 host" "1000 1024 60000 gpu" "1000 4096 60000 gpu"; do
   timeout 600 python scripts/astar_bench.py $args 2>&1 | tail -1 | tee -a gpurun_out/astar_bench_a.jsonl
 done
-PGI_ASTAR_POP=0 timeout 600 python scripts/astar_bench.py 1000 1024 60000 gpu 2>&1 | tail -1 | tee -a gpurun_out/astar_bench_a.jsonl

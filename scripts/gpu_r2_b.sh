@@ -15,8 +15,8 @@ except Exception as e:
     print("no json", e); print(open("gpurun_out/$name.err").read()[-2000:])
 P
 }
-run cfg2_host PGI_GPU_SEARCH=0 python bench.py --config cfg2_300v --steps 2 --warmup 1 --cpu-sample 256
-run cfg2_gpu256 PGI_GPU_SEARCH=1 python bench.py --config cfg2_300v --steps 2 --warmup 1 --cpu-sample 256
-run cfg2_gpu1024 PGI_GPU_SEARCH=1 python bench.py --config cfg2_300v --steps 2 --warmup 1 --cpu-sample 256 --wave 1024
-run cfg2_gpu4096 PGI_GPU_SEARCH=1 python bench.py --config cfg2_300v --steps 2 --warmup 1 --cpu-sample 256 --wave 4096
-run cfg3_gpu2048 PGI_GPU_SEARCH=1 python bench.py --config cfg3_1000v --steps 1 --warmup 1 --cpu-sample 256 --wave 2048
+run cfg2_host python bench.py --config cfg2_300v --steps 2 --warmup 1 --cpu-sample 256
+run cfg2_gpu256 python bench.py --config cfg2_300v --steps 2 --warmup 1 --cpu-sample 256
+run cfg2_gpu1024 python bench.py --config cfg2_300v --steps 2 --warmup 1 --cpu-sample 256 --wave 1024
+run cfg2_gpu4096 python bench.py --config cfg2_300v --steps 2 --warmup 1 --cpu-sample 256 --wave 4096
+run cfg3_gpu2048 python bench.py --config cfg3_1000v --steps 1 --warmup 1 --cpu-sample 256 --wave 2048

@@ -3,9 +3,7 @@ cd $GRAFT_REPO_ROOT
 mkdir -p gpurun_out
 make -C oracle -s 2>&1 | tail -3
 timeout 600 python -m pytest tests/test_gpu_astar.py -x -q 2>&1 | tail -8
-for st in 0 1; do
-  PGI_ASTAR_STAGED=$st timeout 600 python scripts/astar_bench.py 1000 2048 150000 gpu 2>&1 | tail -1 | cut -c1-700
-done
+timeout 600 python scripts/astar_bench.py 1000 2048 150000 gpu 2>&1 | tail -1 | cut -c1-700
 timeout 300 python scripts/astar_bench.py 1000 2048 150000 host 2>&1 | tail -1 | cut -c1-500
 run() { # name, args
   name=$1; shift

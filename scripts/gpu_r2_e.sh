@@ -3,8 +3,8 @@ cd $GRAFT_REPO_ROOT
 mkdir -p gpurun_out
 make -C oracle -s 2>&1 | tail -3
 timeout 600 python -m pytest tests/test_gpu_astar.py -x -q 2>&1 | tail -5
-PGB_HYBRID_SHARE=0.3 timeout 600 python scripts/astar_bench.py 1000 2048 150000 gpu 2>&1 | tail -1 | cut -c1-900
-PGB_HYBRID_SHARE=0.3 timeout 600 python scripts/astar_bench.py 1000 2048 150000 check 2>&1 | tail -1 | cut -c1-500
+timeout 600 python scripts/astar_bench.py 1000 2048 150000 gpu 2>&1 | tail -1 | cut -c1-900
+timeout 600 python scripts/astar_bench.py 1000 2048 150000 check 2>&1 | tail -1 | cut -c1-500
 run() { # name, args
   name=$1; shift
   timeout 1500 python bench.py "$@" > gpurun_out/$name.json 2> gpurun_out/$name.err

@@ -3,7 +3,7 @@ cd $GRAFT_REPO_ROOT
 mkdir -p gpurun_out
 make -C oracle -s 2>&1 | tail -3
 timeout 600 python -m pytest tests/test_gpu_astar.py -x -q 2>&1 | tail -5
-PGB_HYBRID_SHARE=0 timeout 600 python scripts/astar_bench.py 1000 2048 150000 gpu 2>&1 | tail -1 | cut -c1-900
+timeout 600 python scripts/astar_bench.py 1000 2048 150000 gpu 2>&1 | tail -1 | cut -c1-900
 run() { # name, env..., -- args
   name=$1; shift
   timeout 1500 env "$@" > gpurun_out/$name.json 2> gpurun_out/$name.err
@@ -16,6 +16,4 @@ except Exception as e:
     print("no json", e); print(open("gpurun_out/$name.err").read()[-2000:])
 P
 }
-run f_cfg2_w1024_gpuonly PGB_HYBRID_SHARE=0 python bench.py --config cfg2_300v --steps 2 --warmup 1 --wave 1024 --cpu-sample 256 --verify 500 --verify-replay 2000
-run f_cfg3_w2048_gpuonly PGB_HYBRID_SHARE=0 python bench.py --config cfg3_1000v --steps 1 --warmup 1 --wave 2048 --cpu-sample 256
-run f_cfg3_w2048_hybrid PGB_HYBRID_SHARE=0.2 python bench.py --config cfg3_1000v --steps 1 --warmup 1 --wave 2048 --cpu-sample 256 --verify 1000 --verify-replay 20000
+run f_cfg3_w2048_hybrid python bench.py --config cfg3_1000v --steps 1 --warmup 1 --wave 2048 --cpu-sample 256 --verify 1000 --verify-replay 20000

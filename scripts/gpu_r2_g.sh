@@ -14,5 +14,4 @@ except Exception as e:
     print("no json", e); print(open("gpurun_out/$name.err").read()[-2000:])
 P
 }
-run g_cfg3_w2048_gpuonly PGB_HYBRID_SHARE=0 python bench.py --config cfg3_1000v --steps 1 --warmup 0 --wave 2048 --cpu-sample 256
-run g_cfg3_w2048_hybrid PGB_HYBRID_SHARE=0.2 python bench.py --config cfg3_1000v --steps 1 --warmup 0 --wave 2048 --cpu-sample 256 --verify 500 --verify-replay 10000
+run g_cfg3_w2048_hybrid python bench.py --config cfg3_1000v --steps 1 --warmup 0 --wave 2048 --cpu-sample 256 --verify 500 --verify-replay 10000

@@ -2,7 +2,7 @@ cd $GRAFT_REPO_ROOT
 mkdir -p gpurun_out
 make -C oracle -s 2>&1 | tail -3
 timeout 600 python -m pytest tests/test_gpu_astar.py -x -q 2>&1 | tail -5
-PGB_HYBRID_SHARE=0 timeout 600 python scripts/astar_bench.py 1000 2048 150000 check 2>&1 | tail -1 | cut -c1-600
+timeout 600 python scripts/astar_bench.py 1000 2048 150000 check 2>&1 | tail -1 | cut -c1-600
 run() { # name, env..., -- args
   name=$1; shift
   timeout 1500 env "$@" > gpurun_out/$name.json 2> gpurun_out/$name.err
@@ -15,5 +15,4 @@ except Exception as e:
     print("no json", e); print(open("gpurun_out/$name.err").read()[-2000:])
 P
 }
-run i_cfg3_w2048_gpuonly PGB_HYBRID_SHARE=0 python bench.py --config cfg3_1000v --steps 1 --warmup 0 --wave 2048 --cpu-sample 256 --verify 500 --verify-replay 10000
-run i_cfg3_w2048_hybrid PGB_HYBRID_SHARE=0.2 python bench.py --config cfg3_1000v --steps 1 --warmup 0 --wave 2048 --cpu-sample 256
+run i_cfg3_w2048_hybrid python bench.py --config cfg3_1000v --steps 1 --warmup 0 --wave 2048 --cpu-sample 256

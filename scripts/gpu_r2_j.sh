@@ -14,6 +14,6 @@ except Exception as e:
     print("no json", e); print(open("gpurun_out/$name.err").read()[-2000:])
 P
 }
-run j_cfg3_w256_host PGB_HYBRID_SHARE=0.2 python bench.py --config cfg3_1000v --steps 1 --warmup 0 --wave 256 --cpu-sample 64 --host-search
-run j_cfg3_w512_hybrid PGB_HYBRID_SHARE=0.2 python bench.py --config cfg3_1000v --steps 1 --warmup 0 --wave 512 --cpu-sample 64 --search-min-batch 128
-run j_cfg3_w512_host PGB_HYBRID_SHARE=0.2 python bench.py --config cfg3_1000v --steps 1 --warmup 0 --wave 512 --cpu-sample 64 --host-search
+run j_cfg3_w256_host python bench.py --config cfg3_1000v --steps 1 --warmup 0 --wave 256 --cpu-sample 64 --host-search
+run j_cfg3_w512_hybrid python bench.py --config cfg3_1000v --steps 1 --warmup 0 --wave 512 --cpu-sample 64 --search-min-batch 128
+run j_cfg3_w512_host python bench.py --config cfg3_1000v --steps 1 --warmup 0 --wave 512 --cpu-sample 64 --host-search

@@ -14,8 +14,7 @@ except Exception as e:
     print("no json", e); print(open("gpurun_out/$name.err").read()[-2000:])
 P
 }
-run k_cfg2_tma1 PGI_K1_TMA=1 python bench.py --config cfg2_300v --steps 2 --warmup 1
-run k_cfg2_tma0 PGI_K1_TMA=0 python bench.py --config cfg2_300v --steps 2 --warmup 1
+run k_cfg2_tma1 python bench.py --config cfg2_300v --steps 2 --warmup 1
 run k_cfg1 X=1 python bench.py --config cfg1_50v --steps 2 --warmup 1 --verify 0 --dump-tuples gpurun_out/tuples_cfg1_50v.npz
 run k_cfg4 X=1 python bench.py --config cfg4_sparse --steps 2 --warmup 1 --verify 0 --dump-tuples gpurun_out/tuples_cfg4_sparse.npz
 run k_cfg3 X=1 python bench.py --config cfg3_1000v --steps 2 --warmup 1 --verify 4000 --verify-replay 30000

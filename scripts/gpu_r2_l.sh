@@ -3,28 +3,3 @@ mkdir -p gpurun_out
 make -C oracle -s 2>&1 | tail -3
 timeout 600 python -m pytest tests/test_gpu_matcher.py -x -q 2>&1 | tail -40
 timeout 900 python scripts/diag_tuples.py cfg4_sparse 2>&1 | tail -40
-for v in 0 1 2; do
-  PGB_EXPAND=$v timeout 600 python scripts/astar_bench.py 1000 256 150000 host 2>&1 | tail -1 | python -c "import json,sys; d=json.loads(sys.stdin.read()); print('expand $v', d['sec_astar'], d['astar_runs'], d['pushes'])"
-done
-for v in 0 2; do
-  PGB_EXPAND=$v timeout 900 python bench.py --config cfg3_1000v --steps 1 --warmup 0 --cpu-sample 64 > gpurun_out/l_cfg3_expand$v.json 2> gpurun_out/l_cfg3_expand$v.err
-  python - <<P
-import json
-d=json.load(open("gpurun_out/l_cfg3_expand$v.json"))
-print("expand $v", d["ms_per_step"], d["host_counters"]["sec_astar"], d["host_counters"]["astar_runs"], d["host_s_per_step"])
-P
-done
-PGI_K1_TMA=1 timeout 600 ncu --set full --clock-control none --import-source on -k regex:k1_score_hypotheses_tma -s 3 -c 1 -o gpurun_out/prof_k1_tma python - <<P
-import numpy as np, sys
-sys.path.insert(0, ".")
-from pose_graph_initialization_b200 import Engine
-rng = np.random.default_rng(0)
-n, N = 8192, 2000
-corr = rng.uniform(-0.5, 0.5, (n * N, 4))
-eng = Engine(device=0)
-eng.register_pairs(corr, np.arange(n + 1, dtype=np.uint64) * N, np.full(n, 5e-4))
-ident = np.tile(np.array([0.0, 0.0, 0.0, 1.0, 1.0, 0.0, 0.0]), (n, 1))
-for _ in range(5):
-    eng.run_wave(np.arange(n, dtype=np.uint32), np.arange(n + 1, dtype=np.uint32), ident, flags=1)
-print(eng.stats()["ms_score"])
-P

@@ -15,6 +15,5 @@ except Exception as e:
     print("no json", e); print(open("gpurun_out/$name.err").read()[-2000:])
 P
 }
-run m_cfg2_tma1 PGI_K1_TMA=1 python bench.py --config cfg2_300v --steps 2 --warmup 1
-run m_cfg2_tma0 PGI_K1_TMA=0 python bench.py --config cfg2_300v --steps 2 --warmup 1
+run m_cfg2_tma1 python bench.py --config cfg2_300v --steps 2 --warmup 1
 run m_cfg4 X=1 python bench.py --config cfg4_sparse --steps 2 --warmup 1 --verify 0

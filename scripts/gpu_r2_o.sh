@@ -14,6 +14,4 @@ except Exception as e:
 P
 }
 run o_cfg3_floor X=1 python bench.py --config cfg3_1000v --steps 1 --warmup 1 --cpu-sample 512 --verify 0
-run o_cfg3_nofloor PGB_FLOOR_MARGIN=-1 python bench.py --config cfg3_1000v --steps 1 --warmup 0 --cpu-sample 64 --verify 0
-run o_cfg3_m005 PGB_FLOOR_MARGIN=0.005 python bench.py --config cfg3_1000v --steps 1 --warmup 0 --cpu-sample 64 --verify 0
 run o_cfg2_floor X=1 python bench.py --config cfg2_300v --steps 2 --warmup 1 --verify 0

@@ -3,11 +3,10 @@ mkdir -p gpurun_out
 make -C oracle -s 2>&1 | tail -3
 timeout 600 python -m pytest tests -m gpu -q 2>&1 | tail -5
 cp pose_graph_initialization_b200/libpgi.so /tmp/libpgi_A.so
-TAG=A PGI_K1_TMA=1 timeout 120 python scripts/k1_probe.py 2>&1 | tail -1
-TAG=A PGI_K1_TMA=0 timeout 120 python scripts/k1_probe.py 2>&1 | tail -1
+TAG=A timeout 120 python scripts/k1_probe.py 2>&1 | tail -1
 for v in B C D; do
   cp gpurun_variants/libpgi_$v.so pose_graph_initialization_b200/libpgi.so
-  TAG=$v PGI_K1_TMA=1 timeout 120 python scripts/k1_probe.py 2>&1 | tail -1
+  TAG=$v timeout 120 python scripts/k1_probe.py 2>&1 | tail -1
 done
 cp /tmp/libpgi_A.so pose_graph_initialization_b200/libpgi.so
 run() { # name, env..., -- args

@@ -1,6 +1,6 @@
 """K1 throughput probe: 8 192 pairs x 2 000 correspondences (524 MB of FP64 rows, larger than L2), one hypothesis per
-pair, PATH-only waves; prints the scoring time per wave (CUDA events inside the engine) and GB/s.
-PGI_K1_TMA=0/1 selects the direct-load / streaming kernel."""
+pair, PATH-only waves without byte masks, so K1 runs in its streaming form; prints the scoring time per wave (CUDA events
+inside the engine) and GB/s."""
 import json
 import os
 import sys
@@ -24,5 +24,5 @@ reps = 10
 for _ in range(reps):
     eng.run_wave(ids, hoff, ident, flags=1)
 ms = eng.stats()["ms_score"] / reps
-print(json.dumps(dict(tag=os.environ.get("TAG", ""), tma=os.environ.get("PGI_K1_TMA", "1"), ms_per_wave=ms, gbs=n * N * 32 / ms / 1e6,
+print(json.dumps(dict(tag=os.environ.get("TAG", ""), ms_per_wave=ms, gbs=n * N * 32 / ms / 1e6,
                       frac_of_6453=n * N * 32 / ms / 1e6 / 6453.7)))

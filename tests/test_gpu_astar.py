@@ -17,10 +17,8 @@ CFG = dict(similarity_threshold=0.0, minimum_inlier_number=20, minimum_point_num
            traversal_heuristics_weight=0.8, use_path_finding=True)
 
 
-def _run(engine, sc, wave, backend, check, n_corr=2000, max_positions=None, pop=None):
+def _run(engine, sc, wave, backend, check, n_corr=2000, max_positions=None):
     os.environ["PGB_SEARCH_CHECK"] = "1" if check else "0"
-    if pop is not None:
-        os.environ["PGI_ASTAR_POP"] = str(pop)
     host = B.HostBuilder(sc, host_threads=4, lazy_fallback=False, **CFG)
     if backend:
         host.set_search_backend(engine, min_batch=1)
@@ -28,15 +26,14 @@ def _run(engine, sc, wave, backend, check, n_corr=2000, max_positions=None, pop=
     out = host.log().copy(), host.edges().copy(), host.counters()
     host.close()
     os.environ.pop("PGB_SEARCH_CHECK", None)
-    os.environ.pop("PGI_ASTAR_POP", None)
     return out
 
 
-@pytest.mark.parametrize("views,wave,decimals,pop", [(40, 64, 3, 1), (40, 64, 3, 0), (120, 512, 3, 1), (120, 2048, 1, 1), (90, 300, 2, 0)])
-def test_device_search_equals_host_search(engine, views, wave, decimals, pop):
+@pytest.mark.parametrize("views,wave,decimals", [(40, 64, 3), (64, 128, 1), (120, 512, 3), (120, 2048, 1), (90, 300, 2)])
+def test_device_search_equals_host_search(engine, views, wave, decimals):
     sc = dense_scene(views, seed=views + decimals, decimals=decimals)
     hlog, hedges, hc = _run(engine, sc, wave, backend=False, check=False)
-    glog, gedges, gc = _run(engine, sc, wave, backend=True, check=True, pop=pop)
+    glog, gedges, gc = _run(engine, sc, wave, backend=True, check=True)
     assert gc["gpu_searches"] > 0
     assert gc["search_mismatches"] == 0
     assert gc["gpu_search_redo"] == 0
