@@ -97,6 +97,10 @@ typedef struct pgi_stats {
     uint64_t match_rows;        /* matches K9 produced                                */
     double ms_guided;           /* K7 guided matching (pgi_guided_match, pgi_guided_match_views) */
     uint64_t guided_calls;      /* K7 launches timed in ms_guided                     */
+    double ms_guided_pairs;     /* K10 batched guided matching (pgi_guided_match_pairs, all chunks) */
+    uint64_t guided_pairs;      /* pairs matched by K10                               */
+    uint64_t guided_dist_evals; /* K10 descriptor distances computed                  */
+    uint64_t guided_chunks;     /* K10 chunks run (scratch is bounded per chunk)      */
 } pgi_stats;
 
 const char *pgi_version(void);
@@ -265,6 +269,19 @@ pgi_status pgi_guided_match(pgi_ctx *ctx, uint32_t n_src, const float *kp_src, c
  * allocation after the first calls and no descriptor copy.  PGI_ERR_STATE without a scene or without descriptors. */
 pgi_status pgi_guided_match_views(pgi_ctx *ctx, uint32_t src, uint32_t dst, const double *pose_q_t, int32_t bin_number,
                                   uint32_t max_points, uint32_t *matches_out, double *values_out, uint32_t *n_out);
+
+/* guidedMatching (pose_graph_builder.h:717-783) for n_pairs cases of the registered scene in one call (K10, spread over the
+ * whole GPU).  pair_views[n][2] (src, dst); poses_q_t[n][7] T_dst_src; bin_number as pgi_guided_match_views.
+ * max_points > 0: pair k's rows are exactly what pgi_guided_match_views(src, dst, pose, bin_number, max_points) returns.
+ * max_points == 0: match()'s rows and adapted ratios, as pgi_guided_match returns them.
+ * offsets_out[n+1]; matches_out[capacity_rows][2] (src idx, dst idx); values_out[capacity_rows]: pair k's rows are
+ * offsets_out[k] .. offsets_out[k+1] - 1.  capacity_rows >= sum_k (max_points ? min(n_src(k), max_points) : n_src(k)), else
+ * PGI_ERR_INVALID before any work; so is a view of more than 16384 keypoints in the batch.  Device scratch is bounded per
+ * chunk of pairs (512 MB); only the final rows are copied to the host.  PGI_ERR_STATE without a scene, without descriptors
+ * or while a wave is in flight. */
+pgi_status pgi_guided_match_pairs(pgi_ctx *ctx, uint64_t n_pairs, const uint32_t *pair_views, const double *poses_q_t,
+                                  int32_t bin_number, uint32_t max_points, uint64_t *offsets_out,
+                                  uint32_t *matches_out, double *values_out, uint64_t capacity_rows);
 
 /* ---- brute-force descriptor matching (K8) ------------------------------------------------------------------
  * matchFeatures (feature_utils.h:103-210) without its HDF5 cache: BRUTEFORCE_SL2 2-NN in both directions, ratio test

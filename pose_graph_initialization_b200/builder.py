@@ -510,17 +510,20 @@ class PoseGraphBuilder:
         self.gpu_search_min_batch = int(gpu_search_min_batch)
         self.prefetch_streams = int(prefetch_streams)
         self.timing = {}
+        self.graph = None
+        self._desc_resident = False
 
     # -- engine + registration (H2D inside, counted by the engine's stats) -----------------------------------
     def prepare(self):
         if self.engine is None:
             self.engine = _engine.Engine(device=self.device, min_inliers=self.min_inliers)
         registered = False
+        self._desc_resident = False
         if self.world == 1:
             sub = self.scene
             if needs_matching(sub):  # keypoints + descriptors only: matchFeatures on the device, registered in the same call
                 self.engine.register_scene_descriptors(sub, self.thr_px)
-                registered = True
+                registered = self._desc_resident = True
         else:
             # the rank's shard is cut once (a 32 GB scene's shard is gigabytes: not something to copy on every registration)
             if getattr(self, "_sub", None) is None:
@@ -534,6 +537,7 @@ class PoseGraphBuilder:
             self.engine.register_scene(sub, self.thr_px)
             if self.hashing:  # a scene that came with matches: guided matching still needs its descriptors on the device
                 self.engine.set_scene_descriptors(sub["desc"])
+                self._desc_resident = True
         self.prepared = True
         if self.overlap:
             if self.engine_fb is None:
@@ -816,7 +820,33 @@ class PoseGraphBuilder:
         self.log = host.log()
         self.counters = host.counters()
         self.search_stats = self.engine.search_stats() if self.gpu_search else {}
-        return PoseGraph(len(self.scene["focal"]), edges)
+        self.graph = PoseGraph(len(self.scene["focal"]), edges)
+        return self.graph
+
+    def guided_match_edges(self, graph=None, max_points=None, bin_number=45):
+        """guidedMatching (pose_graph_builder.h:717-783) for every edge of `graph` (default: the last run()'s), each with
+        its own (q, t) as T_dst_src, in the graph's edge order, in one device call (K10) on the scene's resident keypoints
+        and descriptors -> (offsets [E + 1] u64, matches [M, 2] u32 (src idx, dst idx), values [M] f64); edge k's rows are
+        offsets[k]:offsets[k + 1].  max_points=None is kMaximumPointNumberForEpipolarHashing_, 0 gives all of match()'s
+        rows with their adapted ratios."""
+        if "desc" not in self.scene:
+            raise ValueError("guided matching needs a scene with descriptors (desc)")
+        if self.world > 1:
+            raise ValueError("guided_match_edges runs on one GPU (world_size must be 1)")
+        if graph is None:
+            graph = getattr(self, "graph", None)
+        if graph is None:
+            raise ValueError("no pose graph: call run() first or pass graph=")
+        if self.engine is None or not getattr(self, "prepared", False):
+            self.prepare()
+        if not self._desc_resident:  # a scene that came with matches: its descriptors go to the device once
+            self.engine.set_scene_descriptors(self.scene["desc"])
+            self._desc_resident = True
+        e = graph.edges
+        pv = np.stack([e["src"], e["dst"]], 1).astype(np.uint32)
+        poses = np.concatenate([e["q"], e["t"]], 1) if len(e) else np.zeros((0, 7))
+        mp = self.max_points_hashing if max_points is None else int(max_points)
+        return self.engine.guided_match_pairs(pv, poses, bin_number, mp)
 
     def _run_hashing(self):
         """The exact sequential epipolar-hashing loop (pgb_run_hashing) with the engine's own entry points."""
@@ -840,4 +870,5 @@ class PoseGraphBuilder:
         self.match_sources = host.match_sources()
         self.counters = host.counters()
         self.search_stats = {}
-        return PoseGraph(len(self.scene["focal"]), edges)
+        self.graph = PoseGraph(len(self.scene["focal"]), edges)
+        return self.graph

@@ -18,6 +18,7 @@
 #include "pgi_kernels.cuh"
 #include "pgi_astar.cuh"
 #include "pgi_matcher.cuh"
+#include "pgi_guided_batch.cuh"
 #include "pgi_features.cuh"
 #include "pgi_match_scene.cuh"
 #include "pgi_nvtx.h"
@@ -222,6 +223,9 @@ struct pgi_ctx {
     std::vector<uint32_t> guidedM;
     std::vector<double> guidedR;
     std::vector<uint32_t> guidedOrder;
+    DevBuf<unsigned char> guidedBatch;  // pgi_guided_match_pairs: K10 scratch of one chunk
+    std::vector<GuidedPairIn> guidedIn;
+    std::vector<uint64_t> guidedOff;
     const Registration *reg = &own;  // own, or the owner's after pgi_share_pairs
     // wave buffers
     DevSlots slots;
@@ -1427,6 +1431,168 @@ pgi_status pgi_guided_match_views(pgi_ctx *ctx, uint32_t src, uint32_t dst, cons
         }
         *n_out = n;
     }
+    return PGI_OK;
+}
+
+pgi_status pgi_guided_match_pairs(pgi_ctx *ctx, uint64_t n_pairs, const uint32_t *pair_views, const double *poses_q_t,
+                                  int32_t bin_number, uint32_t max_points, uint64_t *offsets_out,
+                                  uint32_t *matches_out, double *values_out, uint64_t capacity_rows)
+{
+    PgiNvtxRange nvtxRange("pgi:guided_match_pairs (K10 on the resident scene)");
+    if (!ctx) return PGI_ERR_INVALID;
+    if (ctx->inFlight) { ctx->err = "a wave is in flight"; return PGI_ERR_STATE; }
+    const SceneStaging &sc = ctx->scene;
+    if (!sc.staged) { ctx->err = "pgi_guided_match_pairs needs a scene registration first"; return PGI_ERR_STATE; }
+    if (!sc.hasDesc) {
+        ctx->err = "the registered scene has no descriptors (pgi_register_scene_descriptors or pgi_set_scene_descriptors)";
+        return PGI_ERR_STATE;
+    }
+    if (!offsets_out || (n_pairs && (!pair_views || !poses_q_t)) || bin_number > kMatchMaxBins) {
+        ctx->err = "bad argument";
+        return PGI_ERR_INVALID;
+    }
+    const uint64_t V = sc.hFocal.size();
+    uint64_t need = 0;
+    uint32_t maxS = 0, maxD = 0;
+    for (uint64_t p = 0; p < n_pairs; p++) {
+        const uint32_t src = pair_views[2 * p], dst = pair_views[2 * p + 1];
+        if (src >= V || dst >= V) { ctx->err = "view id out of range"; return PGI_ERR_INVALID; }
+        const uint64_t nS = sc.hKpOff[src + 1] - sc.hKpOff[src], nD = sc.hKpOff[dst + 1] - sc.hKpOff[dst];
+        if (nS > kK10MaxKp || nD > kK10MaxKp) {
+            ctx->err = "batched guided matching supports at most 16384 keypoints per view";
+            return PGI_ERR_INVALID;
+        }
+        need += max_points ? std::min<uint64_t>(nS, max_points) : nS;
+        maxS = std::max<uint32_t>(maxS, (uint32_t)nS);
+        maxD = std::max<uint32_t>(maxD, (uint32_t)nD);
+    }
+    if (need > capacity_rows) { ctx->err = "capacity_rows is below the rows the batch can produce"; return PGI_ERR_INVALID; }
+    if (need && (!matches_out || !values_out)) { ctx->err = "null argument"; return PGI_ERR_INVALID; }
+    CK(cudaSetDevice(ctx->cfg.device));
+    offsets_out[0] = 0;
+    if (n_pairs == 0) return PGI_OK;
+    cudaStream_t s = ctx->stream;
+
+    // K10 per chunk of pairs: every per-pair array is sized for the batch's largest views, the chunk for 512 MB
+    const uint32_t strideS = std::max<uint32_t>(maxS, 1), strideD = std::max<uint32_t>(maxD, 1);
+    const uint32_t dstBlocks = (strideD + kK10DstBlock - 1) / kK10DstBlock;
+    const uint32_t rowCap = max_points ? std::min(strideS, max_points) : strideS;
+    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    const size_t perPair = sizeof(GuidedPairIn) + sizeof(GuidedPairDev) + (size_t)strideD * 5 + (size_t)dstBlocks * kMatchMaxBins * 4 +
+                           (size_t)strideS * (4 + 8 + 8 + 8) + 4 + 8 + (size_t)rowCap * 16;
+    const size_t kScratchBudget = (size_t)512 << 20;
+    const uint64_t chunk = std::max<uint64_t>(1, std::min<uint64_t>({kScratchBudget / perPair, 65535, n_pairs}));
+    const size_t oIn = 0, oDev = oIn + al(chunk * sizeof(GuidedPairIn)), oBin = oDev + al(chunk * sizeof(GuidedPairDev)),
+                 oList = oBin + al(chunk * strideD), oBlk = oList + al(chunk * strideD * 4),
+                 oCand = oBlk + al(chunk * dstBlocks * kMatchMaxBins * 4), oRatio = oCand + al(chunk * strideS * 4),
+                 oSM = oRatio + al(chunk * strideS * 8), oSV = oSM + al(chunk * strideS * 8), oCnt = oSV + al(chunk * strideS * 8),
+                 oOff = oCnt + al(chunk * 4), oRM = oOff + al((chunk + 1) * 8), oRV = oRM + al(chunk * rowCap * 8),
+                 oEv = oRV + al(chunk * rowCap * 8), total = oEv + 256;
+    CK(ctx->guidedBatch.grow(total));
+    unsigned char *d = ctx->guidedBatch.data();
+    GuidedScratch g;
+    g.in = reinterpret_cast<const GuidedPairIn *>(d + oIn);
+    g.dev = reinterpret_cast<GuidedPairDev *>(d + oDev);
+    g.binOfD = d + oBin;
+    g.binList = reinterpret_cast<uint32_t *>(d + oList);
+    g.blockOff = reinterpret_cast<uint32_t *>(d + oBlk);
+    g.cand = reinterpret_cast<uint32_t *>(d + oCand);
+    g.candRatio = reinterpret_cast<double *>(d + oRatio);
+    g.stageM = reinterpret_cast<uint2 *>(d + oSM);
+    g.stageV = reinterpret_cast<double *>(d + oSV);
+    g.counts = reinterpret_cast<uint32_t *>(d + oCnt);
+    g.strideS = strideS; g.strideD = strideD; g.dstBlocks = dstBlocks;
+    uint64_t *d_off = reinterpret_cast<uint64_t *>(d + oOff);
+    uint2 *d_rowsM = reinterpret_cast<uint2 *>(d + oRM);
+    double *d_rowsV = reinterpret_cast<double *>(d + oRV);
+    unsigned long long *d_evals = reinterpret_cast<unsigned long long *>(d + oEv);
+    uint32_t sortCap = 0;
+    if (max_points) {
+        sortCap = 1;
+        while (sortCap < strideS) sortCap <<= 1;
+    }
+    const size_t selectSmem = (size_t)sortCap * (8 + 2);
+    CK(cudaFuncSetAttribute(k10_select, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)selectSmem));
+    CK(cudaMemsetAsync(d_evals, 0, 8, s));
+    CK(cudaMemsetAsync(d_off, 0, 8, s));
+    std::vector<GuidedPairIn> &hin = ctx->guidedIn;
+    std::vector<uint64_t> &hoff = ctx->guidedOff;
+    float msTotal = 0;
+    uint64_t base = 0, chunks = 0;
+    for (uint64_t c0 = 0; c0 < n_pairs; c0 += chunk) {
+        const uint32_t cp = (uint32_t)std::min<uint64_t>(chunk, n_pairs - c0);
+        hin.resize(cp);
+        uint32_t sBlocks = 0, dBlocks = 0;
+        for (uint32_t k = 0; k < cp; k++) {
+            const uint32_t src = pair_views[2 * (c0 + k)], dst = pair_views[2 * (c0 + k) + 1];
+            GuidedPairIn &in = hin[k];
+            memset(&in, 0, sizeof in);
+            essentialOfPose(poses_q_t + 7 * (c0 + k), in.E);
+            // K = [f 0 w/2; 0 f h/2; 0 0 1] of each view (pose_graph_builder.h:284-286), as pgi_guided_match_views builds it
+            const double fS = sc.hFocal[src], wS = sc.hSize[2 * src], hS = sc.hSize[2 * src + 1];
+            const double fD = sc.hFocal[dst], wD = sc.hSize[2 * dst], hD = sc.hSize[2 * dst + 1];
+            const double Ks[9] = {fS, 0.0, wS / 2.0, 0.0, fS, hS / 2.0, 0.0, 0.0, 1.0};
+            const double Kd[9] = {fD, 0.0, wD / 2.0, 0.0, fD, hD / 2.0, 0.0, 0.0, 1.0};
+            memcpy(in.Ks, Ks, sizeof Ks);
+            memcpy(in.Kd, Kd, sizeof Kd);
+            in.wS = (int)wS; in.hS = (int)hS; in.wD = (int)wD; in.hD = (int)hD; in.binNumber = bin_number;
+            in.kS0 = sc.hKpOff[src]; in.kD0 = sc.hKpOff[dst];
+            in.nS = (uint32_t)(sc.hKpOff[src + 1] - in.kS0); in.nD = (uint32_t)(sc.hKpOff[dst + 1] - in.kD0);
+            sBlocks = std::max<uint32_t>(sBlocks, (in.nS + kK10SrcPerCta - 1) / kK10SrcPerCta);
+            dBlocks = std::max<uint32_t>(dBlocks, (in.nD + kK10DstBlock - 1) / kK10DstBlock);
+        }
+        CK(cudaMemcpyAsync(d + oIn, hin.data(), (size_t)cp * sizeof(GuidedPairIn), cudaMemcpyHostToDevice, s));
+        ctx->stats.h2d_bytes += (size_t)cp * sizeof(GuidedPairIn);
+        CK(cudaEventRecord(ctx->evStart, s));
+        {
+            PgiNvtxRange chunkRange("pgi:k10 chunk");
+            k10_prepare<<<(cp + 63) / 64, 64, 0, s>>>(g, cp);
+            if (dBlocks) {
+                k10_bin_count<<<dim3(dBlocks, cp), kK10DstBlock, 0, s>>>(g, sc.kp.data());
+                k10_bin_offsets<<<cp, kMatchMaxBins, 0, s>>>(g);
+                k10_bin_scatter<<<dim3(dBlocks, cp), kK10DstBlock, 0, s>>>(g);
+                ctx->stats.launches += 3;
+            }
+            if (sBlocks) {
+                if (sc.dim == 128)
+                    k10_match<128><<<dim3(sBlocks, cp), kK10Threads, 0, s>>>(g, sc.kp.data(), sc.desc.data(), d_evals);
+                else
+                    k10_match<64><<<dim3(sBlocks, cp), kK10Threads, 0, s>>>(g, sc.kp.data(), sc.desc.data(), d_evals);
+                ctx->stats.launches += 1;
+            }
+            k10_select<<<cp, kK10SelectThreads, selectSmem, s>>>(g, max_points, sortCap);
+            k9_offsets<<<1, 1024, 0, s>>>(g.counts, cp, d_off, 0);
+            k10_scatter<<<cp, 256, 0, s>>>(g, d_off, d_rowsM, d_rowsV);
+            ctx->stats.launches += 4;
+        }
+        CK(cudaEventRecord(ctx->evK1, s));
+        CK(cudaGetLastError());
+        hoff.resize(cp + 1);
+        CK(cudaMemcpyAsync(hoff.data(), d_off, (size_t)(cp + 1) * 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        const uint64_t rows = hoff[cp];
+        if (rows > capacity_rows - base) { ctx->err = "K10 produced more rows than its bound"; return PGI_ERR_CUDA; }
+        for (uint32_t k = 0; k < cp; k++) offsets_out[c0 + k + 1] = base + hoff[k + 1];
+        if (rows) {
+            CK(cudaMemcpyAsync(matches_out + 2 * base, d_rowsM, rows * 8, cudaMemcpyDeviceToHost, s));
+            CK(cudaMemcpyAsync(values_out + base, d_rowsV, rows * 8, cudaMemcpyDeviceToHost, s));
+            CK(cudaStreamSynchronize(s));
+        }
+        float ms = 0;
+        CK(cudaEventElapsedTime(&ms, ctx->evStart, ctx->evK1));
+        msTotal += ms;
+        ctx->stats.d2h_bytes += (size_t)(cp + 1) * 8 + rows * 16;
+        base += rows;
+        chunks++;
+    }
+    unsigned long long evals = 0;
+    CK(cudaMemcpyAsync(&evals, d_evals, 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    ctx->stats.d2h_bytes += 8;
+    ctx->stats.ms_guided_pairs += msTotal;
+    ctx->stats.guided_pairs += n_pairs;
+    ctx->stats.guided_dist_evals += evals;
+    ctx->stats.guided_chunks += chunks;
     return PGI_OK;
 }
 

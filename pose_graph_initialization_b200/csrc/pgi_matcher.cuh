@@ -13,6 +13,8 @@
 //           against 0.75^2, then the 128-D squared descriptor distance (float differences accumulated in double,
 //           matcher.h:371-375), best / second best, count-corrected Lowe ratio (matcher.h:386-406);
 //   phase 4: accepted matches are compacted in source order (block scan).
+// The preparation (guidedPrepare), the bins, the epipolar gate, the descriptor distance, the best / second-best step
+// (pgi_guided_nn.h) and the count-corrected ratio are device functions that K10 (pgi_guided_batch.cuh) calls too.
 // atan2 is evaluated in double-double arithmetic and rounded once (pgi_atan2.h): the correctly rounded value, which is
 // what glibc returns for all but ~2.5e-4 of arguments (CUDA's own atan2 is a 2-ulp function and differed from the host
 // in the angular range of one of five test scenes).
@@ -22,6 +24,7 @@
 #include <cuda_runtime.h>
 
 #include "pgi_atan2.h"
+#include "pgi_guided_nn.h"
 #include "pgi_math.cuh"
 
 namespace pgi {
@@ -82,65 +85,141 @@ PGI_DEV int binOfAngle(double angle, double minAngle, double angularRange, int b
     return lo < binNumber - 1 ? lo : binNumber - 1;
 }
 
+// The per-pair preparation (matcher.h:218-277): F = Kd^-T E Ks^-1, the epipole from the 3x3 Jacobi SVD of F, the angular
+// range from the destination image's corners, the bin count.  K7 and K10 both run it on one thread per pair.
+struct GuidedPrep {
+    double F[9];
+    double ex, ey, minAngle, range;
+    int binsRaw;  // binNumber, or the angular range's integer part for binNumber <= 0
+    int bins;     // binsRaw clamped to [0, kMatchMaxBins]: the bins the kernels use (0: no match)
+};
+
+PGI_DEV void guidedPrepare(const double *E, const double *Ks, const double *Kd, int wS, int hS, int wD, int hD, int binNumber,
+                           GuidedPrep &p)
+{
+    double KdInv[9], KsInv[9], KdInvT[9], T[9];
+    inverse3(Kd, KdInv);
+    inverse3(Ks, KsInv);
+    for (int i = 0; i < 3; i++)
+        for (int j = 0; j < 3; j++) KdInvT[i * 3 + j] = KdInv[j * 3 + i];
+    mul3(KdInvT, E, T);
+    mul3(T, KsInv, p.F);
+    double U[1], V[9], S[3];
+    eigenJacobiSvd<3, false, true>(p.F, U, V, S);
+    const double *F = p.F;
+    const double ez = V[8];
+    const double ex = V[2] / ez, ey = V[5] / ez;
+    const bool inImage = ex >= 0 && ex < wS && ey >= 0 && ey < hS;
+    double minAngle = 180, maxAngle = 0;
+    if (!inImage) {
+        const double corners[8] = {0, 0, (double)wD, 0, (double)wD, (double)hD, 0, (double)hD};
+        for (int c = 0; c < 8; c += 2) {
+            const double x = corners[c], y = corners[c + 1];
+            const double nx = F[0] * x + F[3] * y + F[6];
+            const double ny = F[1] * x + F[4] * y + F[7];
+            const double angle = lineAngle(ny, nx);
+            minAngle = minAngle < angle ? minAngle : angle;
+            maxAngle = maxAngle > angle ? maxAngle : angle;
+        }
+    }
+    p.ex = ex; p.ey = ey;
+    p.minAngle = minAngle;
+    p.range = maxAngle - minAngle;
+    p.binsRaw = binNumber <= 0 ? (int)p.range : binNumber;
+    p.bins = p.binsRaw < 0 ? 0 : (p.binsRaw > kMatchMaxBins ? kMatchMaxBins : p.binsRaw);
+}
+
+// bin of destination keypoint (x, y): the angle of its epipolar line's normal (matcher.h:285-299)
+PGI_DEV int guidedDestinationBin(const double *F, double x, double y, double minAngle, double range, int bins)
+{
+    const double nx = F[0] * x + F[3] * y + F[6];
+    const double ny = F[1] * x + F[4] * y + F[7];
+    return binOfAngle(lineAngle(ny, nx), minAngle, range, bins);
+}
+
+// bin of source keypoint (x1, y1): the angle of its ray from the epipole (matcher.h:333-345)
+PGI_DEV int guidedSourceBin(double x1, double y1, double ex, double ey, double minAngle, double range, int bins)
+{
+    const double vx = x1 - ex, vy = y1 - ey;
+    return binOfAngle(lineAngle(vx, -vy), minAngle, range, bins);
+}
+
+// squared symmetric epipolar distance (FP64, matcher.h:351-360)
+PGI_DEV double guidedEpipolarSq(const double *F, double x1, double y1, double x2, double y2)
+{
+    const double rxc = F[0] * x2 + F[3] * y2 + F[6];
+    const double ryc = F[1] * x2 + F[4] * y2 + F[7];
+    const double rwc = F[2] * x2 + F[5] * y2 + F[8];
+    const double r = (x1 * rxc + y1 * ryc + rwc);
+    const double rx = F[0] * x1 + F[1] * y1 + F[2];
+    const double ry = F[3] * x1 + F[4] * y1 + F[5];
+    const double a1 = rxc * rxc + ryc * ryc;
+    const double b1 = rx * rx + ry * ry;
+    return r * r * (a1 + b1) / (a1 * b1);
+}
+
+// the gate of matcher.h:362, literally: a NaN distance passes it
+PGI_DEV bool guidedIsCandidate(double d2) { return !(d2 >= 0.75 * 0.75); }
+
+// squared descriptor distance: float differences widened to double, accumulated in dimension order (matcher.h:371-375)
+PGI_DEV double guidedDescriptorSq(const float *ds, const float *dd, uint32_t dim)
+{
+    double acc = 0;
+    for (uint32_t m = 0; m < dim; m++) {
+        const double dist = (double)(ds[m] - dd[m]);  // float subtraction, widened (matcher.h:373)
+        acc += dist * dist;
+    }
+    return acc;
+}
+
+// count-corrected Lowe ratio (matcher.h:386-399) of a source keypoint's final scan state
+PGI_DEV double guidedAdaptedRatio(const GuidedNn &s)
+{
+    double corr = 1.0;
+    if (s.count < 20) corr = 0.65 * 0.65;
+    if (s.count < 10) corr = 0.6 * 0.6;
+    if (s.count < 5) corr = 0.5 * 0.5;
+    if (s.count < 3) corr = 0.25 * 0.25;
+    return (s.best / s.second) / corr;
+}
+
+// acceptance (matcher.h:400-406)
+PGI_DEV bool guidedAccepted(const GuidedNn &s, double adapted)
+{
+    bool ok = false;
+    if (!(adapted < 0.00001)) ok = s.bestIndex > -1 && ((adapted < 0.8 * 0.8) || (s.count == 1));
+    return ok;
+}
+
 __global__ void __launch_bounds__(kMatchThreads) k7_guided_match(MatchArgs a)
 {
-    __shared__ double sF[9], sEpi[2], sMinAngle, sRange;
-    __shared__ int sBins;
+    __shared__ GuidedPrep sP;
     __shared__ uint32_t sBinStart[kMatchMaxBins + 1], sBinCount[kMatchMaxBins];
     __shared__ uint32_t sScan[kMatchThreads / 32], sTotal;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (threadIdx.x == 0) {
-        double KdInv[9], KsInv[9], KdInvT[9], T[9], F[9];
-        inverse3(a.Kd, KdInv);
-        inverse3(a.Ks, KsInv);
-        for (int i = 0; i < 3; i++)
-            for (int j = 0; j < 3; j++) KdInvT[i * 3 + j] = KdInv[j * 3 + i];
-        mul3(KdInvT, a.E, T);
-        mul3(T, KsInv, F);
-        double U[1], V[9], S[3];
-        eigenJacobiSvd<3, false, true>(F, U, V, S);
-        const double ez = V[8];
-        const double ex = V[2] / ez, ey = V[5] / ez;
-        const bool inImage = ex >= 0 && ex < a.wS && ey >= 0 && ey < a.hS;
-        double minAngle = 180, maxAngle = 0;
-        if (!inImage) {
-            const double corners[8] = {0, 0, (double)a.wD, 0, (double)a.wD, (double)a.hD, 0, (double)a.hD};
-            for (int c = 0; c < 8; c += 2) {
-                const double x = corners[c], y = corners[c + 1];
-                const double nx = F[0] * x + F[3] * y + F[6];
-                const double ny = F[1] * x + F[4] * y + F[7];
-                const double angle = lineAngle(ny, nx);
-                minAngle = minAngle < angle ? minAngle : angle;
-                maxAngle = maxAngle > angle ? maxAngle : angle;
-            }
-        }
-        for (int k = 0; k < 9; k++) sF[k] = F[k];
-        sEpi[0] = ex; sEpi[1] = ey;
-        sMinAngle = minAngle;
-        sRange = maxAngle - minAngle;
-        int bins = a.binNumber <= 0 ? (int)sRange : a.binNumber;
-        sBins = bins < 0 ? 0 : (bins > kMatchMaxBins ? kMatchMaxBins : bins);
+        GuidedPrep p;
+        guidedPrepare(a.E, a.Ks, a.Kd, a.wS, a.hS, a.wD, a.hD, a.binNumber, p);
+        sP = p;
         if (a.prepOut) {
-            for (int k = 0; k < 9; k++) a.prepOut[k] = F[k];
-            a.prepOut[9] = ex; a.prepOut[10] = ey; a.prepOut[11] = minAngle; a.prepOut[12] = sRange; a.prepOut[13] = bins;
+            for (int k = 0; k < 9; k++) a.prepOut[k] = p.F[k];
+            a.prepOut[9] = p.ex; a.prepOut[10] = p.ey; a.prepOut[11] = p.minAngle; a.prepOut[12] = p.range; a.prepOut[13] = p.binsRaw;
         }
     }
     for (int b = threadIdx.x; b < kMatchMaxBins; b += kMatchThreads) sBinCount[b] = 0;
     __syncthreads();
-    const int bins = sBins;
+    const int bins = sP.bins;
     if (bins <= 0) {
         if (threadIdx.x == 0) *a.nOut = 0;
         return;
     }
-    const double F0 = sF[0], F1 = sF[1], F2 = sF[2], F3 = sF[3], F4 = sF[4], F5 = sF[5], F6 = sF[6], F7 = sF[7], F8 = sF[8];
-    const double minAngle = sMinAngle, range = sRange;
+    double F[9];
+    for (int k = 0; k < 9; k++) F[k] = sP.F[k];
+    const double minAngle = sP.minAngle, range = sP.range;
     // ---- phase 1: bin of every destination keypoint
     for (uint32_t i = threadIdx.x; i < a.nD; i += kMatchThreads) {
         const float2 p = a.kpD[i];
-        const double x = p.x, y = p.y;
-        const double nx = F0 * x + F3 * y + F6;
-        const double ny = F1 * x + F4 * y + F7;
-        const int b = binOfAngle(lineAngle(ny, nx), minAngle, range, bins);
+        const int b = guidedDestinationBin(F, p.x, p.y, minAngle, range, bins);
         a.binOfD[i] = (uint8_t)b;
         atomicAdd(&sBinCount[b], 1u);
     }
@@ -167,43 +246,17 @@ __global__ void __launch_bounds__(kMatchThreads) k7_guided_match(MatchArgs a)
     for (uint32_t i = threadIdx.x; i < a.nS; i += kMatchThreads) {
         const float2 p = a.kpS[i];
         const double x1 = p.x, y1 = p.y;
-        const double vx = x1 - sEpi[0], vy = y1 - sEpi[1];
-        const int bin = binOfAngle(lineAngle(vx, -vy), minAngle, range, bins);
-        double second = DBL_MAX, best = DBL_MAX;
-        int bestIndex = -1, countSnn = 0;
+        const int bin = guidedSourceBin(x1, y1, sP.ex, sP.ey, minAngle, range, bins);
+        GuidedNn s = guidedEmpty();
         const float *ds = a.dS + (size_t)i * a.dim;
         for (uint32_t k = sBinStart[bin]; k < sBinStart[bin + 1]; k++) {
             const uint32_t nb = a.binList[k];
             const float2 q = a.kpD[nb];
-            const double x2 = q.x, y2 = q.y;
-            const double rxc = F0 * x2 + F3 * y2 + F6;
-            const double ryc = F1 * x2 + F4 * y2 + F7;
-            const double rwc = F2 * x2 + F5 * y2 + F8;
-            const double r = (x1 * rxc + y1 * ryc + rwc);
-            const double rx = F0 * x1 + F1 * y1 + F2;
-            const double ry = F3 * x1 + F4 * y1 + F5;
-            const double a1 = rxc * rxc + ryc * ryc;
-            const double b1 = rx * rx + ry * ry;
-            const double d2 = r * r * (a1 + b1) / (a1 * b1);
-            if (d2 >= 0.75 * 0.75) continue;
-            countSnn += 1;
-            const float *dd = a.dD + (size_t)nb * a.dim;
-            double acc = 0;
-            for (uint32_t m = 0; m < a.dim; m++) {
-                const double dist = (double)(ds[m] - dd[m]);  // float subtraction, widened (matcher.h:373)
-                acc += dist * dist;
-            }
-            if (acc < best) { second = best; best = acc; bestIndex = (int)nb; }
+            if (!guidedIsCandidate(guidedEpipolarSq(F, x1, y1, q.x, q.y))) continue;
+            guidedPush(s, guidedDescriptorSq(ds, a.dD + (size_t)nb * a.dim, a.dim), (int32_t)nb);
         }
-        double corr = 1.0;
-        if (countSnn < 20) corr = 0.65 * 0.65;
-        if (countSnn < 10) corr = 0.6 * 0.6;
-        if (countSnn < 5) corr = 0.5 * 0.5;
-        if (countSnn < 3) corr = 0.25 * 0.25;
-        const double adapted = (best / second) / corr;
-        bool ok = false;
-        if (!(adapted < 0.00001)) ok = bestIndex > -1 && ((adapted < 0.8 * 0.8) || (countSnn == 1));
-        a.cand[i] = ok ? (uint32_t)bestIndex : 0xffffffffu;
+        const double adapted = guidedAdaptedRatio(s);
+        a.cand[i] = guidedAccepted(s, adapted) ? (uint32_t)s.bestIndex : 0xffffffffu;
         a.candRatio[i] = adapted;
     }
     __syncthreads();

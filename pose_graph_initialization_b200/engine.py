@@ -37,7 +37,9 @@ class PgiStats(C.Structure):
                 ("ms_total", C.c_double), ("launches", C.c_uint64), ("pairs", C.c_uint64), ("corr_evals", C.c_uint64),
                 ("fallback_pairs", C.c_uint64), ("fallback_models", C.c_uint64), ("h2d_bytes", C.c_uint64),
                 ("d2h_bytes", C.c_uint64), ("ms_match", C.c_double), ("dist_evals", C.c_uint64), ("match_pairs", C.c_uint64),
-                ("match_rows", C.c_uint64), ("ms_guided", C.c_double), ("guided_calls", C.c_uint64)]
+                ("match_rows", C.c_uint64), ("ms_guided", C.c_double), ("guided_calls", C.c_uint64),
+                ("ms_guided_pairs", C.c_double), ("guided_pairs", C.c_uint64), ("guided_dist_evals", C.c_uint64),
+                ("guided_chunks", C.c_uint64)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
@@ -50,7 +52,7 @@ EXPORTS = [
     "pgi_guided_match", "pgi_match_features", "pgi_get_stats", "pgi_reset_stats", "pgi_dbg_sampson",
     "pgi_dbg_five_point", "pgi_dbg_pose_from_essential", "pgi_dbg_fp64_peak", "pgi_register_scene_descriptors",
     "pgi_read_scene_matches", "pgi_set_scene_descriptors", "pgi_register_extra_pairs", "pgi_read_extra_pair",
-    "pgi_guided_match_views",
+    "pgi_guided_match_views", "pgi_guided_match_pairs",
 ]
 
 _lib = None
@@ -128,6 +130,7 @@ class Engine:
         self.n_pairs = 0
         self.offset = None
         self.extra_offset = None
+        self._kp_offset = None
         self._wave_n = 0
         self._wave_rows = 0
 
@@ -165,6 +168,7 @@ class Engine:
         self._ck(self.lib.pgi_register_scene(self.h, C.c_uint64(len(focal)), _ptr(focal), _ptr(size), _ptr(kpo), _ptr(kp),
                                              C.c_uint64(len(pv)), _ptr(pv), _ptr(mo), _ptr(mt), C.c_double(thr_px)))
         self.n_pairs, self.offset = len(pv), mo.copy()
+        self._kp_offset = kpo.copy()
 
     def register_scene_descriptors(self, scene, thr_px=0.4):
         """matchFeatures for every pair of `scene` on the device (K9), then the registration of register_scene from the
@@ -182,6 +186,7 @@ class Engine:
                                                          _ptr(kp), _ptr(desc), C.c_uint32(desc.shape[1]), C.c_uint64(len(pv)),
                                                          _ptr(pv), C.c_double(thr_px), _ptr(mo)))
         self.n_pairs, self.offset = len(pv), mo.copy()
+        self._kp_offset = kpo.copy()
         matches, ratios = self.read_scene_matches(int(mo[-1]))
         scene["m_offset"], scene["matches"], scene["ratios"] = mo, matches, ratios
         return mo
@@ -356,6 +361,28 @@ class Engine:
                                                  C.c_uint32(max_points), _ptr(m), _ptr(r), C.byref(n)))
         k = int(n.value)
         return [(int(m[i, 0]), int(m[i, 1]), float(r[i])) for i in range(k)]
+
+    def guided_match_pairs(self, pair_views, poses, bin_number=45, max_points=100):
+        """guidedMatching (pose_graph_builder.h:717-783) for every (src, dst) row of pair_views [n, 2] with the pose of the
+        same row of poses [n, 7] (T_dst_src) in one device call (K10) on the registered scene -> (offsets [n + 1] u64,
+        matches [M, 2] u32 (src idx, dst idx), values [M] f64): pair k's rows are offsets[k]:offsets[k + 1], those of
+        guided_match_views(src, dst, pose, bin_number, max_points); max_points=0 gives match()'s rows and adapted ratios."""
+        pv = np.ascontiguousarray(pair_views, dtype=np.uint32).reshape(-1, 2)
+        poses = _f64(poses).reshape(-1, 7)
+        if len(poses) != len(pv):
+            raise ValueError("poses must have one row (qx qy qz qw tx ty tz) per pair")
+        # the capacity from the registered keypoint counts (the library itself rejects a missing scene or a bad view id)
+        n_kp = np.diff(self._kp_offset.astype(np.int64)) if self._kp_offset is not None else np.zeros(0, dtype=np.int64)
+        src = pv[:, 0].astype(np.int64)
+        n_src = n_kp[src[src < len(n_kp)]]
+        cap = int(np.minimum(n_src, max_points).sum() if max_points else n_src.sum())
+        off = np.zeros(len(pv) + 1, dtype=np.uint64)
+        m = np.zeros((max(cap, 1), 2), dtype=np.uint32)
+        v = np.zeros(max(cap, 1))
+        self._ck(self.lib.pgi_guided_match_pairs(self.h, C.c_uint64(len(pv)), _ptr(pv), _ptr(poses), C.c_int32(bin_number),
+                                                 C.c_uint32(max_points), _ptr(off), _ptr(m), _ptr(v), C.c_uint64(cap)))
+        k = int(off[-1])
+        return off, m[:k].copy(), v[:k].copy()
 
     def match_features(self, desc_src, desc_dst):
         """matchFeatures (feature_utils.h:103-210) on the device: -> (matches [n, 2] (queryIdx, trainIdx), ratios [n]),

@@ -11,6 +11,7 @@ ValueError on shape errors.
     matches, ratios = ppg.match_features(desc1, desc2)                   # matchFeatures                  feature_utils.h:103-210
     tracks = ppg.Tracklets(n_views); tracks.add(i, j, matches, mask)    # reconstruction::Tracklets      point_track.h:541-712
     graph = ppg.PoseGraphBuilder(**flags, scene=scene).run()            # PoseGraphBuilder::run           PGB:173-239
+    offsets, matches, values = builder.guided_match_edges()             # guidedMatching on every edge    PGB:717-783
     # a scene with keypoint descriptors (scene.make_descriptor_scene) and no matches is matched on the device first
 
 Everything runs on the sm_100a engine through the C-ABI (include/pgi.h, include/pgb.h); there is no CPU path."""
