@@ -95,8 +95,8 @@ typedef struct pgi_stats {
     uint64_t dist_evals;        /* K9 descriptor distances (each pair's n_src x n_dst once) */
     uint64_t match_pairs;       /* pairs matched by K9                                */
     uint64_t match_rows;        /* matches K9 produced                                */
-    double ms_guided;           /* K7 guided matching (pgi_guided_match, pgi_guided_match_views) */
-    uint64_t guided_calls;      /* K7 launches timed in ms_guided                     */
+    double ms_guided;           /* single-pair guided matching (K10: pgi_guided_match, pgi_guided_match_views) */
+    uint64_t guided_calls;      /* single-pair calls timed in ms_guided               */
     double ms_guided_pairs;     /* K10 batched guided matching (pgi_guided_match_pairs, all chunks) */
     uint64_t guided_pairs;      /* pairs matched by K10                               */
     uint64_t guided_dist_evals; /* K10 descriptor distances computed                  */
@@ -141,8 +141,8 @@ pgi_status pgi_register_scene_descriptors(pgi_ctx *ctx, uint64_t n_views, const 
 pgi_status pgi_read_scene_matches(pgi_ctx *ctx, uint32_t *matches_out, double *ratios_or_null, uint64_t capacity_rows);
 
 /* Descriptors for a scene registered with pgi_register_scene (which keeps none): desc[sum K][dim] float, row-aligned with
- * that registration's kp_xy, dim 64 or 128, every value finite (PGI_ERR_INVALID otherwise).  They stay resident for
- * pgi_guided_match_views.  PGI_ERR_STATE before any scene registration. */
+ * that registration's kp_xy, dim 64 or 128, every value finite, at most 16384 keypoints per view (PGI_ERR_INVALID
+ * otherwise).  They stay resident for pgi_guided_match_views.  PGI_ERR_STATE before any scene registration. */
 pgi_status pgi_set_scene_descriptors(pgi_ctx *ctx, const float *desc, uint32_t dim);
 
 /* Pairs whose matches the caller supplies (the quick matches the Tracklets hand out, pose_graph_builder.h:492-520), built
@@ -246,12 +246,14 @@ pgi_status pgi_graph_search(pgi_ctx *ctx, uint32_t n, const pgi_query *queries, 
                             pgi_search_result *results, uint32_t *expanded_bits);
 pgi_status pgi_graph_stats(pgi_ctx *ctx, pgi_search_stats *out, int32_t reset);
 
-/* ---- epipolar-hashing guided matcher (K7) ----------------------------------------------------------------
+/* ---- epipolar-hashing guided matcher (K10) ---------------------------------------------------------------
  * HashingBasedMatcherWithPose<false, 45>::match (matcher.h:199-405), the matcher PoseGraphBuilder::guidedMatching runs
  * on an accepted pair (pose_graph_builder.h:717-783): keypoints of the destination image are hashed by the angle of
  * their epipolar line, every source keypoint searches its bin for the descriptor nearest neighbour among the points
  * within 0.75 px symmetric epipolar distance, count-corrected Lowe ratio.  kp_*: n x 2 float pixels (cv::KeyPoint.pt),
- * desc_*: n x dim float; pose_q_t: T_dst_src; K_*: 3x3 row-major intrinsics; size_*: width, height.
+ * desc_*: n x dim float (dim 64 or 128, else PGI_ERR_INVALID); pose_q_t: T_dst_src; K_*: 3x3 row-major intrinsics;
+ * size_*: width, height.  Any number of keypoints: the pair runs as a batch of one of pgi_guided_match_pairs without
+ * the selection.
  * matches_out (capacity n_src x 2: source index, destination index, in source order) and ratios_out (capacity n_src)
  * receive match()'s output, *n_out their number.  The top-`maximum_points` selection of guidedMatching is host work on
  * that list (pose_graph_builder.h:760-782).  prepared_or_null: 14 doubles (F, epipole, min angle, range, bins). */
@@ -261,7 +263,7 @@ pgi_status pgi_guided_match(pgi_ctx *ctx, uint32_t n_src, const float *kp_src, c
                             int32_t bin_number, uint32_t *matches_out, double *ratios_out, uint32_t *n_out,
                             double *prepared_or_null);
 
-/* PoseGraphBuilder::guidedMatching (pose_graph_builder.h:717-783) of views src -> dst of the registered scene: K7 on the
+/* PoseGraphBuilder::guidedMatching (pose_graph_builder.h:717-783) of views src -> dst of the registered scene: K10 on the
  * device-resident keypoints and descriptors (pgi_register_scene_descriptors or pgi_set_scene_descriptors), K = [f 0 w/2;
  * 0 f h/2; 0 0 1] of each view, then the selection of :760-782.  matches_out (capacity max_points x 2) and values_out
  * (capacity max_points) receive the selected rows: the max_points smallest (value, index) entries in ascending order if
@@ -276,18 +278,20 @@ pgi_status pgi_guided_match_views(pgi_ctx *ctx, uint32_t src, uint32_t dst, cons
  * max_points == 0: match()'s rows and adapted ratios, as pgi_guided_match returns them.
  * offsets_out[n+1]; matches_out[capacity_rows][2] (src idx, dst idx); values_out[capacity_rows]: pair k's rows are
  * offsets_out[k] .. offsets_out[k+1] - 1.  capacity_rows >= sum_k (max_points ? min(n_src(k), max_points) : n_src(k)), else
- * PGI_ERR_INVALID before any work; so is a view of more than 16384 keypoints in the batch.  Device scratch is bounded per
+ * PGI_ERR_INVALID before any work; so is, with max_points > 0, a view of more than 16384 keypoints.  Device scratch is bounded per
  * chunk of pairs (512 MB); only the final rows are copied to the host.  PGI_ERR_STATE without a scene, without descriptors
  * or while a wave is in flight. */
 pgi_status pgi_guided_match_pairs(pgi_ctx *ctx, uint64_t n_pairs, const uint32_t *pair_views, const double *poses_q_t,
                                   int32_t bin_number, uint32_t max_points, uint64_t *offsets_out,
                                   uint32_t *matches_out, double *values_out, uint64_t capacity_rows);
 
-/* ---- brute-force descriptor matching (K8) ------------------------------------------------------------------
+/* ---- brute-force descriptor matching (K9 on one pair) -------------------------------------------------------
  * matchFeatures (feature_utils.h:103-210) without its HDF5 cache: BRUTEFORCE_SL2 2-NN in both directions, ratio test
  * best/second < 0.90 on the squared distances, mutual nearest neighbour, survivors sorted by the ratio.
- * desc_*: n x dim float descriptors (dim 128 or 64).  matches_out (capacity n_src x 2: queryIdx, trainIdx) and ratios_out
- * (capacity n_src) receive the rows the reference appends to `matches_` (:196-204), *n_out their number. */
+ * desc_*: n x dim float descriptors (dim 128 or 64, at most 16384 per side, every value finite: PGI_ERR_INVALID
+ * otherwise).  A row whose distances all overflow has no neighbour and no match.  matches_out (capacity n_src x 2:
+ * queryIdx, trainIdx) and ratios_out (capacity n_src) receive the rows the reference appends to `matches_` (:196-204),
+ * *n_out their number.  The registered scene is left as it is. */
 pgi_status pgi_match_features(pgi_ctx *ctx, uint32_t n_src, const float *desc_src, uint32_t n_dst, const float *desc_dst,
                               uint32_t dim, uint32_t *matches_out, double *ratios_out, uint32_t *n_out);
 

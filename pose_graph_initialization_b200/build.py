@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libpgi.so")
 SOURCES = ["pgi_api.cu", "pgb_host.cpp"]  # pgb_host.cpp includes pgb_tracklets.cpp
-DEPS = ["pgi_api.cu", "pgi_kernels.cuh", "pgi_math.cuh", "pgi_astar.cuh", "pgi_matcher.cuh", "pgi_guided_batch.cuh", "pgi_guided_nn.h", "pgi_features.cuh", "pgi_match_scene.cuh", "pgi_nn2.h", "pgi_atan2.h", "pgi_nvtx.h", "pgb_host.cpp", "pgb_tracklets.cpp", os.path.join("..", "..", "include", "pgi.h"),
+DEPS = ["pgi_api.cu", "pgi_kernels.cuh", "pgi_math.cuh", "pgi_astar.cuh", "pgi_matcher.cuh", "pgi_guided_batch.cuh", "pgi_guided_nn.h", "pgi_match_scene.cuh", "pgi_nn2.h", "pgi_atan2.h", "pgi_nvtx.h", "pgb_host.cpp", "pgb_tracklets.cpp", os.path.join("..", "..", "include", "pgi.h"),
         os.path.join("..", "..", "include", "pgb.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-std=c++17", "-O3", "-lineinfo", "-fmad=false",
               "-Xcompiler", "-fPIC,-O3,-ffp-contract=off,-pthread", "-shared"]

@@ -19,7 +19,6 @@
 #include "pgi_astar.cuh"
 #include "pgi_matcher.cuh"
 #include "pgi_guided_batch.cuh"
-#include "pgi_features.cuh"
 #include "pgi_match_scene.cuh"
 #include "pgi_nvtx.h"
 
@@ -134,25 +133,13 @@ struct FallbackScratch {
     DevBuf<uint32_t> dkList, dkCtl;  // work list of K4b (K4a -> K4b -> K4c)
 };
 
-// The compact inputs of the last scene registration. Kept between registrations: cudaMalloc / cudaFree of GB-sized
-// buffers costs up to hundreds of milliseconds and synchronises the device.
-struct SceneStaging {
-    DevBuf<double> focal, size;
+// What K9 (matchPairs) reads and writes: descriptors, keypoint offsets and pair views of the views it matches, its
+// per-chunk scratch, and the match list with the ratios beside it.
+struct MatchStaging {
     DevBuf<uint64_t> kpOff;
-    DevBuf<float2> kp;
     DevBuf<uint2> pv, m;
-    // pgi_register_scene_descriptors: resident descriptors, the ratios beside m, the per-chunk scratch of K9
     DevBuf<float> desc, ratio;
     DevBuf<unsigned char> k9Scratch;
-    uint64_t rows = 0;
-    bool matches = false;  // m / ratio hold the matches of the last descriptor registration
-    // what pgi_register_extra_pairs and pgi_guided_match_views read on the host: the last registration's views
-    bool staged = false;   // a scene registration completed its upload
-    bool hasDesc = false;  // desc holds dim floats per keypoint of this scene
-    uint32_t dim = 0;
-    double thrPx = 0.0;
-    std::vector<uint64_t> hKpOff;
-    std::vector<double> hFocal, hSize;
 
     // The match list is the one allocation that grows while it is filled: to max(need, 2 x capacity, 1024) rows,
     // with its first `keep` rows copied over.
@@ -172,6 +159,22 @@ struct SceneStaging {
         ratio = std::move(ratio2);
         return cudaSuccess;
     }
+};
+
+// The compact inputs of the last scene registration. Kept between registrations: cudaMalloc / cudaFree of GB-sized
+// buffers costs up to hundreds of milliseconds and synchronises the device.  The descriptors stay resident for K9 and K10.
+struct SceneStaging : MatchStaging {
+    DevBuf<double> focal, size;
+    DevBuf<float2> kp;
+    uint64_t rows = 0;
+    bool matches = false;  // m / ratio hold the matches of the last descriptor registration
+    // what pgi_register_extra_pairs and pgi_guided_match_views read on the host: the last registration's views
+    bool staged = false;   // a scene registration completed its upload
+    bool hasDesc = false;  // desc holds dim floats per keypoint of this scene
+    uint32_t dim = 0;
+    double thrPx = 0.0;
+    std::vector<uint64_t> hKpOff;
+    std::vector<double> hFocal, hSize;
 };
 
 // K6: device mirror of the pose graph and the per-search slabs (pgi_graph_*). V is 0 until pgi_graph_init built it.
@@ -219,13 +222,11 @@ struct pgi_ctx {
     Registration own, tmp;
     Registration extra;            // pgi_register_extra_pairs: rows built from caller-supplied matches (PGI_WAVE_EXTRA)
     DevBuf<uint2> extraPv, extraM; // their pair views and matches, as K0 reads them
-    DevBuf<unsigned char> guided;  // pgi_guided_match_views: K7 scratch
-    std::vector<uint32_t> guidedM;
-    std::vector<double> guidedR;
-    std::vector<uint32_t> guidedOrder;
-    DevBuf<unsigned char> guidedBatch;  // pgi_guided_match_pairs: K10 scratch of one chunk
+    DevBuf<unsigned char> guidedBatch;  // K10 scratch of one chunk
     std::vector<GuidedPairIn> guidedIn;
     std::vector<uint64_t> guidedOff;
+    MatchStaging pairMatch;             // pgi_match_features: its two views, apart from the registered scene
+    DevBuf<uint64_t> pairMatchOff;
     const Registration *reg = &own;  // own, or the owner's after pgi_share_pairs
     // wave buffers
     DevSlots slots;
@@ -587,21 +588,16 @@ pgi_status buildCorrespondences(pgi_ctx *ctx, Registration &r, double thr_px, co
     return buildTables(ctx, r);
 }
 
-// Uploads the scene's descriptors (nKp x dim, row-aligned with the staged keypoints); they stay resident for K9 and K7.
-// Non-finite values are rejected (a NaN distance never enters a 2-NN, so it would silently drop neighbours).
-pgi_status uploadDescriptors(pgi_ctx *ctx, const float *desc, uint64_t nKp, uint32_t dim)
+// PGI_ERR_INVALID if one of the n device values is not finite (a NaN distance never enters a 2-NN, so it would silently
+// drop neighbours).  Synchronises the stream.
+pgi_status checkFinite(pgi_ctx *ctx, const float *x, uint64_t n)
 {
-    SceneStaging &sc = ctx->scene;
     cudaStream_t s = ctx->stream;
-    sc.hasDesc = false;
-    CK(sc.desc.grow(nKp * dim));
-    if (nKp) CK(cudaMemcpyAsync(sc.desc.data(), desc, nKp * dim * 4, cudaMemcpyHostToDevice, s));
-    ctx->stats.h2d_bytes += nKp * dim * 4;
     uint32_t *d_flag = reinterpret_cast<uint32_t *>(ctx->counters.data());
     uint32_t flag = 0;
     CK(cudaMemsetAsync(d_flag, 0, 4, s));
-    if (nKp) {
-        k9_check_finite<<<(uint32_t)std::min<uint64_t>((nKp * dim + 1023) / 1024, 4 * ctx->numSms), 1024, 0, s>>>(sc.desc.data(), nKp * dim, d_flag);
+    if (n) {
+        k9_check_finite<<<(uint32_t)std::min<uint64_t>((n + 1023) / 1024, 4 * ctx->numSms), 1024, 0, s>>>(x, n, d_flag);
         CK(cudaGetLastError());
         ctx->stats.launches += 1;
     }
@@ -609,6 +605,18 @@ pgi_status uploadDescriptors(pgi_ctx *ctx, const float *desc, uint64_t nKp, uint
     CK(cudaStreamSynchronize(s));
     ctx->stats.d2h_bytes += 4;
     if (flag) { ctx->err = "non-finite descriptor value"; return PGI_ERR_INVALID; }
+    return PGI_OK;
+}
+
+// Uploads the scene's descriptors (nKp x dim, row-aligned with the staged keypoints); they stay resident for K9 and K10.
+pgi_status uploadDescriptors(pgi_ctx *ctx, const float *desc, uint64_t nKp, uint32_t dim)
+{
+    SceneStaging &sc = ctx->scene;
+    sc.hasDesc = false;
+    CK(sc.desc.grow(nKp * dim));
+    if (nKp) CK(cudaMemcpyAsync(sc.desc.data(), desc, nKp * dim * 4, cudaMemcpyHostToDevice, ctx->stream));
+    ctx->stats.h2d_bytes += nKp * dim * 4;
+    if (pgi_status st = checkFinite(ctx, sc.desc.data(), nKp * dim); st != PGI_OK) return st;
     sc.hasDesc = true;
     sc.dim = dim;
     return PGI_OK;
@@ -655,16 +663,229 @@ void essentialOfPose(const double *q, double *E)
         for (int j = 0; j < 3; j++) E[i * 3 + j] = Cx[i * 3 + 0] * R[j] + (Cx[i * 3 + 1] * R[3 + j] + Cx[i * 3 + 2] * R[6 + j]);
 }
 
-// K7's device time (evStart -> evK1 around its launch), after the stream was synchronised.
-cudaError_t addGuidedTime(pgi_ctx *ctx)
-{
+// What a K9 or K10 run took: device time of its chunks (CUDA events), descriptor distances, rows, chunks.
+struct MatchRun {
     float ms = 0;
-    const cudaError_t e = cudaEventElapsedTime(&ms, ctx->evStart, ctx->evK1);
-    if (e == cudaSuccess) {
-        ctx->stats.ms_guided += ms;
-        ctx->stats.guided_calls += 1;
+    uint64_t dist = 0, rows = 0, chunks = 0;
+};
+
+// K9 for the n_pairs pairs staged in st (desc, kpOff, pv; kp_offset and pair_views are the host copies of the last two,
+// maxK the largest view): pair p's rows, sorted by (ratio bits, query), go to st.m / st.ratio at offset[p] .. offset[p + 1]
+// - 1.  The caller sets offset[0] = 0.  Scratch (forward states, backward partials, staged sorted rows) is sized for a
+// chunk of pairs only.
+pgi_status matchPairs(pgi_ctx *ctx, MatchStaging &st, uint32_t dim, uint32_t maxK, uint64_t n_pairs, const uint64_t *kp_offset,
+                      const uint32_t *pair_views, uint64_t *offset, MatchRun &run)
+{
+    cudaStream_t s = ctx->stream;
+    const uint32_t stride = std::max<uint32_t>(maxK, 1), maxSB = (stride + kK9Rows - 1) / kK9Rows;
+    uint32_t keyCap = 1;
+    while (keyCap < stride) keyCap <<= 1;
+    const size_t perPair = (size_t)maxSB * stride * sizeof(Nn2) + (size_t)stride * (sizeof(Nn2) + 8 + 4) + 4;
+    const size_t kScratchBudget = (size_t)512 << 20;
+    const uint64_t chunk = std::max<uint64_t>(1, std::min<uint64_t>({kScratchBudget / perPair, 65535, std::max<uint64_t>(n_pairs, 1)}));
+    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    const size_t oF = 0, oB = oF + al(chunk * stride * sizeof(Nn2)), oM = oB + al(chunk * maxSB * stride * sizeof(Nn2)),
+                 oR = oM + al(chunk * stride * 8), oC = oR + al(chunk * stride * 4), total = oC + al(chunk * 4);
+    CK(st.k9Scratch.grow(total));
+    Nn2 *d_fwd = reinterpret_cast<Nn2 *>(st.k9Scratch.data() + oF), *d_bpart = reinterpret_cast<Nn2 *>(st.k9Scratch.data() + oB);
+    uint2 *d_sm = reinterpret_cast<uint2 *>(st.k9Scratch.data() + oM);
+    float *d_sr = reinterpret_cast<float *>(st.k9Scratch.data() + oR);
+    uint32_t *d_cnt = reinterpret_cast<uint32_t *>(st.k9Scratch.data() + oC);
+    const size_t finishSmem = (size_t)keyCap * 8 + (size_t)stride * 4;
+    CK(cudaFuncSetAttribute(k9_finish, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)finishSmem));
+    for (uint64_t c0 = 0; c0 < n_pairs; c0 += chunk) {
+        const uint32_t cp = (uint32_t)std::min<uint64_t>(chunk, n_pairs - c0);
+        uint32_t sbUsed = 0;
+        for (uint64_t p = c0; p < c0 + cp; p++) {
+            const uint64_t nS = kp_offset[pair_views[2 * p] + 1] - kp_offset[pair_views[2 * p]];
+            const uint64_t nD = kp_offset[pair_views[2 * p + 1] + 1] - kp_offset[pair_views[2 * p + 1]];
+            sbUsed = std::max<uint32_t>(sbUsed, (uint32_t)((nS + kK9Rows - 1) / kK9Rows));
+            run.dist += nS * nD;
+        }
+        CK(cudaEventRecord(ctx->evStart, s));
+        {
+            PgiNvtxRange chunkRange("pgi:k9 chunk");
+            if (sbUsed) {
+                if (dim == 128)
+                    k9_knn2_tile<128><<<dim3(sbUsed, cp), kK9Threads, 0, s>>>(st.desc.data(), st.kpOff.data(), st.pv.data(), c0, stride, maxSB, d_fwd, d_bpart);
+                else
+                    k9_knn2_tile<64><<<dim3(sbUsed, cp), kK9Threads, 0, s>>>(st.desc.data(), st.kpOff.data(), st.pv.data(), c0, stride, maxSB, d_fwd, d_bpart);
+                ctx->stats.launches += 1;
+            }
+            k9_finish<<<cp, kK9FinishThreads, finishSmem, s>>>(st.kpOff.data(), st.pv.data(), c0, stride, keyCap, maxSB, d_fwd, d_bpart, d_cnt, d_sm, d_sr);
+            k9_offsets<<<1, 1024, 0, s>>>(d_cnt, cp, offset, c0);
+            CK(cudaGetLastError());
+            ctx->stats.launches += 2;
+        }
+        uint64_t end = 0;
+        CK(cudaMemcpyAsync(&end, offset + c0 + cp, 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        ctx->stats.d2h_bytes += 8;
+        CK(st.growMatches(end, run.rows, s));
+        k9_scatter<<<cp, 256, 0, s>>>(offset, c0, stride, d_cnt, d_sm, d_sr, st.m.data(), st.ratio.data());
+        CK(cudaEventRecord(ctx->evK1, s));
+        CK(cudaGetLastError());
+        ctx->stats.launches += 1;
+        CK(cudaEventSynchronize(ctx->evK1));
+        float ms = 0;
+        CK(cudaEventElapsedTime(&ms, ctx->evStart, ctx->evK1));
+        run.ms += ms;
+        run.rows = end;
+        run.chunks++;
     }
-    return e;
+    return PGI_OK;
+}
+
+// One guided-matching case of the registered scene: views src -> dst at pose q (T_dst_src), K = [f 0 w/2; 0 f h/2; 0 0 1]
+// of each view (pose_graph_builder.h:284-286).
+GuidedPairIn scenePairIn(const SceneStaging &sc, uint32_t src, uint32_t dst, const double *q, int32_t bin_number)
+{
+    GuidedPairIn in;
+    memset(&in, 0, sizeof in);
+    essentialOfPose(q, in.E);
+    const double fS = sc.hFocal[src], wS = sc.hSize[2 * src], hS = sc.hSize[2 * src + 1];
+    const double fD = sc.hFocal[dst], wD = sc.hSize[2 * dst], hD = sc.hSize[2 * dst + 1];
+    const double Ks[9] = {fS, 0.0, wS / 2.0, 0.0, fS, hS / 2.0, 0.0, 0.0, 1.0};
+    const double Kd[9] = {fD, 0.0, wD / 2.0, 0.0, fD, hD / 2.0, 0.0, 0.0, 1.0};
+    memcpy(in.Ks, Ks, sizeof Ks);
+    memcpy(in.Kd, Kd, sizeof Kd);
+    in.wS = (int)wS; in.hS = (int)hS; in.wD = (int)wD; in.hD = (int)hD; in.binNumber = bin_number;
+    in.kS0 = sc.hKpOff[src]; in.kD0 = sc.hKpOff[dst];
+    in.nS = (uint32_t)(sc.hKpOff[src + 1] - in.kS0); in.nD = (uint32_t)(sc.hKpOff[dst + 1] - in.kD0);
+    return in;
+}
+
+// K10 for the n_pairs cases `in` (host array) on the keypoints kp and the descriptors desc (dim 64 or 128) they index:
+// pair k's rows go to offsets_out[k] .. offsets_out[k + 1] - 1 of matches_out / values_out.  max_points > 0: guidedMatching's
+// selection (pose_graph_builder.h:760-782); 0: match()'s rows and adapted ratios in source order.  Every argument error
+// comes before any device work.  Scratch is sized for the batch's largest views and bounded per chunk of pairs (512 MB).
+// prep_or_null receives the first pair's preparation.
+pgi_status runGuided(pgi_ctx *ctx, const float2 *kp, const float *desc, uint32_t dim, const GuidedPairIn *in, uint64_t n_pairs,
+                     uint32_t max_points, uint64_t *offsets_out, uint32_t *matches_out, double *values_out, uint64_t capacity_rows,
+                     GuidedPrep *prep_or_null, MatchRun &run)
+{
+    uint64_t need = 0;
+    uint32_t maxS = 0, maxD = 0;
+    for (uint64_t p = 0; p < n_pairs; p++) {
+        // the selection sorts 16-bit source indices; without it any view size works
+        if (max_points && (in[p].nS > kK10MaxKp || in[p].nD > kK10MaxKp)) {
+            ctx->err = "batched guided matching supports at most 16384 keypoints per view";
+            return PGI_ERR_INVALID;
+        }
+        need += max_points ? std::min<uint64_t>(in[p].nS, max_points) : in[p].nS;
+        maxS = std::max(maxS, in[p].nS);
+        maxD = std::max(maxD, in[p].nD);
+    }
+    if (need > capacity_rows) { ctx->err = "capacity_rows is below the rows the batch can produce"; return PGI_ERR_INVALID; }
+    if (need && (!matches_out || !values_out)) { ctx->err = "null argument"; return PGI_ERR_INVALID; }
+    CK(cudaSetDevice(ctx->cfg.device));
+    offsets_out[0] = 0;
+    if (n_pairs == 0) return PGI_OK;
+    cudaStream_t s = ctx->stream;
+
+    const uint32_t strideS = std::max<uint32_t>(maxS, 1), strideD = std::max<uint32_t>(maxD, 1);
+    const uint32_t dstBlocks = (strideD + kK10DstBlock - 1) / kK10DstBlock;
+    const uint32_t rowCap = max_points ? std::min(strideS, max_points) : strideS;
+    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    const size_t perPair = sizeof(GuidedPairIn) + sizeof(GuidedPairDev) + (size_t)strideD * 5 + (size_t)dstBlocks * kMatchMaxBins * 4 +
+                           (size_t)strideS * (4 + 8 + 8 + 8) + 4 + 8 + (size_t)rowCap * 16;
+    const size_t kScratchBudget = (size_t)512 << 20;
+    const uint64_t chunk = std::max<uint64_t>(1, std::min<uint64_t>({kScratchBudget / perPair, 65535, n_pairs}));
+    const size_t oIn = 0, oDev = oIn + al(chunk * sizeof(GuidedPairIn)), oBin = oDev + al(chunk * sizeof(GuidedPairDev)),
+                 oList = oBin + al(chunk * strideD), oBlk = oList + al(chunk * strideD * 4),
+                 oCand = oBlk + al(chunk * dstBlocks * kMatchMaxBins * 4), oRatio = oCand + al(chunk * strideS * 4),
+                 oSM = oRatio + al(chunk * strideS * 8), oSV = oSM + al(chunk * strideS * 8), oCnt = oSV + al(chunk * strideS * 8),
+                 oOff = oCnt + al(chunk * 4), oRM = oOff + al((chunk + 1) * 8), oRV = oRM + al(chunk * rowCap * 8),
+                 oEv = oRV + al(chunk * rowCap * 8), total = oEv + 256;
+    CK(ctx->guidedBatch.grow(total));
+    unsigned char *d = ctx->guidedBatch.data();
+    GuidedScratch g;
+    g.in = reinterpret_cast<const GuidedPairIn *>(d + oIn);
+    g.dev = reinterpret_cast<GuidedPairDev *>(d + oDev);
+    g.binOfD = d + oBin;
+    g.binList = reinterpret_cast<uint32_t *>(d + oList);
+    g.blockOff = reinterpret_cast<uint32_t *>(d + oBlk);
+    g.cand = reinterpret_cast<uint32_t *>(d + oCand);
+    g.candRatio = reinterpret_cast<double *>(d + oRatio);
+    g.stageM = reinterpret_cast<uint2 *>(d + oSM);
+    g.stageV = reinterpret_cast<double *>(d + oSV);
+    g.counts = reinterpret_cast<uint32_t *>(d + oCnt);
+    g.strideS = strideS; g.strideD = strideD; g.dstBlocks = dstBlocks;
+    uint64_t *d_off = reinterpret_cast<uint64_t *>(d + oOff);
+    uint2 *d_rowsM = reinterpret_cast<uint2 *>(d + oRM);
+    double *d_rowsV = reinterpret_cast<double *>(d + oRV);
+    unsigned long long *d_evals = reinterpret_cast<unsigned long long *>(d + oEv);
+    uint32_t sortCap = 0;
+    if (max_points) {
+        sortCap = 1;
+        while (sortCap < strideS) sortCap <<= 1;
+    }
+    const size_t selectSmem = (size_t)sortCap * (8 + 2);
+    CK(cudaFuncSetAttribute(k10_select, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)selectSmem));
+    CK(cudaMemsetAsync(d_evals, 0, 8, s));
+    CK(cudaMemsetAsync(d_off, 0, 8, s));
+    std::vector<uint64_t> &hoff = ctx->guidedOff;
+    uint64_t base = 0;
+    unsigned long long evals = 0;  // every chunk adds to d_evals: the copy after the last chunk is the total
+    for (uint64_t c0 = 0; c0 < n_pairs; c0 += chunk) {
+        const uint32_t cp = (uint32_t)std::min<uint64_t>(chunk, n_pairs - c0);
+        uint32_t sBlocks = 0, dBlocks = 0;
+        for (uint32_t k = 0; k < cp; k++) {
+            sBlocks = std::max<uint32_t>(sBlocks, (in[c0 + k].nS + kK10SrcPerCta - 1) / kK10SrcPerCta);
+            dBlocks = std::max<uint32_t>(dBlocks, (in[c0 + k].nD + kK10DstBlock - 1) / kK10DstBlock);
+        }
+        CK(cudaMemcpyAsync(d + oIn, in + c0, (size_t)cp * sizeof(GuidedPairIn), cudaMemcpyHostToDevice, s));
+        ctx->stats.h2d_bytes += (size_t)cp * sizeof(GuidedPairIn);
+        CK(cudaEventRecord(ctx->evStart, s));
+        {
+            PgiNvtxRange chunkRange("pgi:k10 chunk");
+            k10_prepare<<<(cp + 63) / 64, 64, 0, s>>>(g, cp);
+            if (dBlocks) {
+                k10_bin_count<<<dim3(dBlocks, cp), kK10DstBlock, 0, s>>>(g, kp);
+                k10_bin_offsets<<<cp, kMatchMaxBins, 0, s>>>(g);
+                k10_bin_scatter<<<dim3(dBlocks, cp), kK10DstBlock, 0, s>>>(g);
+                ctx->stats.launches += 3;
+            }
+            if (sBlocks) {
+                if (dim == 128)
+                    k10_match<128><<<dim3(sBlocks, cp), kK10Threads, 0, s>>>(g, kp, desc, d_evals);
+                else
+                    k10_match<64><<<dim3(sBlocks, cp), kK10Threads, 0, s>>>(g, kp, desc, d_evals);
+                ctx->stats.launches += 1;
+            }
+            k10_select<<<cp, kK10SelectThreads, selectSmem, s>>>(g, max_points, sortCap);
+            k9_offsets<<<1, 1024, 0, s>>>(g.counts, cp, d_off, 0);
+            k10_scatter<<<cp, 256, 0, s>>>(g, d_off, d_rowsM, d_rowsV);
+            ctx->stats.launches += 4;
+        }
+        CK(cudaEventRecord(ctx->evK1, s));
+        CK(cudaGetLastError());
+        hoff.resize(cp + 1);
+        CK(cudaMemcpyAsync(hoff.data(), d_off, (size_t)(cp + 1) * 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(&evals, d_evals, 8, cudaMemcpyDeviceToHost, s));
+        if (prep_or_null && c0 == 0) {
+            CK(cudaMemcpyAsync(prep_or_null, &g.dev[0].p, sizeof(GuidedPrep), cudaMemcpyDeviceToHost, s));
+            ctx->stats.d2h_bytes += sizeof(GuidedPrep);
+        }
+        CK(cudaStreamSynchronize(s));
+        const uint64_t rows = hoff[cp];
+        if (rows > capacity_rows - base) { ctx->err = "K10 produced more rows than its bound"; return PGI_ERR_CUDA; }
+        for (uint32_t k = 0; k < cp; k++) offsets_out[c0 + k + 1] = base + hoff[k + 1];
+        if (rows) {
+            CK(cudaMemcpyAsync(matches_out + 2 * base, d_rowsM, rows * 8, cudaMemcpyDeviceToHost, s));
+            CK(cudaMemcpyAsync(values_out + base, d_rowsV, rows * 8, cudaMemcpyDeviceToHost, s));
+            CK(cudaStreamSynchronize(s));
+        }
+        float ms = 0;
+        CK(cudaEventElapsedTime(&ms, ctx->evStart, ctx->evK1));
+        run.ms += ms;
+        ctx->stats.d2h_bytes += (size_t)(cp + 2) * 8 + rows * 16;
+        base += rows;
+        run.chunks++;
+    }
+    run.dist += evals;
+    run.rows = base;
+    return PGI_OK;
 }
 
 }  // namespace
@@ -831,67 +1052,11 @@ pgi_status pgi_register_scene_descriptors(pgi_ctx *ctx, uint64_t n_views, const 
     if (pgi_status st = stageScene(ctx, n_views, focal, size_wh, kp_offset, kp_xy, n_pairs, pair_views); st != PGI_OK) return st;
     CK(cudaMemsetAsync(r.offset.data(), 0, 8, s));
     if (pgi_status st = uploadDescriptors(ctx, desc, nKp, dim); st != PGI_OK) return st;
-
-    // K9 per chunk of pairs: scratch (forward states, backward partials, staged sorted rows) sized for the chunk only
-    const uint32_t stride = std::max<uint32_t>(maxK, 1), maxSB = (stride + kK9Rows - 1) / kK9Rows;
-    uint32_t keyCap = 1;
-    while (keyCap < stride) keyCap <<= 1;
-    const size_t perPair = (size_t)maxSB * stride * sizeof(Nn2) + (size_t)stride * (sizeof(Nn2) + 8 + 4) + 4;
-    const size_t kScratchBudget = (size_t)512 << 20;
-    const uint64_t chunk = std::max<uint64_t>(1, std::min<uint64_t>({kScratchBudget / perPair, 65535, std::max<uint64_t>(n_pairs, 1)}));
-    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
-    const size_t oF = 0, oB = oF + al(chunk * stride * sizeof(Nn2)), oM = oB + al(chunk * maxSB * stride * sizeof(Nn2)),
-                 oR = oM + al(chunk * stride * 8), oC = oR + al(chunk * stride * 4), total = oC + al(chunk * 4);
-    CK(sc.k9Scratch.grow(total));
-    Nn2 *d_fwd = reinterpret_cast<Nn2 *>(sc.k9Scratch.data() + oF), *d_bpart = reinterpret_cast<Nn2 *>(sc.k9Scratch.data() + oB);
-    uint2 *d_sm = reinterpret_cast<uint2 *>(sc.k9Scratch.data() + oM);
-    float *d_sr = reinterpret_cast<float *>(sc.k9Scratch.data() + oR);
-    uint32_t *d_cnt = reinterpret_cast<uint32_t *>(sc.k9Scratch.data() + oC);
-    const size_t finishSmem = (size_t)keyCap * 8 + (size_t)stride * 4;
-    CK(cudaFuncSetAttribute(k9_finish, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)finishSmem));
-    float msMatch = 0;
-    uint64_t rows = 0, dist = 0;
-    for (uint64_t c0 = 0; c0 < n_pairs; c0 += chunk) {
-        const uint32_t cp = (uint32_t)std::min<uint64_t>(chunk, n_pairs - c0);
-        uint32_t sbUsed = 0;
-        for (uint64_t p = c0; p < c0 + cp; p++) {
-            const uint64_t nS = kp_offset[pair_views[2 * p] + 1] - kp_offset[pair_views[2 * p]];
-            const uint64_t nD = kp_offset[pair_views[2 * p + 1] + 1] - kp_offset[pair_views[2 * p + 1]];
-            sbUsed = std::max<uint32_t>(sbUsed, (uint32_t)((nS + kK9Rows - 1) / kK9Rows));
-            dist += nS * nD;
-        }
-        CK(cudaEventRecord(ctx->evStart, s));
-        {
-            PgiNvtxRange chunkRange("pgi:k9 chunk");
-            if (sbUsed) {
-                if (dim == 128)
-                    k9_knn2_tile<128><<<dim3(sbUsed, cp), kK9Threads, 0, s>>>(sc.desc.data(), sc.kpOff.data(), sc.pv.data(), c0, stride, maxSB, d_fwd, d_bpart);
-                else
-                    k9_knn2_tile<64><<<dim3(sbUsed, cp), kK9Threads, 0, s>>>(sc.desc.data(), sc.kpOff.data(), sc.pv.data(), c0, stride, maxSB, d_fwd, d_bpart);
-                ctx->stats.launches += 1;
-            }
-            k9_finish<<<cp, kK9FinishThreads, finishSmem, s>>>(sc.kpOff.data(), sc.pv.data(), c0, stride, keyCap, maxSB, d_fwd, d_bpart, d_cnt, d_sm, d_sr);
-            k9_offsets<<<1, 1024, 0, s>>>(d_cnt, cp, r.offset.data(), c0);
-            CK(cudaGetLastError());
-            ctx->stats.launches += 2;
-        }
-        uint64_t end = 0;
-        CK(cudaMemcpyAsync(&end, r.offset.data() + c0 + cp, 8, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        ctx->stats.d2h_bytes += 8;
-        CK(sc.growMatches(end, rows, s));
-        k9_scatter<<<cp, 256, 0, s>>>(r.offset.data(), c0, stride, d_cnt, d_sm, d_sr, sc.m.data(), sc.ratio.data());
-        CK(cudaEventRecord(ctx->evK1, s));
-        CK(cudaGetLastError());
-        ctx->stats.launches += 1;
-        CK(cudaEventSynchronize(ctx->evK1));
-        float ms = 0;
-        CK(cudaEventElapsedTime(&ms, ctx->evStart, ctx->evK1));
-        msMatch += ms;
-        rows = end;
-    }
-    ctx->stats.ms_match += msMatch;
-    ctx->stats.dist_evals += dist;
+    MatchRun run;
+    if (pgi_status st = matchPairs(ctx, sc, dim, maxK, n_pairs, kp_offset, pair_views, r.offset.data(), run); st != PGI_OK) return st;
+    const uint64_t rows = run.rows;
+    ctx->stats.ms_match += run.ms;
+    ctx->stats.dist_evals += run.dist;
     ctx->stats.match_pairs += n_pairs;
     ctx->stats.match_rows += rows;
     // the offsets are the caller's m_offset and the registration's host copy; the matches stay on the device for K0
@@ -1023,6 +1188,14 @@ pgi_status pgi_set_scene_descriptors(pgi_ctx *ctx, const float *desc, uint32_t d
     if (dim != 128 && dim != 64) { ctx->err = "descriptors must have 64 or 128 dimensions"; return PGI_ERR_INVALID; }
     const uint64_t nKp = sc.hKpOff.back();
     if (!desc && nKp) { ctx->err = "null argument"; return PGI_ERR_INVALID; }
+    for (size_t v = 0; v + 1 < sc.hKpOff.size(); v++)
+        if (sc.hKpOff[v + 1] - sc.hKpOff[v] > kK10MaxKp) {
+            char buf[160];
+            snprintf(buf, sizeof buf, "view %zu has %llu keypoints; guided matching supports at most %u per view", v,
+                     (unsigned long long)(sc.hKpOff[v + 1] - sc.hKpOff[v]), kK10MaxKp);
+            ctx->err = buf;
+            return PGI_ERR_INVALID;
+        }
     CK(cudaSetDevice(ctx->cfg.device));
     return uploadDescriptors(ctx, desc, nKp, dim);
 }
@@ -1289,66 +1462,58 @@ pgi_status pgi_guided_match(pgi_ctx *ctx, uint32_t n_src, const float *kp_src, c
                             int32_t bin_number, uint32_t *matches_out, double *ratios_out, uint32_t *n_out,
                             double *prepared_or_null)
 {
-    PgiNvtxRange nvtxRange("pgi:guided_match (K7)");
+    PgiNvtxRange nvtxRange("pgi:guided_match (K10 on one pair)");
     if (!ctx) return PGI_ERR_INVALID;
     if (!pose_q_t || !K_src || !K_dst || !size_src || !size_dst || !n_out || (n_src && (!kp_src || !desc_src || !matches_out || !ratios_out)) ||
-        (n_dst && (!kp_dst || !desc_dst)) || dim == 0 || bin_number > kMatchMaxBins) {
+        (n_dst && (!kp_dst || !desc_dst)) || bin_number > kMatchMaxBins) {
         ctx->err = "bad argument";
         return PGI_ERR_INVALID;
     }
+    if (dim != 128 && dim != 64) { ctx->err = "descriptors must have 64 or 128 dimensions"; return PGI_ERR_INVALID; }
     CK(cudaSetDevice(ctx->cfg.device));
     *n_out = 0;
     if (n_src == 0 || n_dst == 0) return PGI_OK;
+    // the pair as a scene of two views: [desc_src; desc_dst], then [kp_src; kp_dst] (256-byte aligned: dim * 4 is)
     cudaStream_t s = ctx->stream;
-    const size_t bS = (size_t)n_src, bD = (size_t)n_dst;
-    // one scratch allocation per call: this entry point is the reference-shaped single-pair call
-    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
-    const size_t oKpS = 0, oDS = oKpS + al(bS * 8), oKpD = oDS + al(bS * dim * 4), oDD = oKpD + al(bD * 8), oBin = oDD + al(bD * dim * 4),
-                 oList = oBin + al(bD), oCand = oList + al(bD * 4), oRatio = oCand + al(bS * 4), oM = oRatio + al(bS * 8),
-                 oR = oM + al(bS * 8), oN = oR + al(bS * 8), oPrep = oN + 256, total = oPrep + 256;
-    DevBuf<unsigned char> scratch;
-    CK(scratch.grow(total));
-    unsigned char *d = scratch.data();
-    CK(cudaMemcpyAsync(d + oKpS, kp_src, bS * 8, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(d + oDS, desc_src, bS * dim * 4, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(d + oKpD, kp_dst, bD * 8, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(d + oDD, desc_dst, bD * dim * 4, cudaMemcpyHostToDevice, s));
-    MatchArgs a;
-    a.kpS = reinterpret_cast<const float2 *>(d + oKpS); a.dS = reinterpret_cast<const float *>(d + oDS);
-    a.kpD = reinterpret_cast<const float2 *>(d + oKpD); a.dD = reinterpret_cast<const float *>(d + oDD);
-    a.nS = n_src; a.nD = n_dst; a.dim = dim;
-    essentialOfPose(pose_q_t, a.E);
-    for (int k = 0; k < 9; k++) { a.Ks[k] = K_src[k]; a.Kd[k] = K_dst[k]; }
-    a.wS = size_src[0]; a.hS = size_src[1]; a.wD = size_dst[0]; a.hD = size_dst[1]; a.binNumber = bin_number;
-    a.binOfD = d + oBin; a.binList = reinterpret_cast<uint32_t *>(d + oList); a.cand = reinterpret_cast<uint32_t *>(d + oCand);
-    a.candRatio = reinterpret_cast<double *>(d + oRatio); a.matches = reinterpret_cast<uint32_t *>(d + oM);
-    a.ratios = reinterpret_cast<double *>(d + oR); a.nOut = reinterpret_cast<uint32_t *>(d + oN);
-    a.prepOut = reinterpret_cast<double *>(d + oPrep);
-    CK(cudaEventRecord(ctx->evStart, s));
-    k7_guided_match<<<1, kMatchThreads, 0, s>>>(a);
-    CK(cudaEventRecord(ctx->evK1, s));
-    CK(cudaGetLastError());
-    uint32_t n = 0;
-    CK(cudaMemcpyAsync(&n, d + oN, 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    CK(addGuidedTime(ctx));
-    if (n > n_src) n = n_src;
-    if (n) {
-        CK(cudaMemcpy(matches_out, d + oM, (size_t)n * 8, cudaMemcpyDeviceToHost));
-        CK(cudaMemcpy(ratios_out, d + oR, (size_t)n * 8, cudaMemcpyDeviceToHost));
+    const size_t nKp = (size_t)n_src + n_dst, oKp = nKp * dim * 4;
+    DevBuf<unsigned char> staged;
+    CK(staged.grow(oKp + nKp * 8));
+    unsigned char *d = staged.data();
+    CK(cudaMemcpyAsync(d, desc_src, (size_t)n_src * dim * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d + (size_t)n_src * dim * 4, desc_dst, (size_t)n_dst * dim * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d + oKp, kp_src, (size_t)n_src * 8, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d + oKp + (size_t)n_src * 8, kp_dst, (size_t)n_dst * 8, cudaMemcpyHostToDevice, s));
+    ctx->stats.h2d_bytes += nKp * (8 + dim * 4);
+    GuidedPairIn in;
+    memset(&in, 0, sizeof in);
+    essentialOfPose(pose_q_t, in.E);
+    memcpy(in.Ks, K_src, sizeof in.Ks);
+    memcpy(in.Kd, K_dst, sizeof in.Kd);
+    in.wS = size_src[0]; in.hS = size_src[1]; in.wD = size_dst[0]; in.hD = size_dst[1]; in.binNumber = bin_number;
+    in.kS0 = 0; in.kD0 = n_src;
+    in.nS = n_src; in.nD = n_dst;
+    uint64_t off[2];
+    GuidedPrep prep;
+    MatchRun run;
+    if (pgi_status st = runGuided(ctx, reinterpret_cast<const float2 *>(d + oKp), reinterpret_cast<const float *>(d), dim, &in, 1, 0,
+                                  off, matches_out, ratios_out, n_src, &prep, run);
+        st != PGI_OK)
+        return st;
+    ctx->stats.ms_guided += run.ms;
+    ctx->stats.guided_calls += 1;
+    *n_out = (uint32_t)off[1];
+    if (prepared_or_null) {
+        for (int k = 0; k < 9; k++) prepared_or_null[k] = prep.F[k];
+        prepared_or_null[9] = prep.ex; prepared_or_null[10] = prep.ey; prepared_or_null[11] = prep.minAngle;
+        prepared_or_null[12] = prep.range; prepared_or_null[13] = prep.binsRaw;
     }
-    if (prepared_or_null) CK(cudaMemcpy(prepared_or_null, d + oPrep, 14 * 8, cudaMemcpyDeviceToHost));
-    *n_out = n;
-    ctx->stats.launches += 1;
-    ctx->stats.h2d_bytes += bS * (8 + dim * 4) + bD * (8 + dim * 4);
-    ctx->stats.d2h_bytes += (size_t)n * 16 + 4;
     return PGI_OK;
 }
 
 pgi_status pgi_guided_match_views(pgi_ctx *ctx, uint32_t src, uint32_t dst, const double *pose_q_t, int32_t bin_number,
                                   uint32_t max_points, uint32_t *matches_out, double *values_out, uint32_t *n_out)
 {
-    PgiNvtxRange nvtxRange("pgi:guided_match_views (K7 on the resident scene)");
+    PgiNvtxRange nvtxRange("pgi:guided_match_views (K10 on one pair of the resident scene)");
     if (!ctx) return PGI_ERR_INVALID;
     if (ctx->inFlight) { ctx->err = "a wave is in flight"; return PGI_ERR_STATE; }
     const SceneStaging &sc = ctx->scene;
@@ -1365,72 +1530,17 @@ pgi_status pgi_guided_match_views(pgi_ctx *ctx, uint32_t src, uint32_t dst, cons
     }
     CK(cudaSetDevice(ctx->cfg.device));
     *n_out = 0;
-    const uint64_t nS = sc.hKpOff[src + 1] - sc.hKpOff[src], nD = sc.hKpOff[dst + 1] - sc.hKpOff[dst];
-    if (nS == 0 || nD == 0 || max_points == 0) return PGI_OK;
-    cudaStream_t s = ctx->stream;
-    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
-    const size_t oBin = 0, oList = oBin + al(nD), oCand = oList + al(nD * 4), oRatio = oCand + al(nS * 4), oM = oRatio + al(nS * 8),
-                 oR = oM + al(nS * 8), oN = oR + al(nS * 8), total = oN + 256;
-    CK(ctx->guided.grow(total));
-    unsigned char *d = ctx->guided.data();
-    MatchArgs a;
-    a.kpS = sc.kp.data() + sc.hKpOff[src]; a.dS = sc.desc.data() + sc.hKpOff[src] * sc.dim;
-    a.kpD = sc.kp.data() + sc.hKpOff[dst]; a.dD = sc.desc.data() + sc.hKpOff[dst] * sc.dim;
-    a.nS = (uint32_t)nS; a.nD = (uint32_t)nD; a.dim = sc.dim;
-    essentialOfPose(pose_q_t, a.E);
-    // K = [f 0 w/2; 0 f h/2; 0 0 1] of each view (pose_graph_builder.h:284-286)
-    const double fS = sc.hFocal[src], wS = sc.hSize[2 * src], hS = sc.hSize[2 * src + 1];
-    const double fD = sc.hFocal[dst], wD = sc.hSize[2 * dst], hD = sc.hSize[2 * dst + 1];
-    const double Ks[9] = {fS, 0.0, wS / 2.0, 0.0, fS, hS / 2.0, 0.0, 0.0, 1.0};
-    const double Kd[9] = {fD, 0.0, wD / 2.0, 0.0, fD, hD / 2.0, 0.0, 0.0, 1.0};
-    for (int k = 0; k < 9; k++) { a.Ks[k] = Ks[k]; a.Kd[k] = Kd[k]; }
-    a.wS = (int)wS; a.hS = (int)hS; a.wD = (int)wD; a.hD = (int)hD; a.binNumber = bin_number;
-    a.binOfD = d + oBin; a.binList = reinterpret_cast<uint32_t *>(d + oList); a.cand = reinterpret_cast<uint32_t *>(d + oCand);
-    a.candRatio = reinterpret_cast<double *>(d + oRatio); a.matches = reinterpret_cast<uint32_t *>(d + oM);
-    a.ratios = reinterpret_cast<double *>(d + oR); a.nOut = reinterpret_cast<uint32_t *>(d + oN);
-    a.prepOut = nullptr;
-    CK(cudaEventRecord(ctx->evStart, s));
-    k7_guided_match<<<1, kMatchThreads, 0, s>>>(a);
-    CK(cudaEventRecord(ctx->evK1, s));
-    CK(cudaGetLastError());
-    uint32_t n = 0;
-    CK(cudaMemcpyAsync(&n, d + oN, 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    CK(addGuidedTime(ctx));
-    if (n > nS) n = (uint32_t)nS;
-    ctx->guidedM.resize((size_t)2 * n);
-    ctx->guidedR.resize(n);
-    if (n) {
-        CK(cudaMemcpyAsync(ctx->guidedM.data(), d + oM, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
-        CK(cudaMemcpyAsync(ctx->guidedR.data(), d + oR, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
-    ctx->stats.launches += 1;
-    ctx->stats.d2h_bytes += (size_t)n * 16 + 4;
-    // guidedMatching's selection (pose_graph_builder.h:760-782): above max_points matches, the max_points smallest
-    // (value, index) entries in the min-heap's pop order; otherwise every match, each carrying the first value (:777-779)
-    const std::vector<uint32_t> &m = ctx->guidedM;
-    const std::vector<double> &r = ctx->guidedR;
-    if (n > max_points) {
-        std::vector<uint32_t> &order = ctx->guidedOrder;
-        order.resize(n);
-        for (uint32_t i = 0; i < n; i++) order[i] = i;
-        const auto less = [&](uint32_t x, uint32_t y) { return r[x] != r[y] ? r[x] < r[y] : x < y; };
-        std::partial_sort(order.begin(), order.begin() + max_points, order.end(), less);
-        for (uint32_t k = 0; k < max_points; k++) {
-            matches_out[2 * k] = m[2 * order[k]];
-            matches_out[2 * k + 1] = m[2 * order[k] + 1];
-            values_out[k] = r[order[k]];
-        }
-        *n_out = max_points;
-    } else {
-        for (uint32_t k = 0; k < n; k++) {
-            matches_out[2 * k] = m[2 * k];
-            matches_out[2 * k + 1] = m[2 * k + 1];
-            values_out[k] = r[0];
-        }
-        *n_out = n;
-    }
+    const GuidedPairIn in = scenePairIn(sc, src, dst, pose_q_t, bin_number);
+    if (in.nS == 0 || in.nD == 0 || max_points == 0) return PGI_OK;
+    uint64_t off[2];
+    MatchRun run;
+    if (pgi_status st = runGuided(ctx, sc.kp.data(), sc.desc.data(), sc.dim, &in, 1, max_points, off, matches_out, values_out,
+                                  std::min(in.nS, max_points), nullptr, run);
+        st != PGI_OK)
+        return st;
+    ctx->stats.ms_guided += run.ms;
+    ctx->stats.guided_calls += 1;
+    *n_out = (uint32_t)off[1];
     return PGI_OK;
 }
 
@@ -1452,208 +1562,73 @@ pgi_status pgi_guided_match_pairs(pgi_ctx *ctx, uint64_t n_pairs, const uint32_t
         return PGI_ERR_INVALID;
     }
     const uint64_t V = sc.hFocal.size();
-    uint64_t need = 0;
-    uint32_t maxS = 0, maxD = 0;
+    std::vector<GuidedPairIn> &in = ctx->guidedIn;
+    in.resize(n_pairs);
     for (uint64_t p = 0; p < n_pairs; p++) {
         const uint32_t src = pair_views[2 * p], dst = pair_views[2 * p + 1];
         if (src >= V || dst >= V) { ctx->err = "view id out of range"; return PGI_ERR_INVALID; }
-        const uint64_t nS = sc.hKpOff[src + 1] - sc.hKpOff[src], nD = sc.hKpOff[dst + 1] - sc.hKpOff[dst];
-        if (nS > kK10MaxKp || nD > kK10MaxKp) {
-            ctx->err = "batched guided matching supports at most 16384 keypoints per view";
-            return PGI_ERR_INVALID;
-        }
-        need += max_points ? std::min<uint64_t>(nS, max_points) : nS;
-        maxS = std::max<uint32_t>(maxS, (uint32_t)nS);
-        maxD = std::max<uint32_t>(maxD, (uint32_t)nD);
+        in[p] = scenePairIn(sc, src, dst, poses_q_t + 7 * p, bin_number);
     }
-    if (need > capacity_rows) { ctx->err = "capacity_rows is below the rows the batch can produce"; return PGI_ERR_INVALID; }
-    if (need && (!matches_out || !values_out)) { ctx->err = "null argument"; return PGI_ERR_INVALID; }
-    CK(cudaSetDevice(ctx->cfg.device));
-    offsets_out[0] = 0;
-    if (n_pairs == 0) return PGI_OK;
-    cudaStream_t s = ctx->stream;
-
-    // K10 per chunk of pairs: every per-pair array is sized for the batch's largest views, the chunk for 512 MB
-    const uint32_t strideS = std::max<uint32_t>(maxS, 1), strideD = std::max<uint32_t>(maxD, 1);
-    const uint32_t dstBlocks = (strideD + kK10DstBlock - 1) / kK10DstBlock;
-    const uint32_t rowCap = max_points ? std::min(strideS, max_points) : strideS;
-    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
-    const size_t perPair = sizeof(GuidedPairIn) + sizeof(GuidedPairDev) + (size_t)strideD * 5 + (size_t)dstBlocks * kMatchMaxBins * 4 +
-                           (size_t)strideS * (4 + 8 + 8 + 8) + 4 + 8 + (size_t)rowCap * 16;
-    const size_t kScratchBudget = (size_t)512 << 20;
-    const uint64_t chunk = std::max<uint64_t>(1, std::min<uint64_t>({kScratchBudget / perPair, 65535, n_pairs}));
-    const size_t oIn = 0, oDev = oIn + al(chunk * sizeof(GuidedPairIn)), oBin = oDev + al(chunk * sizeof(GuidedPairDev)),
-                 oList = oBin + al(chunk * strideD), oBlk = oList + al(chunk * strideD * 4),
-                 oCand = oBlk + al(chunk * dstBlocks * kMatchMaxBins * 4), oRatio = oCand + al(chunk * strideS * 4),
-                 oSM = oRatio + al(chunk * strideS * 8), oSV = oSM + al(chunk * strideS * 8), oCnt = oSV + al(chunk * strideS * 8),
-                 oOff = oCnt + al(chunk * 4), oRM = oOff + al((chunk + 1) * 8), oRV = oRM + al(chunk * rowCap * 8),
-                 oEv = oRV + al(chunk * rowCap * 8), total = oEv + 256;
-    CK(ctx->guidedBatch.grow(total));
-    unsigned char *d = ctx->guidedBatch.data();
-    GuidedScratch g;
-    g.in = reinterpret_cast<const GuidedPairIn *>(d + oIn);
-    g.dev = reinterpret_cast<GuidedPairDev *>(d + oDev);
-    g.binOfD = d + oBin;
-    g.binList = reinterpret_cast<uint32_t *>(d + oList);
-    g.blockOff = reinterpret_cast<uint32_t *>(d + oBlk);
-    g.cand = reinterpret_cast<uint32_t *>(d + oCand);
-    g.candRatio = reinterpret_cast<double *>(d + oRatio);
-    g.stageM = reinterpret_cast<uint2 *>(d + oSM);
-    g.stageV = reinterpret_cast<double *>(d + oSV);
-    g.counts = reinterpret_cast<uint32_t *>(d + oCnt);
-    g.strideS = strideS; g.strideD = strideD; g.dstBlocks = dstBlocks;
-    uint64_t *d_off = reinterpret_cast<uint64_t *>(d + oOff);
-    uint2 *d_rowsM = reinterpret_cast<uint2 *>(d + oRM);
-    double *d_rowsV = reinterpret_cast<double *>(d + oRV);
-    unsigned long long *d_evals = reinterpret_cast<unsigned long long *>(d + oEv);
-    uint32_t sortCap = 0;
-    if (max_points) {
-        sortCap = 1;
-        while (sortCap < strideS) sortCap <<= 1;
-    }
-    const size_t selectSmem = (size_t)sortCap * (8 + 2);
-    CK(cudaFuncSetAttribute(k10_select, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)selectSmem));
-    CK(cudaMemsetAsync(d_evals, 0, 8, s));
-    CK(cudaMemsetAsync(d_off, 0, 8, s));
-    std::vector<GuidedPairIn> &hin = ctx->guidedIn;
-    std::vector<uint64_t> &hoff = ctx->guidedOff;
-    float msTotal = 0;
-    uint64_t base = 0, chunks = 0;
-    for (uint64_t c0 = 0; c0 < n_pairs; c0 += chunk) {
-        const uint32_t cp = (uint32_t)std::min<uint64_t>(chunk, n_pairs - c0);
-        hin.resize(cp);
-        uint32_t sBlocks = 0, dBlocks = 0;
-        for (uint32_t k = 0; k < cp; k++) {
-            const uint32_t src = pair_views[2 * (c0 + k)], dst = pair_views[2 * (c0 + k) + 1];
-            GuidedPairIn &in = hin[k];
-            memset(&in, 0, sizeof in);
-            essentialOfPose(poses_q_t + 7 * (c0 + k), in.E);
-            // K = [f 0 w/2; 0 f h/2; 0 0 1] of each view (pose_graph_builder.h:284-286), as pgi_guided_match_views builds it
-            const double fS = sc.hFocal[src], wS = sc.hSize[2 * src], hS = sc.hSize[2 * src + 1];
-            const double fD = sc.hFocal[dst], wD = sc.hSize[2 * dst], hD = sc.hSize[2 * dst + 1];
-            const double Ks[9] = {fS, 0.0, wS / 2.0, 0.0, fS, hS / 2.0, 0.0, 0.0, 1.0};
-            const double Kd[9] = {fD, 0.0, wD / 2.0, 0.0, fD, hD / 2.0, 0.0, 0.0, 1.0};
-            memcpy(in.Ks, Ks, sizeof Ks);
-            memcpy(in.Kd, Kd, sizeof Kd);
-            in.wS = (int)wS; in.hS = (int)hS; in.wD = (int)wD; in.hD = (int)hD; in.binNumber = bin_number;
-            in.kS0 = sc.hKpOff[src]; in.kD0 = sc.hKpOff[dst];
-            in.nS = (uint32_t)(sc.hKpOff[src + 1] - in.kS0); in.nD = (uint32_t)(sc.hKpOff[dst + 1] - in.kD0);
-            sBlocks = std::max<uint32_t>(sBlocks, (in.nS + kK10SrcPerCta - 1) / kK10SrcPerCta);
-            dBlocks = std::max<uint32_t>(dBlocks, (in.nD + kK10DstBlock - 1) / kK10DstBlock);
-        }
-        CK(cudaMemcpyAsync(d + oIn, hin.data(), (size_t)cp * sizeof(GuidedPairIn), cudaMemcpyHostToDevice, s));
-        ctx->stats.h2d_bytes += (size_t)cp * sizeof(GuidedPairIn);
-        CK(cudaEventRecord(ctx->evStart, s));
-        {
-            PgiNvtxRange chunkRange("pgi:k10 chunk");
-            k10_prepare<<<(cp + 63) / 64, 64, 0, s>>>(g, cp);
-            if (dBlocks) {
-                k10_bin_count<<<dim3(dBlocks, cp), kK10DstBlock, 0, s>>>(g, sc.kp.data());
-                k10_bin_offsets<<<cp, kMatchMaxBins, 0, s>>>(g);
-                k10_bin_scatter<<<dim3(dBlocks, cp), kK10DstBlock, 0, s>>>(g);
-                ctx->stats.launches += 3;
-            }
-            if (sBlocks) {
-                if (sc.dim == 128)
-                    k10_match<128><<<dim3(sBlocks, cp), kK10Threads, 0, s>>>(g, sc.kp.data(), sc.desc.data(), d_evals);
-                else
-                    k10_match<64><<<dim3(sBlocks, cp), kK10Threads, 0, s>>>(g, sc.kp.data(), sc.desc.data(), d_evals);
-                ctx->stats.launches += 1;
-            }
-            k10_select<<<cp, kK10SelectThreads, selectSmem, s>>>(g, max_points, sortCap);
-            k9_offsets<<<1, 1024, 0, s>>>(g.counts, cp, d_off, 0);
-            k10_scatter<<<cp, 256, 0, s>>>(g, d_off, d_rowsM, d_rowsV);
-            ctx->stats.launches += 4;
-        }
-        CK(cudaEventRecord(ctx->evK1, s));
-        CK(cudaGetLastError());
-        hoff.resize(cp + 1);
-        CK(cudaMemcpyAsync(hoff.data(), d_off, (size_t)(cp + 1) * 8, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        const uint64_t rows = hoff[cp];
-        if (rows > capacity_rows - base) { ctx->err = "K10 produced more rows than its bound"; return PGI_ERR_CUDA; }
-        for (uint32_t k = 0; k < cp; k++) offsets_out[c0 + k + 1] = base + hoff[k + 1];
-        if (rows) {
-            CK(cudaMemcpyAsync(matches_out + 2 * base, d_rowsM, rows * 8, cudaMemcpyDeviceToHost, s));
-            CK(cudaMemcpyAsync(values_out + base, d_rowsV, rows * 8, cudaMemcpyDeviceToHost, s));
-            CK(cudaStreamSynchronize(s));
-        }
-        float ms = 0;
-        CK(cudaEventElapsedTime(&ms, ctx->evStart, ctx->evK1));
-        msTotal += ms;
-        ctx->stats.d2h_bytes += (size_t)(cp + 1) * 8 + rows * 16;
-        base += rows;
-        chunks++;
-    }
-    unsigned long long evals = 0;
-    CK(cudaMemcpyAsync(&evals, d_evals, 8, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    ctx->stats.d2h_bytes += 8;
-    ctx->stats.ms_guided_pairs += msTotal;
+    MatchRun run;
+    if (pgi_status st = runGuided(ctx, sc.kp.data(), sc.desc.data(), sc.dim, in.data(), n_pairs, max_points, offsets_out, matches_out,
+                                  values_out, capacity_rows, nullptr, run);
+        st != PGI_OK)
+        return st;
+    ctx->stats.ms_guided_pairs += run.ms;
     ctx->stats.guided_pairs += n_pairs;
-    ctx->stats.guided_dist_evals += evals;
-    ctx->stats.guided_chunks += chunks;
+    ctx->stats.guided_dist_evals += run.dist;
+    ctx->stats.guided_chunks += run.chunks;
     return PGI_OK;
 }
 
 pgi_status pgi_match_features(pgi_ctx *ctx, uint32_t n_src, const float *desc_src, uint32_t n_dst, const float *desc_dst,
                               uint32_t dim, uint32_t *matches_out, double *ratios_out, uint32_t *n_out)
 {
-    PgiNvtxRange nvtxRange("pgi:match_features (K8)");
+    PgiNvtxRange nvtxRange("pgi:match_features (K9 on one pair)");
     if (!ctx) return PGI_ERR_INVALID;
+    // the finite check's flag word and K9's timing events are the ones a wave in flight reads back
+    if (ctx->inFlight) { ctx->err = "a wave is in flight"; return PGI_ERR_STATE; }
     if (!n_out || (n_src && (!desc_src || !matches_out || !ratios_out)) || (n_dst && !desc_dst) || (dim != 128 && dim != 64)) {
         ctx->err = "bad argument (descriptors must have 64 or 128 dimensions)";
+        return PGI_ERR_INVALID;
+    }
+    if (n_src > kK9MaxKp || n_dst > kK9MaxKp) {
+        ctx->err = "descriptor matching supports at most 16384 descriptors per side";
         return PGI_ERR_INVALID;
     }
     CK(cudaSetDevice(ctx->cfg.device));
     *n_out = 0;
     if (n_src == 0 || n_dst == 0) return PGI_OK;
+    // the pair as a scene of two views, staged apart from the registered scene: [desc_src; desc_dst], pair (0, 1)
+    MatchStaging &st = ctx->pairMatch;
     cudaStream_t s = ctx->stream;
-    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
-    const size_t bS = n_src, bD = n_dst;
-    const size_t oA = 0, oB = oA + al(bS * dim * 4), oF = oB + al(bD * dim * 4), oG = oF + al(bS * sizeof(Knn2)),
-                 oM = oG + al(bD * sizeof(Knn2)), oR = oM + al(bS * 8), oN = oR + al(bS * 8), total = oN + 256;
-    DevBuf<unsigned char> scratch;
-    CK(scratch.grow(total));
-    unsigned char *d = scratch.data();
-    CK(cudaMemcpyAsync(d + oA, desc_src, bS * dim * 4, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(d + oB, desc_dst, bD * dim * 4, cudaMemcpyHostToDevice, s));
-    const float *A = reinterpret_cast<const float *>(d + oA), *B = reinterpret_cast<const float *>(d + oB);
-    Knn2 *F = reinterpret_cast<Knn2 *>(d + oF), *G = reinterpret_cast<Knn2 *>(d + oG);
-    if (dim == 128) {
-        k8_knn2<128><<<(n_src + kFeatThreads - 1) / kFeatThreads, kFeatThreads, 0, s>>>(A, n_src, B, n_dst, F);  // feature_utils.h:158-159
-        k8_knn2<128><<<(n_dst + kFeatThreads - 1) / kFeatThreads, kFeatThreads, 0, s>>>(B, n_dst, A, n_src, G);  // :162-163
-    } else {
-        k8_knn2<64><<<(n_src + kFeatThreads - 1) / kFeatThreads, kFeatThreads, 0, s>>>(A, n_src, B, n_dst, F);
-        k8_knn2<64><<<(n_dst + kFeatThreads - 1) / kFeatThreads, kFeatThreads, 0, s>>>(B, n_dst, A, n_src, G);
-    }
-    k8_mutual<<<1, 1024, 0, s>>>(F, n_src, G, n_dst, reinterpret_cast<uint32_t *>(d + oM), reinterpret_cast<double *>(d + oR),
-                                 reinterpret_cast<uint32_t *>(d + oN));
-    CK(cudaGetLastError());
-    uint32_t n = 0;
-    CK(cudaMemcpyAsync(&n, d + oN, 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    if (n > n_src) n = n_src;
-    std::vector<uint32_t> m((size_t)2 * n);
-    std::vector<double> r(n);
+    const uint64_t kpOff[3] = {0, n_src, (uint64_t)n_src + n_dst};
+    const uint32_t pv[2] = {0, 1};
+    CK(st.desc.grow(kpOff[2] * dim));
+    CK(cudaMemcpyAsync(st.desc.data(), desc_src, (size_t)n_src * dim * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(st.desc.data() + (size_t)n_src * dim, desc_dst, (size_t)n_dst * dim * 4, cudaMemcpyHostToDevice, s));
+    ctx->stats.h2d_bytes += kpOff[2] * dim * 4;
+    if (pgi_status e = checkFinite(ctx, st.desc.data(), kpOff[2] * dim); e != PGI_OK) return e;
+    CK(st.kpOff.grow(3));
+    CK(st.pv.grow(1));
+    CK(ctx->pairMatchOff.grow(2));
+    CK(cudaMemcpyAsync(st.kpOff.data(), kpOff, sizeof kpOff, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(st.pv.data(), pv, sizeof pv, cudaMemcpyHostToDevice, s));
+    CK(cudaMemsetAsync(ctx->pairMatchOff.data(), 0, 8, s));
+    ctx->stats.h2d_bytes += sizeof kpOff + sizeof pv;
+    MatchRun run;
+    if (pgi_status e = matchPairs(ctx, st, dim, std::max(n_src, n_dst), 1, kpOff, pv, ctx->pairMatchOff.data(), run); e != PGI_OK)
+        return e;
+    const uint32_t n = (uint32_t)run.rows;
+    std::vector<float> r(n);
     if (n) {
-        CK(cudaMemcpy(m.data(), d + oM, (size_t)n * 8, cudaMemcpyDeviceToHost));
-        CK(cudaMemcpy(r.data(), d + oR, (size_t)n * 8, cudaMemcpyDeviceToHost));
+        CK(cudaMemcpyAsync(matches_out, st.m.data(), (size_t)n * 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(r.data(), st.ratio.data(), (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
     }
-    // std::sort of (ratio, &matches[i]) pairs (feature_utils.h:188): by ratio, then by the address of the query's
-    // match vector, i.e. by query index
-    std::vector<uint32_t> order(n);
-    for (uint32_t i = 0; i < n; i++) order[i] = i;
-    std::sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return r[x] != r[y] ? r[x] < r[y] : m[2 * x] < m[2 * y]; });
-    for (uint32_t i = 0; i < n; i++) {
-        matches_out[2 * i] = m[2 * order[i]];
-        matches_out[2 * i + 1] = m[2 * order[i] + 1];
-        ratios_out[i] = r[order[i]];
-    }
+    for (uint32_t i = 0; i < n; i++) ratios_out[i] = (double)r[i];  // feature_utils.h:182: float widened
     *n_out = n;
-    ctx->stats.launches += 3;
-    ctx->stats.h2d_bytes += (bS + bD) * dim * 4;
-    ctx->stats.d2h_bytes += (size_t)n * 16 + 4;
+    ctx->stats.d2h_bytes += (size_t)n * 12;
     return PGI_OK;
 }
 

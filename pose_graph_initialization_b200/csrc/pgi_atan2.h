@@ -3,7 +3,7 @@
 // matcher.h:285-299 and :330-340 bin keypoints by `atan2` of an epipolar line's normal; the reference calls the host
 // libm, whose last bit depends on the libm version (glibc 2.39: correctly rounded in 99.97 % of random arguments, off by
 // one ulp in the rest — measured against this file and mpmath).  CUDA's atan2 is a 2-ulp function, and an angle that
-// differs in its last bit shows up in the matcher's angular range and, rarely, in a bin index.  K7 therefore evaluates
+// differs in its last bit shows up in the matcher's angular range and, rarely, in a bin index.  The guided matcher therefore evaluates
 // the one canonical answer, the correctly rounded atan2, itself: y/x as a double-double quotient, reduced against a
 // 65-entry table of atan(k/64) (double-double), odd series on the remainder (|z| <= 1/128), quadrant fix-ups with
 // double-double pi — about 100 bits before the final rounding, so the result is the correctly rounded one except for

@@ -1,7 +1,7 @@
 // pgi_guided_batch.cuh — K10: guided matching (HashingBasedMatcherWithPose<false, 45>::match, matcher.h:199-405, and
 // guidedMatching's selection, pose_graph_builder.h:760-782) for a chunk of (view pair, pose) cases of the registered scene,
-// spread over the whole GPU.  Every pair's rows are bit-identical to K7's: the arithmetic is K7's own device functions
-// (pgi_matcher.cuh), only the split of the work differs.
+// spread over the whole GPU.  Every pair's rows are bit-identical to the reference's: the arithmetic is the shared
+// device functions of pgi_matcher.cuh, applied in the reference's order; only the split of the work differs.
 //
 //   k10_prepare       one thread per pair: guidedPrepare (F, epipole, angular range, bin count);
 //   k10_bin_count     CTA (block of kK10DstBlock destination keypoints, pair): each keypoint's bin, per-block bin histogram;
@@ -68,7 +68,7 @@ __global__ void k10_prepare(GuidedScratch g, uint32_t cp)
     const GuidedPairIn &in = g.in[pl];
     GuidedPrep p;
     guidedPrepare(in.E, in.Ks, in.Kd, in.wS, in.hS, in.wD, in.hD, in.binNumber, p);
-    if (in.nS == 0 || in.nD == 0) p.bins = 0;  // nothing to match (K7 is not launched for such a pair)
+    if (in.nS == 0 || in.nD == 0) p.bins = 0;  // nothing to match
     g.dev[pl].p = p;
 }
 
@@ -249,7 +249,7 @@ __global__ void __launch_bounds__(kK10SelectThreads) k10_select(GuidedScratch g,
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     uint32_t base = 0;
     if (g.dev[pl].p.bins > 0)
-        for (uint32_t i0 = 0; i0 < nS; i0 += kK10SelectThreads) {  // compaction in source order (K7's phase 4)
+        for (uint32_t i0 = 0; i0 < nS; i0 += kK10SelectThreads) {  // compaction in source order
             const uint32_t i = i0 + threadIdx.x;
             const bool ok = i < nS && cand[i] != 0xffffffffu;
             const uint32_t m = __ballot_sync(0xffffffffu, ok);

@@ -1,8 +1,9 @@
 // pgi_guided_nn.h — the best / second-best state of the guided matcher's candidate scan (matcher.h:366-384) as a value that
 // merges over consecutive runs of a bin.
 //
-// K7 walks a source keypoint's bin in list order.  Every bin entry whose gate `d2 >= 0.75 * 0.75` is false is a candidate
-// (a NaN d2 is one); for each candidate it computes the descriptor distance acc and steps
+// The reference (matcher.h:362-384) walks a source keypoint's bin in list order.  Every bin entry whose gate
+// `d2 >= 0.75 * 0.75` is false is a candidate (a NaN d2 is one); for each candidate it computes the descriptor distance
+// acc and steps
 //   if (acc < best) { second = best; best = acc; bestIndex = nb; }        (best = second = DBL_MAX, bestIndex = -1 at first)
 // Restated over the candidate sequence:
 //   best, bestIndex = the FIRST strict minimum of acc among candidates with acc < DBL_MAX (DBL_MAX, -1 if there is none);
@@ -34,7 +35,7 @@ struct GuidedNn {
 
 PGI_GNN_FN GuidedNn guidedEmpty() { return GuidedNn{DBL_MAX, DBL_MAX, -1, 0}; }
 
-// one step of K7's sequential loop: candidate nb with descriptor distance acc, after every candidate before it
+// one step of the reference's sequential loop: candidate nb with descriptor distance acc, after every candidate before it
 PGI_GNN_FN void guidedPush(GuidedNn &s, double acc, int32_t nb)
 {
     s.count += 1;

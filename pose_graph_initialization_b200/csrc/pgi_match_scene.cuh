@@ -1,5 +1,5 @@
 // pgi_match_scene.cuh — K9: matchFeatures (feature_utils.h:103-210) for every pair of a scene in one device call, with
-// the result left on the device for K0 (createCorrespondenceMatrix).  Bit-identical to K8 / oracle.match_features.
+// the result left on the device for K0 (createCorrespondenceMatrix).  Bit-identical to oracle.match_features.
 //
 // k9_knn2_tile: one CTA per (pair, block of kK9Rows source keypoints); it walks the destination keypoints in blocks of
 //   kK9Cols.  Each 128 x 128 distance tile is computed ONCE in FP32, dimension order, multiply then add, never fused

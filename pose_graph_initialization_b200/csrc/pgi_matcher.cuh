@@ -1,20 +1,16 @@
-// pgi_matcher.cuh — K7: epipolar-hashing guided matcher (SURVEY §8f-3).
+// pgi_matcher.cuh — the device functions of guided matching (SURVEY §8f-3), which K10 (pgi_guided_batch.cuh) runs:
 //
 //   HashingBasedMatcherWithPose<false, 45>::match     matcher.h:199-405
 //   (called from PoseGraphBuilder::guidedMatching       pose_graph_builder.h:717-783)
 //
-// One CTA per image pair.
-//   phase 0 (thread 0): F = Kd^-T E Ks^-1, epipole from the 3x3 Jacobi SVD of F, angular range from the destination
-//           image's corners (matcher.h:218-277) — the same operations in the same order as oracle/pgo_matcher.hpp;
-//   phase 1: every destination keypoint gets the bin of its epipolar line's normal angle (matcher.h:285-299);
-//   phase 2: the bins are laid out as index lists in keypoint order (the reference appends in that order, and the order
-//           decides ties between equal descriptor distances): warp w gathers bins w, w + 8, ... with ballot compaction;
-//   phase 3: one thread per source keypoint walks its bin: squared symmetric epipolar distance (FP64, matcher.h:351-360)
-//           against 0.75^2, then the 128-D squared descriptor distance (float differences accumulated in double,
-//           matcher.h:371-375), best / second best, count-corrected Lowe ratio (matcher.h:386-406);
-//   phase 4: accepted matches are compacted in source order (block scan).
-// The preparation (guidedPrepare), the bins, the epipolar gate, the descriptor distance, the best / second-best step
-// (pgi_guided_nn.h) and the count-corrected ratio are device functions that K10 (pgi_guided_batch.cuh) calls too.
+//   guidedPrepare: F = Kd^-T E Ks^-1, epipole from the 3x3 Jacobi SVD of F, angular range from the destination image's
+//           corners (matcher.h:218-277) — the same operations in the same order as oracle/pgo_matcher.hpp;
+//   guidedDestinationBin / guidedSourceBin: the bin of a destination keypoint's epipolar line's normal angle
+//           (matcher.h:285-299), of a source keypoint's ray from the epipole (:333-345);
+//   guidedEpipolarSq, guidedIsCandidate: squared symmetric epipolar distance (FP64, matcher.h:351-360) against 0.75^2;
+//   guidedDescriptorSq: the squared descriptor distance (float differences accumulated in double, matcher.h:371-375);
+//   guidedAdaptedRatio, guidedAccepted: the count-corrected Lowe ratio and the acceptance (matcher.h:386-406) of a
+//           source keypoint's best / second-best state (pgi_guided_nn.h).
 // atan2 is evaluated in double-double arithmetic and rounded once (pgi_atan2.h): the correctly rounded value, which is
 // what glibc returns for all but ~2.5e-4 of arguments (CUDA's own atan2 is a 2-ulp function and differed from the host
 // in the angular range of one of five test scenes).
@@ -29,26 +25,7 @@
 
 namespace pgi {
 
-constexpr int kMatchThreads = 256;
 constexpr int kMatchMaxBins = 192;
-
-struct MatchArgs {
-    const float2 *kpS;   // nS source keypoints (pixels)
-    const float *dS;     // nS x dim
-    const float2 *kpD;
-    const float *dD;
-    uint32_t nS, nD, dim;
-    double E[9], Ks[9], Kd[9];
-    int wS, hS, wD, hD, binNumber;
-    uint8_t *binOfD;     // nD scratch
-    uint32_t *binList;   // nD scratch: bins concatenated
-    uint32_t *cand;      // nS scratch: best index (0xffffffff: none)
-    double *candRatio;   // nS scratch
-    uint32_t *matches;   // out: n x 2
-    double *ratios;      // out
-    uint32_t *nOut;
-    double *prepOut;     // 14 doubles (diagnostics / parity)
-};
 
 PGI_DEV void inverse3(const double *m, double *inv)  // Eigen compute_inverse_size3 (see oracle/pgo_matcher.hpp)
 {
@@ -86,7 +63,7 @@ PGI_DEV int binOfAngle(double angle, double minAngle, double angularRange, int b
 }
 
 // The per-pair preparation (matcher.h:218-277): F = Kd^-T E Ks^-1, the epipole from the 3x3 Jacobi SVD of F, the angular
-// range from the destination image's corners, the bin count.  K7 and K10 both run it on one thread per pair.
+// range from the destination image's corners, the bin count.  K10 runs it on one thread per pair.
 struct GuidedPrep {
     double F[9];
     double ex, ey, minAngle, range;
@@ -189,102 +166,6 @@ PGI_DEV bool guidedAccepted(const GuidedNn &s, double adapted)
     bool ok = false;
     if (!(adapted < 0.00001)) ok = s.bestIndex > -1 && ((adapted < 0.8 * 0.8) || (s.count == 1));
     return ok;
-}
-
-__global__ void __launch_bounds__(kMatchThreads) k7_guided_match(MatchArgs a)
-{
-    __shared__ GuidedPrep sP;
-    __shared__ uint32_t sBinStart[kMatchMaxBins + 1], sBinCount[kMatchMaxBins];
-    __shared__ uint32_t sScan[kMatchThreads / 32], sTotal;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (threadIdx.x == 0) {
-        GuidedPrep p;
-        guidedPrepare(a.E, a.Ks, a.Kd, a.wS, a.hS, a.wD, a.hD, a.binNumber, p);
-        sP = p;
-        if (a.prepOut) {
-            for (int k = 0; k < 9; k++) a.prepOut[k] = p.F[k];
-            a.prepOut[9] = p.ex; a.prepOut[10] = p.ey; a.prepOut[11] = p.minAngle; a.prepOut[12] = p.range; a.prepOut[13] = p.binsRaw;
-        }
-    }
-    for (int b = threadIdx.x; b < kMatchMaxBins; b += kMatchThreads) sBinCount[b] = 0;
-    __syncthreads();
-    const int bins = sP.bins;
-    if (bins <= 0) {
-        if (threadIdx.x == 0) *a.nOut = 0;
-        return;
-    }
-    double F[9];
-    for (int k = 0; k < 9; k++) F[k] = sP.F[k];
-    const double minAngle = sP.minAngle, range = sP.range;
-    // ---- phase 1: bin of every destination keypoint
-    for (uint32_t i = threadIdx.x; i < a.nD; i += kMatchThreads) {
-        const float2 p = a.kpD[i];
-        const int b = guidedDestinationBin(F, p.x, p.y, minAngle, range, bins);
-        a.binOfD[i] = (uint8_t)b;
-        atomicAdd(&sBinCount[b], 1u);
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        uint32_t acc = 0;
-        for (int b = 0; b < bins; b++) { sBinStart[b] = acc; acc += sBinCount[b]; }
-        sBinStart[bins] = acc;
-    }
-    __syncthreads();
-    // ---- phase 2: bins as index lists in keypoint order
-    for (int b = warp; b < bins; b += kMatchThreads / 32) {
-        uint32_t out = sBinStart[b];
-        for (uint32_t base = 0; base < a.nD; base += 32) {
-            const uint32_t i = base + lane;
-            const bool in = i < a.nD && a.binOfD[i] == (uint8_t)b;
-            const uint32_t m = __ballot_sync(0xffffffffu, in);
-            if (in) a.binList[out + __popc(m & ((1u << lane) - 1u))] = i;
-            out += __popc(m);
-        }
-    }
-    __syncthreads();
-    // ---- phase 3: best / second best per source keypoint
-    for (uint32_t i = threadIdx.x; i < a.nS; i += kMatchThreads) {
-        const float2 p = a.kpS[i];
-        const double x1 = p.x, y1 = p.y;
-        const int bin = guidedSourceBin(x1, y1, sP.ex, sP.ey, minAngle, range, bins);
-        GuidedNn s = guidedEmpty();
-        const float *ds = a.dS + (size_t)i * a.dim;
-        for (uint32_t k = sBinStart[bin]; k < sBinStart[bin + 1]; k++) {
-            const uint32_t nb = a.binList[k];
-            const float2 q = a.kpD[nb];
-            if (!guidedIsCandidate(guidedEpipolarSq(F, x1, y1, q.x, q.y))) continue;
-            guidedPush(s, guidedDescriptorSq(ds, a.dD + (size_t)nb * a.dim, a.dim), (int32_t)nb);
-        }
-        const double adapted = guidedAdaptedRatio(s);
-        a.cand[i] = guidedAccepted(s, adapted) ? (uint32_t)s.bestIndex : 0xffffffffu;
-        a.candRatio[i] = adapted;
-    }
-    __syncthreads();
-    // ---- phase 4: compaction in source order
-    uint32_t base = 0;
-    for (uint32_t i0 = 0; i0 < a.nS; i0 += kMatchThreads) {
-        const uint32_t i = i0 + threadIdx.x;
-        const bool ok = i < a.nS && a.cand[i] != 0xffffffffu;
-        const uint32_t m = __ballot_sync(0xffffffffu, ok);
-        if (lane == 0) sScan[warp] = __popc(m);
-        __syncthreads();
-        uint32_t off = base;
-        for (int w = 0; w < warp; w++) off += sScan[w];
-        if (ok) {
-            const uint32_t o = off + __popc(m & ((1u << lane) - 1u));
-            a.matches[2 * o] = i;
-            a.matches[2 * o + 1] = a.cand[i];
-            a.ratios[o] = a.candRatio[i];
-        }
-        if (threadIdx.x == 0) {
-            uint32_t t = 0;
-            for (int w = 0; w < kMatchThreads / 32; w++) t += sScan[w];
-            sTotal = t;
-        }
-        __syncthreads();
-        base += sTotal;
-    }
-    if (threadIdx.x == 0) *a.nOut = base;
 }
 
 }  // namespace pgi

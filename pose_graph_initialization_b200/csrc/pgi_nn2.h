@@ -1,6 +1,7 @@
 // pgi_nn2.h — the 2-NN state of matchFeatures' knnMatch(k = 2) scan (feature_utils.h:151-163) as a mergeable value.
 //
-// The reference (and K8) scans train indices in ascending order with strict `<`, starting from d1 = d2 = FLT_MAX:
+// The reference (and oracle.match_features) scans train indices in ascending order with strict `<`, starting from
+// d1 = d2 = FLT_MAX:
 //   if (v < d1) { d2 = d1; d1 = v; i1 = idx; } else if (v < d2) d2 = v;
 // Its result is a function of the multiset of distances, not of the scan:
 //   d1 = the minimum of the distances below FLT_MAX (FLT_MAX if there is none; NaN and values >= FLT_MAX never enter),

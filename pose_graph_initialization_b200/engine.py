@@ -318,7 +318,7 @@ class Engine:
         self._ck(self.lib.pgi_graph_stats(self.h, C.byref(s), C.c_int32(1 if reset else 0)))
         return s.as_dict()
 
-    # ---- epipolar-hashing guided matcher (K7) ---------------------------------------------------------------
+    # ---- epipolar-hashing guided matcher (K10) --------------------------------------------------------------
     def guided_match(self, kp_src, desc_src, kp_dst, desc_dst, pose_qt, K_src, K_dst, size_src, size_dst, bin_number=45,
                      max_points=100):
         """HashingBasedMatcherWithPose<false, 45>::match on the device + guidedMatching's selection

@@ -3,9 +3,10 @@ descriptor scenes of 100 and 300 views with 2 000-4 000 keypoints per view, 128 
 
 Per scene it reports: the hashing pass (positions/s over the wall time of run(), which ends in a device synchronise), the
 share of positions matched quickly from the tracklets, the time split of pgb_hashing_stats (A*, engine, guided matching,
-tracklets); the same scene's default run() without hashing for comparison; and the K7 device time per call of
-pgi_guided_match_views against pgi_guided_match on the same (pair, pose) cases, from the CUDA events the engine records
-around each K7 launch (pgi_stats.ms_guided), averaged over many calls.  Registration (K9 matching) is outside both timed
+tracklets); the same scene's default run() without hashing for comparison; and the device time per call of
+pgi_guided_match_views against pgi_guided_match (K10 on one pair) on the same (pair, pose) cases, from the CUDA events the
+engine records around the launches (pgi_stats.ms_guided), averaged over many calls.  The script exits non-zero if the two
+entry points select different rows on any case.  Registration (K9 matching) is outside both timed
 passes.  The card's name, power limit and SM clock are read in the same call and are part of the result.
 
     python scripts/hashing_bench.py [--views 100 300] [--guided-calls 200] [--out profiles/hashing_bench.json]
@@ -33,7 +34,8 @@ def smi(fields):
 
 
 def guided_device_time(pgb, sc, n_calls, seed):
-    """Mean K7 device time per call (ms) of pgi_guided_match_views and of pgi_guided_match on the same cases."""
+    """Mean device time per call (ms) of pgi_guided_match_views and of pgi_guided_match on the same cases, and whether their
+    selected rows are equal on every case."""
     eng = pgb.engine
     ko = sc["kp_offset"].astype(np.int64)
     rng = np.random.default_rng(seed)
@@ -45,24 +47,26 @@ def guided_device_time(pgb, sc, n_calls, seed):
         f, (w, h) = float(sc["focal"][v]), sc["size"][v]
         return np.array([[f, 0.0, w / 2.0], [0.0, f, h / 2.0], [0.0, 0.0, 1.0]])
 
-    out = {}
+    out, rows = {}, {}
     for name in ("views", "single_pair"):
         s0, d0, qt0 = cases[0]
         eng.guided_match_views(s0, d0, qt0)  # warm
         before = eng.stats()
         t0 = time.perf_counter()
+        rows[name] = got = []
         for s, d, qt in cases:
             if name == "views":
-                eng.guided_match_views(s, d, qt)
+                got.append(eng.guided_match_views(s, d, qt))
             else:
-                eng.guided_match(sc["kp"][ko[s]:ko[s + 1]], sc["desc"][ko[s]:ko[s + 1]], sc["kp"][ko[d]:ko[d + 1]],
-                                 sc["desc"][ko[d]:ko[d + 1]], qt, K(s), K(d), sc["size"][s], sc["size"][d])
+                got.append(eng.guided_match(sc["kp"][ko[s]:ko[s + 1]], sc["desc"][ko[s]:ko[s + 1]], sc["kp"][ko[d]:ko[d + 1]],
+                                            sc["desc"][ko[d]:ko[d + 1]], qt, K(s), K(d), sc["size"][s], sc["size"][d])["selected"])
         wall = time.perf_counter() - t0
         after = eng.stats()
         calls = after["guided_calls"] - before["guided_calls"]
-        out[name] = dict(calls=int(calls), k7_ms_per_call=(after["ms_guided"] - before["ms_guided"]) / max(calls, 1),
+        out[name] = dict(calls=int(calls), device_ms_per_call=(after["ms_guided"] - before["ms_guided"]) / max(calls, 1),
                          wall_ms_per_call=wall / len(cases) * 1e3,
                          h2d_bytes_per_call=(after["h2d_bytes"] - before["h2d_bytes"]) / len(cases))
+    out["rows_equal"] = rows["views"] == rows["single_pair"]
     return out
 
 
@@ -90,7 +94,7 @@ def bench_scene(views, guided_calls, seed):
                tracklet_adds=int(st["tracklet_adds"]), edges=int(g.numEdges()),
                split_s=dict(astar=st["sec_astar"], engine=st["sec_engine"], guided=st["sec_guided"],
                             tracklets=st["sec_tracklets"]),
-               guided_k7=guided)
+               guided_single_pair=guided)
     pgb.close()
     # the same scene (matches already in it) without hashing: the default speculative-wave pass
     ref = B.PoseGraphBuilder(scene=sc)
@@ -123,6 +127,8 @@ def main():
         os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
         with open(a.out, "w") as f:
             f.write(line + "\n")
+    if not all(s["guided_single_pair"]["rows_equal"] for s in res["scenes"]):
+        sys.exit("pgi_guided_match_views and pgi_guided_match select different rows")
 
 
 if __name__ == "__main__":

@@ -1,8 +1,8 @@
-"""Batched descriptor matching (K9, pgi_register_scene_descriptors) against the per-pair matcher (K8, pgi_match_features)
-on descriptor scenes of 300 views: 4 000 and 2 000 keypoints per view, 128 dimensions, all 44 850 pairs.
+"""Batched descriptor matching (K9, pgi_register_scene_descriptors) against the per-pair matcher (pgi_match_features, K9 on
+one pair per call) on descriptor scenes of 300 views: 4 000 and 2 000 keypoints per view, 128 dimensions, all 44 850 pairs.
 
 Per scene it reports: the batched call (matching + registration; the call ends in a device synchronise, so the host clock
-around it is the call's time) with its K9 kernel time from CUDA events; the per-pair K8 loop on a sample of pairs, scaled
+around it is the call's time) with its K9 kernel time from CUDA events; the per-pair loop on a sample of pairs, scaled
 to all pairs; that the sample's matches and ratio bits are equal in both; one PoseGraphBuilder pass on the matched
 scene.  Rates: pairs/s, distance evaluations/s and algorithmic FP32 operations/s (3 non-fused operations per dimension
 per distance, each distance counted once), the last also as a share of the FP32 instruction bound

@@ -1,4 +1,4 @@
-"""pgi_atan2.h (the atan2 K7 evaluates on the device) compiled for the host: it must return the correctly rounded
+"""pgi_atan2.h (the atan2 guided matching evaluates on the device) compiled for the host: it must return the correctly rounded
 atan2.  Wherever it differs from the host libm (glibc is off by one ulp for ~2.5e-4 of arguments) mpmath decides, and
 it must never be the one that is wrong."""
 import math

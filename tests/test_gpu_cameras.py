@@ -1,8 +1,8 @@
 """Scenes in which every view has its own camera (focal length and image size), as 1DSfM's list_with_focals.txt gives them:
 K0's correspondence rows against the oracle's createCorrespondenceMatrix and against a numpy statement of the reference's
 quirk (both images normalised with the SOURCE view's K, threshold by the source focal length; pose_graph_builder.h:908-912,
-:934-937), for scene, descriptor-matched and extra-pair registrations; K7 with K_src != K_dst and different image sizes,
-single-pair and on the resident scene, against the oracle; PoseGraphBuilder (waves and epipolar hashing) against the
+:934-937), for scene, descriptor-matched and extra-pair registrations; guided matching with K_src != K_dst and different
+image sizes, single-pair and on the resident scene, against the oracle; PoseGraphBuilder (waves and epipolar hashing) against the
 oracle's sequential runs.  With one camera for all views, a swapped K or image size could not fail any of these."""
 import numpy as np
 import pytest

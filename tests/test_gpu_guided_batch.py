@@ -1,5 +1,6 @@
 """Batched guided matching (K10, pgi_guided_match_pairs / Engine.guided_match_pairs / PoseGraphBuilder.guided_match_edges),
-bit for bit: every pair of a batch against K7 (guided_match_views and guided_match) and the oracle's guided matcher, on
+bit for bit: every pair of a batch against the oracle's guided matcher and the single-pair calls (guided_match_views and
+guided_match), on
 descriptor scenes (128-D and 64-D), per-view cameras, degenerate epipolar geometry and bin numbers; a pair's rows do not
 depend on its batch, across scratch chunks too; the builder's edges after a wave-mode and a hashing-mode run; errors."""
 import ctypes as C
@@ -48,7 +49,8 @@ def _same(got, matches, values):
 
 
 def _check_against_oracle(eng, sc, cases, oracle, engine=None, max_points_list=(100, 10, 3, 0), bin_number=45):
-    """Every pair of one batch per max_points equals K7 and the oracle; returns the set of (more than max_points?) seen."""
+    """Every pair of one batch per max_points equals the oracle and the single-pair calls; returns the set of (more than
+    max_points?) seen."""
     kp, desc = _views(sc)
     regimes = set()
     for mp in max_points_list:
@@ -63,8 +65,8 @@ def _check_against_oracle(eng, sc, cases, oracle, engine=None, max_points_list=(
             else:
                 assert _same(got[k], ref["matches"], ref["ratios"]), (k, s, d)
                 if engine is not None:
-                    k7 = engine.guided_match(*args, bin_number=bin_number, max_points=10 ** 9)
-                    assert _same(got[k], k7["matches"], k7["ratios"]), (k, s, d)
+                    single = engine.guided_match(*args, bin_number=bin_number, max_points=10 ** 9)
+                    assert _same(got[k], single["matches"], single["ratios"]), (k, s, d)
     return regimes
 
 
@@ -93,7 +95,7 @@ def scenes():
 
 # ---- 1. descriptor scenes ------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("dim", [128, 64])
-def test_batches_equal_k7_and_the_oracle(scenes, engine, oracle, dim):
+def test_batches_equal_the_oracle_and_single_pair_calls(scenes, engine, oracle, dim):
     sc, eng = scenes[dim]
     cases = _guided_cases(sc, np.random.default_rng(dim), 50)  # ground truth and perturbed poses, both directions, empty views
     cases += cases[:6]  # repeated pairs

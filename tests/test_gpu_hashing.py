@@ -1,6 +1,6 @@
 """Epipolar-hashing mode on the device: extra pairs (pgi_register_extra_pairs + PGI_WAVE_EXTRA) against the oracle's
 createCorrespondenceMatrix / estimatePose and against a static registration of the same rows; guided matching on the
-resident scene (pgi_guided_match_views) against K7's single-pair entry point and the oracle; descriptors added to a scene
+resident scene (pgi_guided_match_views) against the oracle and pgi_guided_match on the same pair; descriptors added to a scene
 registered with matches; PoseGraphBuilder(kUseEpipolarHashing_=True) against pgo_run_scene_hashing; bad input."""
 import os
 import subprocess
@@ -118,7 +118,7 @@ def _guided_cases(sc, rng, n):
 
 
 @pytest.mark.parametrize("dim", [128, 64])
-def test_guided_match_views_equals_k7_and_the_oracle(desc_scene, engine, oracle, dim):
+def test_guided_match_views_equals_the_oracle_and_guided_match(desc_scene, engine, oracle, dim):
     if dim == 128:
         sc, eng = desc_scene
     else:
@@ -135,11 +135,11 @@ def test_guided_match_views_equals_k7_and_the_oracle(desc_scene, engine, oracle,
         for max_points in (100, 10, 3):
             got = eng.guided_match_views(s, d, qt, 45, max_points)
             args = (kp[s], desc[s], kp[d], desc[d], qt, _K(sc, s), _K(sc, d), sc["size"][s], sc["size"][d])
-            k7 = engine.guided_match(*args, bin_number=45, max_points=max_points)
+            single = engine.guided_match(*args, bin_number=45, max_points=max_points)
             ref = oracle.guided_match(*args, bin_number=45, max_points=max_points)
             sel = [(int(a), int(b), float(r)) for (a, b), r in zip(ref["selected_matches"], ref["selected_ratios"])]
-            assert got == k7["selected"] == sel, (s, d, max_points)
-            sizes.add((len(k7["matches"]) > max_points, len(got) > 0))
+            assert got == sel == single["selected"], (s, d, max_points)
+            sizes.add((len(ref["matches"]) > max_points, len(got) > 0))
     assert len(cases) >= 50 and {(True, True), (False, True)} <= sizes
     if dim == 64:
         eng.close()
@@ -225,6 +225,13 @@ def test_bad_input(desc_scene):
                  lambda: e.set_scene_descriptors(np.where(np.arange(sc["desc"].size).reshape(sc["desc"].shape) == 5, np.nan, sc["desc"]))):
         with pytest.raises(PgiError, match="status -1"):
             call()
+    # a view of more keypoints than guided matching supports is rejected when its descriptors arrive
+    big = dict(focal=np.array([1000.0, 1000.0]), size=np.array([[1600.0, 1200.0]] * 2), kp=np.zeros((16395, 2), np.float32),
+               kp_offset=np.array([0, 16385, 16395], dtype=np.uint64), pair_views=np.array([[0, 1]], dtype=np.uint32),
+               m_offset=np.zeros(2, dtype=np.uint64), matches=np.zeros((0, 2), dtype=np.uint32))
+    e.register_scene(big, 0.4)
+    with pytest.raises(PgiError, match="at most 16384"):
+        e.set_scene_descriptors(np.zeros((16395, 128), np.float32))
     e.close()
 
 

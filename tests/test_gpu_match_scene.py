@@ -1,5 +1,5 @@
 """Batched descriptor matching on the device (K9, pgi_register_scene_descriptors): every pair's matches and ratio bits equal
-oracle.match_features (and K8 at full size), the registration built from the device-resident matches equals the one
+oracle.match_features (at full size too, where pgi_match_features must agree), the registration built from the device-resident matches equals the one
 built from the oracle's, and PoseGraphBuilder on a keypoints + descriptors scene commits what the sequential oracle
 commits on the same scene matched by oracle.match_features."""
 import multiprocessing as mp
@@ -79,19 +79,22 @@ def test_registration_from_device_matches(matched):
         assert np.array_equal(corr, rc) and thr == rthr, p
 
 
-def test_matches_equal_k8_at_full_size():
+def test_matches_equal_the_oracle_at_full_size():
     sc = S.make_descriptor_scene(40, kp_range=(4000, 4000), seed=41)
     eng = Engine(device=0)
     dev = dict(sc)
     mo = eng.register_scene_descriptors(dev, 0.4).astype(np.int64)
-    ko = sc["kp_offset"].astype(np.int64)
     rng = np.random.default_rng(0)
     pairs = rng.choice(len(sc["pair_views"]), 60, replace=False)
-    for p in pairs:
+    ref = oracle_matches(dict(sc, pair_views=sc["pair_views"][pairs]))
+    ro = ref["m_offset"].astype(np.int64)
+    ko = sc["kp_offset"].astype(np.int64)
+    for k, p in enumerate(pairs):
         s, d = sc["pair_views"][p]
         m, r = eng.match_features(sc["desc"][ko[s]:ko[s + 1]], sc["desc"][ko[d]:ko[d + 1]])
-        assert np.array_equal(dev["matches"][mo[p]:mo[p + 1]], m), p
-        assert dev["ratios"][mo[p]:mo[p + 1]].tobytes() == r.tobytes(), p
+        for got_m, got_r in ((dev["matches"][mo[p]:mo[p + 1]], dev["ratios"][mo[p]:mo[p + 1]]), (m, r)):
+            assert np.array_equal(got_m, ref["matches"][ro[k]:ro[k + 1]]), p
+            assert got_r.tobytes() == ref["ratios"][ro[k]:ro[k + 1]].tobytes(), p
     eng.close()
 
 

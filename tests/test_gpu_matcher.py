@@ -1,4 +1,4 @@
-"""K7 (pgi_guided_match) against the oracle's restatement of HashingBasedMatcherWithPose<false, 45>::match
+"""pgi_guided_match against the oracle's restatement of HashingBasedMatcherWithPose<false, 45>::match
 (matcher.h:199-405) and of guidedMatching's selection (pose_graph_builder.h:760-782): same prepared quantities (F,
 epipole, angular range), same matches in the same order, bit-identical adapted ratios."""
 import numpy as np

@@ -1,4 +1,4 @@
-"""K7 (pgi_guided_match) at its edges, bit for bit against the oracle's guided matcher: prepared quantities (F, epipole,
+"""pgi_guided_match at its edges, bit for bit against the oracle's guided matcher: prepared quantities (F, epipole,
 angular range, bin count), matches in order, adapted-ratio bits and guidedMatching's selection.
 - Degenerate geometry: lateral motion (the epipole at infinity; with t = (1, 1e-7, 0) the angular range is exactly 0
   and every bin argument is NaN or +-inf), a small rotation with lateral motion, backward motion, and the epipole within
@@ -6,13 +6,15 @@ angular range, bin count), matches in order, adapted-ratio bits and guidedMatchi
 - Hand-built destination sets: exact candidate counts around the count-corrected ratio's steps, duplicated destination
   keypoints with identical descriptors (tests/test_matcher_reference.py checks the same cases against a numpy
   restatement).
-- Sizes: source counts around the 256-thread block, one and 16 384 destination keypoints, source keypoints outside the
-  image, 64-d descriptors.
+- Sizes: source counts around the 256-thread block, one and 16 384 destination keypoints, 20 000 source and destination
+  keypoints (more than a view of the registered scene may have), source keypoints outside the image, 64-d descriptors;
+  other descriptor widths are rejected.
 - Bin numbers 1, 2, 45, 180, 192 and 0 (the angular range's integer part).
 - Selection at n == max_points and n == max_points + 1, and with equal values straddling the cut."""
 import numpy as np
 import pytest
 
+from pose_graph_initialization_b200.engine import PgiError
 from helpers import rodrigues, two_view_keypoints_posed
 from test_matcher_reference import (COUNTS, K_DST, K_SRC, LATERAL_POSES, R_GEN, SIZE_DST, SIZE_SRC, T_GEN, count_case,
                                     lateral_case, tie_case)
@@ -120,6 +122,21 @@ def test_16384_destination_keypoints(engine, oracle):
     assert len(d["kp_dst"]) == 16384
     ref = _compare(engine, oracle, _args(d))
     assert len(ref["matches"]) > 1000
+
+
+def test_20000_keypoints(engine, oracle):
+    d = _posed(R_GEN, T_GEN, n=15400, seed=6)
+    d["kp_src"], d["desc_src"] = d["kp_src"][:20000], d["desc_src"][:20000]
+    assert len(d["kp_src"]) == 20000 and len(d["kp_dst"]) > 20000
+    ref = _compare(engine, oracle, _args(d))
+    assert len(ref["matches"]) > 1000
+
+
+def test_descriptor_widths_other_than_64_and_128_are_rejected(engine, generic):
+    args = list(_args(generic))
+    args[1], args[3] = args[1][:, :96], args[3][:, :96]
+    with pytest.raises(PgiError, match="64 or 128"):
+        engine.guided_match(*args)
 
 
 def test_source_keypoints_outside_the_image(engine, oracle, generic):

@@ -1,7 +1,7 @@
 """pgi_guided_nn.h (the best / second-best state K10 merges across the lanes of a warp) compiled for the host: random bins with
 many exact ties, DBL_MAX descriptor distances and inf / NaN / boundary gate values, cut into random runs of consecutive
-entries merged in random grouping (order kept), must give exactly what K7's sequential loop gives.  The harness also
-checks that the variant which takes `second` as the true second-smallest distance disagrees with the loop, so the test
+entries merged in random grouping (order kept), must give exactly what the reference's sequential loop gives.  The harness
+also checks that the variant which takes `second` as the true second-smallest distance disagrees with the loop, so the test
 would catch that mistake.  And the builder's ValueErrors of guided_match_edges, which need no device."""
 import os
 import subprocess
@@ -22,8 +22,8 @@ HARNESS = r"""
 #include <vector>
 using namespace pgi;
 struct Seq { double best, second; int bestIndex, countSnn; };
-// K7's loop (pgi_matcher.cuh phase 3, matcher.h:362-384), restated without the header
-static Seq k7Loop(const std::vector<double> &d2, const std::vector<double> &acc) {
+// the reference's loop (matcher.h:362-384), restated without the header
+static Seq seqLoop(const std::vector<double> &d2, const std::vector<double> &acc) {
     Seq r{DBL_MAX, DBL_MAX, -1, 0};
     for (size_t k = 0; k < d2.size(); k++) {
         if (d2[k] >= 0.75 * 0.75) continue;
@@ -49,7 +49,7 @@ int main() {
             const unsigned q = (unsigned)(g() %% 100);
             acc[k] = q < 8 ? DBL_MAX : q < 12 ? INFINITY : (double)(g() %% levels) * 0.5;
         }
-        const Seq seq = k7Loop(d2, acc);
+        const Seq seq = seqLoop(d2, acc);
         noneFound += seq.bestIndex < 0;
         // the candidates' states, one per entry, cut into runs of consecutive entries at random points
         std::vector<GuidedNn> st;

@@ -1,6 +1,6 @@
 """pgi_nn2.h (the 2-NN state K9 merges across lanes, warps and CTAs) compiled for the host: random distance rows with many
 exact ties, NaN and values >= FLT_MAX, cut into random index subsets merged in random order and grouping, must give
-exactly what the sequential strict-`<` scan over ascending indices gives (the scan of K8 and oracle.match_features).
+exactly what the sequential strict-`<` scan over ascending indices gives (the scan of the reference and oracle.match_features).
 And the 64-bit survivor key (ratio bits << 32 | query) must sort like (ratio, query)."""
 import os
 import struct
