@@ -187,7 +187,8 @@ int32_t pgi_estimate_pose(pgi_ctx *ctx, const double *corr_xy4, uint64_t n, doub
                           uint32_t n_guesses, double *pose_q_t_out, uint8_t *mask_out, uint64_t *inlier_number_out,
                           pgi_verdict *verdict_or_null);
 /* = InTraversalPoseTester::test, graph_traversal.h:194-233.  thr is the tester's threshold (1.5*thr_norm at
- * pose_graph_builder.h:807-811).  Returns 1/0, <0 on error. */
+ * pose_graph_builder.h:807-811), used as given whatever its value: a row counts when its squared Sampson residual is
+ * below thr*thr, so a negative thr tests like -thr and a NaN thr counts no row.  Returns 1/0, <0 on error. */
 int32_t pgi_test_pose(pgi_ctx *ctx, const double *corr_xy4, uint64_t n, double thr, uint64_t min_inliers,
                       const double *pose_q_t, uint64_t *inlier_number_out);
 

@@ -411,7 +411,7 @@ pgi_status ensureWave(pgi_ctx *ctx, const Registration &r, uint32_t n, uint32_t 
 }
 
 pgi_status submitWave(pgi_ctx *ctx, const Registration &r, uint32_t n, const uint32_t *pairId, const uint32_t *hypOffset,
-                      const double *hyp, uint32_t flags, double thrOverride, uint32_t testMinOverride, bool scoreOnly)
+                      const double *hyp, uint32_t flags, const double *thrOverride, uint32_t testMinOverride, bool scoreOnly)
 {
     if (ctx->inFlight) { ctx->err = "a wave is already in flight"; return PGI_ERR_STATE; }
     if (n == 0) { ctx->waveN = 0; ctx->inFlight = true; ctx->fbLaunched = false; ctx->nChunks = 0; ctx->waveFlags = flags; return PGI_OK; }
@@ -454,7 +454,8 @@ pgi_status submitWave(pgi_ctx *ctx, const Registration &r, uint32_t n, const uin
     a.verdicts = d.verdicts.data(); a.flags = flags; a.minInliers = ctx->cfg.min_inliers;
     a.testMinInliers = testMinOverride ? testMinOverride : ctx->cfg.test_min_inliers;
     a.fbMaxIters = ctx->cfg.fallback_max_iters; a.thrMultiplier = ctx->cfg.threshold_multiplier;
-    a.thrOverride = thrOverride;
+    a.thrOverride = thrOverride ? *thrOverride : 0.0;
+    a.hasThrOverride = thrOverride ? 1u : 0u;
     a.fbSols = ctx->fb.sols.data(); a.fbSolsF = ctx->fb.solsF.data(); a.fbCounts = ctx->fb.counts.data(); a.counters = ctx->counters.data();
     a.k3Scratch = d.k3Scratch.data(); a.dkList = ctx->fb.dkList.data(); a.dkCtl = ctx->fb.dkCtl.data();
 
@@ -1208,7 +1209,7 @@ pgi_status pgi_submit_wave(pgi_ctx *ctx, uint32_t n, const uint32_t *pair_id, co
     CK(cudaSetDevice(ctx->cfg.device));
     // PGI_WAVE_EXTRA selects the registration of pgi_register_extra_pairs; the kernels never see the bit
     const Registration &r = (flags & PGI_WAVE_EXTRA) ? ctx->extra : *ctx->reg;
-    return submitWave(ctx, r, n, pair_id, hyp_offset, hyp_q_t, flags & ~(uint32_t)PGI_WAVE_EXTRA, 0.0, 0, false);
+    return submitWave(ctx, r, n, pair_id, hyp_offset, hyp_q_t, flags & ~(uint32_t)PGI_WAVE_EXTRA, nullptr, 0, false);
 }
 
 pgi_status pgi_wait_wave(pgi_ctx *ctx, pgi_verdict *out, uint8_t *masks_or_null)
@@ -1263,7 +1264,7 @@ int32_t pgi_estimate_pose(pgi_ctx *ctx, const double *corr_xy4, uint64_t n, doub
     if (st != PGI_OK) return st;
     const uint32_t pid = 0, hoff[2] = {0, n_guesses};
     const uint32_t flags = PGI_WAVE_PATH | PGI_WAVE_FALLBACK | PGI_WAVE_NO_TEST | (mask_out ? PGI_WAVE_MASKS : 0u);
-    st = submitWave(ctx, ctx->tmp, 1, &pid, hoff, guesses_q_t, flags, 0.0, 0, false);
+    st = submitWave(ctx, ctx->tmp, 1, &pid, hoff, guesses_q_t, flags, nullptr, 0, false);
     if (st != PGI_OK) return st;
     pgi_verdict v;
     st = pgi_wait_wave(ctx, &v, mask_out);
@@ -1289,7 +1290,7 @@ int32_t pgi_test_pose(pgi_ctx *ctx, const double *corr_xy4, uint64_t n, double t
     pgi_status st = registerDense(ctx, ctx->tmp, 1, off, corr_xy4, &thrReg);
     if (st != PGI_OK) return st;
     const uint32_t pid = 0, hoff[2] = {0, 1};
-    st = submitWave(ctx, ctx->tmp, 1, &pid, hoff, pose_q_t, PGI_WAVE_PATH, thr, (uint32_t)min_inliers, true);
+    st = submitWave(ctx, ctx->tmp, 1, &pid, hoff, pose_q_t, PGI_WAVE_PATH, &thr, (uint32_t)min_inliers, true);
     if (st != PGI_OK) return st;
     // score-only wave: read the slot state instead of a verdict
     SlotState s;

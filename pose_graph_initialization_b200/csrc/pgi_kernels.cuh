@@ -82,7 +82,8 @@ struct WaveArgs {
     uint32_t testMinInliers;
     uint32_t fbMaxIters;
     double thrMultiplier;
-    double thrOverride;  // > 0: tester threshold given explicitly (pgi_test_pose)
+    double thrOverride;        // the tester threshold of every pair when hasThrOverride (pgi_test_pose), whatever its value
+    uint32_t hasThrOverride;   // 0: the tester threshold is thrMultiplier * thr[pair]
     // fallback scratch
     double *fbSols;     // n x kFbChunk x 90
     float4 *fbSolsF;    // n x kFbChunk x 10 models x 3 float4 (FP32 copy for the certificate)
@@ -134,7 +135,7 @@ __global__ void __launch_bounds__(kCtaThreads, 3) k1_score_hypotheses(WaveArgs a
     const uint64_t r0 = a.offset[pid];
     const uint32_t N = (uint32_t)(a.offset[pid + 1] - r0);
     const double4 *rows = reinterpret_cast<const double4 *>(a.corr) + r0;
-    const double thrT = a.thrOverride > 0.0 ? a.thrOverride : a.thrMultiplier * a.thr[pid];  // 1.5 * thr_norm  (PGB:800, :964)
+    const double thrT = a.hasThrOverride ? a.thrOverride : a.thrMultiplier * a.thr[pid];  // 1.5 * thr_norm  (PGB:800, :964)
     const double thrTsq = thrT * thrT;                 // GT:184
     // two bit buffers per slot: the one being written and the one of the last hypothesis that reached
     // estimatePose (so a later failing hypothesis cannot clobber the sampler's input)
@@ -365,7 +366,7 @@ __global__ void __launch_bounds__(kK1TmaThreads, 1) k1_score_hypotheses_tma(Wave
             meta.N[t] = (uint32_t)(a.offset[pid + 1] - r0);
             meta.h0[t] = a.hypOffset[w];
             meta.h1[t] = a.hypOffset[w + 1];
-            meta.thr[t] = a.thrOverride > 0.0 ? a.thrOverride : a.thrMultiplier * a.thr[pid];  // 1.5 * thr_norm  (PGB:800, :964)
+            meta.thr[t] = a.hasThrOverride ? a.thrOverride : a.thrMultiplier * a.thr[pid];  // 1.5 * thr_norm  (PGB:800, :964)
             meta.table[t] = a.pairTable[pid];
             if (meta.h1[t] > meta.h0[t]) {
                 double qt[7], E[9];

@@ -214,3 +214,161 @@ def per_view_camera_scene(n_views=12, seed=0, cameras=CAMERAS, group=3, n_points
         sc["m_offset"] = np.array(mo, dtype=np.uint64)
         sc["matches"] = np.concatenate(rows).astype(np.uint32).reshape(-1, 2)
     return sc
+
+
+# ---- pose-path regimes the two_view / make_scene generators never produce ----------------------------------------------
+REGIME_KINDS = ("wide_fov", "off_centre", "forward", "pure_rotation", "tiny_baseline", "planar", "duplicated", "identical",
+                "outliers", "nonfinite", "focal_zero")
+REGIME_SIZES = (5, 6, 9, 19, 20, 21, 2047, 2048, 2049, 4097, 11264, 11265)
+REGIME_OUTLIER_RATIOS = (0.0, 0.05, 0.5, 0.85, 1.0)
+REGIME_THRESHOLDS = (1e-5, 1e-4, 5e-4, 2e-3, 1e-2)  # per-pair thr_norm across three decades (thr_px 0.4 at f 40 000 .. 40)
+
+
+def _view_rows(X, R, t, noise, rng):
+    """Normalised [x1 y1 x2 y2] rows of the 3-D points X (camera 1) seen by camera 2 (X2 = R X + t), plus noise."""
+    x1 = X[:, :2] / X[:, 2:]
+    X2 = X @ R.T + t
+    x2 = X2[:, :2] / X2[:, 2:]
+    c = np.hstack([x1, x2])
+    return c + rng.standard_normal(c.shape) * noise
+
+
+def regime_pair(kind, n, rng, outlier_ratio=0.3, thr=5e-4):
+    """One seeded pair of the given regime kind with n rows -> dict(corr [n, 4], thr, R, t, good (a pose near the truth as
+    q,t), bad (a wrong pose), outliers (rows replaced by random ones)).  The kinds:
+      wide_fov       normalised coordinates up to about +-2.5 (a focal length of 0.2 x the image width)
+      off_centre     destination camera turned by ~0.9 rad: the destination rows sit far from the principal point
+      forward        motion along the optical axis: the epipole lies inside both images
+      pure_rotation  t = 0 exactly
+      tiny_baseline  |t| = 1e-6
+      planar         every point on one plane
+      duplicated     50 distinct rows, each repeated n / 50 times (n a multiple of 50)
+      identical      one row repeated n times
+      outliers       two_view-like geometry with outlier_ratio of the rows replaced by random ones
+      nonfinite      rows with NaN, +inf and -inf coordinates among finite ones
+      focal_zero     what createCorrespondenceMatrix makes of a view with focal length 0.0: +-inf / NaN rows, thr = inf"""
+    noise = 0.5 / 800.0
+    R = rodrigues(rng.uniform(-0.2, 0.2, 3))
+    t = rng.standard_normal(3)
+    t /= np.linalg.norm(t)
+    X = rng.standard_normal((n, 3)) + np.array([0.0, 0.0, 6.0])
+    n_out = 0
+    if kind == "wide_fov":
+        z = rng.uniform(4.0, 8.0, n)
+        X = np.stack([rng.uniform(-2.4, 2.4, n) * z, rng.uniform(-2.4, 2.4, n) * z, z], 1)
+        t = t * 0.3
+        R = rodrigues(rng.uniform(-0.05, 0.05, 3))
+        noise = 0.5 / 200.0
+    elif kind == "off_centre":
+        R = rodrigues(np.array([0.5, -0.9, 0.05]))
+        t = np.array([0.8, -0.3, 0.2])
+    elif kind == "forward":
+        R = rodrigues(rng.uniform(-0.02, 0.02, 3))
+        t = np.array([0.03, -0.02, -1.0])
+    elif kind == "pure_rotation":
+        t = np.zeros(3)
+    elif kind == "tiny_baseline":
+        t = t * 1e-6
+    elif kind == "planar":
+        xy = rng.uniform(-2.0, 2.0, (n, 2))
+        X = np.stack([xy[:, 0], xy[:, 1], 6.0 + 0.3 * xy[:, 0] - 0.2 * xy[:, 1]], 1)
+    corr = _view_rows(X, R, t, noise, rng)
+    if kind == "duplicated":
+        assert n % 50 == 0
+        corr = np.tile(corr[:50], (n // 50, 1))[rng.permutation(n)]
+    elif kind == "identical":
+        corr = np.repeat(corr[:1], n, 0)
+    elif kind == "outliers":
+        n_out = int(round(n * outlier_ratio))
+        corr[:n_out, 2:] = rng.uniform(-0.8, 0.8, (n_out, 2))
+        corr = corr[rng.permutation(n)]
+    elif kind == "nonfinite":
+        bad = rng.choice(n, max(1, n // 10), replace=False)
+        vals = np.array([np.nan, np.inf, -np.inf])
+        for k, i in enumerate(bad):
+            corr[i, k % 4] = vals[k % 3]
+    elif kind == "focal_zero":
+        # ((double)kp - c) / 0.0 per coordinate: +-inf, or NaN where the key point sits on the principal point
+        sgn = np.sign(rng.standard_normal((n, 4)))
+        sgn[rng.random((n, 4)) < 0.05] = 0.0
+        with np.errstate(divide="ignore", invalid="ignore"):
+            corr = sgn / 0.0
+        thr = np.inf
+    good = perturbed_pose(R, t, rng)
+    bad = pose_qt(rodrigues(np.array([0.0, 0.6, 0.0])), np.array([1.0, 0.0, 0.0]))
+    return dict(corr=np.ascontiguousarray(corr), thr=float(thr), R=R, t=t, good=good, bad=bad, n_outliers=n_out)
+
+
+def hypotheses_for(i, good, bad):
+    """0, 1 or 3 hypotheses for the i-th pair of a set (as test_gpu_k1_stream.py): none; a good or a bad one; good, bad,
+    good or bad, good, bad (the last one decides)."""
+    k = (0, 1, 3)[i % 3]
+    first_good = (i // 3) % 2 == 0
+    return [good if (first_good if j % 2 == 0 else not first_good) else bad for j in range(k)]
+
+
+def lo_fixed_point_bound(corr):
+    """The largest of the 45 sums  sum_rows |a_r a_q| 2^40  of the fallback's LO refit (a = [x2x1 x2y1 x2 y2x1 y2y1 y2 x1
+    y1 1]) over every finite row: an upper bound of the int64 accumulators whatever rows the model makes inliers.  Rows
+    with a non-finite coordinate never enter the sums (their Sampson residual is NaN under every E)."""
+    c = corr[np.isfinite(corr).all(1)]
+    x1, y1, x2, y2 = c.T
+    a = np.abs(np.stack([x2 * x1, x2 * y1, x2, y2 * x1, y2 * y1, y2, x1, y1, np.ones(len(c))], 1))
+    return float((a.T @ a).max() * 2.0 ** 40) if len(c) else 0.0
+
+
+# Fallback termination edges: (seed, N, outlier ratio) of two_view(N, ratio, default_rng(seed)) at thr_norm 0.4 / 800,
+# picked by a one-off scan with oracle.fallback, keyed by the iteration count they end at: one iteration, both sides of
+# K5's 16-iteration batch edges, both sides of the 125-iteration chunk edge and one past the second, and "rejected", which
+# runs all 1 000 iterations and keeps a model of fewer than 20 inliers.
+TERMINATION_EDGES = (  # (label, iterations, seed, N, outlier ratio, noise_px)
+    ("one", 1, 0, 100, 0.0, 0.05),
+    ("batch16", 16, 0, 100, 0.23, 0.05),
+    ("batch17", 17, 0, 100, 0.25, 0.05),
+    ("batch32", 32, 3, 100, 0.32, 0.05),
+    ("batch33", 33, 0, 100, 0.24, 0.1),
+    ("chunk124", 124, 2, 200, 0.48, 0.1),
+    ("chunk125", 125, 2, 200, 0.49, 0.05),
+    ("chunk126", 126, 11, 60, 0.1, 0.5),
+    ("chunk251", 251, 0, 300, 0.12, 0.5),
+    ("rejected", 1000, 6, 60, 0.36, 0.5),
+)
+TERMINATION_THR = 0.4 / 800.0
+
+
+def termination_pairs():
+    """[(label, expected iterations, corr, thr)] of TERMINATION_EDGES plus an all-NaN pair, which runs all 1 000 iterations
+    with models that keep no inlier.  (No input the scan tried ends the fallback without any model: identical, collinear,
+    constant-coordinate and zero-motion rows all give the five-point solver solutions to score.)"""
+    out = [(lab, it, two_view(n, ratio, np.random.default_rng(seed), noise_px=noise)[0], TERMINATION_THR)
+           for lab, it, seed, n, ratio, noise in TERMINATION_EDGES]
+    out.append(("no_inlier", 1000, np.full((50, 4), np.nan), TERMINATION_THR))
+    return out
+
+
+def first_finite_pair():
+    """A pair whose hypothesis passes the in-traversal test and makes every row an inlier (k = N = 100), with the first
+    sample of the legacy RANSAC (its ranks depend on k only) replaced by five rows 1e-9 apart: the five-point solver
+    returns a solution for them, but no finite one, so K2 has to keep sampling.  -> (corr, thr, hypothesis, first sample)."""
+    from oracle import pgo_oracle as O
+
+    c, R, t = two_view(100, 0.0, np.random.default_rng(5), noise_px=0.05)
+    sample = O.find_essential_ransac_inf(c)[3].astype(np.int64)  # the first sample: it succeeds on the clean pair
+    c[sample] = c[sample[0]] + np.random.default_rng(0).standard_normal((5, 4)) * 1e-9
+    return c, TERMINATION_THR, pose_qt(R, t), sample
+
+
+def regime_set():
+    """The regime pairs of the pose-path tests: [(label, corr, thr, hypotheses)].  Every geometric kind at every size of
+    REGIME_SIZES, the row-pattern kinds at a few sizes, every outlier ratio; thresholds cycle through REGIME_THRESHOLDS."""
+    rng = np.random.default_rng(2024)
+    specs = [(k, n, 0.3) for k in ("wide_fov", "off_centre", "forward", "pure_rotation", "tiny_baseline", "planar", "nonfinite")
+             for n in REGIME_SIZES]
+    specs += [("duplicated", 500, 0.0), ("duplicated", 1000, 0.0), ("identical", 5, 0.0), ("identical", 21, 0.0),
+              ("identical", 500, 0.0), ("focal_zero", 5, 0.0), ("focal_zero", 300, 0.0)]
+    specs += [("outliers", n, r) for r in REGIME_OUTLIER_RATIOS for n in (21, 2048, 4097)]
+    out = []
+    for i, (kind, n, ratio) in enumerate(specs):
+        p = regime_pair(kind, n, rng, ratio, REGIME_THRESHOLDS[i % len(REGIME_THRESHOLDS)])
+        out.append((f"{kind}-{n}-{ratio}", p["corr"], p["thr"], hypotheses_for(i, p["good"], p["bad"])))
+    return out
